@@ -2,6 +2,7 @@
 """bench.py -- frame-pairs/sec of the hot path at 1080p (BASELINE.json metric), one process per GPU.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c2-strong|c5]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
            --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -21,20 +22,32 @@ Workloads (BASELINE.json configs):
 `value` is measured with the frames already resident in HBM (CUDA events on the library's compute stream);
 `e2e` through the public bracket API from pinned host frames (H2D inside the timed region, wall clock between
 device synchronisations).  Rank 0 prints ONE JSON line.
+
+--dump-outputs DIR: rank 0 writes what the timed path returned in its last timed step as DIR/<name>.npy (float32 or
+float64; integer and boolean outputs as float64, which holds them exactly).  The inputs are generated from fixed
+seeds, so two builds run with the same arguments can be compared output for output.
+
+The benchmark writes nothing into the source tree, which may be read-only: a library older than its sources is
+rebuilt in a temporary directory, and no bytecode is cached.
 """
 from __future__ import annotations
 
 import argparse
+import atexit
 import hashlib
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True
+os.environ["PYTHONDONTWRITEBYTECODE"] = "1"      # for the spawned workers of the CPU baseline too
 
 import numpy as np  # noqa: E402
 
@@ -62,7 +75,21 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the pageable / drop-in / per-level side measurements")
     ap.add_argument("--no-numa-bind", action="store_true", help="do not pin the process to the GPU's NUMA node")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (rank 0)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+def dump_outputs(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        if a.dtype not in (np.float32, np.float64):
+            a = a.astype(np.float64)
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def bench_config(args, world):
@@ -461,6 +488,8 @@ def run_c2(args, rank, world, local, dd, numa_node, all_cpus):
             "wall_ms_per_step_resident": 1000 * wall_res / args.steps,
         }
         line.update(extras)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {k: v for k, v in r.items() if isinstance(v, np.ndarray)})
         if world == 1 and not args.no_cpu_baseline:
             from oracle import cpu_pipeline
             os.sched_setaffinity(0, all_cpus)      # the CPU baseline gets every host core again
@@ -510,7 +539,7 @@ def run_c2_strong(args, rank, world, local, dd, numa_node):
         torch.cuda.synchronize()
         dd.barrier()
 
-    steps = max(1, min(args.steps, 6))
+    steps = args.steps
     for _ in range(max(1, min(args.warmup, 2))):
         ref = step(src_ptr=d_frames.data_ptr())
     fence()
@@ -533,6 +562,8 @@ def run_c2_strong(args, rank, world, local, dd, numa_node):
     clocks = sampler.stop()
     assert len(got) == NP and np.array_equal(got, ref) and np.array_equal(got, got_e)
     line = None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"scalar": got})
     if rank == 0:
         peak, peak_kind = measured_peak()
         value = NP * steps / wall_res
@@ -587,9 +618,12 @@ def run_c5(args, rank, world, local, dd, numa_node):
     prm = {"batch_size": 3000, "detrend_window": 2.0, "norm_window": 3.0, "keyframe_reduction": True,
            "gpu_batch_frames": args.batch_frames or runner.default_batch_frames(W, H)}
 
+    last = {}
+
     def step():
         out = {}
         res = runner.process_many([vids[v] for v in mine], 30.0, prm, ctx=ctx, return_series=True)     # clips pipelined
+        last["res"] = res
         for v, (actions, series) in zip(mine, res):
             out[v] = (len(actions), float(np.sum(series["values"])))
         merged = {}
@@ -602,7 +636,7 @@ def run_c5(args, rank, world, local, dd, numa_node):
         torch.cuda.synchronize()
         dd.barrier()
 
-    steps = max(1, min(args.steps, 4))
+    steps = args.steps
     ref = step()
     fence()
     sampler = ClockSampler(local)
@@ -616,6 +650,16 @@ def run_c5(args, rank, world, local, dd, numa_node):
     clocks = sampler.stop()
     assert got == ref and len(got) == NV
     line = None
+    if rank == 0 and args.dump_outputs:          # this rank's videos, in the order of plan[0], concatenated
+        res = last["res"]
+        dump_outputs(args.dump_outputs, {
+            "videos": mine, "pairs_per_video": [len(series["values"]) for _, series in res],
+            "actions_per_video": [len(actions) for actions, _ in res],
+            "values": np.concatenate([series["values"] for _, series in res]),
+            "cuts": np.concatenate([series["cuts"] for _, series in res]),
+            "frame_indices": np.concatenate([series["frame_indices"] for _, series in res]),
+            "actions_at": [a["at"] for actions, _ in res for a in actions],
+            "actions_pos": [a["pos"] for actions, _ in res for a in actions]})
     if rank == 0:
         pairs = sum(n - 1 for n in lengths)
         peak, peak_kind = measured_peak()
@@ -649,8 +693,11 @@ def main():
         return
 
     import torch
-    from funscript_flow_b200 import build
-    build.build()
+    from funscript_flow_b200 import _native, build
+    if build.needs_build(build.LIB, build.DEPS):
+        tmp = tempfile.mkdtemp(prefix="ffb_bench_")
+        _native.DEFAULT_LIB = build.build(force=True, lib=os.path.join(tmp, "libffb.so"))
+        atexit.register(shutil.rmtree, tmp, True)
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device (there is no CPU fallback)")
     torch.cuda.set_device(local)

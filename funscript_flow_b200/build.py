@@ -44,10 +44,11 @@ def needs_build(target: str, deps) -> bool:
     return any(os.path.getmtime(d) > t for d in deps)
 
 
-def build(force: bool = False, verbose: bool = False, extra=()) -> str:
-    if not force and not needs_build(LIB, DEPS):
-        return LIB
-    cmd = [find_nvcc(), *NVCC_FLAGS, *extra, "-I", os.path.join(ROOT, "include"), "-I", CSRC, "-o", LIB, *SOURCES]
+def build(force: bool = False, verbose: bool = False, extra=(), lib: str = LIB) -> str:
+    """Compile the library to `lib` (default: in-tree) unless it is newer than its sources; returns its path."""
+    if not force and not needs_build(lib, DEPS):
+        return lib
+    cmd = [find_nvcc(), *NVCC_FLAGS, *extra, "-I", os.path.join(ROOT, "include"), "-I", CSRC, "-o", lib, *SOURCES]
     if verbose:
         cmd.insert(1, "-Xptxas")
         cmd.insert(2, "-v")
@@ -57,7 +58,7 @@ def build(force: bool = False, verbose: bool = False, extra=()) -> str:
         raise RuntimeError("nvcc failed:\n" + res.stdout + res.stderr)
     if verbose:
         print(res.stdout + res.stderr)
-    return LIB
+    return lib
 
 
 if __name__ == "__main__":

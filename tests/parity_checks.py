@@ -4,6 +4,7 @@ called through the C ABI, with the oracle (oracle/) and/or golden vectors record
 reference itself (tests/golden/)."""
 from __future__ import annotations
 
+import hashlib
 import json
 import os
 
@@ -381,3 +382,124 @@ def check_bgr_push_equals_gray_push(ctx, width=320, height=200, n=7):
     rb = ctx.bracket_finish()
     for k in ("scalar", "cut", "cx", "cy", "val", "mean_mag"):
         assert np.array_equal(ra[k], rb[k]), k
+
+
+# ---- records of the comparisons with the reference ----------------------------------------------
+# The reference (FunscriptFlow.pyw) is not part of the repository.  Each record_* function runs one implementation of
+# the reference's functions on the inputs of one test and returns what that test compares, in a form JSON stores
+# exactly (Python floats round-trip, flow fields as SHA-256 of their float32 bytes).  tests/golden/reference_records.json
+# holds the records (tests/golden/make_golden_reference_records.py); the tests compare the oracle and the product with
+# them, and the reference's own functions too when oracle/ref_loader.py finds the file.
+
+def flow_digest(flow):
+    a = np.ascontiguousarray(flow, np.float32)
+    return f"{a.shape[0]}x{a.shape[1]}x{a.shape[2]}:" + hashlib.sha256(a.tobytes()).hexdigest()
+
+
+def record_pairs_and_postprocess(impl, postprocess):
+    """precompute_flow_info / radial_motion_weighted on four pairs of a 128x96 clip, and one post-processed series.
+    `postprocess(final_flow_list, fps, step, params) -> actions`."""
+    clip = make_clip(128, 96, 10, seed=4, period=9.0, amplitude=0.3)
+    pairs = []
+    for j in range(4):
+        info = impl.precompute_flow_info(clip[j], clip[j + 1], {"backend": "CPU"})
+        pairs.append({"flow": flow_digest(info["flow"]), "pos_center": [int(v) for v in info["pos_center"]],
+                      "val_pos": float(info["val_pos"]), "mean_mag": float(info["mean_mag"]), "cut": bool(info["cut"]),
+                      "radial": [float(impl.radial_motion_weighted(info["flow"], c, False, pov))
+                                 for c in ([40.5, 30.25], [64.0, 48.0]) for pov in (False, True)]})
+    rng = np.random.default_rng(3)
+    vals = rng.standard_normal(200).cumsum() * 0.1
+    ffl = [(float(vals[i]), i == 77, i) for i in range(200)]
+    prm = {"detrend_window": 1.5, "norm_window": 4, "keyframe_reduction": True}
+    return {"pairs": pairs, "actions": postprocess(ffl, 30.0, 1, prm)}
+
+
+def record_random_fields(impl):
+    """max_divergence / radial_motion_weighted on the field families of check_reductions_random (ties, zero
+    divergence, centres on and off the frame)."""
+    rng = np.random.default_rng(123)
+    out = []
+    for case in range(30):
+        w, h = int(rng.integers(2, 80)), int(rng.integers(2, 80))
+        flow = rng.standard_normal((h, w, 2)).astype(np.float32)
+        if case % 3 == 1:
+            flow = (flow * 8).round()
+        elif case % 3 == 2:
+            flow[:] = np.float32(rng.uniform(-2, 2))
+        x, y, v = impl.max_divergence(flow)
+        centres = ([float(rng.integers(0, w)), float(rng.integers(0, h))], [rng.uniform(0, w), rng.uniform(0, h)], [-3.5, h + 2.25])
+        out.append({"max_divergence": [int(x), int(y), float(np.float32(v))],
+                    "radial": [float(impl.radial_motion_weighted(flow, c, False, pov)) for c in centres for pov in (False, True)],
+                    "radial_cut": float(impl.radial_motion_weighted(flow, [1.0, 1.0], True, False))})
+    return out
+
+
+def random_postproc_cases():
+    """60 random series (lengths 2..500, random cut positions incl. adjacent cuts and cuts at both ends, 24..120 fps
+    containers, both keyframe modes, short and long windows): (vals, cuts, frame indices, fps, step, params)."""
+    rng = np.random.default_rng(11)
+    for case in range(60):
+        n = int(rng.choice([2, 3, 4, 5, 7, 12, 40, 150, 500]))
+        fps = float(rng.choice([23.976, 24.0, 25.0, 29.97, 30.0, 50.0, 59.94, 60.0, 120.0]))
+        step = max(1, int(np.ceil(fps / 30.0)))
+        kind = case % 3
+        if kind == 0:
+            vals = rng.standard_normal(n).cumsum() * 0.2
+        elif kind == 1:
+            vals = np.sin(np.arange(n) * rng.uniform(0.05, 0.9)) * rng.uniform(0.1, 6) + rng.standard_normal(n) * 0.05
+        else:
+            vals = np.zeros(n) if case % 2 else np.full(n, 0.37)          # flat series: the normalisation's degenerate case
+        cuts = rng.random(n) < rng.choice([0.0, 0.02, 0.2])
+        if n > 3 and case % 5 == 0:
+            cuts[0] = cuts[-1] = True
+            cuts[1] = True
+        idx = [i * step for i in range(n)]
+        prm = {"detrend_window": float(rng.choice([0.5, 1.5, 2.0, 5.0])), "norm_window": float(rng.choice([1.0, 3.0, 4.0, 10.0])),
+               "keyframe_reduction": bool(case % 2)}
+        yield vals, cuts, idx, fps, step, prm
+
+
+def oracle_postprocess(final_flow_list, fps, step, params):
+    return mo.postprocess(final_flow_list, fps, params)
+
+
+def reference_postprocess(ref):
+    """The reference's post-processing statements (oracle/ref_loader.postproc_function) in the form of oracle_postprocess."""
+    from oracle import ref_loader
+    pp = ref_loader.postproc_function(ref)
+    return lambda final_flow_list, fps, step, params: pp(final_flow_list, fps, fps / step, params, lambda *_: None)
+
+
+def record_random_postprocess(postprocess):
+    """The actions of every random_postproc_cases() series; `postprocess(final_flow_list, fps, step, params)`."""
+    return [postprocess([(float(v), bool(c), i) for v, c, i in zip(vals, cuts, idx)], fps, step, prm)
+            for vals, cuts, idx, fps, step, prm in random_postproc_cases()]
+
+
+def record_process_video_logs(process_video, tmp_dir):
+    """The log lines of process_video on a 96x64 FFV1 clip, then of a second call that finds the output; the
+    directory reads <dir>, the backend name and the elapsed time are dropped.  None without an FFV1 writer."""
+    import cv2
+    clip = make_clip(96, 64, 8, seed=12, period=5.0, amplitude=0.3)
+    path = os.path.join(tmp_dir, "log.avi")
+    vw = cv2.VideoWriter(path, cv2.VideoWriter_fourcc(*"FFV1"), 30.0, (96, 64), True)
+    if not vw.isOpened():
+        return None
+    for f in clip:
+        vw.write(cv2.cvtColor(f, cv2.COLOR_GRAY2BGR))
+    vw.release()
+    prm = {"threads": 1, "detrend_window": 2.0, "norm_window": 3.0, "batch_size": 3000, "overwrite": True, "vr_mode": False,
+           "pov_mode": True, "keyframe_reduction": False, "backend": "CPU"}
+    first, again = [], []
+    err = bool(process_video(path, prm, first.append))
+    process_video(path, dict(prm, overwrite=False), again.append)
+
+    def shape(lines):
+        out = []
+        for ln in lines:
+            for prefix in ("Using backend:", "Processing time:"):
+                if ln.startswith(prefix):
+                    ln = prefix
+            out.append(ln.replace(tmp_dir, "<dir>"))
+        return out
+    return {"error_occurred": err, "lines": shape(first), "lines_when_output_exists": shape(again)}

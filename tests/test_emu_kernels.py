@@ -287,44 +287,22 @@ def test_integration_stub_from_the_docs_runs(emu_lib, emu_ctx):
     assert got["val_pos"] == want["val_pos"] and got["cut"] == want["cut"] and got["mean_mag"] == want["mean_mag"]
 
 
-def test_process_video_log_lines_follow_the_reference(emu_ctx, tmp_path):
+def test_process_video_log_lines_follow_the_reference(emu_ctx, golden_dir, tmp_path):
     """Same log lines, in the same order, as the reference's process_video on the same file (backend name and the
-    elapsed time excepted) -- checked live against the AST-loaded reference in the build container."""
+    elapsed time excepted): the lines recorded in tests/golden/reference_records.json, and the
+    AST-loaded reference is run as well when oracle/ref_loader.py finds FunscriptFlow.pyw."""
+    import json
     from oracle import ref_loader
-    if not ref_loader.available():
-        pytest.skip("/root/reference only exists in the build container")
-    import cv2
     api.set_context(emu_ctx)
-    clip = make_clip(96, 64, 8, seed=12, period=5.0, amplitude=0.3)
-    path = str(tmp_path / "log.avi")
-    vw = cv2.VideoWriter(path, cv2.VideoWriter_fourcc(*"FFV1"), 30.0, (96, 64), True)
-    if not vw.isOpened():
+    want = json.load(open(os.path.join(golden_dir, "reference_records.json")))["process_video_logs"]
+    ours = pc.record_process_video_logs(runner.process_video, str(tmp_path))
+    if ours is None:
         pytest.skip("FFV1 writer unavailable")
-    for f in clip:
-        vw.write(cv2.cvtColor(f, cv2.COLOR_GRAY2BGR))
-    vw.release()
-    prm = {"threads": 1, "detrend_window": 2.0, "norm_window": 3.0, "batch_size": 3000, "overwrite": True, "vr_mode": False,
-           "pov_mode": True, "keyframe_reduction": False, "backend": "CPU"}
-    ours, theirs = [], []
-    assert runner.process_video(path, prm, ours.append) is False
-    ref = ref_loader.load("ffref_logs", serial_pools=True)
-    assert not ref.process_video(path, prm, theirs.append)
-
-    def shape(lines):
-        out = []
-        for ln in lines:
-            if ln.startswith("Using backend:"):
-                ln = "Using backend:"
-            if ln.startswith("Processing time:"):
-                ln = "Processing time:"
-            out.append(ln)
-        return out
-    assert shape(ours) == shape(theirs), (ours, theirs)
-    # skip-if-exists line (F:1105-1109)
-    ours.clear(); theirs.clear()
-    runner.process_video(path, dict(prm, overwrite=False), ours.append)
-    ref.process_video(path, dict(prm, overwrite=False), theirs.append)
-    assert ours == theirs
+    assert ours == want
+    if ref_loader.available():
+        (tmp_path / "ref").mkdir()
+        ref = ref_loader.load("ffref_logs", serial_pools=True)
+        assert pc.record_process_video_logs(ref.process_video, str(tmp_path / "ref")) == want
 
 
 def test_configure_is_incremental(emu_lib):

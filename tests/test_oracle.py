@@ -1,7 +1,7 @@
 """CPU suite, part 1: pin the ORACLE.
   * the NumPy Farneback restatement against the installed cv2 (the dependency the reference calls, F:878)
   * the motion-function restatements against golden vectors recorded from the reference itself, and
-    live against the AST-loaded reference when /root/reference is present (build container only)."""
+    live against the AST-loaded reference when oracle/ref_loader.py finds it."""
 import json
 import os
 
@@ -92,25 +92,16 @@ def test_postproc_vs_golden(golden_dir):
     check_postproc_golden(golden_dir)
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference only exists in the build container")
-def test_oracle_vs_live_reference():
-    ref = ref_loader.load("ffref_live", serial_pools=True)
-    clip = make_clip(128, 96, 10, seed=4, period=9.0, amplitude=0.3)
-    cfg = {"backend": "CPU"}
-    for j in range(4):
-        a = ref.precompute_flow_info(clip[j], clip[j + 1], cfg)
-        b = mo.precompute_flow_info(clip[j], clip[j + 1], cfg)
-        assert np.array_equal(a["flow"], b["flow"]) and tuple(a["pos_center"]) == tuple(b["pos_center"])
-        assert a["val_pos"] == b["val_pos"] and a["mean_mag"] == b["mean_mag"] and a["cut"] == b["cut"]
-        for c in ([40.5, 30.25], [64.0, 48.0]):
-            for pov in (False, True):
-                assert ref.radial_motion_weighted(a["flow"], c, False, pov) == mo.radial_motion_weighted(a["flow"], c, False, pov)
-    pp = ref_loader.postproc_function(ref)
-    rng = np.random.default_rng(3)
-    vals = rng.standard_normal(200).cumsum() * 0.1
-    ffl = [(float(vals[i]), i == 77, i) for i in range(200)]
-    prm = {"detrend_window": 1.5, "norm_window": 4, "keyframe_reduction": True}
-    assert pp(ffl, 30.0, 30.0, prm, lambda *_: None) == mo.postprocess(ffl, 30.0, prm)
+def test_oracle_vs_live_reference(golden_dir):
+    """precompute_flow_info / radial_motion_weighted on four pairs and one post-processed series: the oracle against
+    the records of tests/golden/reference_records.json, and against the AST-loaded reference
+    itself when oracle/ref_loader.py finds FunscriptFlow.pyw."""
+    import parity_checks as pc
+    want = json.load(open(os.path.join(golden_dir, "reference_records.json")))["pairs_and_postprocess"]
+    assert pc.record_pairs_and_postprocess(mo, pc.oracle_postprocess) == want
+    if ref_loader.available():
+        ref = ref_loader.load("ffref_live", serial_pools=True)
+        assert pc.record_pairs_and_postprocess(ref, pc.reference_postprocess(ref)) == want
 
 
 def test_preprocess_oracle_bit_exact_vs_cv2():
@@ -161,56 +152,33 @@ def test_oracle_pipeline_vs_golden_video_modes(golden_dir):
         assert acts == case["actions"], case["name"]
 
 
-def test_postproc_product_equals_oracle_on_random_series():
-    """Row N1 beyond the five golden cases: 60 random series (lengths 2..500, random cut positions incl. adjacent
-    cuts and cuts at both ends, 24..120 fps containers, both keyframe modes, short and long windows) through the
-    shipped post-processing and through the oracle restatement -- and through the reference's own statements
-    when /root/reference exists (build container)."""
+def test_postproc_product_equals_oracle_on_random_series(golden_dir):
+    """Row N1 beyond the five golden cases: 60 random series (parity_checks.random_postproc_cases) through the
+    shipped post-processing and through the oracle restatement, against the actions recorded in
+    tests/golden/reference_records.json -- and through the reference's own statements when oracle/ref_loader.py
+    finds FunscriptFlow.pyw."""
+    import parity_checks as pc
     from funscript_flow_b200 import postproc
-    rng = np.random.default_rng(11)
-    pp = ref_loader.postproc_function(ref_loader.load("ffref_pp", serial_pools=True)) if ref_loader.available() else None
-    for case in range(60):
-        n = int(rng.choice([2, 3, 4, 5, 7, 12, 40, 150, 500]))
-        fps = float(rng.choice([23.976, 24.0, 25.0, 29.97, 30.0, 50.0, 59.94, 60.0, 120.0]))
-        step = max(1, int(np.ceil(fps / 30.0)))
-        kind = case % 3
-        if kind == 0:
-            vals = rng.standard_normal(n).cumsum() * 0.2
-        elif kind == 1:
-            vals = np.sin(np.arange(n) * rng.uniform(0.05, 0.9)) * rng.uniform(0.1, 6) + rng.standard_normal(n) * 0.05
-        else:
-            vals = np.zeros(n) if case % 2 else np.full(n, 0.37)          # flat series: the normalisation's degenerate case
-        cuts = rng.random(n) < rng.choice([0.0, 0.02, 0.2])
-        if n > 3 and case % 5 == 0:
-            cuts[0] = cuts[-1] = True
-            cuts[1] = True
-        idx = [i * step for i in range(n)]
-        prm = {"detrend_window": float(rng.choice([0.5, 1.5, 2.0, 5.0])), "norm_window": float(rng.choice([1.0, 3.0, 4.0, 10.0])),
-               "keyframe_reduction": bool(case % 2)}
-        ffl = [(float(vals[i]), bool(cuts[i]), idx[i]) for i in range(n)]
-        want = mo.postprocess(ffl, fps, prm)
+    recorded = json.load(open(os.path.join(golden_dir, "reference_records.json")))["random_postprocess"]
+    cases = list(pc.random_postproc_cases())
+    assert len(recorded) == len(cases)
+    for case, ((vals, cuts, idx, fps, step, prm), want) in enumerate(zip(cases, recorded)):
+        ffl = [(float(vals[i]), bool(cuts[i]), idx[i]) for i in range(len(vals))]
+        assert mo.postprocess(ffl, fps, prm) == want, (case, len(vals), fps, prm)
         got = postproc.scalars_to_actions(vals.tolist(), cuts.tolist(), idx, fps, prm)
-        assert got == want, (case, n, fps, prm)
-        if pp is not None:
-            assert pp(ffl, fps, fps / step, prm, lambda *_: None) == want, (case, n, fps, prm)
+        assert got == want, (case, len(vals), fps, prm)
+    if ref_loader.available():
+        ref = ref_loader.load("ffref_pp", serial_pools=True)
+        assert pc.record_random_postprocess(pc.reference_postprocess(ref)) == recorded
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference only exists in the build container")
-def test_motion_oracle_equals_live_reference_on_random_fields():
-    """The restated max_divergence / radial_motion_weighted against the reference's own functions on the field
-    families of parity_checks.check_reductions_random (ties, zero divergence, centres on and off the frame)."""
-    ref = ref_loader.load("ffref_rand", serial_pools=True)
-    rng = np.random.default_rng(123)
-    for case in range(30):
-        w, h = int(rng.integers(2, 80)), int(rng.integers(2, 80))
-        flow = rng.standard_normal((h, w, 2)).astype(np.float32)
-        if case % 3 == 1:
-            flow = (flow * 8).round()
-        elif case % 3 == 2:
-            flow[:] = np.float32(rng.uniform(-2, 2))
-        a, b = ref.max_divergence(flow), mo.max_divergence(flow)
-        assert (int(a[0]), int(a[1])) == (int(b[0]), int(b[1])) and np.float32(a[2]) == np.float32(b[2])
-        for c in ([float(rng.integers(0, w)), float(rng.integers(0, h))], [rng.uniform(0, w), rng.uniform(0, h)], [-3.5, h + 2.25]):
-            for pov in (False, True):
-                assert ref.radial_motion_weighted(flow, c, False, pov) == mo.radial_motion_weighted(flow, c, False, pov)
-        assert ref.radial_motion_weighted(flow, [1.0, 1.0], True, False) == mo.radial_motion_weighted(flow, [1.0, 1.0], True, False) == 0.0
+def test_motion_oracle_equals_live_reference_on_random_fields(golden_dir):
+    """The restated max_divergence / radial_motion_weighted on the field families of parity_checks.check_reductions_random
+    (ties, zero divergence, centres on and off the frame) against the records of
+    tests/golden/reference_records.json, and against the reference's own functions when oracle/ref_loader.py finds
+    FunscriptFlow.pyw."""
+    import parity_checks as pc
+    want = json.load(open(os.path.join(golden_dir, "reference_records.json")))["random_fields"]
+    assert pc.record_random_fields(mo) == want and all(r["radial_cut"] == 0.0 for r in want)
+    if ref_loader.available():
+        assert pc.record_random_fields(ref_loader.load("ffref_rand", serial_pools=True)) == want
