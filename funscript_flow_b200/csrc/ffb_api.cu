@@ -161,6 +161,10 @@ FfbPolyConsts make_poly_consts() {
 }
 
 // ------------------------------------------------------------------ context
+// k_flow_iter launch of one pyramid level: variant (threads per CTA = matrix columns per strip x rows per step x
+// outputs per horizontal task), strip width and rows per march segment.  nt = 0: no variant forced.
+struct FlowIterPlan { int nt = 0, u = 0, ho = 0, sw = 0, sh = 0; };
+
 struct Level {
     int k = 0, w = 0, h = 0, ksize = 3;
     double sigma = 0;
@@ -174,10 +178,12 @@ struct Level {
     float *xa = nullptr, *ya = nullptr, *uxa = nullptr, *uya = nullptr;
     float* I = nullptr;    // [B][h][rp]
     float2 *fA = nullptr, *fB = nullptr;   // [B][h][fp]
+    FlowIterPlan iter;
+    bool up2x = false;     // exact 2x refinement of the coarser level: its first iteration up-samples the flow itself
 };
 
 struct ProfRec { int kid; int level; double bytes; cudaEvent_t e0, e1; };
-typedef int PtrKindTag;
+struct ProfMark { cudaEvent_t e1 = nullptr; cudaStream_t stream = nullptr; };   // end event of an open record
 
 }  // namespace
 
@@ -185,12 +191,10 @@ struct ffb_ctx {
     int device = 0;
     std::string err;
     cudaStream_t s_comp = nullptr, s_copy = nullptr;
-    cudaStream_t s_aux[3] = {nullptr, nullptr, nullptr};   // extra streams for the sliced flow phase
-    cudaStream_t launch_stream = nullptr;              // stream of the flow-iteration launch in flight
-    cudaStream_t aux_stream = nullptr;                 // stream of the divergence / magnitude launch in flight
+    cudaStream_t s_aux = nullptr;                      // second slice of the sliced flow phase
     cudaStream_t s_time = nullptr;                     // only carries the end-of-flow-phase timing event
-    cudaEvent_t ev_flow_end[4] = {nullptr, nullptr, nullptr, nullptr};
-    cudaEvent_t ev_fork = nullptr, ev_join[3] = {nullptr, nullptr, nullptr};
+    cudaEvent_t ev_flow_end[2] = {nullptr, nullptr};
+    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     cudaEvent_t ev_chain = nullptr;                    // "everything queued on s_comp so far": ffb_chain_after
     cudaEvent_t ev_h2d[2] = {nullptr, nullptr}, ev_expand[2] = {nullptr, nullptr};
     FfbPolyConsts poly;
@@ -202,7 +206,6 @@ struct ffb_ctx {
     Level lev[FFB_MAX_LEVELS];
     float* R = nullptr;
     size_t r_slot_floats = 0;
-    long long seg_frame_px = 0;      // pixels of the frame whose levels are being iterated (segmentation rule)
     float2* ring = nullptr;
     size_t ring_stride = 0;   // float2 per ring element
     uint8_t* d_u8[2] = {nullptr, nullptr};
@@ -215,7 +218,7 @@ struct ffb_ctx {
     double *d_centers = nullptr, *d_scalar = nullptr;
     unsigned long long* d_pkey = nullptr;
     double *d_psum = nullptr, *d_rpart = nullptr;
-    int div_nblk = 0, div_rpb = 0, div_gx = 0, div_gy = 0, rad_gx = 0, rad_gy = 0, rad_rpb = 0;
+    int div_nblk = 0, div_rpb = 0, rad_gx = 0, rad_gy = 0, rad_rpb = 0;
     char* h_res = nullptr;    // pinned result staging
     // frame pre-processing (row N2): source geometry, tables, chunked colour staging
     // source size -> resize target (TW x TH) -> kept window [y0, y0+OH) x [x0, x0+OW) of the target
@@ -235,7 +238,6 @@ struct ffb_ctx {
     bool deferred = false;      // shard mode: the radial pass waits for ffb_bracket_radial (external raw centres)
     bool phase1_read = false;   // ffb_bracket_phase1_finish has been called for the open bracket
     int pend = 0;               // pre-processed gray frames waiting in d_u8[batch_no & 1] for a full batch
-    PtrKindTag pend_kind = 0;   // source kind of the colour frames they came from (first-batch policy)
     // instrumentation
     bool prof = false;
     std::vector<ProfRec> recs;
@@ -249,13 +251,8 @@ struct ffb_ctx {
     size_t pyr_smem_max = 48 * 1024;
     bool attr_poly = false, attr_pyr2 = false;
     std::set<const void*> attr_iter;                     // k_flow_iter instantiations already configured
-    int cur_level = -1;                                  // level k of the flow iteration being launched
-    bool phase_timing = false;                           // sliced flow phase: time the phase, not the launches
-    bool sliced_divmag = false;                          // flow_pairs already launched k_divmag per slice
-    cudaEvent_t phase_rec_e1 = nullptr;
-    bool prof_open = false;                              // a per-launch record is waiting for its end event
+    FlowIterPlan iter_cfg;                               // variant forced by FFB_ITER_CFG for every level
     int flow_streams = 2;
-    int copy_threads = 4;                                // host threads that stage pageable frames into pinned memory
     int64_t launches = 0;
     cudaEvent_t timers[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
 };
@@ -312,55 +309,42 @@ int upload_vec(ffb_ctx* c, T** dptr, const std::vector<T>& v) {
 }
 
 // ---- profiling helpers
-void prof_begin(ffb_ctx* c, int kid, double bytes) {
-    c->launches++;
-    c->k_launches[kid]++;
-    c->k_bytes[kid] += bytes;
-    const int lvl = (kid == FFB_K_FLOW_ITER && c->cur_level >= 0 && c->cur_level < FFB_MAX_LEVELS) ? c->cur_level : -1;
-    if (lvl >= 0) { c->it_launches[lvl]++; c->it_bytes[lvl] += bytes; }
-    if (!c->prof || (kid == FFB_K_FLOW_ITER && c->phase_timing)) return;
-    ProfRec r;
-    r.kid = kid;
-    r.level = lvl;
-    r.bytes = bytes;
+// Opens a timed record of kernel `kid`: its start event is recorded on `stream` now, its end event by prof_end.
+ProfMark prof_record(ffb_ctx* c, int kid, int level, double bytes, cudaStream_t stream) {
+    ProfRec r{kid, level, bytes, nullptr, nullptr};
     for (cudaEvent_t* e : {&r.e0, &r.e1}) {
         if (!c->ev_pool.empty()) { *e = c->ev_pool.back(); c->ev_pool.pop_back(); }
         else cudaEventCreate(e);
     }
-    cudaEventRecord(r.e0, kid == FFB_K_FLOW_ITER ? c->launch_stream : (kid == FFB_K_DIVMAG ? c->aux_stream : c->s_comp));
+    cudaEventRecord(r.e0, stream);
     c->recs.push_back(r);
-    c->prof_open = true;
+    return ProfMark{r.e1, stream};
 }
-void prof_end(ffb_ctx* c) {
-    if (!c->prof_open) return;          // prof_begin did not open a per-launch record
-    c->prof_open = false;
-    const int kid_ = c->recs.back().kid;
-    cudaEventRecord(c->recs.back().e1, kid_ == FFB_K_FLOW_ITER ? c->launch_stream : (kid_ == FFB_K_DIVMAG ? c->aux_stream : c->s_comp));
+// Counts a launch of `kid` on `stream` (a k_flow_iter launch also under its pyramid level; -1: no level) and, when
+// profiling is on and the launch is timed on its own, brackets it with events on that stream.
+ProfMark prof_begin(ffb_ctx* c, int kid, int level, double bytes, cudaStream_t stream, bool timed = true) {
+    c->launches++;
+    c->k_launches[kid]++;
+    c->k_bytes[kid] += bytes;
+    if (level >= 0) { c->it_launches[level]++; c->it_bytes[level] += bytes; }
+    return c->prof && timed ? prof_record(c, kid, level, bytes, stream) : ProfMark{};
+}
+void prof_end(const ProfMark& m) {
+    if (m.e1) cudaEventRecord(m.e1, m.stream);
 }
 // Sliced flow phase: the launch chains of the slices overlap, so per-launch event times would count
 // the same device time several times.  The phase is timed as a whole on s_comp instead
 // (fork ... join) and attributed to k_flow_iter.
-void prof_phase_begin(ffb_ctx* c) {
-    if (!c->prof) return;
-    ProfRec r;
-    r.kid = FFB_K_FLOW_ITER;
-    r.level = -1;
-    r.bytes = 0;
-    for (cudaEvent_t* e : {&r.e0, &r.e1}) {
-        if (!c->ev_pool.empty()) { *e = c->ev_pool.back(); c->ev_pool.pop_back(); }
-        else cudaEventCreate(e);
-    }
-    cudaEventRecord(r.e0, c->s_comp);
-    c->phase_rec_e1 = r.e1;
-    c->recs.push_back(r);
+ProfMark prof_phase_begin(ffb_ctx* c) {
+    return c->prof ? prof_record(c, FFB_K_FLOW_ITER, -1, 0, c->s_comp) : ProfMark{};
 }
 // the phase ends when the last slice's last flow iteration does: a side stream waits for every slice's
 // end-of-flow event and records the timing event, so that the per-slice reductions that follow on the
 // slice streams are not counted
-void prof_phase_end(ffb_ctx* c, int nslice) {
-    if (!c->prof) return;
+void prof_phase_end(ffb_ctx* c, const ProfMark& phase, int nslice) {
+    if (!phase.e1) return;
     for (int i = 0; i < nslice; ++i) cudaStreamWaitEvent(c->s_time, c->ev_flow_end[i], 0);
-    cudaEventRecord(c->phase_rec_e1, c->s_time);
+    cudaEventRecord(phase.e1, c->s_time);
 }
 
 void prof_collect(ffb_ctx* c) {
@@ -409,9 +393,9 @@ int launch_pyramid(ffb_ctx* c, const uint8_t* src, size_t src_stride, int src_pi
         c->pyr_smem_max = smem;
     }
     dim3 grid((w + PYR_TW - 1) / PYR_TW, (h + PYR_TH - 1) / PYR_TH, nframes);
-    prof_begin(c, FFB_K_PYRAMID, (double)nframes * ((double)W * H + 4.0 * w * h));
+    const ProfMark pm = prof_begin(c, FFB_K_PYRAMID, -1, (double)nframes * ((double)W * H + 4.0 * w * h), c->s_comp);
     FFB_LAUNCH(kfn, grid, dim3(PYR_TW * PYR_TH), smem, c->s_comp, a);
-    prof_end(c);
+    prof_end(pm);
     CKL(c);
     return FFB_OK;
 }
@@ -432,9 +416,9 @@ int launch_polyexp(ffb_ctx* c, const float* src, size_t src_stride, int sp, int 
     // against 3.92 ms per 257 1080p frames for this scalar kernel; the packed instructions issue at half rate and the
     // 114 registers they need halve the occupancy.  profiles/r2_other_kernels.txt)
     dim3 grid((w + POLY_OW - 1) / POLY_OW, (h + POLY_ROWS - 1) / POLY_ROWS, nframes);
-    prof_begin(c, FFB_K_POLYEXP, (double)nframes * 24.0 * w * h);
+    const ProfMark pm = prof_begin(c, FFB_K_POLYEXP, -1, (double)nframes * 24.0 * w * h, c->s_comp);
     FFB_LAUNCH(k_polyexp, grid, dim3(256), POLY_SMEM, c->s_comp, a);
-    prof_end(c);
+    prof_end(pm);
     CKL(c);
     return FFB_OK;
 }
@@ -447,78 +431,63 @@ int launch_upsample(ffb_ctx* c, const float2* src, size_t src_stride, int sp, in
     a.dst = dst; a.dst_stride = dst_stride; a.dp = dp; a.w = w; a.h = h;
     a.xi = xi; a.xa = xa; a.yi = yi; a.ya = ya;
     dim3 grid((w + 31) / 32, (h + 7) / 8, npairs);
-    prof_begin(c, FFB_K_UPSAMPLE, (double)npairs * (8.0 * wc * hc + 8.0 * w * h));
+    const ProfMark pm = prof_begin(c, FFB_K_UPSAMPLE, -1, (double)npairs * (8.0 * wc * hc + 8.0 * w * h), c->s_comp);
     FFB_LAUNCH(k_upsample_flow, grid, dim3(256), 0, c->s_comp, a);
-    prof_end(c);
+    prof_end(pm);
     CKL(c);
     return FFB_OK;
 }
 
-// Tunables of the fused iteration kernel.  The defaults are compiled in; the environment overrides exist for
-// tuning runs and for the tests that force a variant onto small frames (parsed per launch):
-//   FFB_ITER_CFG=NTxUxHO   threads per CTA (= matrix columns per strip) x rows per step x outputs per horizontal task;
-//                          compiled in: 256x4x8, 128x2x4, 160x2x4, 96x2x4, 64x2x4 (the round-2 sweeps measured and dropped 192 /
-//                          512-thread strips, 8-output tasks on 2-row steps, 4-output tasks on 4-row steps, non-allocating
-//                          loads, bulk L2 prefetch, early issue of the second row pair, and a barrier-free variant in which
-//                          neighbouring warps synchronise through shared-memory flags: profiles/r2_sweep_flow_iter.txt)
-//   FFB_ITER_CFG_K<k>      the same for pyramid level k only
-//   FFB_ITER_SH / FFB_ITER_MINSEG   rows per march segment (upper bound) / minimum segments per level
-//   FFB_ITER_SWMAX=0       equal-width strips (round 1) instead of full-width strips plus a narrow last one
-struct IterCfg { int nt, u, ho, sh, swmax; };
-IterCfg iter_cfg() {
-    IterCfg c{0, 2, 4, 270, 1};
-    if (const char* e = getenv("FFB_ITER_CFG")) {
-        int nt = 0, u = 0, ho = 0;
-        if (sscanf(e, "%dx%dx%d", &nt, &u, &ho) == 3) { c.nt = nt; c.u = u; c.ho = ho; }
+// Launch plan of k_flow_iter on a w x h level of frame_w x frame_h frames (the frame the context is configured for;
+// a stage hook passes the level itself).  It depends on this geometry alone, never on the batch, so a pair's result is
+// bit-identical however frames are batched or sharded.  `forced`: a variant forced for every level (FFB_ITER_CFG).
+FlowIterPlan flow_iter_plan(int frame_w, int frame_h, int w, int h, const FlowIterPlan& forced) {
+    const bool large = (long long)frame_w * frame_h >= 1280LL * 720;
+    FlowIterPlan p = forced;
+    if (p.nt == 0) {
+        // Defaults from the round-2 sweeps on a B200 (profiles/r2_sweep_flow_iter.txt):
+        //   1280x720 and larger   256 threads, 4 rows per step, 8 outputs per horizontal task: 242-column strips carry
+        //                         5.5 % halo columns instead of 10.9 %, and the 120 horizontal tasks of a step fill 4 of
+        //                         the 8 warps (1080p: +8.4 % over 128x2x4, 4K: +7 %, 720p: +1 %)
+        //   up to 320 columns     160 threads x 2 rows x 4 outputs (the reference's 256x256 product mode: 2 strips); its
+        //                         64- and 32-column levels take 96- and 64-thread strips (5 / 8 CTAs per SM instead of
+        //                         mostly idle 160-thread ones) and a single row segment per level: +3 % together
+        //   in between            128 threads x 2 rows x 4 outputs (640x360: +8 % over 160x2x4)
+        if (large) { p.nt = 256; p.u = 4; p.ho = 8; }
+        else if (frame_w <= 320) { p.nt = w <= 48 ? 64 : (w <= 80 ? 96 : 160); p.u = 2; p.ho = 4; }     // by LEVEL width
+        else { p.nt = 128; p.u = 2; p.ho = 4; }
     }
-    if (const char* e = getenv("FFB_ITER_SH")) { const int v = atoi(e); if (v >= 16) c.sh = v; }
-    if (const char* e = getenv("FFB_ITER_SWMAX")) c.swmax = atoi(e) != 0;
-    return c;
-}
-
-template <int NT, int U, int MINB, int HO>
-int launch_flow_iter_t(ffb_ctx* c, FfbIterArgs a, int npairs, int sh_target, double bytes) {
-    const int w = a.w, h = a.h;
-    const int sw_max = (NT - 2 * FFB_WIN_R) / HO * HO;
-    if (iter_cfg().swmax) {
-        // full-width strips; the last one is narrower and its idle warps skip the gather (k_flow_iter `live`)
-        a.SW = sw_max;
-    } else {
-        const int nstrips = (w + sw_max - 1) / sw_max;
-        a.SW = ffb_round_up((w + nstrips - 1) / nstrips, HO);
-        if (a.SW > sw_max) a.SW = sw_max;
-    }
-    const int gx = (w + a.SW - 1) / a.SW;
-    // Row segments depend on the level geometry only (never on the batch composition), so a pair's
-    // result is bit-identical however frames are batched or sharded.
-    // at most sh_target rows per segment, at least min_seg segments per level (coarse levels would
-    // otherwise be a handful of long, latency-bound marches), never under 32 rows
-    const int min_seg_env = getenv("FFB_ITER_MINSEG") ? atoi(getenv("FFB_ITER_MINSEG")) : 0;
-    // frames of 1280x720 and more: at least 3 segments on every level (parallelism for their 64-pair batches; 2 .. 4
-    // measure the same at 1080p, 5 and more lose); smaller frames come in batches of hundreds, and every segment pays
-    // 14 halo rows: 2 (+7 % at 256x256, +3.5 % at 640x360) -- profiles/r1_sweep_segments.txt, r2_sweep_flow_iter.txt.
-    // The rule looks at the frame the context is configured for, never at the batch.
-    const long long frame_px = c->seg_frame_px > 0 ? c->seg_frame_px : (long long)w * h;      // stage hooks: the level itself
-    const int frame_w0 = c->seg_frame_px > 0 ? c->W : w;
-    const int min_seg = min_seg_env > 0 ? min_seg_env : (frame_px >= 1280LL * 720 ? 3 : (frame_w0 <= 320 ? 1 : 2));
-    int nseg = (h + sh_target - 1) / sh_target;
+    if (p.u < 1 || p.ho < 1) return p;      // no such variant: launch_flow_iter refuses it
+    // full-width strips; the last one is narrower and its idle warps skip the gather (k_flow_iter `live`)
+    p.sw = (p.nt - 2 * FFB_WIN_R) / p.ho * p.ho;
+    // at most 270 rows per segment, at least min_seg segments per level (coarse levels would otherwise be a handful of
+    // long, latency-bound marches), never under 32 rows.  Frames of 1280x720 and more: at least 3 segments on every
+    // level (parallelism for their 64-pair batches; 2 .. 4 measure the same at 1080p, 5 and more lose); smaller frames
+    // come in batches of hundreds, and every segment pays 14 halo rows: 2 (+7 % at 256x256, +3.5 % at 640x360) --
+    // profiles/r1_sweep_segments.txt, r2_sweep_flow_iter.txt.
+    const int min_seg = large ? 3 : (frame_w <= 320 ? 1 : 2);
+    int nseg = (h + 269) / 270;
     if (nseg < min_seg) nseg = min_seg;
     if (nseg > (h + 31) / 32) nseg = (h + 31) / 32;
     if (nseg < 1) nseg = 1;
-    a.SH = ffb_round_up((h + nseg - 1) / nseg, U);     // even: see the fused up-sampling in k_flow_iter
-    const int gy = (h + a.SH - 1) / a.SH;
+    p.sh = ffb_round_up((h + nseg - 1) / nseg, p.u);     // even: see the fused up-sampling in k_flow_iter
+    return p;
+}
+
+template <int NT, int U, int MINB, int HO>
+int launch_flow_iter_t(ffb_ctx* c, const FfbIterArgs& a, int npairs, int level, double bytes, cudaStream_t stream, bool timed) {
     auto kfn = a.up_src ? k_flow_iter<NT, U, MINB, true, HO> : k_flow_iter<NT, U, MINB, false, HO>;
     const size_t smem = ffb_flow_iter_smem<NT, U, HO>();
     if (!c->attr_iter.count((const void*)kfn)) {
         CK(c, cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         c->attr_iter.insert((const void*)kfn);
     }
-    prof_begin(c, FFB_K_FLOW_ITER, bytes);
+    const ProfMark pm = prof_begin(c, FFB_K_FLOW_ITER, level, bytes, stream, timed);
     // pair index varies fastest in launch order: the CTAs working on one spatial tile of consecutive
     // pairs are co-resident, so frame j+1's expansion (R1 of pair j, R0 of pair j+1) is read from
     // HBM once and hit in L2 the second time.
-    FFB_LAUNCH(kfn, dim3(npairs, gx, gy), dim3(NT), smem, c->launch_stream, a);
-    prof_end(c);
+    FFB_LAUNCH(kfn, dim3(npairs, (a.w + a.SW - 1) / a.SW, (a.h + a.SH - 1) / a.SH), dim3(NT), smem, stream, a);
+    prof_end(pm);
     CKL(c);
     return FFB_OK;
 }
@@ -527,12 +496,15 @@ struct UpSrc {   // coarser-level flow to be up-sampled inside the iteration ker
     const float2* src = nullptr; size_t stride = 0; int sp = 0, wc = 0, hc = 0;
 };
 
-int launch_flow_iter(ffb_ctx* c, FfbRing R, size_t plane, int rp, int w, int h, const float2* fin, size_t fin_stride,
-                     int fip, FfbRing fout, int fop, int npairs, const UpSrc* up = nullptr) {
+// One k_flow_iter launch of plan `p` on `stream`, counted under pyramid level `level` (-1: none).  timed = false inside
+// the sliced flow phase, which is timed as a whole.
+int launch_flow_iter(ffb_ctx* c, const FlowIterPlan& p, int level, cudaStream_t stream, bool timed, FfbRing R, size_t plane,
+                     int rp, int w, int h, const float2* fin, size_t fin_stride, int fip, FfbRing fout, int fop, int npairs,
+                     const UpSrc* up = nullptr) {
     FfbIterArgs a;
     a.R = R; a.plane = (int)plane; a.rp = rp; a.w = w; a.h = h;
     a.fin = fin; a.fin_stride = fin_stride; a.fip = fip; a.fout = fout; a.fop = fop;
-    a.SW = a.SH = 0;
+    a.SW = p.sw; a.SH = p.sh;
     a.up_src = nullptr; a.up_stride = 0; a.usp = a.wc = a.hc = 0;
     double bpp = fin ? 56.0 : 48.0;
     if (up && up->src) {
@@ -544,41 +516,20 @@ int launch_flow_iter(ffb_ctx* c, FfbRing R, size_t plane, int rp, int w, int h, 
     // the kernel stores four flow vectors with one 32-byte instruction
     if (fop % 4 != 0 || ((uintptr_t)fout.base | (uintptr_t)fout.stride) % 32 != 0)
         return fail(c, FFB_E_INVALID, "flow output is not 32-byte aligned (pitch %d, stride %zu)", fop, fout.stride);
-    const IterCfg k = iter_cfg();
-    int nt = k.nt, u = k.u, ho = k.ho;
-    if (c->cur_level >= 0 && c->cur_level < FFB_MAX_LEVELS) {      // FFB_ITER_CFG_K<k>: one level only
-        char name[24];
-        snprintf(name, sizeof(name), "FFB_ITER_CFG_K%d", c->cur_level);
-        if (const char* e = getenv(name)) {
-            int a1 = 0, a2 = 0, a3 = 0;
-            if (sscanf(e, "%dx%dx%d", &a1, &a2, &a3) == 3) { nt = a1; u = a2; ho = a3; }
-        }
-    }
-    if (nt == 0) {
-        // Defaults from the round-2 sweeps on a B200 (profiles/r2_sweep_flow_iter.txt), keyed on the frame the context
-        // is configured for (never on the batch):
-        //   1280x720 and larger   256 threads, 4 rows per step, 8 outputs per horizontal task: 242-column strips carry
-        //                         5.5 % halo columns instead of 10.9 %, and the 120 horizontal tasks of a step fill 4 of
-        //                         the 8 warps (1080p: +8.4 % over 128x2x4, 4K: +7 %, 720p: +1 %)
-        //   up to 320 columns     160 threads x 2 rows x 4 outputs (the reference's 256x256 product mode: 2 strips); its
-        //                         64- and 32-column levels take 96- and 64-thread strips (5 / 8 CTAs per SM instead of
-        //                         mostly idle 160-thread ones) and a single row segment per level: +3 % together
-        //   in between            128 threads x 2 rows x 4 outputs (640x360: +8 % over 160x2x4)
-        const long long frame_px = c->seg_frame_px > 0 ? c->seg_frame_px : (long long)w * h;
-        const int frame_w = c->seg_frame_px > 0 ? c->W : w;
-        if (frame_px >= 1280LL * 720) { nt = 256; u = 4; ho = 8; }
-        else if (frame_w <= 320) { nt = w <= 48 ? 64 : (w <= 80 ? 96 : 160); u = 2; ho = 4; }     // by LEVEL width
-        else { nt = 128; u = 2; ho = 4; }
-    }
-    switch (nt * 100 + u * 10 + ho) {
-        case 25648: return launch_flow_iter_t<256, 4, 2, 8>(c, a, npairs, k.sh, bytes);
-        case 12824: return launch_flow_iter_t<128, 2, 4, 4>(c, a, npairs, k.sh, bytes);
-        case 16024: return launch_flow_iter_t<160, 2, 3, 4>(c, a, npairs, k.sh, bytes);
-        case 9624:  return launch_flow_iter_t<96, 2, 5, 4>(c, a, npairs, k.sh, bytes);
-        case 6424:  return launch_flow_iter_t<64, 2, 8, 4>(c, a, npairs, k.sh, bytes);
+    // compiled in: 256x4x8, 128x2x4, 160x2x4, 96x2x4, 64x2x4 (the round-2 sweeps measured and dropped 192 / 512-thread
+    // strips, 8-output tasks on 2-row steps, 4-output tasks on 4-row steps, non-allocating loads, bulk L2 prefetch, early
+    // issue of the second row pair, and a barrier-free variant in which neighbouring warps synchronise through
+    // shared-memory flags: profiles/r2_sweep_flow_iter.txt)
+    switch (p.nt * 100 + p.u * 10 + p.ho) {
+        case 25648: return launch_flow_iter_t<256, 4, 2, 8>(c, a, npairs, level, bytes, stream, timed);
+        case 12824: return launch_flow_iter_t<128, 2, 4, 4>(c, a, npairs, level, bytes, stream, timed);
+        case 16024: return launch_flow_iter_t<160, 2, 3, 4>(c, a, npairs, level, bytes, stream, timed);
+        case 9624:  return launch_flow_iter_t<96, 2, 5, 4>(c, a, npairs, level, bytes, stream, timed);
+        case 6424:  return launch_flow_iter_t<64, 2, 8, 4>(c, a, npairs, level, bytes, stream, timed);
         default: break;
     }
-    return fail(c, FFB_E_INVALID, "FFB_ITER_CFG: no k_flow_iter variant %dx%dx%d (compiled in: 256x4x8, 128x2x4, 160x2x4, 96x2x4, 64x2x4)", nt, u, ho);
+    return fail(c, FFB_E_INVALID, "FFB_ITER_CFG: no k_flow_iter variant %dx%dx%d (compiled in: 256x4x8, 128x2x4, 160x2x4, 96x2x4, 64x2x4)",
+                p.nt, p.u, p.ho);
 }
 
 // ------------------------------------------------------------------ geometry
@@ -658,7 +609,7 @@ bool pyramid_fast_ok(int W, int H, const LevelPlan& p);
 int quiesce(ffb_ctx* c) {
     CK(c, cudaStreamSynchronize(c->s_comp));
     CK(c, cudaStreamSynchronize(c->s_copy));
-    for (int i = 0; i < 3; ++i) CK(c, cudaStreamSynchronize(c->s_aux[i]));
+    CK(c, cudaStreamSynchronize(c->s_aux));
     return FFB_OK;
 }
 
@@ -692,6 +643,8 @@ int configure(ffb_ctx* c, int W, int H, int B, int maxPairs, int ring_pairs = 0)
             off += 5 * L.plane;
             off = (off + 63) / 64 * 64;
             L.taps = make_taps(L.ksize, L.sigma);
+            L.iter = flow_iter_plan(W, H, L.w, L.h, c->iter_cfg);
+            L.up2x = l > 0 && L.w == 2 * c->lev[l - 1].w && L.h == 2 * c->lev[l - 1].h;
             TRY(build_level_tables(c, L, W, H, l > 0 ? c->lev[l - 1].w : 0, l > 0 ? c->lev[l - 1].h : 0));
         }
         c->r_slot_floats = (off + 127) / 128 * 128;      // 512-byte multiples
@@ -699,9 +652,7 @@ int configure(ffb_ctx* c, int W, int H, int B, int maxPairs, int ring_pairs = 0)
         c->ring_stride = (size_t)c->fp0 * H;
         // reduction geometry: fixed per frame size so results do not depend on batch composition
         c->div_rpb = 8;       // whole rows per block: long contiguous reads (a column-marching variant measured slower)
-        c->div_gx = (H + c->div_rpb - 1) / c->div_rpb;
-        c->div_gy = 1;
-        c->div_nblk = c->div_gx;
+        c->div_nblk = (H + c->div_rpb - 1) / c->div_rpb;
         c->rad_gx = (W + 255) / 256;
         c->rad_rpb = 32;
         c->rad_gy = (H + c->rad_rpb - 1) / c->rad_rpb;
@@ -754,8 +705,7 @@ int configure(ffb_ctx* c, int W, int H, int B, int maxPairs, int ring_pairs = 0)
 // ------------------------------------------------------------------ the per-batch pipeline
 // All levels in one pass when every level is an exact 2^k decimation (W, H multiples of 8).
 bool pyramid_fast_ok(int W, int H, const LevelPlan& p) {
-    static const bool generic = getenv("FFB_PYR_GENERIC") && atoi(getenv("FFB_PYR_GENERIC")) != 0;
-    if (generic || W % 8 || H % 8 || W < 64 || H < 64) return false;
+    if (W % 8 || H % 8 || W < 64 || H < 64) return false;
     static const int want[FFB_MAX_LEVELS] = {3, 3, 9, 19};
     for (int l = 0; l < p.n; ++l)
         if (p.ksize[l] != want[p.k[l]] || p.w[l] != (W >> p.k[l]) || p.h[l] != (H >> p.k[l])) return false;
@@ -782,9 +732,9 @@ int launch_pyramid_pow2(ffb_ctx* c, const uint8_t* src, size_t stride, int pitch
         c->attr_pyr2 = true;
     }
     dim3 grid((W + PYR2_TX - 1) / PYR2_TX, (H + PYR2_TY - 1) / PYR2_TY, nb);
-    prof_begin(c, FFB_K_PYRAMID, (double)nb * ((double)W * H + 4.0 * px));
+    const ProfMark pm = prof_begin(c, FFB_K_PYRAMID, -1, (double)nb * ((double)W * H + 4.0 * px), c->s_comp);
     FFB_LAUNCH(k_pyramid_pow2, grid, dim3(256), PYR2_SMEM, c->s_comp, a);
-    prof_end(c);
+    prof_end(pm);
     CKL(c);
     return FFB_OK;
 }
@@ -816,38 +766,44 @@ int expand_frames(ffb_ctx* c, const uint8_t* src, size_t stride, int pitch, int 
     return FFB_OK;
 }
 
-int launch_divmag(ffb_ctx* c, int p0, int off, int cnt, cudaStream_t stream);
+// divergence / magnitude partials of `cnt` pairs starting at pair p0 + off of the bracket, on `stream`
+int launch_divmag(ffb_ctx* c, int p0, int off, int cnt, cudaStream_t stream) {
+    FfbDivArgs d;
+    d.flow = FfbRing{(char*)c->ring, c->ring_stride * sizeof(float2), (p0 + off) % c->ring_n, c->ring_n};
+    d.fp = c->fp0; d.w = c->W; d.h = c->H; d.rows_per_block = c->div_rpb;
+    d.pkey = c->d_pkey + (size_t)off * c->div_nblk;
+    d.psum = c->d_psum + (size_t)off * c->div_nblk;
+    const ProfMark pm = prof_begin(c, FFB_K_DIVMAG, -1, (double)cnt * 8.0 * c->W * c->H, stream);
+    FFB_LAUNCH(k_divmag, dim3(c->div_nblk, 1, cnt), dim3(256), 0, stream, d);
+    prof_end(pm);
+    CKL(c);
+    return FFB_OK;
+}
 
+// Final flows of bracket pairs [p0, p0 + np) into the ring, and their divergence / magnitude partials.
 int flow_pairs(ffb_ctx* c, int p0, int np) {
-    c->phase_timing = false;
-    c->seg_frame_px = (long long)c->W * c->H;
-    static const bool fuse_up = !(getenv("FFB_FUSE_UP") && atoi(getenv("FFB_FUSE_UP")) == 0);
-    // FFB_FLOW_STREAMS=n (1..4): the pairs of a batch are split in n slices whose launch chains run on
-    // n streams, so that the short coarse-level launches (and the tail of every launch) of one slice
-    // overlap the other slices' work.  Every buffer is indexed by pair; the slices share nothing that
-    // is written.
-    const int want_slices = c->flow_streams;
-    bool all_fused = fuse_up;
-    for (int l = 1; l < c->nlev; ++l)
-        all_fused = all_fused && c->lev[l].w == 2 * c->lev[l - 1].w && c->lev[l].h == 2 * c->lev[l - 1].h;
-    int nslice = want_slices < 1 ? 1 : (want_slices > 4 ? 4 : want_slices);
-    if (!all_fused || np < 4 * nslice) nslice = 1;
-    int soff[5];
-    for (int i = 0; i <= nslice; ++i) soff[i] = (int)((long long)np * i / nslice);
-    if (nslice > 1) {
-        prof_phase_begin(c);
-        c->phase_timing = true;
+    // The pairs of a batch are split in two slices whose launch chains run on two streams, so that the short
+    // coarse-level launches (and the tail of every launch) of one slice overlap the other slice's work (+4 %; 3-4 slices
+    // measured no better).  Every buffer is indexed by pair; the slices share nothing that is written.
+    // FFB_FLOW_STREAMS=1 keeps one chain, whose launches can be timed one by one.
+    bool all_fused = true;
+    for (int l = 1; l < c->nlev; ++l) all_fused = all_fused && c->lev[l].up2x;
+    const int nslice = c->flow_streams > 1 && all_fused && np >= 8 ? 2 : 1;
+    const bool sliced = nslice > 1;
+    const int soff[3] = {0, np / nslice, np};
+    const cudaStream_t streams[2] = {c->s_comp, c->s_aux};
+    ProfMark phase;
+    if (sliced) {
+        phase = prof_phase_begin(c);
         CK(c, cudaEventRecord(c->ev_fork, c->s_comp));
-        for (int i = 1; i < nslice; ++i) CK(c, cudaStreamWaitEvent(c->s_aux[i - 1], c->ev_fork, 0));
+        CK(c, cudaStreamWaitEvent(c->s_aux, c->ev_fork, 0));
     }
     for (int l = 0; l < c->nlev; ++l) {
         Level& L = c->lev[l];
-        c->cur_level = L.k;
         const size_t fstride = (size_t)L.fp * L.h;
         const bool last = l == c->nlev - 1;
         const float2* fin0 = nullptr;
-        const bool fused = l > 0 && fuse_up && L.w == 2 * c->lev[l - 1].w && L.h == 2 * c->lev[l - 1].h;
-        if (l > 0 && !fused) {
+        if (l > 0 && !L.up2x) {
             Level& C = c->lev[l - 1];
             TRY(launch_upsample(c, C.fB, (size_t)C.fp * C.h, C.fp, C.w, C.h, L.fA, fstride, L.fp, L.w, L.h, L.uxi,
                                 L.uxa, L.uyi, L.uya, np));
@@ -856,7 +812,6 @@ int flow_pairs(ffb_ctx* c, int p0, int np) {
         for (int it = 0; it < FFB_ITERS; ++it) {
             for (int sl = 0; sl < nslice; ++sl) {
                 const int off = soff[sl], cnt = soff[sl + 1] - soff[sl];
-                c->launch_stream = sl == 0 ? c->s_comp : c->s_aux[sl - 1];
                 FfbRing R;
                 R.base = (char*)(c->R + L.r_off);
                 R.stride = c->r_slot_floats * sizeof(float);
@@ -865,78 +820,65 @@ int flow_pairs(ffb_ctx* c, int p0, int np) {
                 FfbRing toB{(char*)(L.fB + (size_t)off * fstride), fstride * sizeof(float2), 0, 1 << 30};
                 FfbRing toA{(char*)(L.fA + (size_t)off * fstride), fstride * sizeof(float2), 0, 1 << 30};
                 FfbRing toRing{(char*)c->ring, c->ring_stride * sizeof(float2), (p0 + off) % c->ring_n, c->ring_n};
-                int rc;
-                if (it == 0) {
-                    UpSrc up;
-                    if (fused) {
-                        Level& C = c->lev[l - 1];
-                        up.stride = (size_t)C.fp * C.h;
-                        up.src = C.fB + (size_t)off * up.stride; up.sp = C.fp; up.wc = C.w; up.hc = C.h;
-                    }
-                    rc = launch_flow_iter(c, R, L.plane, L.rp, L.w, L.h, fin0 ? fin0 + (size_t)off * fstride : nullptr, fstride,
-                                          L.fp, toB, L.fp, cnt, &up);
-                } else if (it == 1) {
-                    rc = launch_flow_iter(c, R, L.plane, L.rp, L.w, L.h, L.fB + (size_t)off * fstride, fstride, L.fp, toA, L.fp, cnt);
-                } else {
-                    rc = launch_flow_iter(c, R, L.plane, L.rp, L.w, L.h, L.fA + (size_t)off * fstride, fstride, L.fp,
-                                          last ? toRing : toB, L.fp, cnt);
+                UpSrc up;
+                if (l > 0 && L.up2x) {
+                    Level& C = c->lev[l - 1];
+                    up.stride = (size_t)C.fp * C.h;
+                    up.src = C.fB + (size_t)off * up.stride; up.sp = C.fp; up.wc = C.w; up.hc = C.h;
                 }
-                c->launch_stream = c->s_comp;
-                TRY(rc);
+                // iteration 0 starts from the up-sampled coarser flow (or zero) into fB, 1 runs fB -> fA, 2 fA -> ring | fB
+                const float2* fin = it == 0 ? (fin0 ? fin0 + (size_t)off * fstride : nullptr)
+                                            : (it == 1 ? L.fB : L.fA) + (size_t)off * fstride;
+                const FfbRing& fout = it == 1 ? toA : (it == 2 && last ? toRing : toB);
+                TRY(launch_flow_iter(c, L.iter, L.k, streams[sl], !sliced, R, L.plane, L.rp, L.w, L.h, fin, fstride, L.fp,
+                                     fout, L.fp, cnt, it == 0 ? &up : nullptr));
             }
         }
     }
-    if (nslice > 1) {
-        c->phase_timing = false;
-        for (int sl = 0; sl < nslice; ++sl) CK(c, cudaEventRecord(c->ev_flow_end[sl], sl == 0 ? c->s_comp : c->s_aux[sl - 1]));
-        prof_phase_end(c, nslice);
-        // each slice reduces its own pairs as soon as its chain is done (overlaps the other slice's tail)
-        for (int sl = 0; sl < nslice; ++sl)
-            TRY(launch_divmag(c, p0, soff[sl], soff[sl + 1] - soff[sl], sl == 0 ? c->s_comp : c->s_aux[sl - 1]));
+    if (sliced) {
+        for (int sl = 0; sl < nslice; ++sl) CK(c, cudaEventRecord(c->ev_flow_end[sl], streams[sl]));
+        prof_phase_end(c, phase, nslice);
     }
-    for (int i = 1; i < nslice; ++i) {
-        CK(c, cudaEventRecord(c->ev_join[i - 1], c->s_aux[i - 1]));
-        CK(c, cudaStreamWaitEvent(c->s_comp, c->ev_join[i - 1], 0));
+    // each slice reduces its own pairs as soon as its chain is done (overlaps the other slice's tail)
+    for (int sl = 0; sl < nslice; ++sl) TRY(launch_divmag(c, p0, soff[sl], soff[sl + 1] - soff[sl], streams[sl]));
+    if (sliced) {
+        CK(c, cudaEventRecord(c->ev_join, c->s_aux));
+        CK(c, cudaStreamWaitEvent(c->s_comp, c->ev_join, 0));
     }
-    c->sliced_divmag = nslice > 1;
-    c->cur_level = -1;
-    c->seg_frame_px = 0;
     return FFB_OK;
 }
 
-// divergence / magnitude partials of `cnt` pairs starting at pair p0 + off of the bracket, on `stream`
-int launch_divmag(ffb_ctx* c, int p0, int off, int cnt, cudaStream_t stream) {
-    FfbDivArgs d;
-    d.flow = FfbRing{(char*)c->ring, c->ring_stride * sizeof(float2), (p0 + off) % c->ring_n, c->ring_n};
-    d.fp = c->fp0; d.w = c->W; d.h = c->H; d.rows_per_block = c->div_rpb;
-    d.pkey = c->d_pkey + (size_t)off * c->div_nblk;
-    d.psum = c->d_psum + (size_t)off * c->div_nblk;
-    c->aux_stream = stream;
-    prof_begin(c, FFB_K_DIVMAG, (double)cnt * 8.0 * c->W * c->H);
-    FFB_LAUNCH(k_divmag, dim3(c->div_gx, c->div_gy, cnt), dim3(256), 0, stream, d);
-    prof_end(c);
-    c->aux_stream = c->s_comp;
-    CKL(c);
-    return FFB_OK;
-}
-
-int launch_phase1_finish(ffb_ctx* c, int p0, int np) {
+// per-pair centre, value, mean magnitude and cut flag of pairs [p0, p0 + np) from their divergence / magnitude partials
+int launch_phase1_finish(ffb_ctx* c, int p0, int np, int pov, float cut_threshold) {
     FfbP1Args f;
     f.flow = FfbRing{(char*)c->ring, c->ring_stride * sizeof(float2), p0 % c->ring_n, c->ring_n};
     f.fp = c->fp0; f.w = c->W; f.h = c->H;
     f.pkey = c->d_pkey; f.psum = c->d_psum; f.nblk = c->div_nblk;
-    f.pov = c->pov; f.cut_threshold = c->thr; f.out0 = p0;
+    f.pov = pov; f.cut_threshold = cut_threshold; f.out0 = p0;
     f.cx = c->d_cx; f.cy = c->d_cy; f.val = c->d_val; f.mean_mag = c->d_mm; f.cut = c->d_cut;
-    prof_begin(c, FFB_K_SMALL, 0);
+    const ProfMark pm = prof_begin(c, FFB_K_SMALL, -1, 0, c->s_comp);
     FFB_LAUNCH(k_phase1_finish, dim3(np), dim3(32), 0, c->s_comp, f);
-    prof_end(c);
+    prof_end(pm);
     CKL(c);
     return FFB_OK;
 }
 
-int phase1_reduce(ffb_ctx* c, int p0, int np) {
-    TRY(launch_divmag(c, p0, 0, np, c->s_comp));
-    return launch_phase1_finish(c, p0, np);
+// k_radial + k_radial_finish of ring pairs [j0, j0 + cnt) (cnt <= ring_n): d_scalar[j0 ..] from d_centers and d_cut
+int launch_radial(ffb_ctx* c, int j0, int cnt, int pov) {
+    FfbRadArgs r;
+    r.flow = FfbRing{(char*)c->ring, c->ring_stride * sizeof(float2), j0 % c->ring_n, c->ring_n};
+    r.fp = c->fp0; r.w = c->W; r.h = c->H; r.rows_per_block = c->rad_rpb;
+    r.centers = c->d_centers; r.cut = c->d_cut; r.out0 = j0; r.pov = pov; r.partial = c->d_rpart;
+    const ProfMark pm = prof_begin(c, FFB_K_RADIAL, -1, (double)cnt * 8.0 * c->W * c->H, c->s_comp);
+    FFB_LAUNCH(k_radial, dim3(c->rad_gx, c->rad_gy, cnt), dim3(256), 0, c->s_comp, r);
+    prof_end(pm);
+    CKL(c);
+    const ProfMark pf = prof_begin(c, FFB_K_SMALL, -1, 0, c->s_comp);
+    FFB_LAUNCH(k_radial_finish, dim3(cnt), dim3(32), 0, c->s_comp, (const double*)c->d_rpart, c->rad_gx * c->rad_gy, c->W,
+               c->H, j0, c->d_scalar);
+    prof_end(pf);
+    CKL(c);
+    return FFB_OK;
 }
 
 // radial pass for bracket pairs [j0, j1); n = number of pairs known so far (window truncation).
@@ -945,25 +887,13 @@ int radial_range(ffb_ctx* c, int j0, int j1, int n, bool smooth = true) {
     while (j0 < j1) {
         const int cnt = (j1 - j0 < c->ring_n) ? j1 - j0 : c->ring_n;
         if (smooth) {
-            prof_begin(c, FFB_K_SMALL, 0);
+            const ProfMark pm = prof_begin(c, FFB_K_SMALL, -1, 0, c->s_comp);
             FFB_LAUNCH(k_smooth_centers, dim3((cnt + 127) / 128), dim3(128), 0, c->s_comp, c->d_cx, c->d_cy, n, j0,
                        j0 + cnt, 0, c->d_centers);
-            prof_end(c);
+            prof_end(pm);
             CKL(c);
         }
-        FfbRadArgs r;
-        r.flow = FfbRing{(char*)c->ring, c->ring_stride * sizeof(float2), j0 % c->ring_n, c->ring_n};
-        r.fp = c->fp0; r.w = c->W; r.h = c->H; r.rows_per_block = c->rad_rpb;
-        r.centers = c->d_centers; r.cut = c->d_cut; r.out0 = j0; r.pov = c->pov; r.partial = c->d_rpart;
-        prof_begin(c, FFB_K_RADIAL, (double)cnt * 8.0 * c->W * c->H);
-        FFB_LAUNCH(k_radial, dim3(c->rad_gx, c->rad_gy, cnt), dim3(256), 0, c->s_comp, r);
-        prof_end(c);
-        CKL(c);
-        prof_begin(c, FFB_K_SMALL, 0);
-        FFB_LAUNCH(k_radial_finish, dim3(cnt), dim3(32), 0, c->s_comp, (const double*)c->d_rpart,
-                   c->rad_gx * c->rad_gy, c->W, c->H, j0, c->d_scalar);
-        prof_end(c);
-        CKL(c);
+        TRY(launch_radial(c, j0, cnt, c->pov));
         j0 += cnt;
     }
     return FFB_OK;
@@ -971,10 +901,12 @@ int radial_range(ffb_ctx* c, int j0, int j1, int n, bool smooth = true) {
 
 // Pageable frames reach the pinned staging buffer through host memcpy: one thread moves ~7 GB/s, less than the
 // GPU consumes at 1080p (a 257-frame bracket is 533 MB every 36 ms), so large copies are cut into row ranges and
-// moved by a few threads (FFB_COPY_THREADS, default 4; they inherit the caller's CPU affinity, i.e. the NUMA
-// node of the GPU when the process was bound to it).  n frames of `rows` rows of `row` bytes each.
+// moved by kCopyThreads threads (they inherit the caller's CPU affinity, i.e. the NUMA node of the GPU when the
+// process was bound to it; one thread: 3 700 pairs/s at 1080p, four: 5 990 -- profiles/r2_host_paths.txt).
+// n frames of `rows` rows of `row` bytes each.
+constexpr int kCopyThreads = 4;
 void copy_frames(uint8_t* dst, size_t dst_frame, const uint8_t* src, size_t src_frame, size_t src_pitch, int n, int rows,
-                 size_t row, int max_threads) {
+                 size_t row) {
     const long long total_rows = (long long)n * rows;
     auto work = [=](long long r0, long long r1) {
         while (r0 < r1) {
@@ -988,7 +920,7 @@ void copy_frames(uint8_t* dst, size_t dst_frame, const uint8_t* src, size_t src_
         }
     };
     int t = (int)(((size_t)total_rows * row) >> 21);          // at least 2 MB per thread
-    if (t > max_threads) t = max_threads;
+    if (t > kCopyThreads) t = kCopyThreads;
     if (t <= 1) { work(0, total_rows); return; }
     std::vector<std::thread> pool;
     for (int i = 1; i < t; ++i) pool.emplace_back(work, total_rows * i / t, total_rows * (i + 1) / t);
@@ -1008,6 +940,30 @@ PtrKind classify(const void* p) {
     return PTR_PAGEABLE;
 }
 
+// H2D on s_copy of n host frames (`rows` rows of `row` bytes, `pitch` bytes apart; frames `stride` bytes apart) into
+// the dense device buffer `dst`, which the kernels before `ev_consumer` read.  Pinned input is copied directly,
+// pageable input through the pinned staging buffer `pin`.  `ev_dma` marks the end of the copy (and so the end of
+// the last DMA out of `pin`); s_comp waits for it.
+int upload_frames(ffb_ctx* c, uint8_t* dst, uint8_t* pin, cudaEvent_t ev_dma, cudaEvent_t ev_consumer, const uint8_t* src,
+                  PtrKind kind, int n, int rows, size_t row, size_t pitch, size_t stride) {
+    const size_t fbytes = row * rows;
+    CK(c, cudaStreamWaitEvent(c->s_copy, ev_consumer, 0));
+    if (kind == PTR_PAGEABLE) {
+        CK(c, cudaEventSynchronize(ev_dma));
+        copy_frames(pin, fbytes, src, stride, pitch, n, rows, row);
+        CK(c, cudaMemcpyAsync(dst, pin, (size_t)n * fbytes, cudaMemcpyHostToDevice, c->s_copy));
+    } else if (pitch == row && stride == fbytes) {
+        CK(c, cudaMemcpyAsync(dst, src, (size_t)n * fbytes, cudaMemcpyHostToDevice, c->s_copy));
+    } else {
+        for (int f = 0; f < n; ++f)
+            CK(c, cudaMemcpy2DAsync(dst + (size_t)f * fbytes, row, src + (size_t)f * stride, pitch, row, rows,
+                                    cudaMemcpyHostToDevice, c->s_copy));
+    }
+    CK(c, cudaEventRecord(ev_dma, c->s_copy));
+    CK(c, cudaStreamWaitEvent(c->s_comp, ev_dma, 0));
+    return FFB_OK;
+}
+
 int process_batch(ffb_ctx* c, const uint8_t* frames, int nb, size_t pitch, size_t stride, PtrKind kind) {
     const int b = c->batch_no & 1;
     const size_t fbytes = (size_t)c->W * c->H;
@@ -1016,20 +972,8 @@ int process_batch(ffb_ctx* c, const uint8_t* frames, int nb, size_t pitch, size_
     int s_pitch = (int)pitch;
     if (kind != PTR_DEVICE) {
         // staging buffer b was last read by the expansion kernels two batches ago
-        CK(c, cudaStreamWaitEvent(c->s_copy, c->ev_expand[b], 0));
-        if (kind == PTR_PAGEABLE) {
-            CK(c, cudaEventSynchronize(c->ev_h2d[b]));   // previous DMA out of h_pin[b] finished
-            copy_frames(c->h_pin[b], fbytes, frames, stride, pitch, nb, c->H, (size_t)c->W, c->copy_threads);
-            CK(c, cudaMemcpyAsync(c->d_u8[b], c->h_pin[b], (size_t)nb * fbytes, cudaMemcpyHostToDevice, c->s_copy));
-        } else if (pitch == (size_t)c->W && stride == fbytes) {
-            CK(c, cudaMemcpyAsync(c->d_u8[b], frames, (size_t)nb * fbytes, cudaMemcpyHostToDevice, c->s_copy));
-        } else {
-            for (int f = 0; f < nb; ++f)
-                CK(c, cudaMemcpy2DAsync(c->d_u8[b] + (size_t)f * fbytes, c->W, frames + (size_t)f * stride, pitch, c->W,
-                                        c->H, cudaMemcpyHostToDevice, c->s_copy));
-        }
-        CK(c, cudaEventRecord(c->ev_h2d[b], c->s_copy));
-        CK(c, cudaStreamWaitEvent(c->s_comp, c->ev_h2d[b], 0));
+        TRY(upload_frames(c, c->d_u8[b], c->h_pin[b], c->ev_h2d[b], c->ev_expand[b], frames, kind, nb, c->H, (size_t)c->W,
+                          pitch, stride));
         src = c->d_u8[b];
         s_stride = fbytes;
         s_pitch = c->W;
@@ -1044,8 +988,7 @@ int process_batch(ffb_ctx* c, const uint8_t* frames, int nb, size_t pitch, size_
         if (c->deferred && p0 + np > c->ring_n)
             return fail(c, FFB_E_INVALID, "shard exceeds the %d pairs announced to ffb_bracket_begin_shard", c->ring_n);
         TRY(flow_pairs(c, p0, np));
-        if (c->sliced_divmag) TRY(launch_phase1_finish(c, p0, np));
-        else TRY(phase1_reduce(c, p0, np));
+        TRY(launch_phase1_finish(c, p0, np, c->pov, c->thr));
         c->pairs_done += np;
         const int r1 = c->pairs_done - 6;
         if (!c->deferred && r1 > c->radial_done) {
@@ -1127,9 +1070,9 @@ int launch_preprocess(ffb_ctx* c, const uint8_t* src, size_t stride, int pitch, 
     a.dst = dst; a.dst_frame_stride = (size_t)p.OW * p.OH; a.dst_pitch = p.OW;
     a.xt = xt; a.yt = yt; a.TW = p.TW; a.TH = p.TH; a.x_off = p.x0; a.y_off = p.y0; a.OW = p.OW; a.OH = p.OH;
     // algorithmic bytes: the 2x2 footprint of every output pixel (3 bytes each) + the gray output
-    prof_begin(c, FFB_K_PREPROC, (double)n * ((double)p.OW * p.OH * 13.0));
+    const ProfMark pm = prof_begin(c, FFB_K_PREPROC, -1, (double)n * ((double)p.OW * p.OH * 13.0), c->s_comp);
     FFB_LAUNCH(k_preprocess, dim3((p.OW + 31) / 32, (p.OH + 7) / 8, n), dim3(256), 0, c->s_comp, a);
-    prof_end(c);
+    prof_end(pm);
     CKL(c);
     return FFB_OK;
 }
@@ -1200,15 +1143,16 @@ int ffb_create(int device, ffb_ctx** out) {
     cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming);
     cudaEventCreateWithFlags(&c->ev_chain, cudaEventDisableTiming);
     cudaStreamCreateWithFlags(&c->s_time, cudaStreamNonBlocking);
-    for (int i = 0; i < 4; ++i) cudaEventCreateWithFlags(&c->ev_flow_end[i], cudaEventDisableTiming);
-    for (int i = 0; i < 3; ++i) {
-        cudaStreamCreateWithFlags(&c->s_aux[i], cudaStreamNonBlocking);
-        cudaEventCreateWithFlags(&c->ev_join[i], cudaEventDisableTiming);
-    }
-    c->launch_stream = c->s_comp;
-    c->aux_stream = c->s_comp;
+    for (int i = 0; i < 2; ++i) cudaEventCreateWithFlags(&c->ev_flow_end[i], cudaEventDisableTiming);
+    cudaStreamCreateWithFlags(&c->s_aux, cudaStreamNonBlocking);
+    cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming);
+    // FFB_FLOW_STREAMS=1: one launch chain for the flow phase, so that bench.py can time its launches one by one
     if (const char* e = getenv("FFB_FLOW_STREAMS")) c->flow_streams = atoi(e);
-    if (const char* e = getenv("FFB_COPY_THREADS")) { const int v = atoi(e); if (v >= 1 && v <= 64) c->copy_threads = v; }
+    // FFB_ITER_CFG=NTxUxHO forces one k_flow_iter variant on every level (the CPU tests run each variant on small frames)
+    if (const char* e = getenv("FFB_ITER_CFG")) {
+        int nt = 0, u = 0, ho = 0;
+        if (sscanf(e, "%dx%dx%d", &nt, &u, &ho) == 3) { c->iter_cfg.nt = nt; c->iter_cfg.u = u; c->iter_cfg.ho = ho; }
+    }
     for (int b = 0; b < 2; ++b) {
         cudaEventCreateWithFlags(&c->ev_h2d[b], cudaEventDisableTiming);
         cudaEventCreateWithFlags(&c->ev_expand[b], cudaEventDisableTiming);
@@ -1240,9 +1184,10 @@ void ffb_destroy(ffb_ctx* c) {
     }
     cudaEventDestroy(c->ev_fork);
     cudaEventDestroy(c->ev_chain);
-    for (int i = 0; i < 4; ++i) cudaEventDestroy(c->ev_flow_end[i]);
+    for (int i = 0; i < 2; ++i) cudaEventDestroy(c->ev_flow_end[i]);
     cudaStreamDestroy(c->s_time);
-    for (int i = 0; i < 3; ++i) { cudaEventDestroy(c->ev_join[i]); cudaStreamDestroy(c->s_aux[i]); }
+    cudaEventDestroy(c->ev_join);
+    cudaStreamDestroy(c->s_aux);
     cudaStreamDestroy(c->s_comp);
     cudaStreamDestroy(c->s_copy);
     delete c;
@@ -1257,7 +1202,6 @@ int ffb_host_free(void* p) { return cudaFreeHost(p) == cudaSuccess ? FFB_OK : FF
 static int configure_checked(ffb_ctx* c, int w, int h, int batch_frames, int max_pairs, int ring_pairs) {
     if (!c) return FFB_E_INVALID;
     CK(c, cudaSetDevice(c->device));
-    const int W0 = c->W;
     const int rc = configure(c, w, h, batch_frames, max_pairs, ring_pairs);
     // an allocation that failed half-way leaves no half-built geometry behind (argument errors change nothing)
     if (rc != FFB_OK && rc != FFB_E_INVALID && !c->in_bracket) {
@@ -1265,7 +1209,6 @@ static int configure_checked(ffb_ctx* c, int w, int h, int batch_frames, int max
         free_geometry(c);
         c->err = msg;
     }
-    (void)W0;
     return rc;
 }
 
@@ -1363,7 +1306,7 @@ int ffb_bracket_abort(ffb_ctx* c) {
     // queued work reads the caller's buffers and the staging rings: let it drain (errors are already recorded)
     cudaStreamSynchronize(c->s_copy);
     cudaStreamSynchronize(c->s_comp);
-    for (int i = 0; i < 3; ++i) cudaStreamSynchronize(c->s_aux[i]);
+    cudaStreamSynchronize(c->s_aux);
     cudaGetLastError();
     c->in_bracket = false;
     c->deferred = c->phase1_read = false;
@@ -1467,10 +1410,10 @@ int ffb_bracket_radial(ffb_ctx* c, const int32_t* cx_ext, const int32_t* cy_ext,
         // the raw centres of the shard and of up to 6 neighbours on each side, as the neighbours computed them
         CK(c, cudaMemcpyAsync(c->d_cx_ext, cx_ext, (size_t)n_ext * 4, cudaMemcpyHostToDevice, c->s_comp));
         CK(c, cudaMemcpyAsync(c->d_cy_ext, cy_ext, (size_t)n_ext * 4, cudaMemcpyHostToDevice, c->s_comp));
-        prof_begin(c, FFB_K_SMALL, 0);
+        const ProfMark pm = prof_begin(c, FFB_K_SMALL, -1, 0, c->s_comp);
         FFB_LAUNCH(k_smooth_centers, dim3((n + 127) / 128), dim3(128), 0, c->s_comp, c->d_cx_ext, c->d_cy_ext, n_ext, first,
                    first + n, first, c->d_centers);
-        prof_end(c);
+        prof_end(pm);
         CKL(c);
         TRY(radial_range(c, 0, n, n, false));
         c->radial_done = n;
@@ -1518,14 +1461,8 @@ static int flow_stats(ffb_ctx* c, const float* flow, int w, int h, int32_t* x, i
     if (!c || !flow) return FFB_E_INVALID;
     CK(c, cudaSetDevice(c->device));
     TRY(upload_flow(c, flow, w, h));
-    const int pov = c->pov;
-    const float thr = c->thr;
-    c->pov = 0;
-    c->thr = std::numeric_limits<float>::infinity();
-    const int rc = phase1_reduce(c, 0, 1);
-    c->pov = pov;
-    c->thr = thr;
-    TRY(rc);
+    TRY(launch_divmag(c, 0, 0, 1, c->s_comp));
+    TRY(launch_phase1_finish(c, 0, 1, 0, std::numeric_limits<float>::infinity()));
     int hx = 0, hy = 0;
     float hv = 0, hm = 0;
     CK(c, cudaMemcpyAsync(&hx, c->d_cx, 4, cudaMemcpyDeviceToHost, c->s_comp));
@@ -1556,19 +1493,7 @@ int ffb_radial_motion(ffb_ctx* c, const float* flow, int w, int h, double cx, do
     const unsigned char zero = 0;
     CK(c, cudaMemcpyAsync(c->d_centers, cen, 16, cudaMemcpyHostToDevice, c->s_comp));
     CK(c, cudaMemcpyAsync(c->d_cut, &zero, 1, cudaMemcpyHostToDevice, c->s_comp));
-    FfbRadArgs r;
-    r.flow = FfbRing{(char*)c->ring, c->ring_stride * sizeof(float2), 0, c->ring_n};
-    r.fp = c->fp0; r.w = w; r.h = h; r.rows_per_block = c->rad_rpb;
-    r.centers = c->d_centers; r.cut = c->d_cut; r.out0 = 0; r.pov = pov ? 1 : 0; r.partial = c->d_rpart;
-    prof_begin(c, FFB_K_RADIAL, 8.0 * w * h);
-    FFB_LAUNCH(k_radial, dim3(c->rad_gx, c->rad_gy, 1), dim3(256), 0, c->s_comp, r);
-    prof_end(c);
-    CKL(c);
-    prof_begin(c, FFB_K_SMALL, 0);
-    FFB_LAUNCH(k_radial_finish, dim3(1), dim3(32), 0, c->s_comp, (const double*)c->d_rpart, c->rad_gx * c->rad_gy, w, h, 0,
-               c->d_scalar);
-    prof_end(c);
-    CKL(c);
+    TRY(launch_radial(c, 0, 1, pov ? 1 : 0));
     CK(c, cudaMemcpyAsync(out, c->d_scalar, 8, cudaMemcpyDeviceToHost, c->s_comp));
     CK(c, cudaStreamSynchronize(c->s_comp));
     return FFB_OK;
@@ -1681,9 +1606,9 @@ int ffb_stage_update_matrices(ffb_ctx* c, const float* R0, const float* R1, cons
     if (flow) TRY(s.upload(c, &df, (const float2*)flow, (size_t)w * h));
     TRY(s.alloc(c, &dM, (size_t)5 * w * h));
     FfbMatArgs a{d0, d1, (size_t)w * h, w, w, h, df, w, dM};
-    prof_begin(c, FFB_K_SMALL, 0);
+    const ProfMark pm = prof_begin(c, FFB_K_SMALL, -1, 0, c->s_comp);
     FFB_LAUNCH(k_update_matrices, dim3((w + 31) / 32, (h + 7) / 8), dim3(256), 0, c->s_comp, a);
-    prof_end(c);
+    prof_end(pm);
     CKL(c);
     CK(c, cudaStreamSynchronize(c->s_comp));
     CK(c, cudaMemcpy(out, dM, (size_t)5 * w * h * 4, cudaMemcpyDeviceToHost));
@@ -1710,7 +1635,8 @@ int ffb_stage_flow_iter(ffb_ctx* c, const float* R0, const float* R1, const floa
     TRY(s.alloc(c, &dfo, plane));
     FfbRing R{(char*)dR, 5 * plane * sizeof(float), 0, 2};
     FfbRing fo{(char*)dfo, 0, 0, 1};
-    TRY(launch_flow_iter(c, R, plane, rp, w, h, dfi, 0, rp, fo, rp, 1));
+    TRY(launch_flow_iter(c, flow_iter_plan(w, h, w, h, c->iter_cfg), -1, c->s_comp, true, R, plane, rp, w, h, dfi, 0, rp, fo,
+                         rp, 1));
     CK(c, cudaStreamSynchronize(c->s_comp));
     CK(c, cudaMemcpy2D(flow_out, (size_t)w * 8, dfo, (size_t)rp * 8, (size_t)w * 8, h, cudaMemcpyDeviceToHost));
     return FFB_OK;
@@ -1794,20 +1720,8 @@ int ffb_bracket_push_bgr(ffb_ctx* c, const uint8_t* bgr, int n, size_t pitch, si
         if (kind != PTR_DEVICE) {
             const int cb = c->color_no & 1;
             c->color_no++;
-            CK(c, cudaStreamWaitEvent(c->s_copy, c->ev_pre[cb], 0));      // kernel that last read d_color[cb]
-            if (kind == PTR_PAGEABLE) {
-                CK(c, cudaEventSynchronize(c->ev_ch2d[cb]));              // DMA that last read h_color[cb]
-                copy_frames(c->h_color[cb], fbytes, src, stride, pitch, m, pp.H, row, c->copy_threads);
-                CK(c, cudaMemcpyAsync(c->d_color[cb], c->h_color[cb], (size_t)m * fbytes, cudaMemcpyHostToDevice, c->s_copy));
-            } else if (pitch == row && stride == fbytes) {
-                CK(c, cudaMemcpyAsync(c->d_color[cb], src, (size_t)m * fbytes, cudaMemcpyHostToDevice, c->s_copy));
-            } else {
-                for (int f = 0; f < m; ++f)
-                    CK(c, cudaMemcpy2DAsync(c->d_color[cb] + (size_t)f * fbytes, row, src + (size_t)f * stride, pitch, row,
-                                            pp.H, cudaMemcpyHostToDevice, c->s_copy));
-            }
-            CK(c, cudaEventRecord(c->ev_ch2d[cb], c->s_copy));
-            CK(c, cudaStreamWaitEvent(c->s_comp, c->ev_ch2d[cb], 0));
+            TRY(upload_frames(c, c->d_color[cb], c->h_color[cb], c->ev_ch2d[cb], c->ev_pre[cb], src, kind, m, pp.H, row,
+                              pitch, stride));
             TRY(launch_preprocess(c, c->d_color[cb], fbytes, (int)row, dst, pp, c->pre_xt, c->pre_yt, m));
             CK(c, cudaEventRecord(c->ev_pre[cb], c->s_comp));
         } else {
