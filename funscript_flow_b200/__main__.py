@@ -3,6 +3,8 @@
     python -m funscript_flow_b200 INPUT [--threads N] [--detrend_window S] [--norm_window S] [--batch_size N]
                                   [--overwrite] [--vr_mode] [--pov_mode] [--disable_keyframe_reduction]
                                   [--native_resolution] [--vr_eye left|right|both]      (extensions, SURVEY row N4)
+                                  [--flow_pyr_scale S] [--flow_levels N] [--flow_winsize N] [--flow_iterations N]
+                                  [--flow_poly_n 5|7] [--flow_poly_sigma S]             (Farneback parameters)
 
 Under `torchrun --nproc-per-node N` every rank takes each N-th video of the folder on its own GPU.
 The reference's quirk is kept (SURVEY Q4): `--disable_keyframe_reduction` is a store_false flag whose
@@ -14,7 +16,7 @@ import argparse
 import os
 import sys
 
-from . import runner
+from . import api, runner
 
 
 def build_parser() -> argparse.ArgumentParser:
@@ -33,6 +35,14 @@ def build_parser() -> argparse.ArgumentParser:
     p.add_argument("--native_resolution", action="store_true", help="run the flow on the decoded frame size instead of 256x256")
     p.add_argument("--vr_eye", choices=["left", "right", "both"], default="left",
                    help="which eye of a side-by-side VR frame (with --vr_mode); both = mean of the two eyes' scalars")
+    # cv2.calcOpticalFlowFarneback's parameters; the defaults are the reference's call (F:878-879)
+    ref = api.REFERENCE_FARNEBACK
+    p.add_argument("--flow_pyr_scale", type=float, default=ref["pyr_scale"], help="pyramid scale between levels, 0 < s < 1")
+    p.add_argument("--flow_levels", type=int, default=ref["levels"], help="pyramid levels above the frame (>= 0)")
+    p.add_argument("--flow_winsize", type=int, default=ref["winsize"], help="averaging window, 3 .. 63")
+    p.add_argument("--flow_iterations", type=int, default=ref["iterations"], help="iterations per level, 1 .. 20")
+    p.add_argument("--flow_poly_n", type=int, choices=[5, 7], default=ref["poly_n"], help="polynomial expansion size")
+    p.add_argument("--flow_poly_sigma", type=float, default=ref["poly_sigma"], help="polynomial expansion sigma (>= 0)")
     return p
 
 
@@ -53,6 +63,10 @@ def settings_from_args(args) -> dict:
         settings["native_resolution"] = True
     if getattr(args, "vr_eye", "left") != "left":
         settings["vr_eye"] = args.vr_eye
+    for key, name in api.FARNEBACK_SETTINGS.items():
+        value = getattr(args, key, None)
+        if value is not None and value != api.REFERENCE_FARNEBACK[name]:
+            settings[key] = value
     return settings
 
 

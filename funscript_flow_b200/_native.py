@@ -68,6 +68,9 @@ def load(path: Optional[str] = None) -> C.CDLL:
         "ffb_mean_magnitude": (i32, [vp, f32p, i32, i32, f32p]),
         "ffb_radial_motion": (i32, [vp, f32p, i32, i32, C.c_double, C.c_double, i32, i32, f64p]),
         "ffb_level_plan": (i32, [i32, i32, i32p, i32p, i32p, i32p, f64p]),
+        "ffb_set_farneback": (i32, [vp, C.c_double, i32, i32, i32, i32, C.c_double, i32]),
+        "ffb_get_farneback": (i32, [vp, f64p, i32p, i32p, i32p, i32p, f64p, i32p]),
+        "ffb_level_plan_ex": (i32, [i32, i32, C.c_double, i32, i32, i32p, i32p, i32p, i32p, f64p]),
         "ffb_stage_pyramid": (i32, [vp, u8p, i32, i32, sz, i32, f32p]),
         "ffb_stage_polyexp": (i32, [vp, f32p, i32, i32, f32p]),
         "ffb_stage_update_matrices": (i32, [vp, f32p, f32p, f32p, i32, i32, f32p]),
@@ -127,6 +130,21 @@ def level_plan(width: int, height: int, lib_path: Optional[str] = None):
     if rc:
         raise FFBError(rc, "ffb_level_plan")
     return [dict(w=w[i], h=h[i], ksize=ks[i], sigma=sg[i]) for i in range(n.value)]
+
+
+MAX_PLAN_LEVELS = 16
+
+
+def level_plan_ex(width: int, height: int, pyr_scale: float, levels: int, lib_path: Optional[str] = None):
+    """Level geometry (coarsest first) for any (pyr_scale, levels): list of dicts k, w, h, ksize, sigma."""
+    lib = load(lib_path)
+    n = C.c_int32(0)
+    w, h, ks = ((C.c_int32 * MAX_PLAN_LEVELS)() for _ in range(3))
+    sg = (C.c_double * MAX_PLAN_LEVELS)()
+    rc = lib.ffb_level_plan_ex(int(width), int(height), float(pyr_scale), int(levels), MAX_PLAN_LEVELS, C.byref(n), w, h, ks, sg)
+    if rc:
+        raise FFBError(rc, f"ffb_level_plan_ex({width}, {height}, {pyr_scale}, {levels})")
+    return [dict(k=n.value - 1 - i, w=w[i], h=h[i], ksize=ks[i], sigma=sg[i]) for i in range(n.value)]
 
 
 def _u8(a):
@@ -216,6 +234,23 @@ class FlowContext:
         d, h = C.c_int64(0), C.c_int64(0)
         self._ck(self._lib.ffb_alloc_counts(self._h, C.byref(d), C.byref(h)))
         return int(d.value), int(h.value)
+
+    def set_farneback(self, pyr_scale: float = 0.5, levels: int = 3, winsize: int = 15, iterations: int = 3,
+                      poly_n: int = 5, poly_sigma: float = 1.2, flags: int = 0):
+        """Parameters of every flow this context computes (cv2.calcOpticalFlowFarneback's, after `flow`); the defaults
+        are the reference's call.  Equal parameters change nothing; refused inside a bracket."""
+        self._ck(self._lib.ffb_set_farneback(self._h, float(pyr_scale), int(levels), int(winsize), int(iterations), int(poly_n),
+                                             float(poly_sigma), int(flags)))
+
+    @property
+    def farneback_params(self) -> dict:
+        """The parameters set_farneback took last (the reference's for a new context)."""
+        ps, sg = C.c_double(), C.c_double()
+        lv, ws, it, pn, fl = (C.c_int32() for _ in range(5))
+        self._ck(self._lib.ffb_get_farneback(self._h, C.byref(ps), C.byref(lv), C.byref(ws), C.byref(it), C.byref(pn),
+                                             C.byref(sg), C.byref(fl)))
+        return dict(pyr_scale=ps.value, levels=lv.value, winsize=ws.value, iterations=it.value, poly_n=pn.value,
+                    poly_sigma=sg.value, flags=fl.value)
 
     def bracket_begin(self, pov_mode: bool = False, cut_threshold: float = 7.0):
         self._ck(self._lib.ffb_bracket_begin(self._h, int(bool(pov_mode)), float(cut_threshold)))
@@ -373,7 +408,8 @@ class FlowContext:
     def stage_pyramid(self, img: np.ndarray, level_k: int) -> np.ndarray:
         img = np.ascontiguousarray(img, dtype=np.uint8)
         h, w = img.shape
-        plan = level_plan(w, h, self._lib._name)
+        fp = self.farneback_params
+        plan = level_plan_ex(w, h, fp["pyr_scale"], fp["levels"], self._lib._name)
         lv = plan[len(plan) - 1 - level_k]
         out = np.empty((lv["h"], lv["w"]), np.float32)
         self._ck(self._lib.ffb_stage_pyramid(self._h, _u8(img), w, h, w, int(level_k), _f32(out)))
@@ -431,10 +467,11 @@ class FlowContext:
             out[name] = dict(launches=int(n.value), ms=float(ms.value), alg_bytes=float(by.value))
         return out
 
-    def flow_iter_level_stats(self):
-        """k_flow_iter launches / device ms / algorithmic bytes per pyramid level k (0 = full resolution)."""
+    def flow_iter_level_stats(self, levels: int = 4):
+        """Flow-iteration launches / device ms / algorithmic bytes per pyramid level k (0 = full resolution) for
+        k < levels (at most 16; the reference's plans have 4)."""
         out = {}
-        for k in range(4):
+        for k in range(levels):
             n, ms, by = C.c_int64(), C.c_double(), C.c_double()
             self._ck(self._lib.ffb_flow_iter_level_stats(self._h, k, C.byref(n), C.byref(ms), C.byref(by)))
             if n.value:

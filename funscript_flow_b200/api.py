@@ -7,6 +7,12 @@
     max_divergence(flow)                            F:748-758
     radial_motion_weighted(flow, center, is_cut, pov_mode=False)   F:761-785
     get_available_backends()                        F:32-63
+    calc_optical_flow_farneback(prev, next, None, pyr_scale, levels, winsize, iterations, poly_n, poly_sigma, 0)
+                                                    cv2's signature (F:878), any parameter set
+
+Every entry point that configures a context first sets its Farneback parameters from the settings keys
+flow_pyr_scale, flow_levels, flow_winsize, flow_iterations, flow_poly_n, flow_poly_sigma (farneback_params;
+a missing key means the reference's value).
 
 plus the batched entry the GPU runner uses, because per-pair calls from forked pool workers
 (F:1190-1191) cannot drive a GPU:
@@ -26,6 +32,26 @@ from . import _native
 
 DEFAULT_CUT_THRESHOLD = 7          # F:876
 DEFAULT_BATCH_FRAMES = 64
+
+# cv2.calcOpticalFlowFarneback's parameters in the reference's call (F:878-879) and the settings keys that override them
+REFERENCE_FARNEBACK = dict(pyr_scale=0.5, levels=3, winsize=15, iterations=3, poly_n=5, poly_sigma=1.2)
+FARNEBACK_SETTINGS = {"flow_pyr_scale": "pyr_scale", "flow_levels": "levels", "flow_winsize": "winsize",
+                      "flow_iterations": "iterations", "flow_poly_n": "poly_n", "flow_poly_sigma": "poly_sigma"}
+
+
+def farneback_params(params: Optional[Dict]) -> Dict:
+    """The Farneback parameters a settings dict asks for: the flow_* keys, the reference's value where one is missing."""
+    params = params or {}
+    out = dict(REFERENCE_FARNEBACK)
+    for key, name in FARNEBACK_SETTINGS.items():
+        if params.get(key) is not None:
+            out[name] = type(REFERENCE_FARNEBACK[name])(params[key])
+    return out
+
+
+def apply_farneback(ctx: "_native.FlowContext", params: Optional[Dict]) -> None:
+    """Set the context's Farneback parameters from a settings dict (a no-op when they are already set)."""
+    ctx.set_farneback(**farneback_params(params))
 
 _contexts: Dict[int, _native.FlowContext] = {}
 
@@ -119,6 +145,7 @@ def process_bracket(frames, params: Optional[Dict] = None, *, ctx: Optional[_nat
     ctx = ctx or get_context()
     arr = _as_frames(frames)
     n, h, w = arr.shape
+    apply_farneback(ctx, params)
     ctx.configure(w, h, max(1, min(batch_frames, n)), max(n - 1, 1))
     ctx.bracket_begin(bool(params.get("pov_mode", False)), float(params.get("cut_threshold", DEFAULT_CUT_THRESHOLD)))
     try:
@@ -148,6 +175,7 @@ def shard_phase1(ctx: _native.FlowContext, frames, a: int, b: int, params: Optio
     params = params or {}
     arr = _as_frames(frames[a:b + 1])
     n, h, w = arr.shape
+    apply_farneback(ctx, params)
     ctx.configure(w, h, max(1, min(batch_frames, n)), max(n - 1, 1))
     ctx.bracket_begin_shard(n - 1, bool(params.get("pov_mode", False)), float(params.get("cut_threshold", DEFAULT_CUT_THRESHOLD)))
     try:
@@ -207,6 +235,7 @@ class BracketPipeline:
         n, h, w = arr.shape
         ctx = self.ctxs[self._turn]
         other = self.ctxs[self._turn ^ 1]
+        apply_farneback(ctx, params)
         ctx.configure(w, h, max(1, min(self.batch_frames, n)), max(n - 1, 1))
         if self._pending is not None:
             ctx.chain_after(other)
@@ -240,6 +269,7 @@ def precompute_flow_info(p0: np.ndarray, p1: np.ndarray, config: Dict) -> Dict:
         raise ValueError("p0 and p1 must be equal-sized 2-D uint8 arrays")
     h, w = p0.shape
     pov = bool(config.get("pov_mode"))
+    apply_farneback(ctx, config)    # the context is shared: a call without flow_* keys switches back to the reference's
     ctx.configure(w, h, 2, 1)       # incremental: a context already configured for this frame size is left alone
     ctx.bracket_begin(pov, float(config.get("cut_threshold", DEFAULT_CUT_THRESHOLD)))
     try:
@@ -264,6 +294,18 @@ def precompute_flow_info(p0: np.ndarray, p1: np.ndarray, config: Dict) -> Dict:
         "cut_center": pos_center[0],
         "mean_mag": np.float32(r["mean_mag"][0]),
     }
+
+
+def calc_optical_flow_farneback(prev: np.ndarray, next: np.ndarray, flow, pyr_scale: float, levels: int, winsize: int,
+                                iterations: int, poly_n: int, poly_sigma: float, flags: int = 0, *,
+                                ctx: Optional[_native.FlowContext] = None) -> np.ndarray:
+    """cv2.calcOpticalFlowFarneback with cv2's positional order, on the GPU: float32 [H, W, 2] (x, y displacement).
+    `flow` must be None (an initial flow, OPTFLOW_USE_INITIAL_FLOW, is not supported) and `flags` 0."""
+    if flow is not None:
+        raise ValueError("calc_optical_flow_farneback: flow must be None (an initial flow is not supported)")
+    ctx = ctx or get_context()
+    ctx.set_farneback(pyr_scale, levels, winsize, iterations, poly_n, poly_sigma, flags)
+    return ctx.farneback(prev, next)
 
 
 def precompute_flow_info_gpu(p0: np.ndarray, p1: np.ndarray, cut_threshold) -> Dict:

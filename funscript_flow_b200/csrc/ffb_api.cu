@@ -4,7 +4,8 @@
 //   host (pageable | pinned) --cudaMemcpyAsync on s_copy, double-buffered--> device u8 staging
 //   --k_pyramid_pow2 | k_pyramid_level / k_polyexp--> per-frame expansion slots (ring of S = B+2 frames; each frame
 //     is expanded once and used as `next` of pair j-1 and `prev` of pair j: streaming mode)
-//   --k_flow_iter x3 per level (flow up-sampling fused, k_upsample_flow otherwise)--> final-flow ring (>= B+8 pairs)
+//   --k_flow_iter x iterations per level (flow up-sampling fused, k_upsample_flow otherwise; winsize != 15:
+//     k_flow_matrices + k_box_solve)--> final-flow ring (>= B+8 pairs)
 //   --k_divmag / k_phase1_finish--> per-pair centre, value, mean magnitude, cut flag (device arrays)
 //   --k_smooth_centers / k_radial / k_radial_finish (lagging 6 pairs)--> per-pair scalar
 // and only the 1-D per-pair results are copied back at ffb_bracket_finish.
@@ -32,27 +33,42 @@ const char* const kKernelNames[FFB_K_COUNT] = {"k_pyramid_level", "k_polyexp",  
 // ------------------------------------------------------------------ host-side constant builders
 int cv_round(double v) { return (int)nearbyint(v); }   // round-half-even in the default FP mode
 
-struct LevelPlan {
-    int n;
-    int k[FFB_MAX_LEVELS], w[FFB_MAX_LEVELS], h[FFB_MAX_LEVELS], ksize[FFB_MAX_LEVELS];
-    double sigma[FFB_MAX_LEVELS];
+// calcOpticalFlowFarneback's parameters (flags is always 0: the two flags are refused).  A new context holds the
+// reference's call (F:878-879).
+struct FarnebackParams {
+    double pyr_scale = 0.5;
+    int levels = 3, winsize = 15, iterations = 3, poly_n = 5;
+    double poly_sigma = 1.2;
+    bool operator==(const FarnebackParams& o) const {
+        return pyr_scale == o.pyr_scale && levels == o.levels && winsize == o.winsize && iterations == o.iterations &&
+               poly_n == o.poly_n && poly_sigma == o.poly_sigma;
+    }
 };
 
-// calcOpticalFlowFarneback level geometry for pyr_scale 0.5, levels 3 (SURVEY.md 3.4 steps 1-2).
-LevelPlan make_plan(int W, int H) {
+struct LevelPlan {
+    int n;                  // may exceed FFB_PLAN_LEVELS: then only the first FFB_PLAN_LEVELS entries are filled
+    double pyr_scale;
+    int k[FFB_PLAN_LEVELS], w[FFB_PLAN_LEVELS], h[FFB_PLAN_LEVELS], ksize[FFB_PLAN_LEVELS];
+    double sigma[FFB_PLAN_LEVELS];
+};
+
+// calcOpticalFlowFarneback level geometry (SURVEY.md 3.4 steps 1-2): levels stop where the coarsest one would be
+// narrower or lower than 32 px.
+LevelPlan make_plan(int W, int H, double pyr_scale, int levels) {
     LevelPlan p;
+    p.pyr_scale = pyr_scale;
     int k = 0;
     double scale = 1.0;
-    while (k < 3) {
-        scale *= 0.5;
+    while (k < levels) {
+        scale *= pyr_scale;
         if (W * scale < 32 || H * scale < 32) break;
         ++k;
     }
     p.n = k + 1;
-    for (int i = 0; i < p.n; ++i) {
+    for (int i = 0; i < p.n && i < FFB_PLAN_LEVELS; ++i) {
         const int kk = k - i;   // coarsest first
         double s = 1.0;
-        for (int j = 0; j < kk; ++j) s *= 0.5;
+        for (int j = 0; j < kk; ++j) s *= pyr_scale;
         const double sigma = (1.0 / s - 1.0) * 0.5;
         int ks = cv_round(sigma * 5) | 1;
         if (ks < 3) ks = 3;
@@ -64,17 +80,12 @@ LevelPlan make_plan(int W, int H) {
     }
     return p;
 }
+LevelPlan make_plan(int W, int H, const FarnebackParams& fp) { return make_plan(W, H, fp.pyr_scale, fp.levels); }
 
-// cv::getGaussianKernel(ksize, sigma, CV_32F), half kernel.
-FfbTaps make_taps(int ksize, double sigma) {
-    FfbTaps t;
-    memset(&t, 0, sizeof(t));
-    t.r = ksize / 2;
-    if (sigma <= 0 && ksize == 3) {
-        t.k[0] = 0.5f;
-        t.k[1] = 0.25f;
-        return t;
-    }
+// cv::getGaussianKernel(ksize, sigma, CV_32F), half kernel (ksize / 2 + 1 taps).
+std::vector<float> gaussian_half(int ksize, double sigma) {
+    const int r = ksize / 2;
+    if (sigma <= 0 && ksize == 3) return {0.5f, 0.25f};
     if (sigma <= 0) sigma = ((ksize - 1) * 0.5 - 1) * 0.3 + 0.8;
     std::vector<double> v(ksize);
     double sum = 0;
@@ -83,9 +94,21 @@ FfbTaps make_taps(int ksize, double sigma) {
         v[i] = exp(-0.5 / (sigma * sigma) * x * x);
         sum += v[i];
     }
-    for (int i = 0; i <= t.r; ++i) t.k[i] = (float)(v[t.r + i] / sum);
+    std::vector<float> k(r + 1);
+    for (int i = 0; i <= r; ++i) k[i] = (float)(v[r + i] / sum);
+    return k;
+}
+
+// The same half kernel in the fixed-size form the shared-memory pyramid kernels take (radius <= 9).
+FfbTaps make_taps(int ksize, double sigma) {
+    FfbTaps t;
+    memset(&t, 0, sizeof(t));
+    t.r = ksize / 2;
+    const std::vector<float> k = gaussian_half(ksize, sigma);
+    for (int i = 0; i <= t.r && i < 10; ++i) t.k[i] = k[i];
     return t;
 }
+constexpr int kTapsMaxR = 9;
 
 // cv::resize INTER_LINEAR per-axis table.
 void make_linear_table(int dst_n, int src_n, std::vector<int>& idx, std::vector<float>& alpha) {
@@ -103,7 +126,7 @@ void make_linear_table(int dst_n, int src_n, std::vector<int>& idx, std::vector<
     }
 }
 
-// FarnebackPrepareGaussian(n = 5, sigma = 1.2): taps in float32, inverse moments in double.
+// FarnebackPrepareGaussian(n, sigma): taps in float32, inverse moments in double.
 void invert6(double G[6][6], double inv[6][6]) {
     double a[6][12];
     for (int i = 0; i < 6; ++i)
@@ -124,10 +147,11 @@ void invert6(double G[6][6], double inv[6][6]) {
         for (int j = 0; j < 6; ++j) inv[i][j] = a[i][j + 6];
 }
 
-FfbPolyConsts make_poly_consts() {
-    const int n = FFB_POLY_N;
-    const double sigma = 1.2;
-    float g[2 * FFB_POLY_N + 1], xg[2 * FFB_POLY_N + 1], xxg[2 * FFB_POLY_N + 1];
+template <int N>
+FfbPolyConsts<N> make_poly_consts(double sigma) {
+    const int n = N;
+    if (sigma < std::numeric_limits<float>::epsilon()) sigma = n * 0.3;
+    float g[2 * N + 1], xg[2 * N + 1], xxg[2 * N + 1];
     double s = 0;
     for (int x = -n; x <= n; ++x) { g[x + n] = (float)exp(-x * x / (2 * sigma * sigma)); s += g[x + n]; }
     s = 1.0 / s;
@@ -151,7 +175,7 @@ FfbPolyConsts make_poly_consts() {
     G[3][4] = G[4][3] = G[5][5];
     double inv[6][6];
     invert6(G, inv);
-    FfbPolyConsts c;
+    FfbPolyConsts<N> c;
     for (int i = 0; i <= n; ++i) { c.g[i] = g[n + i]; c.xg[i] = xg[n + i]; c.xxg[i] = xxg[n + i]; }
     c.ig11 = (float)inv[1][1];
     c.ig03 = (float)inv[0][3];
@@ -174,8 +198,10 @@ struct Level {
     size_t r_off = 0;      // float offset of this level inside a frame's expansion slot
     FfbTaps taps;
     int RW = 0, RH = 0;    // source window bound of one 32x8 output tile
+    bool wide = false;     // blur radius or tile window beyond k_pyramid_level: k_pyramid_wide_rows / _cols
     int *xi = nullptr, *yi = nullptr, *uxi = nullptr, *uyi = nullptr;
     float *xa = nullptr, *ya = nullptr, *uxa = nullptr, *uya = nullptr;
+    float* wk = nullptr;   // half kernel of a wide level (device)
     float* I = nullptr;    // [B][h][rp]
     float2 *fA = nullptr, *fB = nullptr;   // [B][h][fp]
     FlowIterPlan iter;
@@ -197,13 +223,18 @@ struct ffb_ctx {
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     cudaEvent_t ev_chain = nullptr;                    // "everything queued on s_comp so far": ffb_chain_after
     cudaEvent_t ev_h2d[2] = {nullptr, nullptr}, ev_expand[2] = {nullptr, nullptr};
-    FfbPolyConsts poly;
+    FarnebackParams fb;
+    FfbPolyConsts<5> poly5;
+    FfbPolyConsts<7> poly7;
     // geometry
     int W = 0, H = 0, B = 0, maxPairs = 0, nlev = 0, S = 0, ring_n = 0, fp0 = 0;
     int Bcap = 0, pairsCap = 0;                 // allocated capacities (B / maxPairs are the limits of the last ffb_configure)
     int64_t n_dev_alloc = 0, n_host_alloc = 0;  // cudaMalloc / cudaHostAlloc calls made for this context so far
     bool pyr_fast = false;
-    Level lev[FFB_MAX_LEVELS];
+    Level lev[FFB_PLAN_LEVELS];
+    int wide_w = 0;                 // widest level that takes the large-radius pyramid (0: none)
+    float* pyr_tmp = nullptr;       // its scratch image, (Bcap + 1) x H x wide_w floats
+    float* M = nullptr;             // matrices of the unfused flow iteration (winsize != 15), Bcap pairs at level 0
     float* R = nullptr;
     size_t r_slot_floats = 0;
     float2* ring = nullptr;
@@ -244,12 +275,12 @@ struct ffb_ctx {
     std::vector<cudaEvent_t> ev_pool;
     int64_t k_launches[FFB_K_COUNT] = {0};
     double k_ms[FFB_K_COUNT] = {0}, k_bytes[FFB_K_COUNT] = {0};
-    int64_t it_launches[FFB_MAX_LEVELS] = {0};          // k_flow_iter split by level k
-    double it_ms[FFB_MAX_LEVELS] = {0}, it_bytes[FFB_MAX_LEVELS] = {0};
+    int64_t it_launches[FFB_PLAN_LEVELS] = {0};         // k_flow_iter (or k_flow_matrices + k_box_solve) split by level k
+    double it_ms[FFB_PLAN_LEVELS] = {0}, it_bytes[FFB_PLAN_LEVELS] = {0};
     // cudaFuncSetAttribute is per device: remember per context which kernels already had their
     // dynamic shared-memory limit raised (a process may own contexts on several GPUs)
     size_t pyr_smem_max = 48 * 1024;
-    bool attr_poly = false, attr_pyr2 = false;
+    bool attr_poly = false, attr_poly7 = false, attr_pyr2 = false;
     std::set<const void*> attr_iter;                     // k_flow_iter instantiations already configured
     FlowIterPlan iter_cfg;                               // variant forced by FFB_ITER_CFG for every level
     int flow_streams = 2;
@@ -376,6 +407,14 @@ void pyramid_window(const std::vector<int>& idx, int dst_n, int src_n, int tile,
     *bound = best;
 }
 
+// k_pyramid_level's dynamic shared memory for a source window bound RW x RH (the staged window + the row-pass plane)
+size_t pyramid_smem(int RW, int RH) {
+    return ((size_t)ffb_round_up((RW | 1) * RH, 4) + (size_t)RH * PYR_TW) * sizeof(float);
+}
+// A level takes the large-radius kernels when its radius exceeds FfbTaps or its tile window exceeds the 227 KB of
+// shared memory a B200 block may use.
+bool pyramid_wide(int r, int RW, int RH) { return r > kTapsMaxR || pyramid_smem(RW, RH) > 227u * 1024u; }
+
 int launch_pyramid(ffb_ctx* c, const uint8_t* src, size_t src_stride, int src_pitch, int W, int H, float* dst,
                    size_t dst_stride, int dp, int w, int h, const int* xi, const float* xa, const int* yi,
                    const float* ya, const FfbTaps& taps, int RW, int RH, int nframes) {
@@ -385,7 +424,7 @@ int launch_pyramid(ffb_ctx* c, const uint8_t* src, size_t src_stride, int src_pi
     a.xi = xi; a.xa = xa; a.yi = yi; a.ya = ya; a.taps = taps;
     a.RWp = RW | 1;                       // odd pitch: column walks of pass 1 stay conflict-free
     a.p_off = ffb_round_up(a.RWp * RH, 4);
-    const size_t smem = ((size_t)a.p_off + (size_t)RH * PYR_TW) * sizeof(float);
+    const size_t smem = pyramid_smem(RW, RH);
     if (taps.r >= W || taps.r >= H) return fail(c, FFB_E_INVALID, "frame smaller than the blur radius");
     auto kfn = k_pyramid_level<PYR_TW, PYR_TH>;
     if (smem > c->pyr_smem_max) {
@@ -400,29 +439,66 @@ int launch_pyramid(ffb_ctx* c, const uint8_t* src, size_t src_stride, int src_pi
     return FFB_OK;
 }
 
-int launch_polyexp(ffb_ctx* c, const float* src, size_t src_stride, int sp, int w, int h, FfbRing dst, size_t plane,
-                   int rp, int nframes) {
-    FfbPolyArgs a;
-    a.src = src; a.src_frame_stride = src_stride; a.sp = sp; a.w = w; a.h = h;
-    a.dst = dst; a.plane = plane; a.rp = rp; a.c = c->poly;
+// Large-radius pyramid level (Level::wide): row pass into `tmp` (H x w per frame), column pass into dst.
+int launch_pyramid_wide(ffb_ctx* c, const uint8_t* src, size_t src_stride, int src_pitch, int W, int H, float* tmp, float* dst,
+                        size_t dst_stride, int dp, int w, int h, const int* xi, const float* xa, const int* yi, const float* ya,
+                        const float* k, int r, int nframes) {
+    if (r >= W || r >= H) return fail(c, FFB_E_INVALID, "frame smaller than the blur radius");
+    FfbPyrWideArgs a;
+    a.src = src; a.src_frame_stride = src_stride; a.src_pitch = src_pitch; a.W = W; a.H = H;
+    a.tmp = tmp; a.tmp_frame_stride = (size_t)H * w;
+    a.dst = dst; a.dst_frame_stride = dst_stride; a.dp = dp; a.w = w; a.h = h;
+    a.xi = xi; a.xa = xa; a.yi = yi; a.ya = ya; a.k = k; a.r = r;
+    const ProfMark pr = prof_begin(c, FFB_K_PYRAMID, -1, (double)nframes * ((double)W * H + 4.0 * H * w), c->s_comp);
+    FFB_LAUNCH(k_pyramid_wide_rows, dim3((w + 31) / 32, (H + 7) / 8, nframes), dim3(256), 0, c->s_comp, a);
+    prof_end(pr);
+    CKL(c);
+    const ProfMark pc = prof_begin(c, FFB_K_PYRAMID, -1, (double)nframes * (4.0 * H * w + 4.0 * w * h), c->s_comp);
+    FFB_LAUNCH(k_pyramid_wide_cols, dim3((w + 31) / 32, (h + 7) / 8, nframes), dim3(256), 0, c->s_comp, a);
+    prof_end(pc);
+    CKL(c);
+    return FFB_OK;
+}
+
+template <int N>
+int launch_polyexp_t(ffb_ctx* c, FfbPolyArgs<N>& a, const FfbPolyConsts<N>& consts, bool& attr, int nframes) {
+    a.c = consts;
     // the kernel stores two pixels (32 bytes) of the float4 image per instruction
-    if (rp % 4 != 0 || ((uintptr_t)dst.base | (uintptr_t)dst.stride) % 32 != 0)
-        return fail(c, FFB_E_INVALID, "expansion output is not 32-byte aligned (pitch %d, stride %zu)", rp, dst.stride);
-    if (!c->attr_poly) {
-        CK(c, cudaFuncSetAttribute(k_polyexp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)POLY_SMEM));
-        c->attr_poly = true;
+    if (a.rp % 4 != 0 || ((uintptr_t)a.dst.base | (uintptr_t)a.dst.stride) % 32 != 0)
+        return fail(c, FFB_E_INVALID, "expansion output is not 32-byte aligned (pitch %d, stride %zu)", a.rp, a.dst.stride);
+    if (!attr) {
+        CK(c, cudaFuncSetAttribute(k_polyexp<N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)POLY_SMEM));
+        attr = true;
     }
     // (a variant with packed fp32 arithmetic -- FFMA2 / FADD2 / FMUL2 on row pairs -- was measured in round 2: 4.60 ms
     // against 3.92 ms per 257 1080p frames for this scalar kernel; the packed instructions issue at half rate and the
     // 114 registers they need halve the occupancy.  profiles/r2_other_kernels.txt)
-    dim3 grid((w + POLY_OW - 1) / POLY_OW, (h + POLY_ROWS - 1) / POLY_ROWS, nframes);
-    const ProfMark pm = prof_begin(c, FFB_K_POLYEXP, -1, (double)nframes * 24.0 * w * h, c->s_comp);
-    FFB_LAUNCH(k_polyexp, grid, dim3(256), POLY_SMEM, c->s_comp, a);
+    dim3 grid((a.w + POLY_OW - 1) / POLY_OW, (a.h + POLY_ROWS - 1) / POLY_ROWS, nframes);
+    const ProfMark pm = prof_begin(c, FFB_K_POLYEXP, -1, (double)nframes * 24.0 * a.w * a.h, c->s_comp);
+    FFB_LAUNCH(k_polyexp<N>, grid, dim3(256), POLY_SMEM, c->s_comp, a);
     prof_end(pm);
     CKL(c);
     return FFB_OK;
 }
 
+// the context's poly_n selects the instantiation (5 or 7)
+int launch_polyexp(ffb_ctx* c, const float* src, size_t src_stride, int sp, int w, int h, FfbRing dst, size_t plane,
+                   int rp, int nframes) {
+    auto fill = [&](auto& a) {
+        a.src = src; a.src_frame_stride = src_stride; a.sp = sp; a.w = w; a.h = h;
+        a.dst = dst; a.plane = plane; a.rp = rp;
+    };
+    if (c->fb.poly_n == 7) {
+        FfbPolyArgs<7> a;
+        fill(a);
+        return launch_polyexp_t(c, a, c->poly7, c->attr_poly7, nframes);
+    }
+    FfbPolyArgs<5> a;
+    fill(a);
+    return launch_polyexp_t(c, a, c->poly5, c->attr_poly, nframes);
+}
+
+// k_upsample_flow: the flow is doubled with pyr_scale 0.5, multiplied by 1 / pyr_scale otherwise
 int launch_upsample(ffb_ctx* c, const float2* src, size_t src_stride, int sp, int wc, int hc, float2* dst,
                     size_t dst_stride, int dp, int w, int h, const int* xi, const float* xa, const int* yi,
                     const float* ya, int npairs) {
@@ -430,9 +506,11 @@ int launch_upsample(ffb_ctx* c, const float2* src, size_t src_stride, int sp, in
     a.src = src; a.src_stride = src_stride; a.sp = sp; a.wc = wc; a.hc = hc;
     a.dst = dst; a.dst_stride = dst_stride; a.dp = dp; a.w = w; a.h = h;
     a.xi = xi; a.xa = xa; a.yi = yi; a.ya = ya;
+    a.scale = (float)(1.0 / c->fb.pyr_scale);
     dim3 grid((w + 31) / 32, (h + 7) / 8, npairs);
     const ProfMark pm = prof_begin(c, FFB_K_UPSAMPLE, -1, (double)npairs * (8.0 * wc * hc + 8.0 * w * h), c->s_comp);
-    FFB_LAUNCH(k_upsample_flow, grid, dim3(256), 0, c->s_comp, a);
+    if (c->fb.pyr_scale == 0.5) FFB_LAUNCH(k_upsample_flow<false>, grid, dim3(256), 0, c->s_comp, a);
+    else FFB_LAUNCH(k_upsample_flow<true>, grid, dim3(256), 0, c->s_comp, a);
     prof_end(pm);
     CKL(c);
     return FFB_OK;
@@ -532,6 +610,36 @@ int launch_flow_iter(ffb_ctx* c, const FlowIterPlan& p, int level, cudaStream_t 
                 p.nt, p.u, p.ho);
 }
 
+// One flow iteration with the context's winsize != 15: k_flow_matrices into the scratch M (npairs x 5 planes), then
+// k_box_solve into fout.  Same arguments, counters and output layout as launch_flow_iter.
+int launch_flow_unfused(ffb_ctx* c, int level, float* M, FfbRing R, size_t plane, int rp, int w, int h, const float2* fin,
+                        size_t fin_stride, int fip, FfbRing fout, int fop, int npairs) {
+    const int win = c->fb.winsize, r = win / 2;
+    if (BOX_NT - 2 * r < 1) return fail(c, FFB_E_INVALID, "winsize %d too large for k_box_solve", win);
+    FfbMatrixArgs m;
+    m.R = R; m.plane = (int)plane; m.rp = rp; m.w = w; m.h = h;
+    m.fin = fin; m.fin_stride = fin_stride; m.fip = fip;
+    m.M = M; m.m_stride = 5 * plane;
+    // algorithmic bytes: the fused kernel's reads (expansions + incoming flow) plus the matrices written (20 B/px) ...
+    const double px = (double)npairs * w * h;
+    const ProfMark pm = prof_begin(c, FFB_K_FLOW_ITER, level, px * ((fin ? 48.0 : 40.0) + 20.0), c->s_comp);
+    FFB_LAUNCH(k_flow_matrices, dim3((w + 31) / 32, (h + 7) / 8, npairs), dim3(256), 0, c->s_comp, m);
+    prof_end(pm);
+    CKL(c);
+    FfbBoxArgs b;
+    b.M = M; b.m_stride = 5 * plane; b.plane = (int)plane; b.rp = rp; b.w = w; b.h = h;
+    b.r = r; b.scale = (float)(1.0 / ((double)win * win));
+    b.fout = fout; b.fop = fop;
+    b.SW = BOX_NT - 2 * r;
+    b.SH = 64;     // 2r rows of every segment are re-read to start its sums
+    // ... read back (20 B/px) and the flow written (8 B/px)
+    const ProfMark pb = prof_begin(c, FFB_K_FLOW_ITER, level, px * 28.0, c->s_comp);
+    FFB_LAUNCH(k_box_solve, dim3(npairs, (w + b.SW - 1) / b.SW, (h + b.SH - 1) / b.SH), dim3(BOX_NT), 0, c->s_comp, b);
+    prof_end(pb);
+    CKL(c);
+    return FFB_OK;
+}
+
 // ------------------------------------------------------------------ geometry
 // Device / pinned memory comes in four groups with their own lifetimes, so that ffb_configure only
 // re-allocates what a request outgrows:
@@ -540,11 +648,13 @@ int launch_flow_iter(ffb_ctx* c, const FlowIterPlan& p, int level, cudaStream_t 
 //   flow ring    final-flow ring and the reduction partials indexed by ring slot  capacity ring_n pairs
 //   pairs        per-pair results and their pinned staging                        capacity pairsCap pairs
 void free_batch_group(ffb_ctx* c) {
-    for (int l = 0; l < FFB_MAX_LEVELS; ++l) {
+    for (int l = 0; l < FFB_PLAN_LEVELS; ++l) {
         Level& L = c->lev[l];
         dev_free(L.I); dev_free(L.fA); dev_free(L.fB);
     }
     dev_free(c->R);
+    dev_free(c->M);
+    dev_free(c->pyr_tmp);
     for (int b = 0; b < 2; ++b) {
         dev_free(c->d_u8[b]);
         if (c->h_pin[b]) cudaFreeHost(c->h_pin[b]);
@@ -568,13 +678,14 @@ void free_geometry(ffb_ctx* c) {
     free_batch_group(c);
     free_ring_group(c);
     free_pairs_group(c);
-    for (int l = 0; l < FFB_MAX_LEVELS; ++l) {
+    for (int l = 0; l < FFB_PLAN_LEVELS; ++l) {
         Level& L = c->lev[l];
         dev_free(L.xi); dev_free(L.yi); dev_free(L.uxi); dev_free(L.uyi);
         dev_free(L.xa); dev_free(L.ya); dev_free(L.uxa); dev_free(L.uya);
+        dev_free(L.wk);
         L = Level();
     }
-    c->W = c->H = c->B = c->maxPairs = c->nlev = 0;
+    c->W = c->H = c->B = c->maxPairs = c->nlev = c->wide_w = 0;
 }
 
 int host_alloc(ffb_ctx* c, void** p, size_t bytes) {
@@ -593,6 +704,8 @@ int build_level_tables(ffb_ctx* c, Level& L, int W, int H, int wc, int hc) {
     make_linear_table(L.h, H, yi, ya);
     pyramid_window(xi, L.w, W, PYR_TW, L.taps.r, &L.RW);
     pyramid_window(yi, L.h, H, PYR_TH, L.taps.r, &L.RH);
+    L.wide = pyramid_wide(L.taps.r, L.RW, L.RH);
+    if (L.wide) TRY(upload_vec(c, &L.wk, gaussian_half(L.ksize, L.sigma)));
     TRY(upload_vec(c, &L.xi, xi)); TRY(upload_vec(c, &L.xa, xa));
     TRY(upload_vec(c, &L.yi, yi)); TRY(upload_vec(c, &L.ya, ya));
     if (wc > 0) {
@@ -626,10 +739,13 @@ int configure(ffb_ctx* c, int W, int H, int B, int maxPairs, int ring_pairs = 0)
         c->maxPairs = maxPairs;
         return FFB_OK;
     }
+    const LevelPlan p = make_plan(W, H, c->fb);
+    if (p.n > FFB_PLAN_LEVELS)
+        return fail(c, FFB_E_INVALID, "ffb_configure: %dx%d with pyr_scale %g, levels %d plans %d pyramid levels (at most %d)",
+                    W, H, c->fb.pyr_scale, c->fb.levels, p.n, FFB_PLAN_LEVELS);
     TRY(quiesce(c));
     if (new_frame) {
         free_geometry(c);
-        const LevelPlan p = make_plan(W, H);
         c->W = W; c->H = H; c->nlev = p.n;
         c->pyr_fast = pyramid_fast_ok(W, H, p);
         size_t off = 0;
@@ -644,8 +760,10 @@ int configure(ffb_ctx* c, int W, int H, int B, int maxPairs, int ring_pairs = 0)
             off = (off + 63) / 64 * 64;
             L.taps = make_taps(L.ksize, L.sigma);
             L.iter = flow_iter_plan(W, H, L.w, L.h, c->iter_cfg);
-            L.up2x = l > 0 && L.w == 2 * c->lev[l - 1].w && L.h == 2 * c->lev[l - 1].h;
+            // the fused up-sampling doubles the flow: pyr_scale 0.5 only
+            L.up2x = l > 0 && c->fb.pyr_scale == 0.5 && L.w == 2 * c->lev[l - 1].w && L.h == 2 * c->lev[l - 1].h;
             TRY(build_level_tables(c, L, W, H, l > 0 ? c->lev[l - 1].w : 0, l > 0 ? c->lev[l - 1].h : 0));
+            if (L.wide && L.w > c->wide_w) c->wide_w = L.w;
         }
         c->r_slot_floats = (off + 127) / 128 * 128;      // 512-byte multiples
         c->fp0 = c->lev[p.n - 1].fp;
@@ -667,6 +785,8 @@ int configure(ffb_ctx* c, int W, int H, int B, int maxPairs, int ring_pairs = 0)
         }
         c->S = B + 2;      // the first batch of a bracket may carry B + 1 frames (= B pairs)
         TRY(dev_alloc(c, &c->R, (size_t)c->S * c->r_slot_floats));
+        if (c->fb.winsize != FFB_WIN) TRY(dev_alloc(c, &c->M, (size_t)B * 5 * c->lev[c->nlev - 1].plane));
+        if (c->wide_w > 0) TRY(dev_alloc(c, &c->pyr_tmp, (size_t)(B + 1) * H * c->wide_w));
         const size_t fbytes = (size_t)W * H;
         for (int b = 0; b < 2; ++b) {
             TRY(dev_alloc(c, &c->d_u8[b], (size_t)(B + 1) * fbytes));
@@ -706,6 +826,7 @@ int configure(ffb_ctx* c, int W, int H, int B, int maxPairs, int ring_pairs = 0)
 // All levels in one pass when every level is an exact 2^k decimation (W, H multiples of 8).
 bool pyramid_fast_ok(int W, int H, const LevelPlan& p) {
     if (W % 8 || H % 8 || W < 64 || H < 64) return false;
+    if (p.pyr_scale != 0.5 || p.n > FFB_MAX_LEVELS) return false;
     static const int want[FFB_MAX_LEVELS] = {3, 3, 9, 19};
     for (int l = 0; l < p.n; ++l)
         if (p.ksize[l] != want[p.k[l]] || p.w[l] != (W >> p.k[l]) || p.h[l] != (H >> p.k[l])) return false;
@@ -753,7 +874,10 @@ int expand_frames(ffb_ctx* c, const uint8_t* src, size_t stride, int pitch, int 
     }
     for (int l = 0; l < c->nlev; ++l) {
         Level& L = c->lev[l];
-        if (!fast)
+        if (!fast && L.wide)
+            TRY(launch_pyramid_wide(c, src, stride, pitch, c->W, c->H, c->pyr_tmp, L.I, L.plane, L.rp, L.w, L.h, L.xi, L.xa,
+                                    L.yi, L.ya, L.wk, L.taps.r, nb));
+        else if (!fast)
             TRY(launch_pyramid(c, src, stride, pitch, c->W, c->H, L.I, L.plane, L.rp, L.w, L.h, L.xi, L.xa, L.yi, L.ya,
                                L.taps, L.RW, L.RH, nb));
         FfbRing dst;
@@ -786,7 +910,10 @@ int flow_pairs(ffb_ctx* c, int p0, int np) {
     // coarse-level launches (and the tail of every launch) of one slice overlap the other slice's work (+4 %; 3-4 slices
     // measured no better).  Every buffer is indexed by pair; the slices share nothing that is written.
     // FFB_FLOW_STREAMS=1 keeps one chain, whose launches can be timed one by one.
-    bool all_fused = true;
+    // winsize 15: the fused k_flow_iter; any other: k_flow_matrices + k_box_solve through the scratch c->M, whose pairs
+    // are those of one launch chain (so the unfused path keeps one chain)
+    const bool fused = c->fb.winsize == FFB_WIN;
+    bool all_fused = fused;
     for (int l = 1; l < c->nlev; ++l) all_fused = all_fused && c->lev[l].up2x;
     const int nslice = c->flow_streams > 1 && all_fused && np >= 8 ? 2 : 1;
     const bool sliced = nslice > 1;
@@ -798,18 +925,22 @@ int flow_pairs(ffb_ctx* c, int p0, int np) {
         CK(c, cudaEventRecord(c->ev_fork, c->s_comp));
         CK(c, cudaStreamWaitEvent(c->s_aux, c->ev_fork, 0));
     }
+    // iteration it writes fB (it even) or fA (it odd), the last one of level 0 the final-flow ring instead
+    const int iters = c->fb.iterations;
+    auto level_out = [&](const Level& X) { return (iters - 1) % 2 == 0 ? X.fB : X.fA; };
     for (int l = 0; l < c->nlev; ++l) {
         Level& L = c->lev[l];
         const size_t fstride = (size_t)L.fp * L.h;
         const bool last = l == c->nlev - 1;
+        const bool fuse_up = fused && L.up2x;
         const float2* fin0 = nullptr;
-        if (l > 0 && !L.up2x) {
+        if (l > 0 && !fuse_up) {
             Level& C = c->lev[l - 1];
-            TRY(launch_upsample(c, C.fB, (size_t)C.fp * C.h, C.fp, C.w, C.h, L.fA, fstride, L.fp, L.w, L.h, L.uxi,
+            TRY(launch_upsample(c, level_out(C), (size_t)C.fp * C.h, C.fp, C.w, C.h, L.fA, fstride, L.fp, L.w, L.h, L.uxi,
                                 L.uxa, L.uyi, L.uya, np));
             fin0 = L.fA;
         }
-        for (int it = 0; it < FFB_ITERS; ++it) {
+        for (int it = 0; it < iters; ++it) {
             for (int sl = 0; sl < nslice; ++sl) {
                 const int off = soff[sl], cnt = soff[sl + 1] - soff[sl];
                 FfbRing R;
@@ -821,17 +952,21 @@ int flow_pairs(ffb_ctx* c, int p0, int np) {
                 FfbRing toA{(char*)(L.fA + (size_t)off * fstride), fstride * sizeof(float2), 0, 1 << 30};
                 FfbRing toRing{(char*)c->ring, c->ring_stride * sizeof(float2), (p0 + off) % c->ring_n, c->ring_n};
                 UpSrc up;
-                if (l > 0 && L.up2x) {
+                if (l > 0 && fuse_up) {
                     Level& C = c->lev[l - 1];
                     up.stride = (size_t)C.fp * C.h;
-                    up.src = C.fB + (size_t)off * up.stride; up.sp = C.fp; up.wc = C.w; up.hc = C.h;
+                    up.src = level_out(C) + (size_t)off * up.stride; up.sp = C.fp; up.wc = C.w; up.hc = C.h;
                 }
-                // iteration 0 starts from the up-sampled coarser flow (or zero) into fB, 1 runs fB -> fA, 2 fA -> ring | fB
+                // iteration 0 starts from the up-sampled coarser flow (or zero); with the reference's 3 iterations:
+                // fB, fB -> fA, fA -> ring | fB
                 const float2* fin = it == 0 ? (fin0 ? fin0 + (size_t)off * fstride : nullptr)
-                                            : (it == 1 ? L.fB : L.fA) + (size_t)off * fstride;
-                const FfbRing& fout = it == 1 ? toA : (it == 2 && last ? toRing : toB);
-                TRY(launch_flow_iter(c, L.iter, L.k, streams[sl], !sliced, R, L.plane, L.rp, L.w, L.h, fin, fstride, L.fp,
-                                     fout, L.fp, cnt, it == 0 ? &up : nullptr));
+                                            : ((it - 1) % 2 == 0 ? L.fB : L.fA) + (size_t)off * fstride;
+                const FfbRing& fout = it == iters - 1 && last ? toRing : (it % 2 == 0 ? toB : toA);
+                if (fused)
+                    TRY(launch_flow_iter(c, L.iter, L.k, streams[sl], !sliced, R, L.plane, L.rp, L.w, L.h, fin, fstride, L.fp,
+                                         fout, L.fp, cnt, it == 0 ? &up : nullptr));
+                else
+                    TRY(launch_flow_unfused(c, L.k, c->M, R, L.plane, L.rp, L.w, L.h, fin, fstride, L.fp, fout, L.fp, cnt));
             }
         }
     }
@@ -1163,7 +1298,8 @@ int ffb_create(int device, ffb_ctx** out) {
         cudaEventRecord(c->ev_ch2d[b], c->s_copy);
         cudaEventRecord(c->ev_pre[b], c->s_comp);
     }
-    c->poly = make_poly_consts();
+    c->poly5 = make_poly_consts<5>(c->fb.poly_sigma);
+    c->poly7 = make_poly_consts<7>(c->fb.poly_sigma);
     *out = c;
     return FFB_OK;
 }
@@ -1214,6 +1350,69 @@ static int configure_checked(ffb_ctx* c, int w, int h, int batch_frames, int max
 
 int ffb_configure(ffb_ctx* c, int w, int h, int batch_frames, int max_pairs) {
     return configure_checked(c, w, h, batch_frames, max_pairs, 0);
+}
+
+// Parameter domain of ffb_set_farneback (include/ffb.h); nothing is touched when a value is outside it.
+static int check_farneback(ffb_ctx* c, const FarnebackParams& p, int flags) {
+    if (flags & 4) return fail(c, FFB_E_INVALID, "ffb_set_farneback: OPTFLOW_USE_INITIAL_FLOW (4) is not supported");
+    if (flags & 256) return fail(c, FFB_E_INVALID, "ffb_set_farneback: OPTFLOW_FARNEBACK_GAUSSIAN (256) is not supported");
+    if (flags != 0) return fail(c, FFB_E_INVALID, "ffb_set_farneback: unknown flags %d", flags);
+    if (!(p.pyr_scale > 0.0 && p.pyr_scale < 1.0))
+        return fail(c, FFB_E_INVALID, "ffb_set_farneback: pyr_scale %g outside (0, 1)", p.pyr_scale);
+    if (p.levels < 0) return fail(c, FFB_E_INVALID, "ffb_set_farneback: levels %d < 0", p.levels);
+    if (p.winsize < 3 || p.winsize > 63) return fail(c, FFB_E_INVALID, "ffb_set_farneback: winsize %d outside 3 .. 63", p.winsize);
+    if (p.iterations < 1 || p.iterations > 20)
+        return fail(c, FFB_E_INVALID, "ffb_set_farneback: iterations %d outside 1 .. 20", p.iterations);
+    if (p.poly_n != 5 && p.poly_n != 7) return fail(c, FFB_E_INVALID, "ffb_set_farneback: poly_n %d is not 5 or 7", p.poly_n);
+    if (!(p.poly_sigma >= 0.0 && isfinite(p.poly_sigma)))
+        return fail(c, FFB_E_INVALID, "ffb_set_farneback: poly_sigma %g is not a finite value >= 0", p.poly_sigma);
+    return FFB_OK;
+}
+
+int ffb_set_farneback(ffb_ctx* c, double pyr_scale, int levels, int winsize, int iterations, int poly_n, double poly_sigma,
+                      int flags) {
+    if (!c) return FFB_E_INVALID;
+    FarnebackParams p;
+    p.pyr_scale = pyr_scale; p.levels = levels; p.winsize = winsize; p.iterations = iterations;
+    p.poly_n = poly_n; p.poly_sigma = poly_sigma;
+    TRY(check_farneback(c, p, flags));
+    if (c->in_bracket) return fail(c, FFB_E_INVALID, "ffb_set_farneback inside a bracket");
+    if (p == c->fb) return FFB_OK;
+    if (c->W > 0) {
+        const LevelPlan lp = make_plan(c->W, c->H, p);
+        if (lp.n > FFB_PLAN_LEVELS)
+            return fail(c, FFB_E_INVALID, "ffb_set_farneback: %dx%d with pyr_scale %g, levels %d plans %d pyramid levels (at most %d)",
+                        c->W, c->H, pyr_scale, levels, lp.n, FFB_PLAN_LEVELS);
+    }
+    CK(c, cudaSetDevice(c->device));
+    // re-plan the configured geometry with the same capacities, as a new frame size would
+    const int W = c->W, H = c->H, B = c->B, maxPairs = c->maxPairs, Bcap = c->Bcap, pairsCap = c->pairsCap, ring = c->ring_n;
+    if (W > 0) {
+        TRY(quiesce(c));
+        free_geometry(c);
+    }
+    c->fb = p;
+    c->poly5 = make_poly_consts<5>(p.poly_sigma);
+    c->poly7 = make_poly_consts<7>(p.poly_sigma);
+    if (W > 0) {
+        TRY(configure_checked(c, W, H, Bcap, pairsCap, ring));
+        c->B = B;
+        c->maxPairs = maxPairs;
+    }
+    return FFB_OK;
+}
+
+int ffb_get_farneback(const ffb_ctx* c, double* pyr_scale, int* levels, int* winsize, int* iterations, int* poly_n,
+                      double* poly_sigma, int* flags) {
+    if (!c) return FFB_E_INVALID;
+    if (pyr_scale) *pyr_scale = c->fb.pyr_scale;
+    if (levels) *levels = c->fb.levels;
+    if (winsize) *winsize = c->fb.winsize;
+    if (iterations) *iterations = c->fb.iterations;
+    if (poly_n) *poly_n = c->fb.poly_n;
+    if (poly_sigma) *poly_sigma = c->fb.poly_sigma;
+    if (flags) *flags = 0;
+    return FFB_OK;
 }
 
 int ffb_get_geometry(const ffb_ctx* c, int* w, int* h, int* batch_frames, int* max_pairs) {
@@ -1500,11 +1699,9 @@ int ffb_radial_motion(ffb_ctx* c, const float* flow, int w, int h, double cx, do
 }
 
 // ---- stage hooks ---------------------------------------------------------------------------
-int ffb_level_plan(int W, int H, int* n, int* w, int* h, int* ksize, double* sigma) {
-    if (!n || W < 1 || H < 1) return FFB_E_INVALID;
-    const LevelPlan p = make_plan(W, H);
+static int level_plan_fill(const LevelPlan& p, int max_n, int* n, int* w, int* h, int* ksize, double* sigma) {
     *n = p.n;
-    for (int i = 0; i < p.n; ++i) {
+    for (int i = 0; i < p.n && i < max_n; ++i) {
         if (w) w[i] = p.w[i];
         if (h) h[i] = p.h[i];
         if (ksize) ksize[i] = p.ksize[i];
@@ -1513,11 +1710,23 @@ int ffb_level_plan(int W, int H, int* n, int* w, int* h, int* ksize, double* sig
     return FFB_OK;
 }
 
+int ffb_level_plan(int W, int H, int* n, int* w, int* h, int* ksize, double* sigma) {
+    if (!n || W < 1 || H < 1) return FFB_E_INVALID;
+    return level_plan_fill(make_plan(W, H, FarnebackParams()), FFB_MAX_LEVELS, n, w, h, ksize, sigma);
+}
+
+int ffb_level_plan_ex(int W, int H, double pyr_scale, int levels, int max_n, int* n, int* w, int* h, int* ksize, double* sigma) {
+    if (!n || W < 1 || H < 1 || !(pyr_scale > 0.0 && pyr_scale < 1.0) || levels < 0 || max_n < 0) return FFB_E_INVALID;
+    const LevelPlan p = make_plan(W, H, pyr_scale, levels);
+    if (p.n > FFB_PLAN_LEVELS) return FFB_E_INVALID;
+    return level_plan_fill(p, max_n, n, w, h, ksize, sigma);
+}
 
 int ffb_stage_pyramid(ffb_ctx* c, const uint8_t* img, int W, int H, size_t pitch, int level_k, float* out) {
     if (!c || !img || !out) return FFB_E_INVALID;
     CK(c, cudaSetDevice(c->device));
-    const LevelPlan p = make_plan(W, H);
+    const LevelPlan p = make_plan(W, H, c->fb);
+    if (p.n > FFB_PLAN_LEVELS) return fail(c, FFB_E_INVALID, "%dx%d plans more than %d pyramid levels", W, H, FFB_PLAN_LEVELS);
     int li = -1;
     for (int i = 0; i < p.n; ++i) if (p.k[i] == level_k) li = i;
     if (li < 0) return fail(c, FFB_E_INVALID, "level %d does not exist for %dx%d", level_k, W, H);
@@ -1550,7 +1759,16 @@ int ffb_stage_pyramid(ffb_ctx* c, const uint8_t* img, int W, int H, size_t pitch
     TRY(s.alloc(c, &d_out, (size_t)w * h));
     TRY(s.upload(c, &dxi, xi.data(), xi.size())); TRY(s.upload(c, &dxa, xa.data(), xa.size()));
     TRY(s.upload(c, &dyi, yi.data(), yi.size())); TRY(s.upload(c, &dya, ya.data(), ya.size()));
-    TRY(launch_pyramid(c, d_img, (size_t)W * H, W, W, H, d_out, (size_t)w * h, w, w, h, dxi, dxa, dyi, dya, taps, RW, RH, 1));
+    if (pyramid_wide(taps.r, RW, RH)) {
+        const std::vector<float> k = gaussian_half(p.ksize[li], p.sigma[li]);
+        float *dk = nullptr, *dtmp = nullptr;
+        TRY(s.upload(c, &dk, k.data(), k.size()));
+        TRY(s.alloc(c, &dtmp, (size_t)H * w));
+        TRY(launch_pyramid_wide(c, d_img, (size_t)W * H, W, W, H, dtmp, d_out, (size_t)w * h, w, w, h, dxi, dxa, dyi, dya, dk,
+                                taps.r, 1));
+    } else {
+        TRY(launch_pyramid(c, d_img, (size_t)W * H, W, W, H, d_out, (size_t)w * h, w, w, h, dxi, dxa, dyi, dya, taps, RW, RH, 1));
+    }
     CK(c, cudaStreamSynchronize(c->s_comp));
     CK(c, cudaMemcpy(out, d_out, (size_t)w * h * 4, cudaMemcpyDeviceToHost));
     return FFB_OK;
@@ -1635,8 +1853,14 @@ int ffb_stage_flow_iter(ffb_ctx* c, const float* R0, const float* R1, const floa
     TRY(s.alloc(c, &dfo, plane));
     FfbRing R{(char*)dR, 5 * plane * sizeof(float), 0, 2};
     FfbRing fo{(char*)dfo, 0, 0, 1};
-    TRY(launch_flow_iter(c, flow_iter_plan(w, h, w, h, c->iter_cfg), -1, c->s_comp, true, R, plane, rp, w, h, dfi, 0, rp, fo,
-                         rp, 1));
+    if (c->fb.winsize == FFB_WIN) {
+        TRY(launch_flow_iter(c, flow_iter_plan(w, h, w, h, c->iter_cfg), -1, c->s_comp, true, R, plane, rp, w, h, dfi, 0, rp, fo,
+                             rp, 1));
+    } else {
+        float* dM = nullptr;
+        TRY(s.alloc(c, &dM, 5 * plane));
+        TRY(launch_flow_unfused(c, -1, dM, R, plane, rp, w, h, dfi, 0, rp, fo, rp, 1));
+    }
     CK(c, cudaStreamSynchronize(c->s_comp));
     CK(c, cudaMemcpy2D(flow_out, (size_t)w * 8, dfo, (size_t)rp * 8, (size_t)w * 8, h, cudaMemcpyDeviceToHost));
     return FFB_OK;
@@ -1775,7 +1999,7 @@ int ffb_profile_reset(ffb_ctx* c) {
     CK(c, cudaStreamSynchronize(c->s_comp));
     prof_collect(c);
     for (int i = 0; i < FFB_K_COUNT; ++i) { c->k_launches[i] = 0; c->k_ms[i] = 0; c->k_bytes[i] = 0; }
-    for (int i = 0; i < FFB_MAX_LEVELS; ++i) { c->it_launches[i] = 0; c->it_ms[i] = 0; c->it_bytes[i] = 0; }
+    for (int i = 0; i < FFB_PLAN_LEVELS; ++i) { c->it_launches[i] = 0; c->it_ms[i] = 0; c->it_bytes[i] = 0; }
     return FFB_OK;
 }
 int ffb_kernel_stats(ffb_ctx* c, int kid, int64_t* launches, double* ms, double* bytes) {
@@ -1788,7 +2012,7 @@ int ffb_kernel_stats(ffb_ctx* c, int kid, int64_t* launches, double* ms, double*
     return FFB_OK;
 }
 int ffb_flow_iter_level_stats(ffb_ctx* c, int k, int64_t* launches, double* ms, double* bytes) {
-    if (!c || k < 0 || k >= FFB_MAX_LEVELS) return FFB_E_INVALID;
+    if (!c || k < 0 || k >= FFB_PLAN_LEVELS) return FFB_E_INVALID;
     CK(c, cudaStreamSynchronize(c->s_comp));
     prof_collect(c);
     if (launches) *launches = c->it_launches[k];

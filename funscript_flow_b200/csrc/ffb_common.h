@@ -48,11 +48,13 @@ __device__ __forceinline__ void ffb_load_f8(const float* p, float4& lo, float4& 
 }
 #endif
 
+// FFB_MAX_LEVELS sizes the single-pass pyramid (k_pyramid_pow2, levels 0..3); a context's level table holds up to
+// FFB_PLAN_LEVELS levels.  FFB_WIN is the window of the fused k_flow_iter (other window sizes take k_flow_matrices +
+// k_box_solve).
 #define FFB_MAX_LEVELS 4
-#define FFB_POLY_N 5
+#define FFB_PLAN_LEVELS 16
 #define FFB_WIN 15
 #define FFB_WIN_R 7
-#define FFB_ITERS 3
 
 // Half of a symmetric 1-D kernel: k[0] is the centre tap, k[i] the taps at +-i.
 struct FfbTaps {
@@ -60,11 +62,12 @@ struct FfbTaps {
     float k[10];
 };
 
-// Polynomial-expansion constants (FarnebackPrepareGaussian, computed on the host in double).
+// Polynomial-expansion constants of a (2N+1)-tap expansion (FarnebackPrepareGaussian, computed on the host in double).
+template <int N>
 struct FfbPolyConsts {
-    float g[FFB_POLY_N + 1];
-    float xg[FFB_POLY_N + 1];
-    float xxg[FFB_POLY_N + 1];
+    float g[N + 1];
+    float xg[N + 1];
+    float xxg[N + 1];
     float ig11, ig03, ig33, ig55;
 };
 

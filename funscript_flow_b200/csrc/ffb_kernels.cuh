@@ -307,6 +307,57 @@ __global__ void __launch_bounds__(256) k_pyramid_pow2(FfbPyr2Args a) {
 }
 
 // ======================================================================================
+// K1'' pyramid level with a large blur radius (deep levels: r > 9, or a tile window beyond shared memory)
+// ======================================================================================
+// The two passes of k_pyramid_level as two launches through a scratch image T[H][w]: the row pass evaluates the
+// horizontal blur at the two resize taps of every output column on every source row and lerps them; the column pass
+// evaluates the vertical blur of T at the two resize rows of every output row and lerps them.  Same taps, pairing and
+// order as k_pyramid_level; the half kernel lives in device memory (any radius < min(W, H), REFLECT_101).
+struct FfbPyrWideArgs {
+    const uint8_t* src; size_t src_frame_stride; int src_pitch; int W, H;
+    float* tmp; size_t tmp_frame_stride;                          // T[H][w] per frame (floats)
+    float* dst; size_t dst_frame_stride; int dp; int w, h;        // strides in floats
+    const int* xi; const float* xa; const int* yi; const float* ya;
+    const float* k; int r;
+};
+
+__global__ void __launch_bounds__(256) k_pyramid_wide_rows(FfbPyrWideArgs a) {
+    const int dx = blockIdx.x * 32 + (threadIdx.x & 31);
+    const int y = blockIdx.y * 8 + (threadIdx.x >> 5);
+    if (dx >= a.w || y >= a.H) return;
+    const uint8_t* row = a.src + (size_t)blockIdx.z * a.src_frame_stride + (size_t)y * a.src_pitch;
+    auto blur = [&](int c) {
+        float s = __ldg(a.k) * (float)__ldg(row + c);
+        for (int i = 1; i <= a.r; ++i)
+            s += __ldg(a.k + i) * ((float)__ldg(row + ffb_reflect1(c - i, a.W)) + (float)__ldg(row + ffb_reflect1(c + i, a.W)));
+        return s;
+    };
+    const int s0 = a.xi[dx];
+    const float al = a.xa[dx];
+    float v = blur(s0);
+    if (al != 0.f) v = v * (1.f - al) + blur(min(s0 + 1, a.W - 1)) * al;
+    a.tmp[(size_t)blockIdx.z * a.tmp_frame_stride + (size_t)y * a.w + dx] = v;
+}
+
+__global__ void __launch_bounds__(256) k_pyramid_wide_cols(FfbPyrWideArgs a) {
+    const int dx = blockIdx.x * 32 + (threadIdx.x & 31);
+    const int dy = blockIdx.y * 8 + (threadIdx.x >> 5);
+    if (dx >= a.w || dy >= a.h) return;
+    const float* col = a.tmp + (size_t)blockIdx.z * a.tmp_frame_stride + dx;
+    auto blur = [&](int c) {
+        float s = __ldg(a.k) * __ldg(col + (size_t)c * a.w);
+        for (int i = 1; i <= a.r; ++i)
+            s += __ldg(a.k + i) * (__ldg(col + (size_t)ffb_reflect1(c - i, a.H) * a.w) + __ldg(col + (size_t)ffb_reflect1(c + i, a.H) * a.w));
+        return s;
+    };
+    const int s0 = a.yi[dy];
+    const float be = a.ya[dy];
+    float v = blur(s0);
+    if (be != 0.f) v = v * (1.f - be) + blur(min(s0 + 1, a.H - 1)) * be;
+    a.dst[(size_t)blockIdx.z * a.dst_frame_stride + (size_t)dy * a.dp + dx] = v;
+}
+
+// ======================================================================================
 // K2  polynomial expansion: f32 image -> 5 planes (d/dy, d/dx, yy, xx, xy)
 // ======================================================================================
 // CTA = 256 threads = 128 columns x 2 row halves; it produces POLY_OW = 112 output columns (the
@@ -316,11 +367,13 @@ __global__ void __launch_bounds__(256) k_pyramid_pow2(FfbPyr2Args a) {
 //            every row of its half from registers -> shared rows vrow[3][POLY_ROWS][132]
 //   phase H: each task = 4 adjacent outputs of one row: 4 aligned 16-byte shared loads per vertical
 //            sum, six horizontal sums with the CPU code's symmetric pairing, 5 x 16-byte stores.
+// N = poly_n: 5 (the reference's) or 7; the 112 output columns plus 2N halo columns fit the 128 loaded ones for both.
+template <int N>
 struct FfbPolyArgs {
     const float* src; size_t src_frame_stride; int sp; int w, h;  // strides in floats
     FfbRing dst;            // per frame-level: float4 [h][rp] (c0..c3) then float [h][rp] (c4); plane = rp * h
     size_t plane; int rp;
-    FfbPolyConsts c;
+    FfbPolyConsts<N> c;
 };
 
 constexpr int POLY_OW = 112;
@@ -328,8 +381,10 @@ constexpr int POLY_ROWS = 32;
 constexpr int POLY_VP = 132;    // shared row pitch (floats)
 constexpr size_t POLY_SMEM = sizeof(float) * 3 * POLY_ROWS * POLY_VP;
 
-__global__ void __launch_bounds__(256) k_polyexp(FfbPolyArgs a) {
-    constexpr int N = FFB_POLY_N;
+template <int N>
+__global__ void __launch_bounds__(256) k_polyexp(FfbPolyArgs<N> a) {
+    static_assert(POLY_OW + 2 * N <= 128, "halo of the expansion");
+    constexpr int NQ = (2 * N + 7) / 4;        // 16-byte loads per vertical sum in phase H (4 outputs + 2N halo)
     constexpr int HR = POLY_ROWS / 2;          // rows per half
     FFB_DYN_SMEM(float, vrow);                 // [3][POLY_ROWS][POLY_VP]
     const int tid = threadIdx.x;
@@ -375,12 +430,12 @@ __global__ void __launch_bounds__(256) k_polyexp(FfbPolyArgs a) {
         const int r = t / QUADS, q = t - r * QUADS;
         const int x = x0 + 4 * q, y = y0 + r;
         if (x >= w || y >= h) continue;
-        float v[3][16];
+        float v[3][4 * NQ];
 #pragma unroll
         for (int k = 0; k < 3; ++k) {
             const float4* p4 = reinterpret_cast<const float4*>(vrow + (k * POLY_ROWS + r) * POLY_VP + 4 * q);
 #pragma unroll
-            for (int j = 0; j < 4; ++j) {
+            for (int j = 0; j < NQ; ++j) {
                 const float4 t4 = p4[j];
                 v[k][4 * j] = t4.x; v[k][4 * j + 1] = t4.y; v[k][4 * j + 2] = t4.z; v[k][4 * j + 3] = t4.w;
             }
@@ -437,8 +492,10 @@ struct FfbUpArgs {
     const float2* src; size_t src_stride; int sp; int wc, hc;     // strides in float2
     float2* dst; size_t dst_stride; int dp; int w, h;
     const int* xi; const float* xa; const int* yi; const float* ya;
+    float scale;      // 1 / pyr_scale (SCALED only; otherwise the flow is doubled)
 };
 
+template <bool SCALED>
 __global__ void __launch_bounds__(256) k_upsample_flow(FfbUpArgs a) {
     const int x = blockIdx.x * 32 + (threadIdx.x & 31);
     const int y = blockIdx.y * 8 + (threadIdx.x >> 5);
@@ -451,9 +508,10 @@ __global__ void __launch_bounds__(256) k_upsample_flow(FfbUpArgs a) {
     const float2 p10 = src[(size_t)y1 * a.sp + x0], p11 = src[(size_t)y1 * a.sp + x1];
     const float tx = p00.x * (1.f - al) + p01.x * al, ty = p00.y * (1.f - al) + p01.y * al;
     const float bx = p10.x * (1.f - al) + p11.x * al, by = p10.y * (1.f - al) + p11.y * al;
+    const float s = SCALED ? a.scale : 2.f;
     float2 o;
-    o.x = (tx * (1.f - be) + bx * be) * 2.f;
-    o.y = (ty * (1.f - be) + by * be) * 2.f;
+    o.x = (tx * (1.f - be) + bx * be) * s;
+    o.y = (ty * (1.f - be) + by * be) * s;
     a.dst[(size_t)blockIdx.z * a.dst_stride + (size_t)y * a.dp + x] = o;
 }
 
@@ -662,9 +720,9 @@ __device__ __forceinline__ void ffb_up2(int d, int src_n, int& i0, int& i1, floa
     i1 = min(i0 + 1, src_n - 1);
 }
 
-// box mean -> 2x2 solve of one output (sums of the 15x15 window of the five matrix channels)
-__device__ __forceinline__ float2 ffb_solve(float s0, float s1, float s2, float s3, float s4) {
-    const float sc = 1.f / (float)(FFB_WIN * FFB_WIN);
+// box mean -> 2x2 solve of one output (sums of the window of the five matrix channels; sc = 1 / winsize^2)
+__device__ __forceinline__ float2 ffb_solve(float s0, float s1, float s2, float s3, float s4,
+                                            float sc = 1.f / (float)(FFB_WIN * FFB_WIN)) {
     const float g11 = s0 * sc, g12 = s1 * sc, g22 = s2 * sc, h1 = s3 * sc, h2 = s4 * sc;
     // det = g11*g22 - g12*g12 with an exact-product correction (Kahan's ad-bc)
     const float wq = g12 * g12;
@@ -914,6 +972,94 @@ __global__ void __launch_bounds__(NT, MINB) k_flow_iter(FfbIterArgs a) {
         for (int u = 0; u < U; ++u) d[u] = dn[u];
     }
     horizontal(nsteps - 1, NB == 2 ? ((nsteps - 1) & 1) : 0);
+}
+
+// ======================================================================================
+// K3'  flow iteration for window sizes other than 15: matrices to HBM, then box sum + solve
+// ======================================================================================
+// k_flow_matrices: one thread per pixel gathers the production expansion layout (ffb_gather_*) and writes
+// M = (G11, G12, G22, h1, h2) as five planes of rp x h floats per pair.
+struct FfbMatrixArgs {
+    FfbRing R; int plane; int rp; int w, h;          // as FfbIterArgs
+    const float2* fin; size_t fin_stride; int fip;   // flow in (NULL = zero), strides in float2
+    float* M; size_t m_stride;                       // per pair: 5 planes of `plane` floats
+};
+
+__global__ void __launch_bounds__(256) k_flow_matrices(FfbMatrixArgs a) {
+    const int x = blockIdx.x * 32 + (threadIdx.x & 31);
+    const int y = blockIdx.y * 8 + (threadIdx.x >> 5);
+    if (x >= a.w || y >= a.h) return;
+    const int pair = blockIdx.z;
+    const float4* A0 = reinterpret_cast<const float4*>(ffb_ring_at(a.R, pair));
+    const float4* A1 = reinterpret_cast<const float4*>(ffb_ring_at(a.R, pair + 1));
+    const float* B0 = reinterpret_cast<const float*>(A0 + a.plane);
+    const float* B1 = reinterpret_cast<const float*>(A1 + a.plane);
+    const float2 d = a.fin ? __ldg(a.fin + (size_t)pair * a.fin_stride + (size_t)y * a.fip + x) : make_float2(0.f, 0.f);
+    FfbGather g;
+    ffb_gather_issue(A0, B0, A1, B1, a.rp, a.w, a.h, x, y, d, g);
+    float m[5];
+    ffb_gather_finish(g, a.w, a.h, x, y, m);
+    float* M = a.M + (size_t)pair * a.m_stride + (size_t)y * a.rp + x;
+#pragma unroll
+    for (int c = 0; c < 5; ++c) M[(size_t)c * a.plane] = m[c];
+}
+
+// k_box_solve: (2r+1) x (2r+1) box sums of M with replicate border, then the 2x2 solve with scale 1 / winsize^2
+// (an even winsize sums 2 * (winsize / 2) + 1 taps, as OpenCV does).  One CTA = BOX_NT matrix columns (a strip of
+// BOX_NT - 2r outputs) marching down a segment of SH rows; each thread keeps the vertical sums of its column in double
+// (add the entering row, subtract the leaving one -- OpenCV keeps double sliding sums too), the outputs sum 2r+1 of
+// them from shared memory in double.
+constexpr int BOX_NT = 256;
+struct FfbBoxArgs {
+    const float* M; size_t m_stride; int plane; int rp; int w, h;
+    int r; float scale;
+    FfbRing fout; int fop;   // flow out ring (element = pair), pitch in float2
+    int SW, SH;              // outputs per strip (BOX_NT - 2r), rows per segment
+};
+
+__global__ void __launch_bounds__(BOX_NT) k_box_solve(FfbBoxArgs a) {
+    __shared__ double vrow[5][BOX_NT];
+    const int tid = threadIdx.x;
+    const int pair = blockIdx.x;
+    const int w = a.w, h = a.h, r = a.r;
+    const float* M = a.M + (size_t)pair * a.m_stride;
+    float2* fout = reinterpret_cast<float2*>(ffb_ring_at(a.fout, pair));
+    const int xo0 = (int)blockIdx.y * a.SW;
+    const int useful = min(a.SW, w - xo0);
+    const bool live = tid < useful + 2 * r;
+    const int xc = ffb_clampi(xo0 - r + tid, 0, w - 1);
+    const int y0 = (int)blockIdx.z * a.SH, y1 = min(y0 + a.SH, h);
+    double vs[5] = {0.0, 0.0, 0.0, 0.0, 0.0};
+    if (live) {
+        for (int i = -r; i <= r; ++i) {
+            const float* p = M + (size_t)ffb_clampi(y0 + i, 0, h - 1) * a.rp + xc;
+#pragma unroll
+            for (int c = 0; c < 5; ++c) vs[c] += (double)__ldg(p + (size_t)c * a.plane);
+        }
+    }
+    for (int y = y0; y < y1; ++y) {
+#pragma unroll
+        for (int c = 0; c < 5; ++c) vrow[c][tid] = vs[c];
+        __syncthreads();
+        if (tid < useful) {
+            float s[5];
+#pragma unroll
+            for (int c = 0; c < 5; ++c) {
+                double t = 0.0;
+                for (int j = 0; j <= 2 * r; ++j) t += vrow[c][tid + j];
+                s[c] = (float)t;
+            }
+            fout[(size_t)y * a.fop + xo0 + tid] = ffb_solve(s[0], s[1], s[2], s[3], s[4], a.scale);
+        }
+        __syncthreads();
+        if (live && y + 1 < y1) {
+            const float* pin = M + (size_t)ffb_clampi(y + 1 + r, 0, h - 1) * a.rp + xc;
+            const float* pout = M + (size_t)ffb_clampi(y - r, 0, h - 1) * a.rp + xc;
+#pragma unroll
+            for (int c = 0; c < 5; ++c)
+                vs[c] += (double)__ldg(pin + (size_t)c * a.plane) - (double)__ldg(pout + (size_t)c * a.plane);
+        }
+    }
 }
 
 // ======================================================================================

@@ -295,6 +295,7 @@ def process_video_series(video_path: str, params: Dict, ctx=None, progress_callb
     # so the shorter last bracket re-allocates nothing)
     max_pairs = min(bracket, len(indices)) - 1
     for c in ctxs:
+        api.apply_farneback(c, params)
         c.configure(out_w, out_h, max(1, min(batch, max_pairs + 1)), max(1, max_pairs))
     done = 0
     for a in range(0, len(indices), bracket):

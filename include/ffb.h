@@ -61,8 +61,8 @@ int  ffb_host_free(void* ptr);
  * (Re)allocate device buffers for width x height frames.
  *   batch_frames       frames expanded per launch group (>= 1); pairs of a batch share launches
  *   max_bracket_pairs  upper bound on pairs between bracket_begin and bracket_finish
- * Farneback parameters are fixed to the reference's call (F:878-879):
- *   pyr_scale 0.5, levels 3, winsize 15, iterations 3, poly_n 5, poly_sigma 1.2, flags 0. */
+ * The Farneback parameters are the context's (ffb_set_farneback below); a new context holds the reference's call
+ * (F:878-879): pyr_scale 0.5, levels 3, winsize 15, iterations 3, poly_n 5, poly_sigma 1.2, flags 0. */
 int  ffb_configure(ffb_ctx* ctx, int width, int height, int batch_frames, int max_bracket_pairs);
 /* ffb_configure is incremental: a call with the frame size already configured and limits that fit the
  * allocated capacities changes nothing on the device (no cudaMalloc, no cudaHostAlloc, no synchronisation);
@@ -73,6 +73,24 @@ int  ffb_configure(ffb_ctx* ctx, int width, int height, int batch_frames, int ma
  * configures once per video must see them stand still after the first bracket). */
 int  ffb_get_geometry(const ffb_ctx* ctx, int* width, int* height, int* batch_frames, int* max_bracket_pairs);
 int  ffb_alloc_counts(const ffb_ctx* ctx, int64_t* device_allocs, int64_t* host_allocs);
+
+/* ---- Farneback parameters (cv2.calcOpticalFlowFarneback's arguments after the flow) ---------------------------
+ * ffb_set_farneback sets the parameters every flow of the context uses: ffb_farneback, the bracket and shard APIs and
+ * the stage hooks.  Accepted (anything else is FFB_E_INVALID with a message, and changes nothing):
+ *   0 < pyr_scale < 1;  levels >= 0 (levels stop where the coarsest one would be under 32 px, as in OpenCV; a plan of
+ *   more than 16 levels is refused);  3 <= winsize <= 63 (an even size sums 2 * (winsize / 2) + 1 taps with mean
+ *   scale 1 / winsize^2, as OpenCV does);  1 <= iterations <= 20;  poly_n 5 or 7;  poly_sigma >= 0 (below FLT_EPSILON
+ *   it becomes poly_n * 0.3);  flags 0 (OPTFLOW_USE_INITIAL_FLOW = 4 and OPTFLOW_FARNEBACK_GAUSSIAN = 256 are refused).
+ * Parameters equal to the current ones change nothing (no allocation, no synchronisation); others re-plan the
+ * configured geometry as a new frame size does.  Refused inside a bracket.
+ * ffb_level_plan_ex: the level geometry of a frame size for (pyr_scale, levels), coarsest level first; fills at most
+ * max_n entries and returns the level count in *n_levels. */
+int  ffb_set_farneback(ffb_ctx* ctx, double pyr_scale, int levels, int winsize, int iterations,
+                       int poly_n, double poly_sigma, int flags);
+int  ffb_get_farneback(const ffb_ctx* ctx, double* pyr_scale, int* levels, int* winsize, int* iterations,
+                       int* poly_n, double* poly_sigma, int* flags);
+int  ffb_level_plan_ex(int width, int height, double pyr_scale, int levels, int max_n,
+                       int* n_levels, int* w, int* h, int* ksize, double* sigma);
 
 /* ---- streaming bracket API (replaces the bracket loop body F:1188-1242) ------------------
  * A bracket is a run of consecutive sampled frames; pairs never span brackets (F:1150-1153,
@@ -137,7 +155,8 @@ int  ffb_bracket_get_flow(ffb_ctx* ctx, int pair, float* flow_hw2);
 int  ffb_flow_ring_size(const ffb_ctx* ctx);
 
 /* ---- per-call functions on host arrays (drop-ins for the module-level functions) ----------
- * ffb_farneback   == cv2.calcOpticalFlowFarneback(p0, p1, None, .5, 3, 15, 3, 5, 1.2, 0) F:878
+ * ffb_farneback   == cv2.calcOpticalFlowFarneback(p0, p1, None, <the context's parameters>)  F:878
+ *                    (a new context: .5, 3, 15, 3, 5, 1.2, 0)
  * ffb_max_divergence     == max_divergence(flow)                                         F:748
  * ffb_mean_magnitude     == np.mean(cv2.cartToPolar(u, v)[0])                            F:889-890
  * ffb_radial_motion      == radial_motion_weighted(flow, (cx, cy), is_cut, pov_mode)     F:761 */
@@ -149,23 +168,23 @@ int  ffb_mean_magnitude(ffb_ctx* ctx, const float* flow_hw2, int width, int heig
 int  ffb_radial_motion(ffb_ctx* ctx, const float* flow_hw2, int width, int height,
                        double cx, double cy, int is_cut, int pov_mode, double* out);
 
-/* ---- per-stage hooks (each runs exactly the production kernel of that stage) --------------
- * Level geometry of the Farneback pyramid for a frame size (coarsest level first):
- * fills up to 4 entries of w[], h[], ksize[], sigma[]; returns the level count in *n_levels. */
+/* ---- per-stage hooks (each runs exactly the production kernel of that stage, for the context's parameters) -----
+ * Level geometry of the Farneback pyramid for a frame size with the reference's pyr_scale 0.5, levels 3 (coarsest
+ * level first): fills up to 4 entries of w[], h[], ksize[], sigma[]; returns the level count in *n_levels. */
 int  ffb_level_plan(int width, int height, int* n_levels, int* w, int* h, int* ksize, double* sigma);
 /* A1a: u8 frame -> float32 level image (GaussianBlur REFLECT_101 at full res + bilinear resize). */
 int  ffb_stage_pyramid(ffb_ctx* ctx, const uint8_t* img, int width, int height, size_t pitch,
                        int level_k, float* out_hw);
-/* A1b: float32 image -> float32 [5][h][w] planes (d/dy, d/dx, yy, xx, xy). */
+/* A1b: float32 image -> float32 [5][h][w] planes (d/dy, d/dx, yy, xx, xy), with the context's poly_n / poly_sigma. */
 int  ffb_stage_polyexp(ffb_ctx* ctx, const float* img, int w, int h, float* out_5hw);
 /* A1c: R0, R1 ([5][h][w] planes), flow [h][w][2] -> M [5][h][w] planes (G11,G12,G22,h1,h2). */
 int  ffb_stage_update_matrices(ffb_ctx* ctx, const float* R0, const float* R1, const float* flow,
                                int w, int h, float* out_5hw);
-/* A1c+A1d fused (the production flow iteration): R0, R1, flow_in -> flow_out [h][w][2].
- * flow_in may be NULL (zero initial flow). */
+/* A1c+A1d (the production flow iteration for the context's winsize: fused for 15, matrices + box solve otherwise):
+ * R0, R1, flow_in -> flow_out [h][w][2].  flow_in may be NULL (zero initial flow). */
 int  ffb_stage_flow_iter(ffb_ctx* ctx, const float* R0, const float* R1, const float* flow_in,
                          int w, int h, float* flow_out);
-/* A1e: coarse flow [hc][wc][2] -> [h][w][2], bilinear, x2. */
+/* A1e: coarse flow [hc][wc][2] -> [h][w][2], bilinear, x (1 / the context's pyr_scale). */
 int  ffb_stage_upsample_flow(ffb_ctx* ctx, const float* flow_c, int wc, int hc, int w, int h, float* out);
 
 /* ---- frame pre-processing on the device (SURVEY row N2; replaces F:173-189 + F:1074-1082) ------
@@ -210,7 +229,7 @@ int  ffb_stage_preprocess_window(ffb_ctx* ctx, const uint8_t* bgr, int width, in
 int  ffb_profile(ffb_ctx* ctx, int enable);
 int  ffb_profile_reset(ffb_ctx* ctx);
 int  ffb_kernel_stats(ffb_ctx* ctx, int kernel_id, int64_t* launches, double* ms, double* alg_bytes);
-/* The same three figures for k_flow_iter alone, split by pyramid level k (0 = full resolution). */
+/* The same three figures for the flow iteration alone, split by pyramid level k (0 = full resolution, up to 15). */
 int  ffb_flow_iter_level_stats(ffb_ctx* ctx, int level_k, int64_t* launches, double* ms, double* alg_bytes);
 int64_t ffb_launch_count(const ffb_ctx* ctx);   /* kernels launched by this context so far */
 /* Device-side stopwatch on the compute stream (the stream every kernel is launched on):
