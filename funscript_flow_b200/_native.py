@@ -64,6 +64,8 @@ def load(path: Optional[str] = None) -> C.CDLL:
         "ffb_bracket_get_flow": (i32, [vp, i32, f32p]),
         "ffb_flow_ring_size": (i32, [vp]),
         "ffb_farneback": (i32, [vp, u8p, u8p, i32, i32, sz, f32p]),
+        "ffb_farneback_pairs": (i32, [vp, vp, vp, i32, i32, i32, sz, sz, vp, sz, sz, i32, C.c_double, i32p, i32p, f32p, f32p,
+                                      u8p, vp]),
         "ffb_max_divergence": (i32, [vp, f32p, i32, i32, i32p, i32p, f32p]),
         "ffb_mean_magnitude": (i32, [vp, f32p, i32, i32, f32p]),
         "ffb_radial_motion": (i32, [vp, f32p, i32, i32, C.c_double, C.c_double, i32, i32, f64p]),
@@ -381,6 +383,55 @@ class FlowContext:
         out = np.empty((h, w, 2), np.float32)
         self._ck(self._lib.ffb_farneback(self._h, _u8(prev), _u8(nxt), w, h, w, _f32(out)))
         return out
+
+    def farneback_pairs(self, prev: np.ndarray, nxt: np.ndarray, *, flow: bool = True, pov: bool = False,
+                        cut_threshold: float = float("inf")) -> dict:
+        """n independent pairs (prev[i], nxt[i]), uint8 [n, H, W] each, in one call (ffb_farneback_pairs): flow f32
+        [n, H, W, 2] (None with flow=False), cx / cy (int32), val / mean_mag (float32) and cut (bool) per pair.  Each
+        flow is bit-identical to farneback(prev[i], nxt[i]).  Pairs run in chunks of (batch_frames + 1) / 2 of the last
+        configure(); a context never configured runs one pair per chunk, so configure it first (api's batch functions
+        do)."""
+        prev = np.ascontiguousarray(prev, dtype=np.uint8)
+        nxt = np.ascontiguousarray(nxt, dtype=np.uint8)
+        if prev.shape != nxt.shape or prev.ndim != 3:
+            raise ValueError(f"farneback_pairs: prev and nxt must be uint8 [n, H, W] of one shape, not {prev.shape} and {nxt.shape}")
+        n, h, w = prev.shape
+        out = self.farneback_pairs_ptr(prev.ctypes.data, nxt.ctypes.data, n, w, h, w, w * h, stats=True, pov=pov,
+                                       cut_threshold=cut_threshold,
+                                       flow=np.empty((n, h, w, 2), np.float32) if flow else None)
+        return out
+
+    def farneback_pairs_ptr(self, prev_ptr: int, next_ptr: int, n: int, width: int, height: int, pitch: int,
+                            frame_stride: int, flow=None, flow_pitch: int = 0, flow_stride: int = 0, stream: int = 0, *,
+                            stats: bool = False, pov: bool = False, cut_threshold: float = float("inf")):
+        """Raw-pointer variant of farneback_pairs, like bracket_push_ptr: frames anywhere (e.g. torch_tensor.data_ptr()),
+        `flow` a pointer (int; 0 = no flow) or a float32 NumPy array, `stream` a cudaStream_t handle (0 = none; e.g.
+        torch.cuda.current_stream().cuda_stream).  stats=True returns the per-pair dict (then the call waits for the
+        device), otherwise None."""
+        flow_arr = flow if isinstance(flow, np.ndarray) else None
+        if flow_arr is not None:
+            assert flow_arr.dtype == np.float32 and flow_arr.flags.c_contiguous and flow_arr.shape == (n, height, width, 2)
+            flow_ptr, flow_pitch, flow_stride = flow_arr.ctypes.data, width * 8, width * height * 8
+        else:
+            flow_ptr = int(flow or 0)
+        res = None
+        args = [None] * 5
+        if stats:
+            res = dict(cx=np.empty(max(n, 1), np.int32), cy=np.empty(max(n, 1), np.int32), val=np.empty(max(n, 1), np.float32),
+                       mean_mag=np.empty(max(n, 1), np.float32), cut=np.empty(max(n, 1), np.uint8))
+            i32p = C.POINTER(C.c_int32)
+            args = [res["cx"].ctypes.data_as(i32p), res["cy"].ctypes.data_as(i32p), _f32(res["val"]), _f32(res["mean_mag"]),
+                    _u8(res["cut"])]
+        self._ck(self._lib.ffb_farneback_pairs(self._h, C.c_void_p(prev_ptr), C.c_void_p(next_ptr), int(n), int(width),
+                                               int(height), int(pitch), int(frame_stride), C.c_void_p(flow_ptr or None),
+                                               int(flow_pitch), int(flow_stride), int(bool(pov)), float(cut_threshold), *args,
+                                               C.c_void_p(int(stream) or None)))
+        if res is None:
+            return None
+        res = {k: v[:n] for k, v in res.items()}
+        res["cut"] = res["cut"].astype(bool)
+        res["flow"] = flow_arr
+        return res
 
     def max_divergence(self, flow: np.ndarray):
         flow = np.ascontiguousarray(flow, dtype=np.float32)

@@ -9,6 +9,9 @@
     get_available_backends()                        F:32-63
     calc_optical_flow_farneback(prev, next, None, pyr_scale, levels, winsize, iterations, poly_n, poly_sigma, 0)
                                                     cv2's signature (F:878), any parameter set
+    calc_optical_flow_farneback_batch(prev, next, None, ...)   the same for n independent pairs ([n, H, W]; NumPy
+                                                    arrays or torch CUDA tensors, which stay on the device)
+    precompute_flow_info_batch(pairs, config)       [precompute_wrapper(p, config) for p in pairs] in one call
 
 Every entry point that configures a context first sets its Farneback parameters from the settings keys
 flow_pyr_scale, flow_levels, flow_winsize, flow_iterations, flow_poly_n, flow_poly_sigma (farneback_params;
@@ -306,6 +309,95 @@ def calc_optical_flow_farneback(prev: np.ndarray, next: np.ndarray, flow, pyr_sc
     ctx = ctx or get_context()
     ctx.set_farneback(pyr_scale, levels, winsize, iterations, poly_n, poly_sigma, flags)
     return ctx.farneback(prev, next)
+
+
+def _pairs_batch(width: int, height: int, n: int) -> int:
+    """batch_frames for n independent pairs of width x height: the runner's batch for the frame size (chunks of
+    (batch_frames + 1) / 2 pairs fill the GPU as a bracket's batches do), no more than n pairs need."""
+    from .runner import default_batch_frames
+    return max(1, min(default_batch_frames(width, height), 2 * n - 1))
+
+
+def _is_torch_tensor(x) -> bool:
+    return type(x).__module__.split(".")[0] == "torch"
+
+
+def calc_optical_flow_farneback_batch(prev, next, flow, pyr_scale: float, levels: int, winsize: int, iterations: int,
+                                      poly_n: int, poly_sigma: float, flags: int = 0, *,
+                                      ctx: Optional[_native.FlowContext] = None):
+    """calc_optical_flow_farneback for n independent pairs (prev[i], next[i]) in one call, cv2's order with a leading
+    batch axis: uint8 [n, H, W] -> float32 [n, H, W, 2].  NumPy arrays give a NumPy array.  torch.uint8 CUDA tensors on
+    the context's device give a tensor on that device, ordered on torch.cuda.current_stream(): the frames and the flow
+    never pass through host memory.  `flow` must be None and `flags` 0.  Like precompute_flow_info, it (re)configures the
+    context: this frame size, the runner's batch for it (at most 2n - 1 frames) and max_pairs n become its limits."""
+    if flow is not None:
+        raise ValueError("calc_optical_flow_farneback_batch: flow must be None (an initial flow is not supported)")
+    ctx = ctx or get_context()
+    tensors = _is_torch_tensor(prev), _is_torch_tensor(next)
+    if tensors[0] != tensors[1]:
+        raise TypeError("calc_optical_flow_farneback_batch: prev and next must both be NumPy arrays or both torch tensors")
+    if tensors[0]:
+        import torch
+        if prev.dtype != torch.uint8 or next.dtype != torch.uint8 or not prev.is_cuda or not next.is_cuda:
+            raise TypeError("calc_optical_flow_farneback_batch: tensors must be torch.uint8 on a CUDA device")
+        if prev.device != next.device or prev.device.index != ctx.device:
+            raise ValueError(f"calc_optical_flow_farneback_batch: tensors on {prev.device} / {next.device}, "
+                             f"the context on cuda:{ctx.device}")
+    else:
+        prev, next = np.asarray(prev), np.asarray(next)
+        if prev.dtype != np.uint8 or next.dtype != np.uint8:
+            raise TypeError("calc_optical_flow_farneback_batch: frames must be uint8")
+    if tuple(prev.shape) != tuple(next.shape) or prev.ndim != 3:
+        raise ValueError(f"calc_optical_flow_farneback_batch: prev and next must be [n, H, W] of one shape, "
+                         f"not {tuple(prev.shape)} and {tuple(next.shape)}")
+    ctx.set_farneback(pyr_scale, levels, winsize, iterations, poly_n, poly_sigma, flags)
+    n, h, w = prev.shape
+    if n == 0:
+        return torch.empty((0, h, w, 2), dtype=torch.float32, device=prev.device) if tensors[0] else np.empty((0, h, w, 2), np.float32)
+    ctx.configure(w, h, _pairs_batch(w, h, n), n)
+    if not tensors[0]:
+        return ctx.farneback_pairs(prev, next)["flow"]
+    prev, next = prev.contiguous(), next.contiguous()
+    out = torch.empty((n, h, w, 2), dtype=torch.float32, device=prev.device)
+    ctx.farneback_pairs_ptr(prev.data_ptr(), next.data_ptr(), n, w, h, w, w * h, out.data_ptr(), w * 8, w * h * 8,
+                            torch.cuda.current_stream(prev.device).cuda_stream)
+    return out
+
+
+def precompute_flow_info_batch(pairs, config: Dict) -> list:
+    """[precompute_wrapper(p, config) for p in pairs] in one call: the same 8-key dicts (F:898-907) with the same types.
+    Every pair must have the frame size of the first.  The shared context is configured as calc_optical_flow_farneback_batch
+    configures it."""
+    pairs = list(pairs)
+    if not pairs:
+        return []
+    prev = np.stack([np.asarray(p[0], dtype=np.uint8) for p in pairs])
+    nxt = np.stack([np.asarray(p[1], dtype=np.uint8) for p in pairs])
+    if prev.shape != nxt.shape or prev.ndim != 3:
+        raise ValueError("every pair must be two equal-sized 2-D uint8 arrays of one frame size")
+    ctx = get_context()
+    n, h, w = prev.shape
+    pov = bool(config.get("pov_mode"))
+    apply_farneback(ctx, config)
+    ctx.configure(w, h, _pairs_batch(w, h, n), n)
+    r = ctx.farneback_pairs(prev, nxt, pov=pov, cut_threshold=float(config.get("cut_threshold", DEFAULT_CUT_THRESHOLD)))
+    out = []
+    for i in range(n):
+        if pov:   # F:882: plain Python ints and the int 0
+            pos_center, val = (w // 2, h - 1), 0
+        else:     # F:757-758: NumPy integer / float32 scalars
+            pos_center, val = (np.int64(r["cx"][i]), np.int64(r["cy"][i])), np.float32(r["val"][i])
+        out.append({
+            "flow": r["flow"][i],
+            "pos_center": pos_center,
+            "neg_center": pos_center,
+            "val_pos": val,
+            "val_neg": val,
+            "cut": bool(r["cut"][i]),
+            "cut_center": pos_center[0],
+            "mean_mag": np.float32(r["mean_mag"][i]),
+        })
+    return out
 
 
 def precompute_flow_info_gpu(p0: np.ndarray, p1: np.ndarray, cut_threshold) -> Dict:

@@ -3,7 +3,8 @@
 // One context = one GPU = one host thread.  Frames flow
 //   host (pageable | pinned) --cudaMemcpyAsync on s_copy, double-buffered--> device u8 staging
 //   --k_pyramid_pow2 | k_pyramid_level / k_polyexp--> per-frame expansion slots (ring of S = B+2 frames; each frame
-//     is expanded once and used as `next` of pair j-1 and `prev` of pair j: streaming mode)
+//     is expanded once and used as `next` of pair j-1 and `prev` of pair j: streaming mode; ffb_farneback_pairs stages
+//     independent pairs as prev_0, next_0, prev_1, ... and reads them with pair stride 2)
 //   --k_flow_iter x iterations per level (flow up-sampling fused, k_upsample_flow otherwise; winsize != 15:
 //     k_flow_matrices + k_box_solve)--> final-flow ring (>= B+8 pairs)
 //   --k_divmag / k_phase1_finish--> per-pair centre, value, mean magnitude, cut flag (device arrays)
@@ -223,6 +224,13 @@ struct ffb_ctx {
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     cudaEvent_t ev_chain = nullptr;                    // "everything queued on s_comp so far": ffb_chain_after
     cudaEvent_t ev_h2d[2] = {nullptr, nullptr}, ev_expand[2] = {nullptr, nullptr};
+    // ffb_farneback_pairs: final flows leave the final-flow ring on s_out.  ev_fin[h] / ev_out[h]: the flows of the
+    // chunk in ring half h are complete / have been copied out; ev_user / ev_done order the call after / before the
+    // caller's stream; ev_h2d_next[b]: the upload of a chunk's `next` frames through staging buffer b is done (the
+    // `prev` frames use ev_h2d[b]), so that the host stages them without waiting for the `prev` frames' DMA.
+    cudaStream_t s_out = nullptr;
+    cudaEvent_t ev_fin[2] = {nullptr, nullptr}, ev_out[2] = {nullptr, nullptr}, ev_user = nullptr, ev_done = nullptr;
+    cudaEvent_t ev_h2d_next[2] = {nullptr, nullptr};
     FarnebackParams fb;
     FfbPolyConsts<5> poly5;
     FfbPolyConsts<7> poly7;
@@ -552,9 +560,9 @@ FlowIterPlan flow_iter_plan(int frame_w, int frame_h, int w, int h, const FlowIt
     return p;
 }
 
-template <int NT, int U, int MINB, int HO>
+template <int NT, int U, int MINB, int HO, int PS>
 int launch_flow_iter_t(ffb_ctx* c, const FfbIterArgs& a, int npairs, int level, double bytes, cudaStream_t stream, bool timed) {
-    auto kfn = a.up_src ? k_flow_iter<NT, U, MINB, true, HO> : k_flow_iter<NT, U, MINB, false, HO>;
+    auto kfn = a.up_src ? k_flow_iter<NT, U, MINB, true, HO, PS> : k_flow_iter<NT, U, MINB, false, HO, PS>;
     const size_t smem = ffb_flow_iter_smem<NT, U, HO>();
     if (!c->attr_iter.count((const void*)kfn)) {
         CK(c, cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -574,11 +582,31 @@ struct UpSrc {   // coarser-level flow to be up-sampled inside the iteration ker
     const float2* src = nullptr; size_t stride = 0; int sp = 0, wc = 0, hc = 0;
 };
 
+// the k_flow_iter variant of plan `p` with pair stride PS
+template <int PS>
+int launch_flow_iter_ps(ffb_ctx* c, const FlowIterPlan& p, const FfbIterArgs& a, int npairs, int level, double bytes,
+                        cudaStream_t stream, bool timed) {
+    // compiled in: 256x4x8, 128x2x4, 160x2x4, 96x2x4, 64x2x4 (the round-2 sweeps measured and dropped 192 / 512-thread
+    // strips, 8-output tasks on 2-row steps, 4-output tasks on 4-row steps, non-allocating loads, bulk L2 prefetch, early
+    // issue of the second row pair, and a barrier-free variant in which neighbouring warps synchronise through
+    // shared-memory flags: profiles/r2_sweep_flow_iter.txt)
+    switch (p.nt * 100 + p.u * 10 + p.ho) {
+        case 25648: return launch_flow_iter_t<256, 4, 2, 8, PS>(c, a, npairs, level, bytes, stream, timed);
+        case 12824: return launch_flow_iter_t<128, 2, 4, 4, PS>(c, a, npairs, level, bytes, stream, timed);
+        case 16024: return launch_flow_iter_t<160, 2, 3, 4, PS>(c, a, npairs, level, bytes, stream, timed);
+        case 9624:  return launch_flow_iter_t<96, 2, 5, 4, PS>(c, a, npairs, level, bytes, stream, timed);
+        case 6424:  return launch_flow_iter_t<64, 2, 8, 4, PS>(c, a, npairs, level, bytes, stream, timed);
+        default: break;
+    }
+    return fail(c, FFB_E_INVALID, "FFB_ITER_CFG: no k_flow_iter variant %dx%dx%d (compiled in: 256x4x8, 128x2x4, 160x2x4, 96x2x4, 64x2x4)",
+                p.nt, p.u, p.ho);
+}
+
 // One k_flow_iter launch of plan `p` on `stream`, counted under pyramid level `level` (-1: none).  timed = false inside
-// the sliced flow phase, which is timed as a whole.
+// the sliced flow phase, which is timed as a whole.  pair_stride: 1 (bracket) or 2 (independent pairs), see k_flow_iter.
 int launch_flow_iter(ffb_ctx* c, const FlowIterPlan& p, int level, cudaStream_t stream, bool timed, FfbRing R, size_t plane,
                      int rp, int w, int h, const float2* fin, size_t fin_stride, int fip, FfbRing fout, int fop, int npairs,
-                     const UpSrc* up = nullptr) {
+                     const UpSrc* up = nullptr, int pair_stride = 1) {
     FfbIterArgs a;
     a.R = R; a.plane = (int)plane; a.rp = rp; a.w = w; a.h = h;
     a.fin = fin; a.fin_stride = fin_stride; a.fip = fip; a.fout = fout; a.fop = fop;
@@ -594,26 +622,14 @@ int launch_flow_iter(ffb_ctx* c, const FlowIterPlan& p, int level, cudaStream_t 
     // the kernel stores four flow vectors with one 32-byte instruction
     if (fop % 4 != 0 || ((uintptr_t)fout.base | (uintptr_t)fout.stride) % 32 != 0)
         return fail(c, FFB_E_INVALID, "flow output is not 32-byte aligned (pitch %d, stride %zu)", fop, fout.stride);
-    // compiled in: 256x4x8, 128x2x4, 160x2x4, 96x2x4, 64x2x4 (the round-2 sweeps measured and dropped 192 / 512-thread
-    // strips, 8-output tasks on 2-row steps, 4-output tasks on 4-row steps, non-allocating loads, bulk L2 prefetch, early
-    // issue of the second row pair, and a barrier-free variant in which neighbouring warps synchronise through
-    // shared-memory flags: profiles/r2_sweep_flow_iter.txt)
-    switch (p.nt * 100 + p.u * 10 + p.ho) {
-        case 25648: return launch_flow_iter_t<256, 4, 2, 8>(c, a, npairs, level, bytes, stream, timed);
-        case 12824: return launch_flow_iter_t<128, 2, 4, 4>(c, a, npairs, level, bytes, stream, timed);
-        case 16024: return launch_flow_iter_t<160, 2, 3, 4>(c, a, npairs, level, bytes, stream, timed);
-        case 9624:  return launch_flow_iter_t<96, 2, 5, 4>(c, a, npairs, level, bytes, stream, timed);
-        case 6424:  return launch_flow_iter_t<64, 2, 8, 4>(c, a, npairs, level, bytes, stream, timed);
-        default: break;
-    }
-    return fail(c, FFB_E_INVALID, "FFB_ITER_CFG: no k_flow_iter variant %dx%dx%d (compiled in: 256x4x8, 128x2x4, 160x2x4, 96x2x4, 64x2x4)",
-                p.nt, p.u, p.ho);
+    return pair_stride == 2 ? launch_flow_iter_ps<2>(c, p, a, npairs, level, bytes, stream, timed)
+                            : launch_flow_iter_ps<1>(c, p, a, npairs, level, bytes, stream, timed);
 }
 
 // One flow iteration with the context's winsize != 15: k_flow_matrices into the scratch M (npairs x 5 planes), then
 // k_box_solve into fout.  Same arguments, counters and output layout as launch_flow_iter.
 int launch_flow_unfused(ffb_ctx* c, int level, float* M, FfbRing R, size_t plane, int rp, int w, int h, const float2* fin,
-                        size_t fin_stride, int fip, FfbRing fout, int fop, int npairs) {
+                        size_t fin_stride, int fip, FfbRing fout, int fop, int npairs, int pair_stride = 1) {
     const int win = c->fb.winsize, r = win / 2;
     if (BOX_NT - 2 * r < 1) return fail(c, FFB_E_INVALID, "winsize %d too large for k_box_solve", win);
     FfbMatrixArgs m;
@@ -623,7 +639,9 @@ int launch_flow_unfused(ffb_ctx* c, int level, float* M, FfbRing R, size_t plane
     // algorithmic bytes: the fused kernel's reads (expansions + incoming flow) plus the matrices written (20 B/px) ...
     const double px = (double)npairs * w * h;
     const ProfMark pm = prof_begin(c, FFB_K_FLOW_ITER, level, px * ((fin ? 48.0 : 40.0) + 20.0), c->s_comp);
-    FFB_LAUNCH(k_flow_matrices, dim3((w + 31) / 32, (h + 7) / 8, npairs), dim3(256), 0, c->s_comp, m);
+    const dim3 mgrid((w + 31) / 32, (h + 7) / 8, npairs);
+    if (pair_stride == 2) FFB_LAUNCH(k_flow_matrices<2>, mgrid, dim3(256), 0, c->s_comp, m);
+    else FFB_LAUNCH(k_flow_matrices<1>, mgrid, dim3(256), 0, c->s_comp, m);
     prof_end(pm);
     CKL(c);
     FfbBoxArgs b;
@@ -723,6 +741,7 @@ int quiesce(ffb_ctx* c) {
     CK(c, cudaStreamSynchronize(c->s_comp));
     CK(c, cudaStreamSynchronize(c->s_copy));
     CK(c, cudaStreamSynchronize(c->s_aux));
+    CK(c, cudaStreamSynchronize(c->s_out));
     return FFB_OK;
 }
 
@@ -904,8 +923,10 @@ int launch_divmag(ffb_ctx* c, int p0, int off, int cnt, cudaStream_t stream) {
     return FFB_OK;
 }
 
-// Final flows of bracket pairs [p0, p0 + np) into the ring, and their divergence / magnitude partials.
-int flow_pairs(ffb_ctx* c, int p0, int np) {
+// Final flows of np pairs into final-flow ring slots f0 .. (mod ring_n), and their divergence / magnitude partials.
+// Pair j reads the expansions in slots r0 + pair_stride * j and the one after it (mod S): bracket pairs [p0, p0 + np)
+// are r0 = f0 = p0 with stride 1, a chunk of independent pairs r0 = 0 with stride 2.
+int flow_pairs(ffb_ctx* c, int r0, int pair_stride, int f0, int np) {
     // The pairs of a batch are split in two slices whose launch chains run on two streams, so that the short
     // coarse-level launches (and the tail of every launch) of one slice overlap the other slice's work (+4 %; 3-4 slices
     // measured no better).  Every buffer is indexed by pair; the slices share nothing that is written.
@@ -946,11 +967,11 @@ int flow_pairs(ffb_ctx* c, int p0, int np) {
                 FfbRing R;
                 R.base = (char*)(c->R + L.r_off);
                 R.stride = c->r_slot_floats * sizeof(float);
-                R.first = (p0 + off) % c->S;
+                R.first = (r0 + pair_stride * off) % c->S;
                 R.mod = c->S;
                 FfbRing toB{(char*)(L.fB + (size_t)off * fstride), fstride * sizeof(float2), 0, 1 << 30};
                 FfbRing toA{(char*)(L.fA + (size_t)off * fstride), fstride * sizeof(float2), 0, 1 << 30};
-                FfbRing toRing{(char*)c->ring, c->ring_stride * sizeof(float2), (p0 + off) % c->ring_n, c->ring_n};
+                FfbRing toRing{(char*)c->ring, c->ring_stride * sizeof(float2), (f0 + off) % c->ring_n, c->ring_n};
                 UpSrc up;
                 if (l > 0 && fuse_up) {
                     Level& C = c->lev[l - 1];
@@ -964,9 +985,10 @@ int flow_pairs(ffb_ctx* c, int p0, int np) {
                 const FfbRing& fout = it == iters - 1 && last ? toRing : (it % 2 == 0 ? toB : toA);
                 if (fused)
                     TRY(launch_flow_iter(c, L.iter, L.k, streams[sl], !sliced, R, L.plane, L.rp, L.w, L.h, fin, fstride, L.fp,
-                                         fout, L.fp, cnt, it == 0 ? &up : nullptr));
+                                         fout, L.fp, cnt, it == 0 ? &up : nullptr, pair_stride));
                 else
-                    TRY(launch_flow_unfused(c, L.k, c->M, R, L.plane, L.rp, L.w, L.h, fin, fstride, L.fp, fout, L.fp, cnt));
+                    TRY(launch_flow_unfused(c, L.k, c->M, R, L.plane, L.rp, L.w, L.h, fin, fstride, L.fp, fout, L.fp, cnt,
+                                            pair_stride));
             }
         }
     }
@@ -975,7 +997,7 @@ int flow_pairs(ffb_ctx* c, int p0, int np) {
         prof_phase_end(c, phase, nslice);
     }
     // each slice reduces its own pairs as soon as its chain is done (overlaps the other slice's tail)
-    for (int sl = 0; sl < nslice; ++sl) TRY(launch_divmag(c, p0, soff[sl], soff[sl + 1] - soff[sl], streams[sl]));
+    for (int sl = 0; sl < nslice; ++sl) TRY(launch_divmag(c, f0, soff[sl], soff[sl + 1] - soff[sl], streams[sl]));
     if (sliced) {
         CK(c, cudaEventRecord(c->ev_join, c->s_aux));
         CK(c, cudaStreamWaitEvent(c->s_comp, c->ev_join, 0));
@@ -983,13 +1005,14 @@ int flow_pairs(ffb_ctx* c, int p0, int np) {
     return FFB_OK;
 }
 
-// per-pair centre, value, mean magnitude and cut flag of pairs [p0, p0 + np) from their divergence / magnitude partials
-int launch_phase1_finish(ffb_ctx* c, int p0, int np, int pov, float cut_threshold) {
+// per-pair centre, value, mean magnitude and cut flag of the np pairs in final-flow ring slots f0 .. from their
+// divergence / magnitude partials, into the per-pair arrays at out0 ..
+int launch_phase1_finish(ffb_ctx* c, int f0, int out0, int np, int pov, float cut_threshold) {
     FfbP1Args f;
-    f.flow = FfbRing{(char*)c->ring, c->ring_stride * sizeof(float2), p0 % c->ring_n, c->ring_n};
+    f.flow = FfbRing{(char*)c->ring, c->ring_stride * sizeof(float2), f0 % c->ring_n, c->ring_n};
     f.fp = c->fp0; f.w = c->W; f.h = c->H;
     f.pkey = c->d_pkey; f.psum = c->d_psum; f.nblk = c->div_nblk;
-    f.pov = pov; f.cut_threshold = cut_threshold; f.out0 = p0;
+    f.pov = pov; f.cut_threshold = cut_threshold; f.out0 = out0;
     f.cx = c->d_cx; f.cy = c->d_cy; f.val = c->d_val; f.mean_mag = c->d_mm; f.cut = c->d_cut;
     const ProfMark pm = prof_begin(c, FFB_K_SMALL, -1, 0, c->s_comp);
     FFB_LAUNCH(k_phase1_finish, dim3(np), dim3(32), 0, c->s_comp, f);
@@ -1064,35 +1087,41 @@ void copy_frames(uint8_t* dst, size_t dst_frame, const uint8_t* src, size_t src_
 }
 
 enum PtrKind { PTR_PAGEABLE, PTR_PINNED, PTR_DEVICE };
-PtrKind classify(const void* p) {
+// `device`: where a device pointer lives
+PtrKind classify(const void* p, int* device = nullptr) {
     cudaPointerAttributes at;
     if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
         cudaGetLastError();
         return PTR_PAGEABLE;
     }
+    if (device) *device = at.device;
     if (at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged) return PTR_DEVICE;
     if (at.type == cudaMemoryTypeHost) return PTR_PINNED;
     return PTR_PAGEABLE;
 }
 
-// H2D on s_copy of n host frames (`rows` rows of `row` bytes, `pitch` bytes apart; frames `stride` bytes apart) into
-// the dense device buffer `dst`, which the kernels before `ev_consumer` read.  Pinned input is copied directly,
-// pageable input through the pinned staging buffer `pin`.  `ev_dma` marks the end of the copy (and so the end of
-// the last DMA out of `pin`); s_comp waits for it.
+// Copy on s_copy of n frames (`rows` rows of `row` bytes, `pitch` bytes apart; frames `stride` bytes apart) into the
+// device buffer `dst` (frames dst_frame bytes apart; 0: dense), which the kernels before `ev_consumer` read.  Pinned
+// and device input is copied directly, pageable input through the pinned staging buffer `pin` (same layout as dst).
+// `ev_dma` marks the end of the copy (and so the end of the last DMA out of `pin`); s_comp waits for it.
 int upload_frames(ffb_ctx* c, uint8_t* dst, uint8_t* pin, cudaEvent_t ev_dma, cudaEvent_t ev_consumer, const uint8_t* src,
-                  PtrKind kind, int n, int rows, size_t row, size_t pitch, size_t stride) {
+                  PtrKind kind, int n, int rows, size_t row, size_t pitch, size_t stride, size_t dst_frame = 0) {
     const size_t fbytes = row * rows;
+    if (dst_frame == 0) dst_frame = fbytes;
+    const cudaMemcpyKind dir = kind == PTR_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
     CK(c, cudaStreamWaitEvent(c->s_copy, ev_consumer, 0));
     if (kind == PTR_PAGEABLE) {
         CK(c, cudaEventSynchronize(ev_dma));
-        copy_frames(pin, fbytes, src, stride, pitch, n, rows, row);
-        CK(c, cudaMemcpyAsync(dst, pin, (size_t)n * fbytes, cudaMemcpyHostToDevice, c->s_copy));
-    } else if (pitch == row && stride == fbytes) {
-        CK(c, cudaMemcpyAsync(dst, src, (size_t)n * fbytes, cudaMemcpyHostToDevice, c->s_copy));
+        copy_frames(pin, dst_frame, src, stride, pitch, n, rows, row);
+        if (dst_frame == fbytes) CK(c, cudaMemcpyAsync(dst, pin, (size_t)n * fbytes, cudaMemcpyHostToDevice, c->s_copy));
+        else CK(c, cudaMemcpy2DAsync(dst, dst_frame, pin, dst_frame, fbytes, n, cudaMemcpyHostToDevice, c->s_copy));
+    } else if (pitch == row && stride == fbytes && dst_frame == fbytes) {
+        CK(c, cudaMemcpyAsync(dst, src, (size_t)n * fbytes, dir, c->s_copy));
+    } else if (pitch == row && stride >= fbytes) {     // whole frames as the rows of one 2-D copy
+        CK(c, cudaMemcpy2DAsync(dst, dst_frame, src, stride, fbytes, n, dir, c->s_copy));
     } else {
         for (int f = 0; f < n; ++f)
-            CK(c, cudaMemcpy2DAsync(dst + (size_t)f * fbytes, row, src + (size_t)f * stride, pitch, row, rows,
-                                    cudaMemcpyHostToDevice, c->s_copy));
+            CK(c, cudaMemcpy2DAsync(dst + (size_t)f * dst_frame, row, src + (size_t)f * stride, pitch, row, rows, dir, c->s_copy));
     }
     CK(c, cudaEventRecord(ev_dma, c->s_copy));
     CK(c, cudaStreamWaitEvent(c->s_comp, ev_dma, 0));
@@ -1122,8 +1151,8 @@ int process_batch(ffb_ctx* c, const uint8_t* frames, int nb, size_t pitch, size_
         if (p0 + np > c->maxPairs) return fail(c, FFB_E_INVALID, "bracket exceeds max_bracket_pairs=%d", c->maxPairs);
         if (c->deferred && p0 + np > c->ring_n)
             return fail(c, FFB_E_INVALID, "shard exceeds the %d pairs announced to ffb_bracket_begin_shard", c->ring_n);
-        TRY(flow_pairs(c, p0, np));
-        TRY(launch_phase1_finish(c, p0, np, c->pov, c->thr));
+        TRY(flow_pairs(c, p0, 1, p0, np));
+        TRY(launch_phase1_finish(c, p0, p0, np, c->pov, c->thr));
         c->pairs_done += np;
         const int r1 = c->pairs_done - 6;
         if (!c->deferred && r1 > c->radial_done) {
@@ -1281,6 +1310,10 @@ int ffb_create(int device, ffb_ctx** out) {
     for (int i = 0; i < 2; ++i) cudaEventCreateWithFlags(&c->ev_flow_end[i], cudaEventDisableTiming);
     cudaStreamCreateWithFlags(&c->s_aux, cudaStreamNonBlocking);
     cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming);
+    cudaStreamCreateWithFlags(&c->s_out, cudaStreamNonBlocking);
+    for (cudaEvent_t* e : {&c->ev_fin[0], &c->ev_fin[1], &c->ev_out[0], &c->ev_out[1], &c->ev_user, &c->ev_done,
+                           &c->ev_h2d_next[0], &c->ev_h2d_next[1]})
+        cudaEventCreateWithFlags(e, cudaEventDisableTiming);
     // FFB_FLOW_STREAMS=1: one launch chain for the flow phase, so that bench.py can time its launches one by one
     if (const char* e = getenv("FFB_FLOW_STREAMS")) c->flow_streams = atoi(e);
     // FFB_ITER_CFG=NTxUxHO forces one k_flow_iter variant on every level (the CPU tests run each variant on small frames)
@@ -1309,6 +1342,7 @@ void ffb_destroy(ffb_ctx* c) {
     cudaSetDevice(c->device);
     cudaStreamSynchronize(c->s_comp);
     cudaStreamSynchronize(c->s_copy);
+    cudaStreamSynchronize(c->s_out);
     prof_collect(c);
     for (cudaEvent_t e : c->ev_pool) cudaEventDestroy(e);
     for (cudaEvent_t e : c->timers) if (e) cudaEventDestroy(e);
@@ -1324,6 +1358,10 @@ void ffb_destroy(ffb_ctx* c) {
     cudaStreamDestroy(c->s_time);
     cudaEventDestroy(c->ev_join);
     cudaStreamDestroy(c->s_aux);
+    for (cudaEvent_t e : {c->ev_fin[0], c->ev_fin[1], c->ev_out[0], c->ev_out[1], c->ev_user, c->ev_done, c->ev_h2d_next[0],
+                          c->ev_h2d_next[1]})
+        cudaEventDestroy(e);
+    cudaStreamDestroy(c->s_out);
     cudaStreamDestroy(c->s_comp);
     cudaStreamDestroy(c->s_copy);
     delete c;
@@ -1648,6 +1686,100 @@ int ffb_farneback(ffb_ctx* c, const uint8_t* prev, const uint8_t* next, int w, i
     return ffb_bracket_get_flow(c, 0, flow);
 }
 
+// Independent pairs: chunks of P = (B + 1) / 2 pairs.  A chunk stages its 2P frames as prev_0, next_0, prev_1, ... in
+// the frame staging buffer and expands them into expansion slots 0 .. 2P-1; the flow phase reads them with pair stride
+// 2.  Consecutive chunks alternate between the final-flow ring slots [0, P) and [P, 2P) (ring_n >= B + 8 > 2P), so the
+// copy-out of one chunk on s_out overlaps the next chunk's kernels.
+int ffb_farneback_pairs(ffb_ctx* c, const uint8_t* prev, const uint8_t* next, int n_pairs, int width, int height,
+                        size_t pitch, size_t frame_stride, float* flow, size_t flow_pitch, size_t flow_stride,
+                        int pov_mode, double cut_threshold, int32_t* cx, int32_t* cy, float* val, float* mean_mag,
+                        uint8_t* cut, void* stream) {
+    if (!c) return FFB_E_INVALID;
+    if (c->in_bracket) return fail(c, FFB_E_INVALID, "ffb_farneback_pairs inside a bracket");
+    if (n_pairs < 0) return fail(c, FFB_E_INVALID, "ffb_farneback_pairs: n_pairs %d < 0", n_pairs);
+    if (n_pairs == 0) return FFB_OK;
+    if (!prev || !next || width < 1 || height < 1)
+        return fail(c, FFB_E_INVALID, "ffb_farneback_pairs: bad frames (%dx%d)", width, height);
+    if (pitch < (size_t)width) return fail(c, FFB_E_INVALID, "ffb_farneback_pairs: pitch %zu below the width %d", pitch, width);
+    if (n_pairs > 1 && frame_stride < pitch * (size_t)(height - 1) + width)
+        return fail(c, FFB_E_INVALID, "ffb_farneback_pairs: frame_stride %zu shorter than a frame", frame_stride);
+    if (flow && flow_pitch < (size_t)width * 8)
+        return fail(c, FFB_E_INVALID, "ffb_farneback_pairs: flow_pitch %zu below 8 * width (%d)", flow_pitch, 8 * width);
+    if (flow && n_pairs > 1 && flow_stride < flow_pitch * (size_t)(height - 1) + (size_t)width * 8)
+        return fail(c, FFB_E_INVALID, "ffb_farneback_pairs: flow_stride %zu shorter than a flow", flow_stride);
+    CK(c, cudaSetDevice(c->device));
+    int dev[3] = {c->device, c->device, c->device};
+    const PtrKind kp = classify(prev, &dev[0]), kn = classify(next, &dev[1]);
+    const PtrKind kf = flow ? classify(flow, &dev[2]) : PTR_DEVICE;
+    const PtrKind kinds[3] = {kp, kn, kf};
+    for (int i = 0; i < 3; ++i)
+        if (kinds[i] == PTR_DEVICE && dev[i] != c->device)
+            return fail(c, FFB_E_INVALID, "ffb_farneback_pairs: %s is on device %d, the context on device %d",
+                        i == 0 ? "prev" : (i == 1 ? "next" : "flow"), dev[i], c->device);
+    const bool stats = cx || cy || val || mean_mag || cut;
+    // the per-pair results of the whole call stay on the device until the end: max_pairs covers n_pairs
+    const int maxPairs = stats && n_pairs > c->maxPairs ? n_pairs : (c->maxPairs > 0 ? c->maxPairs : 1);
+    TRY(configure_checked(c, width, height, c->B > 0 ? c->B : 2, maxPairs, 0));
+    const int P = (c->B + 1) / 2;
+    const size_t fbytes = (size_t)width * height;
+    const cudaStream_t us = (cudaStream_t)stream;
+    c->pairs_done = 0;   // the final-flow ring no longer holds a bracket's flows
+    CK(c, cudaEventRecord(c->ev_user, us));
+    CK(c, cudaStreamWaitEvent(c->s_copy, c->ev_user, 0));
+    CK(c, cudaStreamWaitEvent(c->s_comp, c->ev_user, 0));
+    // flows of pairs [i0, i0 + np) from ring half `half` to the caller's buffer
+    auto copy_out = [&](int i0, int np, int half) -> int {
+        CK(c, cudaStreamWaitEvent(c->s_out, c->ev_fin[half], 0));
+        const cudaMemcpyKind dir = kf == PTR_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+        const float2* src = c->ring + (size_t)half * P * c->ring_stride;
+        char* dst = (char*)flow + (size_t)i0 * flow_stride;
+        const size_t row = (size_t)width * 8, spitch = (size_t)c->fp0 * 8;
+        if (flow_stride == flow_pitch * height)     // the pairs' rows are evenly spaced on both sides
+            CK(c, cudaMemcpy2DAsync(dst, flow_pitch, src, spitch, row, (size_t)np * height, dir, c->s_out));
+        else
+            for (int j = 0; j < np; ++j)
+                CK(c, cudaMemcpy2DAsync(dst + (size_t)j * flow_stride, flow_pitch, src + (size_t)j * c->ring_stride, spitch, row,
+                                        height, dir, c->s_out));
+        CK(c, cudaEventRecord(c->ev_out[half], c->s_out));
+        return FFB_OK;
+    };
+    int pend_i0 = -1, pend_np = 0, pend_half = 0;   // chunk whose copy-out has not been issued yet
+    for (int i0 = 0, k = 0; i0 < n_pairs; i0 += P, ++k) {
+        const int np = n_pairs - i0 < P ? n_pairs - i0 : P, half = k & 1, b = c->batch_no & 1;
+        const size_t off = (size_t)i0 * frame_stride;
+        TRY(upload_frames(c, c->d_u8[b], c->h_pin[b], c->ev_h2d[b], c->ev_expand[b], prev + off, kp, np, height,
+                          (size_t)width, pitch, frame_stride, 2 * fbytes));
+        TRY(upload_frames(c, c->d_u8[b] + fbytes, c->h_pin[b] + fbytes, c->ev_h2d_next[b], c->ev_expand[b], next + off, kn, np,
+                          height, (size_t)width, pitch, frame_stride, 2 * fbytes));
+        TRY(expand_frames(c, c->d_u8[b], fbytes, width, 2 * np, 0));
+        CK(c, cudaEventRecord(c->ev_expand[b], c->s_comp));
+        c->batch_no++;
+        // ring half `half` is free once the copy-out of chunk k - 2 (or of an earlier call) has read it
+        CK(c, cudaStreamWaitEvent(c->s_comp, c->ev_out[half], 0));
+        TRY(flow_pairs(c, 0, 2, half * P, np));
+        if (stats) TRY(launch_phase1_finish(c, half * P, i0, np, pov_mode ? 1 : 0, (float)cut_threshold));
+        if (!flow) continue;
+        CK(c, cudaEventRecord(c->ev_fin[half], c->s_comp));
+        // issued one chunk late: a copy into pageable memory returns only when it is done
+        if (pend_i0 >= 0) TRY(copy_out(pend_i0, pend_np, pend_half));
+        pend_i0 = i0; pend_np = np; pend_half = half;
+    }
+    if (pend_i0 >= 0) TRY(copy_out(pend_i0, pend_np, pend_half));
+    if (flow) {   // later work of the context (a bracket, the next call) overwrites the ring after the copy-out
+        CK(c, cudaEventRecord(c->ev_done, c->s_out));
+        CK(c, cudaStreamWaitEvent(c->s_comp, c->ev_done, 0));
+    }
+    // s_comp has waited for every upload and copy-out: the caller's stream continues when the inputs have been read
+    // and the flows written
+    CK(c, cudaEventRecord(c->ev_done, c->s_comp));
+    CK(c, cudaStreamWaitEvent(us, c->ev_done, 0));
+    const bool host_io = kp != PTR_DEVICE || kn != PTR_DEVICE || kf != PTR_DEVICE || stats;
+    if (stream && !host_io) return FFB_OK;
+    if (stats) return fetch_results(c, n_pairs, false, nullptr, cut, cx, cy, val, mean_mag, nullptr);
+    CK(c, cudaStreamSynchronize(c->s_comp));
+    return FFB_OK;
+}
+
 static int upload_flow(ffb_ctx* c, const float* flow, int w, int h) {
     TRY(ensure_config(c, w, h));
     if (c->in_bracket) return fail(c, FFB_E_INVALID, "per-call function inside a bracket");
@@ -1661,7 +1793,7 @@ static int flow_stats(ffb_ctx* c, const float* flow, int w, int h, int32_t* x, i
     CK(c, cudaSetDevice(c->device));
     TRY(upload_flow(c, flow, w, h));
     TRY(launch_divmag(c, 0, 0, 1, c->s_comp));
-    TRY(launch_phase1_finish(c, 0, 1, 0, std::numeric_limits<float>::infinity()));
+    TRY(launch_phase1_finish(c, 0, 0, 1, 0, std::numeric_limits<float>::infinity()));
     int hx = 0, hy = 0;
     float hv = 0, hm = 0;
     CK(c, cudaMemcpyAsync(&hx, c->d_cx, 4, cudaMemcpyDeviceToHost, c->s_comp));

@@ -601,7 +601,7 @@ __global__ void __launch_bounds__(256) k_update_matrices(FfbMatArgs a) {
 // Warps whose 32 columns lie entirely beyond the strip's last needed column (the last strip of a level,
 // narrow levels) skip the gather and the vertical sums; they only meet the barriers.
 struct FfbIterArgs {
-    FfbRing R;              // frame expansions: pair j uses elements j (prev) and j+1 (next)
+    FfbRing R;              // frame expansions: pair j uses elements PS*j (prev) and PS*j + 1 (next)
     int plane; int rp; int w, h;                     // plane = rp * h floats (< 2^31 / 5)
     const float2* fin; size_t fin_stride; int fip;   // flow in (NULL = zero), strides in float2
     FfbRing fout; int fop;                           // flow out ring (element j), pitch in float2
@@ -737,7 +737,9 @@ __device__ __forceinline__ float2 ffb_solve(float s0, float s1, float s2, float 
     return o;
 }
 
-template <int NT, int U, int MINB, bool UP2X, int HO>
+// PS (pair stride): pair j reads the expansions in ring elements PS*j and PS*j + 1.  1: consecutive frames of a bracket
+// (frame j+1 is `next` of pair j and `prev` of pair j+1); 2: independent pairs, staged as prev_0, next_0, prev_1, ...
+template <int NT, int U, int MINB, bool UP2X, int HO, int PS>
 __global__ void __launch_bounds__(NT, MINB) k_flow_iter(FfbIterArgs a) {
     static_assert(HO == 4 || HO == 8, "outputs per horizontal task");
     static_assert(U == 2 || U == 4, "rows per step");
@@ -750,8 +752,8 @@ __global__ void __launch_bounds__(NT, MINB) k_flow_iter(FfbIterArgs a) {
     RingT ring = reinterpret_cast<RingT>(smem_f + NB * U * HL::RSTRIDE);   // [FFB_WIN][5][NT]
     const int tid = threadIdx.x;
     const int pair = blockIdx.x;      // fastest-varying: see the launcher
-    const float4* A0 = reinterpret_cast<const float4*>(ffb_ring_at(a.R, pair));
-    const float4* A1 = reinterpret_cast<const float4*>(ffb_ring_at(a.R, pair + 1));
+    const float4* A0 = reinterpret_cast<const float4*>(ffb_ring_at(a.R, PS * pair));
+    const float4* A1 = reinterpret_cast<const float4*>(ffb_ring_at(a.R, PS * pair + 1));
     const float* B0 = reinterpret_cast<const float*>(A0 + a.plane);
     const float* B1 = reinterpret_cast<const float*>(A1 + a.plane);
     const float2* fin = a.fin ? a.fin + (size_t)pair * a.fin_stride : nullptr;
@@ -985,13 +987,14 @@ struct FfbMatrixArgs {
     float* M; size_t m_stride;                       // per pair: 5 planes of `plane` floats
 };
 
+template <int PS>   // pair stride, as k_flow_iter's
 __global__ void __launch_bounds__(256) k_flow_matrices(FfbMatrixArgs a) {
     const int x = blockIdx.x * 32 + (threadIdx.x & 31);
     const int y = blockIdx.y * 8 + (threadIdx.x >> 5);
     if (x >= a.w || y >= a.h) return;
     const int pair = blockIdx.z;
-    const float4* A0 = reinterpret_cast<const float4*>(ffb_ring_at(a.R, pair));
-    const float4* A1 = reinterpret_cast<const float4*>(ffb_ring_at(a.R, pair + 1));
+    const float4* A0 = reinterpret_cast<const float4*>(ffb_ring_at(a.R, PS * pair));
+    const float4* A1 = reinterpret_cast<const float4*>(ffb_ring_at(a.R, PS * pair + 1));
     const float* B0 = reinterpret_cast<const float*>(A0 + a.plane);
     const float* B1 = reinterpret_cast<const float*>(A1 + a.plane);
     const float2 d = a.fin ? __ldg(a.fin + (size_t)pair * a.fin_stride + (size_t)y * a.fip + x) : make_float2(0.f, 0.f);

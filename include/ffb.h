@@ -168,6 +168,26 @@ int  ffb_mean_magnitude(ffb_ctx* ctx, const float* flow_hw2, int width, int heig
 int  ffb_radial_motion(ffb_ctx* ctx, const float* flow_hw2, int width, int height,
                        double cx, double cy, int is_cut, int pov_mode, double* out);
 
+/* ---- independent pairs: ffb_farneback for n pairs in one call, through the batched launch chains of a bracket ----
+ * Independent pairs (prev + i*frame_stride, next + i*frame_stride), i < n_pairs, uint8 width x height, the context's
+ * Farneback parameters.  Outputs may be NULL: flow [n][height][width][2] at flow + i*flow_stride (rows flow_pitch bytes
+ * apart); cx, cy, val (max_divergence or the POV shortcut), mean_mag, cut (mean |flow| > cut_threshold) per pair.
+ *
+ * prev, next and flow may each be pageable host, pinned host or device memory (of the context's device); the per-pair
+ * outputs are host arrays.  Every pair's flow is bit-identical to ffb_farneback on that pair.  Pairs run in chunks of
+ * (batch_frames + 1) / 2; the call configures the frame size incrementally (the current batch_frames, 2 on a new
+ * context; max_pairs grows to n_pairs when a per-pair output is requested).  There is no +-6 centre smoothing and no
+ * radial scalar: those are defined along a bracket only.  The flows of an earlier bracket are no longer resident.
+ * stream: a cudaStream_t or NULL.  Non-NULL: the work starts after what is queued on `stream`, and `stream` waits
+ * until the inputs have been read and the flow written; with every buffer on the device and no per-pair output the
+ * call returns without waiting for the device.  NULL, or any host buffer: the call returns when the outputs are
+ * complete.  FFB_E_INVALID inside a bracket, for n_pairs < 0, pitch < width, flow_pitch < 8 * width, strides shorter
+ * than a frame, and a device pointer on another device; n_pairs == 0 does nothing. */
+int  ffb_farneback_pairs(ffb_ctx* ctx, const uint8_t* prev, const uint8_t* next, int n_pairs, int width, int height,
+                         size_t pitch, size_t frame_stride, float* flow, size_t flow_pitch, size_t flow_stride,
+                         int pov_mode, double cut_threshold, int32_t* cx, int32_t* cy, float* val, float* mean_mag,
+                         uint8_t* cut, void* stream);
+
 /* ---- per-stage hooks (each runs exactly the production kernel of that stage, for the context's parameters) -----
  * Level geometry of the Farneback pyramid for a frame size with the reference's pyr_scale 0.5, levels 3 (coarsest
  * level first): fills up to 4 entries of w[], h[], ksize[], sigma[]; returns the level count in *n_levels. */
