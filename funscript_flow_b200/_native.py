@@ -66,6 +66,8 @@ def load(path: Optional[str] = None) -> C.CDLL:
         "ffb_farneback": (i32, [vp, u8p, u8p, i32, i32, sz, f32p]),
         "ffb_farneback_pairs": (i32, [vp, vp, vp, i32, i32, i32, sz, sz, vp, sz, sz, i32, C.c_double, i32p, i32p, f32p, f32p,
                                       u8p, vp]),
+        "ffb_farneback_sequence": (i32, [vp, vp, i32, i32, i32, sz, sz, vp, sz, sz, i32, C.c_double, f64p, u8p, i32p, i32p,
+                                         f32p, f32p, f64p, vp]),
         "ffb_max_divergence": (i32, [vp, f32p, i32, i32, i32p, i32p, f32p]),
         "ffb_mean_magnitude": (i32, [vp, f32p, i32, i32, f32p]),
         "ffb_radial_motion": (i32, [vp, f32p, i32, i32, C.c_double, C.c_double, i32, i32, f64p]),
@@ -430,6 +432,59 @@ class FlowContext:
             return None
         res = {k: v[:n] for k, v in res.items()}
         res["cut"] = res["cut"].astype(bool)
+        res["flow"] = flow_arr
+        return res
+
+    def farneback_sequence(self, frames: np.ndarray, *, flow: bool = True, stats: bool = False, pov: bool = False,
+                           cut_threshold: float = float("inf")) -> dict:
+        """The n - 1 pairs of consecutive frames of uint8 [n, H, W] in one call (ffb_farneback_sequence), each frame
+        expanded once: {"flow": f32 [n - 1, H, W, 2]} (None with flow=False).  Each flow is bit-identical to
+        farneback(frames[j], frames[j + 1]).  stats=True adds bracket_finish's per-pair arrays (scalar, cut, cx, cy, val,
+        mean_mag, centers, n_pairs), bit-identical to a bracket of these frames with pov / cut_threshold.  Batches are
+        those of the last configure(); a context never configured runs batches of 2 frames, so configure it first
+        (api.calc_optical_flow_farneback_sequence does)."""
+        frames = np.ascontiguousarray(frames, dtype=np.uint8)
+        if frames.ndim != 3:
+            raise ValueError(f"farneback_sequence: frames must be uint8 [n, H, W], not {frames.shape}")
+        n, h, w = frames.shape
+        out = np.empty((max(n - 1, 0), h, w, 2), np.float32) if flow else None
+        res = self.farneback_sequence_ptr(frames.ctypes.data, n, w, h, w, w * h, out, stats=stats, pov=pov,
+                                          cut_threshold=cut_threshold)
+        return res if stats else {"flow": out}
+
+    def farneback_sequence_ptr(self, frames_ptr: int, n_frames: int, width: int, height: int, pitch: int,
+                               frame_stride: int, flow=None, flow_pitch: int = 0, flow_stride: int = 0, stream: int = 0, *,
+                               stats: bool = False, pov: bool = False, cut_threshold: float = float("inf")):
+        """Raw-pointer variant of farneback_sequence, like farneback_pairs_ptr: frames anywhere (e.g.
+        torch_tensor.data_ptr()), `flow` a pointer (int; 0 = no flow) or a float32 NumPy array [n_frames - 1, H, W, 2],
+        `stream` a cudaStream_t handle (0 = none).  stats=True returns the per-pair dict with "flow" (then the call waits
+        for the device), otherwise None."""
+        n = max(int(n_frames) - 1, 0)
+        flow_arr = flow if isinstance(flow, np.ndarray) else None
+        if flow_arr is not None:
+            assert flow_arr.dtype == np.float32 and flow_arr.flags.c_contiguous and flow_arr.shape == (n, height, width, 2)
+            flow_ptr, flow_pitch, flow_stride = flow_arr.ctypes.data, width * 8, width * height * 8
+        else:
+            flow_ptr = int(flow or 0)
+        res = None
+        args = [None] * 7
+        if stats:
+            m = max(n, 1)
+            res = dict(scalar=np.empty(m, np.float64), cut=np.empty(m, np.uint8), cx=np.empty(m, np.int32),
+                       cy=np.empty(m, np.int32), val=np.empty(m, np.float32), mean_mag=np.empty(m, np.float32),
+                       centers=np.empty((m, 2), np.float64))
+            i32p, f64p = C.POINTER(C.c_int32), C.POINTER(C.c_double)
+            args = [res["scalar"].ctypes.data_as(f64p), _u8(res["cut"]), res["cx"].ctypes.data_as(i32p),
+                    res["cy"].ctypes.data_as(i32p), _f32(res["val"]), _f32(res["mean_mag"]), res["centers"].ctypes.data_as(f64p)]
+        self._ck(self._lib.ffb_farneback_sequence(self._h, C.c_void_p(frames_ptr), int(n_frames), int(width), int(height),
+                                                  int(pitch), int(frame_stride), C.c_void_p(flow_ptr or None), int(flow_pitch),
+                                                  int(flow_stride), int(bool(pov)), float(cut_threshold), *args,
+                                                  C.c_void_p(int(stream) or None)))
+        if res is None:
+            return None
+        res = {k: v[:n].copy() for k, v in res.items()}
+        res["cut"] = res["cut"].astype(bool)
+        res["n_pairs"] = n
         res["flow"] = flow_arr
         return res
 

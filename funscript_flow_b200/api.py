@@ -12,6 +12,8 @@
     calc_optical_flow_farneback_batch(prev, next, None, ...)   the same for n independent pairs ([n, H, W]; NumPy
                                                     arrays or torch CUDA tensors, which stay on the device)
     precompute_flow_info_batch(pairs, config)       [precompute_wrapper(p, config) for p in pairs] in one call
+    calc_optical_flow_farneback_sequence(frames, None, ...)    the same for every pair of consecutive frames ([n, H, W]
+                                                    -> [n - 1, H, W, 2]; each frame expanded once)
 
 Every entry point that configures a context first sets its Farneback parameters from the settings keys
 flow_pyr_scale, flow_levels, flow_winsize, flow_iterations, flow_poly_n, flow_poly_sigma (farneback_params;
@@ -21,6 +23,7 @@ plus the batched entry the GPU runner uses, because per-pair calls from forked p
 (F:1190-1191) cannot drive a GPU:
 
     process_bracket(frames, params) -> dict of per-pair arrays   (F:1188-1242 in one call)
+    process_sequence(frames, params)                the same dict plus the flow of every pair
 
 There is no CPU path here: every function raises if libffb.so or a CUDA device is missing.
 """
@@ -362,6 +365,69 @@ def calc_optical_flow_farneback_batch(prev, next, flow, pyr_scale: float, levels
     ctx.farneback_pairs_ptr(prev.data_ptr(), next.data_ptr(), n, w, h, w, w * h, out.data_ptr(), w * 8, w * h * 8,
                             torch.cuda.current_stream(prev.device).cuda_stream)
     return out
+
+
+def _sequence_batch(width: int, height: int, n_frames: int) -> int:
+    """batch_frames for a sequence of n_frames frames: the runner's batch for the frame size, no more than the
+    sequence needs (its first batch takes batch_frames + 1 frames)."""
+    from .runner import default_batch_frames
+    return max(1, min(default_batch_frames(width, height), n_frames - 1))
+
+
+def calc_optical_flow_farneback_sequence(frames, flow, pyr_scale: float, levels: int, winsize: int, iterations: int,
+                                         poly_n: int, poly_sigma: float, flags: int = 0, *,
+                                         ctx: Optional[_native.FlowContext] = None):
+    """calc_optical_flow_farneback for every pair of consecutive frames (frames[j], frames[j + 1]) in one call, cv2's
+    order after a leading frame axis: uint8 [n, H, W] -> float32 [n - 1, H, W, 2].  Each frame is expanded once (a
+    bracket), where the batch function would expand it twice.  NumPy arrays give a NumPy array.  A torch.uint8 CUDA
+    tensor on the context's device gives a tensor on that device, ordered on torch.cuda.current_stream(): the frames and
+    the flows never pass through host memory.  `flow` must be None and `flags` 0.  It (re)configures the context: this
+    frame size and the runner's batch for it (at most n - 1 frames) become its limits."""
+    if flow is not None:
+        raise ValueError("calc_optical_flow_farneback_sequence: flow must be None (an initial flow is not supported)")
+    ctx = ctx or get_context()
+    tensor = _is_torch_tensor(frames)
+    if tensor:
+        import torch
+        if frames.dtype != torch.uint8 or not frames.is_cuda:
+            raise TypeError("calc_optical_flow_farneback_sequence: a tensor must be torch.uint8 on a CUDA device")
+        if frames.device.index != ctx.device:
+            raise ValueError(f"calc_optical_flow_farneback_sequence: frames on {frames.device}, the context on cuda:{ctx.device}")
+    else:
+        frames = np.asarray(frames)
+        if frames.dtype != np.uint8:
+            raise TypeError("calc_optical_flow_farneback_sequence: frames must be uint8")
+    if frames.ndim != 3:
+        raise ValueError(f"calc_optical_flow_farneback_sequence: frames must be [n, H, W], not {tuple(frames.shape)}")
+    ctx.set_farneback(pyr_scale, levels, winsize, iterations, poly_n, poly_sigma, flags)
+    n, h, w = frames.shape
+    if n < 2:
+        shape = (0, h, w, 2)
+        return torch.empty(shape, dtype=torch.float32, device=frames.device) if tensor else np.empty(shape, np.float32)
+    ctx.configure(w, h, _sequence_batch(w, h, n), 1)
+    if not tensor:
+        return ctx.farneback_sequence(frames)["flow"]
+    frames = frames.contiguous()
+    out = torch.empty((n - 1, h, w, 2), dtype=torch.float32, device=frames.device)
+    ctx.farneback_sequence_ptr(frames.data_ptr(), n, w, h, w, w * h, out.data_ptr(), w * 8, w * h * 8,
+                               torch.cuda.current_stream(frames.device).cuda_stream)
+    return out
+
+
+def process_sequence(frames, params: Optional[Dict] = None, *, ctx: Optional[_native.FlowContext] = None,
+                     batch_frames: int = DEFAULT_BATCH_FRAMES) -> Dict:
+    """process_bracket(frames, params) plus `flows` (f32 [N-1, H, W, 2]), the flow of every pair, in one pass: the same
+    per-pair arrays bit for bit, each flow bit-identical to calc_optical_flow_farneback on that pair."""
+    params = params or {}
+    ctx = ctx or get_context()
+    arr = _as_frames(frames)
+    n, h, w = arr.shape
+    apply_farneback(ctx, params)
+    ctx.configure(w, h, max(1, min(batch_frames, n)), max(n - 1, 1))
+    res = ctx.farneback_sequence(arr, stats=True, pov=bool(params.get("pov_mode", False)),
+                                 cut_threshold=float(params.get("cut_threshold", DEFAULT_CUT_THRESHOLD)))
+    res["flows"] = res.pop("flow")
+    return res
 
 
 def precompute_flow_info_batch(pairs, config: Dict) -> list:

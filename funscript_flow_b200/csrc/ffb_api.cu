@@ -6,7 +6,8 @@
 //     is expanded once and used as `next` of pair j-1 and `prev` of pair j: streaming mode; ffb_farneback_pairs stages
 //     independent pairs as prev_0, next_0, prev_1, ... and reads them with pair stride 2)
 //   --k_flow_iter x iterations per level (flow up-sampling fused, k_upsample_flow otherwise; winsize != 15:
-//     k_flow_matrices + k_box_solve)--> final-flow ring (>= B+8 pairs)
+//     k_flow_matrices + k_box_solve)--> final-flow ring (>= B+8 pairs; ffb_farneback_pairs and ffb_farneback_sequence
+//     copy the flows out of it on s_out, the sequence with a ring of >= 2B+8 pairs)
 //   --k_divmag / k_phase1_finish--> per-pair centre, value, mean magnitude, cut flag (device arrays)
 //   --k_smooth_centers / k_radial / k_radial_finish (lagging 6 pairs)--> per-pair scalar
 // and only the 1-D per-pair results are copied back at ffb_bracket_finish.
@@ -224,10 +225,11 @@ struct ffb_ctx {
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     cudaEvent_t ev_chain = nullptr;                    // "everything queued on s_comp so far": ffb_chain_after
     cudaEvent_t ev_h2d[2] = {nullptr, nullptr}, ev_expand[2] = {nullptr, nullptr};
-    // ffb_farneback_pairs: final flows leave the final-flow ring on s_out.  ev_fin[h] / ev_out[h]: the flows of the
-    // chunk in ring half h are complete / have been copied out; ev_user / ev_done order the call after / before the
-    // caller's stream; ev_h2d_next[b]: the upload of a chunk's `next` frames through staging buffer b is done (the
-    // `prev` frames use ev_h2d[b]), so that the host stages them without waiting for the `prev` frames' DMA.
+    // ffb_farneback_pairs / _sequence: final flows leave the final-flow ring on s_out.  ev_fin[h] / ev_out[h]: the flows
+    // of the chunk in ring half h (of the sequence batch of parity h) are complete / have been copied out; ev_user /
+    // ev_done order the call after / before the caller's stream; ev_h2d_next[b]: the upload of a chunk's `next` frames
+    // through staging buffer b is done (the `prev` frames use ev_h2d[b]), so that the host stages them without waiting
+    // for the `prev` frames' DMA.
     cudaStream_t s_out = nullptr;
     cudaEvent_t ev_fin[2] = {nullptr, nullptr}, ev_out[2] = {nullptr, nullptr}, ev_user = nullptr, ev_done = nullptr;
     cudaEvent_t ev_h2d_next[2] = {nullptr, nullptr};
@@ -923,10 +925,11 @@ int launch_divmag(ffb_ctx* c, int p0, int off, int cnt, cudaStream_t stream) {
     return FFB_OK;
 }
 
-// Final flows of np pairs into final-flow ring slots f0 .. (mod ring_n), and their divergence / magnitude partials.
-// Pair j reads the expansions in slots r0 + pair_stride * j and the one after it (mod S): bracket pairs [p0, p0 + np)
-// are r0 = f0 = p0 with stride 1, a chunk of independent pairs r0 = 0 with stride 2.
-int flow_pairs(ffb_ctx* c, int r0, int pair_stride, int f0, int np) {
+// Final flows of np pairs into final-flow ring slots f0 .. (mod ring_n), and their divergence / magnitude partials
+// (divmag = false: flows only).  Pair j reads the expansions in slots r0 + pair_stride * j and the one after it
+// (mod S): bracket pairs [p0, p0 + np) are r0 = f0 = p0 with stride 1, a chunk of independent pairs r0 = 0 with
+// stride 2.
+int flow_pairs(ffb_ctx* c, int r0, int pair_stride, int f0, int np, bool divmag = true) {
     // The pairs of a batch are split in two slices whose launch chains run on two streams, so that the short
     // coarse-level launches (and the tail of every launch) of one slice overlap the other slice's work (+4 %; 3-4 slices
     // measured no better).  Every buffer is indexed by pair; the slices share nothing that is written.
@@ -997,7 +1000,8 @@ int flow_pairs(ffb_ctx* c, int r0, int pair_stride, int f0, int np) {
         prof_phase_end(c, phase, nslice);
     }
     // each slice reduces its own pairs as soon as its chain is done (overlaps the other slice's tail)
-    for (int sl = 0; sl < nslice; ++sl) TRY(launch_divmag(c, f0, soff[sl], soff[sl + 1] - soff[sl], streams[sl]));
+    if (divmag)
+        for (int sl = 0; sl < nslice; ++sl) TRY(launch_divmag(c, f0, soff[sl], soff[sl + 1] - soff[sl], streams[sl]));
     if (sliced) {
         CK(c, cudaEventRecord(c->ev_join, c->s_aux));
         CK(c, cudaStreamWaitEvent(c->s_comp, c->ev_join, 0));
@@ -1128,7 +1132,10 @@ int upload_frames(ffb_ctx* c, uint8_t* dst, uint8_t* pin, cudaEvent_t ev_dma, cu
     return FFB_OK;
 }
 
-int process_batch(ffb_ctx* c, const uint8_t* frames, int nb, size_t pitch, size_t stride, PtrKind kind) {
+// One batch of the open bracket (or sequence): upload, expansion, final flows and, with stats, the per-pair results
+// and the radial pass lagging 6 pairs.  stats = false computes the flows only (ffb_farneback_sequence without per-pair
+// outputs): no k_divmag, phase-1 finish, centre smoothing or radial pass, and max_pairs does not bound the pairs.
+int process_batch(ffb_ctx* c, const uint8_t* frames, int nb, size_t pitch, size_t stride, PtrKind kind, bool stats = true) {
     const int b = c->batch_no & 1;
     const size_t fbytes = (size_t)c->W * c->H;
     const uint8_t* src = frames;
@@ -1148,14 +1155,14 @@ int process_batch(ffb_ctx* c, const uint8_t* frames, int nb, size_t pitch, size_
     const int np = nb - (g0 == 0 ? 1 : 0);
     if (np > 0) {
         const int p0 = c->pairs_done;
-        if (p0 + np > c->maxPairs) return fail(c, FFB_E_INVALID, "bracket exceeds max_bracket_pairs=%d", c->maxPairs);
+        if (stats && p0 + np > c->maxPairs) return fail(c, FFB_E_INVALID, "bracket exceeds max_bracket_pairs=%d", c->maxPairs);
         if (c->deferred && p0 + np > c->ring_n)
             return fail(c, FFB_E_INVALID, "shard exceeds the %d pairs announced to ffb_bracket_begin_shard", c->ring_n);
-        TRY(flow_pairs(c, p0, 1, p0, np));
-        TRY(launch_phase1_finish(c, p0, p0, np, c->pov, c->thr));
+        TRY(flow_pairs(c, p0, 1, p0, np, stats));
+        if (stats) TRY(launch_phase1_finish(c, p0, p0, np, c->pov, c->thr));
         c->pairs_done += np;
         const int r1 = c->pairs_done - 6;
-        if (!c->deferred && r1 > c->radial_done) {
+        if (stats && !c->deferred && r1 > c->radial_done) {
             TRY(radial_range(c, c->radial_done, r1, c->pairs_done));
             c->radial_done = r1;
         }
@@ -1686,6 +1693,21 @@ int ffb_farneback(ffb_ctx* c, const uint8_t* prev, const uint8_t* next, int w, i
     return ffb_bracket_get_flow(c, 0, flow);
 }
 
+// Copy on s_out of the final flows in ring slots s0 .. s0 + np - 1 (no wrap) to `dst`: flows flow_stride bytes apart,
+// rows flow_pitch bytes apart, in host memory or on the device (`kind`).
+static int copy_flows_out(ffb_ctx* c, int s0, int np, char* dst, size_t flow_pitch, size_t flow_stride, PtrKind kind) {
+    const cudaMemcpyKind dir = kind == PTR_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+    const float2* src = c->ring + (size_t)s0 * c->ring_stride;
+    const size_t row = (size_t)c->W * 8, spitch = (size_t)c->fp0 * 8;
+    if (flow_stride == flow_pitch * c->H)     // the pairs' rows are evenly spaced on both sides
+        CK(c, cudaMemcpy2DAsync(dst, flow_pitch, src, spitch, row, (size_t)np * c->H, dir, c->s_out));
+    else
+        for (int j = 0; j < np; ++j)
+            CK(c, cudaMemcpy2DAsync(dst + (size_t)j * flow_stride, flow_pitch, src + (size_t)j * c->ring_stride, spitch, row,
+                                    c->H, dir, c->s_out));
+    return FFB_OK;
+}
+
 // Independent pairs: chunks of P = (B + 1) / 2 pairs.  A chunk stages its 2P frames as prev_0, next_0, prev_1, ... in
 // the frame staging buffer and expands them into expansion slots 0 .. 2P-1; the flow phase reads them with pair stride
 // 2.  Consecutive chunks alternate between the final-flow ring slots [0, P) and [P, 2P) (ring_n >= B + 8 > 2P), so the
@@ -1730,16 +1752,7 @@ int ffb_farneback_pairs(ffb_ctx* c, const uint8_t* prev, const uint8_t* next, in
     // flows of pairs [i0, i0 + np) from ring half `half` to the caller's buffer
     auto copy_out = [&](int i0, int np, int half) -> int {
         CK(c, cudaStreamWaitEvent(c->s_out, c->ev_fin[half], 0));
-        const cudaMemcpyKind dir = kf == PTR_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
-        const float2* src = c->ring + (size_t)half * P * c->ring_stride;
-        char* dst = (char*)flow + (size_t)i0 * flow_stride;
-        const size_t row = (size_t)width * 8, spitch = (size_t)c->fp0 * 8;
-        if (flow_stride == flow_pitch * height)     // the pairs' rows are evenly spaced on both sides
-            CK(c, cudaMemcpy2DAsync(dst, flow_pitch, src, spitch, row, (size_t)np * height, dir, c->s_out));
-        else
-            for (int j = 0; j < np; ++j)
-                CK(c, cudaMemcpy2DAsync(dst + (size_t)j * flow_stride, flow_pitch, src + (size_t)j * c->ring_stride, spitch, row,
-                                        height, dir, c->s_out));
+        TRY(copy_flows_out(c, half * P, np, (char*)flow + (size_t)i0 * flow_stride, flow_pitch, flow_stride, kf));
         CK(c, cudaEventRecord(c->ev_out[half], c->s_out));
         return FFB_OK;
     };
@@ -1776,6 +1789,98 @@ int ffb_farneback_pairs(ffb_ctx* c, const uint8_t* prev, const uint8_t* next, in
     const bool host_io = kp != PTR_DEVICE || kn != PTR_DEVICE || kf != PTR_DEVICE || stats;
     if (stream && !host_io) return FFB_OK;
     if (stats) return fetch_results(c, n_pairs, false, nullptr, cut, cx, cy, val, mean_mag, nullptr);
+    CK(c, cudaStreamSynchronize(c->s_comp));
+    return FFB_OK;
+}
+
+// Consecutive pairs of a sequence: one bracket over the n_frames frames (the batches of ffb_bracket_push, with the
+// ramp for host input; every frame expanded once; flow_pairs with pair stride 1), whose final flows are also copied
+// out.  Pair p sits in final-flow ring slot p mod ring_n, and the copy-out of batch k on s_out is issued after batch
+// k + 1 has been queued, so it overlaps that batch's kernels.  With ring_n >= 2B + 8, batch k + 1 (at most B pairs)
+// writes no slot of batch k (at most B) nor of the 6 pairs before it that its radial pass still reads; the slots it
+// does overwrite held batch k - 1 or earlier, so it waits for the copy-out of batch k - 1 (ev_out[(k + 1) & 1]).  The
+// radial pass runs on s_comp, in order with every later write.
+int ffb_farneback_sequence(ffb_ctx* c, const uint8_t* frames, int n_frames, int width, int height, size_t pitch,
+                           size_t frame_stride, float* flow, size_t flow_pitch, size_t flow_stride, int pov_mode,
+                           double cut_threshold, double* scalar, uint8_t* cut, int32_t* cx, int32_t* cy, float* val,
+                           float* mean_mag, double* centers, void* stream) {
+    if (!c) return FFB_E_INVALID;
+    if (c->in_bracket) return fail(c, FFB_E_INVALID, "ffb_farneback_sequence inside a bracket");
+    if (n_frames < 0) return fail(c, FFB_E_INVALID, "ffb_farneback_sequence: n_frames %d < 0", n_frames);
+    if (n_frames < 2) return FFB_OK;
+    const int n_pairs = n_frames - 1;
+    if (!frames || width < 1 || height < 1)
+        return fail(c, FFB_E_INVALID, "ffb_farneback_sequence: bad frames (%dx%d)", width, height);
+    if (pitch < (size_t)width) return fail(c, FFB_E_INVALID, "ffb_farneback_sequence: pitch %zu below the width %d", pitch, width);
+    if (frame_stride < pitch * (size_t)(height - 1) + width)
+        return fail(c, FFB_E_INVALID, "ffb_farneback_sequence: frame_stride %zu shorter than a frame", frame_stride);
+    if (flow && flow_pitch < (size_t)width * 8)
+        return fail(c, FFB_E_INVALID, "ffb_farneback_sequence: flow_pitch %zu below 8 * width (%d)", flow_pitch, 8 * width);
+    if (flow && n_pairs > 1 && flow_stride < flow_pitch * (size_t)(height - 1) + (size_t)width * 8)
+        return fail(c, FFB_E_INVALID, "ffb_farneback_sequence: flow_stride %zu shorter than a flow", flow_stride);
+    CK(c, cudaSetDevice(c->device));
+    int dev[2] = {c->device, c->device};
+    const PtrKind kfr = classify(frames, &dev[0]);
+    const PtrKind kf = flow ? classify(flow, &dev[1]) : PTR_DEVICE;
+    if (kfr == PTR_DEVICE && dev[0] != c->device)
+        return fail(c, FFB_E_INVALID, "ffb_farneback_sequence: frames are on device %d, the context on device %d", dev[0], c->device);
+    if (kf == PTR_DEVICE && dev[1] != c->device)
+        return fail(c, FFB_E_INVALID, "ffb_farneback_sequence: flow is on device %d, the context on device %d", dev[1], c->device);
+    const bool stats = scalar || cut || cx || cy || val || mean_mag || centers;
+    // the per-pair results of the whole call stay on the device until the end: max_pairs covers n_pairs
+    const int maxPairs = stats && n_pairs > c->maxPairs ? n_pairs : (c->maxPairs > 0 ? c->maxPairs : 1);
+    const int B = c->B > 0 ? c->B : 2;
+    TRY(configure_checked(c, width, height, B, maxPairs, flow ? 2 * B + 8 : 0));
+    const cudaStream_t us = (cudaStream_t)stream;
+    // ffb_bracket_begin's state; the final-flow ring no longer holds an earlier bracket's flows
+    c->deferred = c->phase1_read = false;
+    c->pend = 0;
+    c->pov = pov_mode ? 1 : 0;
+    c->thr = (float)cut_threshold;
+    c->frames_seen = c->pairs_done = c->radial_done = 0;
+    CK(c, cudaEventRecord(c->ev_user, us));
+    CK(c, cudaStreamWaitEvent(c->s_copy, c->ev_user, 0));
+    CK(c, cudaStreamWaitEvent(c->s_comp, c->ev_user, 0));
+    // flows of pairs [p0, p0 + np) of batch parity `par` to the caller's buffer: one or two runs of ring slots
+    auto copy_out = [&](int p0, int np, int par) -> int {
+        CK(c, cudaStreamWaitEvent(c->s_out, c->ev_fin[par], 0));
+        for (int p = p0; p < p0 + np;) {
+            const int s = p % c->ring_n, m = p0 + np - p < c->ring_n - s ? p0 + np - p : c->ring_n - s;
+            TRY(copy_flows_out(c, s, m, (char*)flow + (size_t)p * flow_stride, flow_pitch, flow_stride, kf));
+            p += m;
+        }
+        CK(c, cudaEventRecord(c->ev_out[par], c->s_out));
+        return FFB_OK;
+    };
+    int k = 0, pend_p0 = 0, pend_np = 0;   // batch k - 1, whose copy-out has not been issued yet
+    for (int i = 0; i < n_frames; ++k) {
+        const int cap = batch_cap(c, kfr);
+        const int nb = n_frames - i < cap ? n_frames - i : cap;
+        const int p0 = c->pairs_done;
+        if (flow) CK(c, cudaStreamWaitEvent(c->s_comp, c->ev_out[k & 1], 0));   // copy-out of batch k - 2 done
+        TRY(process_batch(c, frames + (size_t)i * frame_stride, nb, pitch, frame_stride, kfr, stats));
+        i += nb;
+        if (!flow) continue;
+        CK(c, cudaEventRecord(c->ev_fin[k & 1], c->s_comp));
+        // issued one batch late: a copy into pageable memory returns only when it is done
+        if (pend_np > 0) TRY(copy_out(pend_p0, pend_np, (k - 1) & 1));
+        pend_p0 = p0;
+        pend_np = c->pairs_done - p0;
+    }
+    if (stats && n_pairs > c->radial_done) TRY(radial_range(c, c->radial_done, n_pairs, n_pairs));
+    if (pend_np > 0) TRY(copy_out(pend_p0, pend_np, (k - 1) & 1));
+    c->frames_seen = c->pairs_done = c->radial_done = 0;
+    if (flow) {   // later work of the context (a bracket, the next call) overwrites the ring after the copy-out
+        CK(c, cudaEventRecord(c->ev_done, c->s_out));
+        CK(c, cudaStreamWaitEvent(c->s_comp, c->ev_done, 0));
+    }
+    // s_comp has waited for every upload and copy-out: the caller's stream continues when the inputs have been read
+    // and the flows written
+    CK(c, cudaEventRecord(c->ev_done, c->s_comp));
+    CK(c, cudaStreamWaitEvent(us, c->ev_done, 0));
+    const bool host_io = kfr != PTR_DEVICE || kf != PTR_DEVICE || stats;
+    if (stream && !host_io) return FFB_OK;
+    if (stats) return fetch_results(c, n_pairs, true, scalar, cut, cx, cy, val, mean_mag, centers);
     CK(c, cudaStreamSynchronize(c->s_comp));
     return FFB_OK;
 }

@@ -188,6 +188,26 @@ int  ffb_farneback_pairs(ffb_ctx* ctx, const uint8_t* prev, const uint8_t* next,
                          int pov_mode, double cut_threshold, int32_t* cx, int32_t* cy, float* val, float* mean_mag,
                          uint8_t* cut, void* stream);
 
+/* ---- sequences: the flows of every pair of consecutive frames, each frame expanded once (a bracket) -----------------
+ * Pair j = (frame j, frame j+1), j < n_frames - 1, frames uint8 width x height at frames + j*frame_stride, the context's
+ * Farneback parameters.  Outputs may be NULL: flow of pair j at flow + j*flow_stride (rows flow_pitch bytes apart, the
+ * layout of ffb_farneback_pairs); scalar, cut, cx, cy, val, mean_mag, centers as ffb_bracket_finish returns them.
+ *
+ * The call is a bracket: ffb_bracket_begin(pov_mode, cut_threshold) + ffb_bracket_push(frames) + ffb_bracket_finish,
+ * whose final flows are also copied out, one batch behind the kernels.  Every flow is bit-identical to ffb_farneback
+ * on that pair, and the per-pair outputs (the +-6 smoothed centres and the radial scalar included) to that bracket's.
+ * With no per-pair output only the flows are computed.  frames and flow may each be pageable host, pinned host or
+ * device memory (of the context's device); the per-pair outputs are host arrays.  The call configures the frame size
+ * incrementally like ffb_farneback_pairs (the current batch_frames, 2 on a new context; max_pairs grows to
+ * n_frames - 1 when a per-pair output is requested; with a flow, a final-flow ring of 2*batch_frames + 8 pairs).  The
+ * flows of an earlier bracket are no longer resident.  stream: as in ffb_farneback_pairs.  FFB_E_INVALID inside a
+ * bracket, for n_frames < 0, pitch < width, flow_pitch < 8 * width, strides shorter than a frame or a flow, and a device
+ * pointer on another device; n_frames of 0 or 1 does nothing. */
+int  ffb_farneback_sequence(ffb_ctx* ctx, const uint8_t* frames, int n_frames, int width, int height, size_t pitch,
+                            size_t frame_stride, float* flow, size_t flow_pitch, size_t flow_stride, int pov_mode,
+                            double cut_threshold, double* scalar, uint8_t* cut, int32_t* cx, int32_t* cy, float* val,
+                            float* mean_mag, double* centers, void* stream);
+
 /* ---- per-stage hooks (each runs exactly the production kernel of that stage, for the context's parameters) -----
  * Level geometry of the Farneback pyramid for a frame size with the reference's pyr_scale 0.5, levels 3 (coarsest
  * level first): fills up to 4 entries of w[], h[], ksize[], sigma[]; returns the level count in *n_levels. */

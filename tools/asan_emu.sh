@@ -20,6 +20,14 @@ ctx = _native.FlowContext(0, lib_path="$OUT/libffb_emu_asan.so")
 for (w, h) in [(256, 256), (150, 101), (33, 20), (264, 72), (97, 131)]:
     r = api.process_bracket(make_clip(w, h, 4, seed=w), {}, ctx=ctx, batch_frames=2)
     print(w, h, "ok", float(np.sum(r["scalar"])))
+for (w, h, b) in [(97, 70, 3), (33, 20, 16)]:   # sequences that wrap the final-flow ring; b = 16: host-input ramp
+    seq = make_clip(w, h, 41, seed=b)
+    ctx.configure(w, h, b, 8)
+    r = ctx.farneback_sequence(seq, stats=True)
+    flow = np.zeros((40, h + 1, w + 3, 2), np.float32)
+    ctx.farneback_sequence_ptr(seq.ctypes.data, 41, w, h, w, w * h, flow.ctypes.data, (w + 3) * 8, (h + 1) * (w + 3) * 8)
+    assert np.array_equal(flow[:, :h, :w], r["flow"])
+    print(w, h, "sequence ok", float(np.sum(r["scalar"])))
 pc.check_reductions_random(ctx, n_cases=8, max_side=70)
 pc.check_preprocess(ctx, sizes=((97, 131), (64, 48)))
 pc.check_preprocess_window(ctx)
