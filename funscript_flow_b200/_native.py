@@ -15,7 +15,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 DEFAULT_LIB = os.path.join(_HERE, "libffb.so")
 
-K_NAMES = ["pyramid", "polyexp", "upsample", "flow_iter", "divmag", "radial", "small", "preprocess"]
+K_NAMES = ["pyramid", "polyexp", "upsample", "flow_iter", "divmag", "radial", "small", "preprocess", "fb_check"]
 K_FLOW_ITER = 3
 
 
@@ -68,6 +68,8 @@ def load(path: Optional[str] = None) -> C.CDLL:
                                       u8p, vp]),
         "ffb_farneback_sequence": (i32, [vp, vp, i32, i32, i32, sz, sz, vp, sz, sz, i32, C.c_double, f64p, u8p, i32p, i32p,
                                          f32p, f32p, f64p, vp]),
+        "ffb_farneback_sequence_bidir": (i32, [vp, vp, i32, i32, i32, sz, sz, vp, vp, sz, sz, vp, sz, sz, C.c_double,
+                                               C.c_double, C.POINTER(C.c_int64), vp]),
         "ffb_max_divergence": (i32, [vp, f32p, i32, i32, i32p, i32p, f32p]),
         "ffb_mean_magnitude": (i32, [vp, f32p, i32, i32, f32p]),
         "ffb_radial_motion": (i32, [vp, f32p, i32, i32, C.c_double, C.c_double, i32, i32, f64p]),
@@ -80,6 +82,7 @@ def load(path: Optional[str] = None) -> C.CDLL:
         "ffb_stage_update_matrices": (i32, [vp, f32p, f32p, f32p, i32, i32, f32p]),
         "ffb_stage_flow_iter": (i32, [vp, f32p, f32p, f32p, i32, i32, f32p]),
         "ffb_stage_upsample_flow": (i32, [vp, f32p, i32, i32, i32, i32, f32p]),
+        "ffb_stage_fb_check": (i32, [vp, f32p, f32p, i32, i32, C.c_double, C.c_double, u8p, C.POINTER(C.c_int64)]),
         "ffb_preprocess_configure": (i32, [vp, i32, i32, i32]),
         "ffb_bracket_push_bgr": (i32, [vp, vp, i32, sz, sz]),
         "ffb_stage_preprocess": (i32, [vp, u8p, i32, i32, sz, i32, u8p]),
@@ -488,6 +491,57 @@ class FlowContext:
         res["flow"] = flow_arr
         return res
 
+    def farneback_sequence_bidir(self, frames: np.ndarray, *, forward: bool = True, backward: bool = True,
+                                 mask: bool = True, counts: bool = True, alpha: float = 0.01, beta: float = 0.5) -> dict:
+        """farneback_sequence plus, for pair j, the backward flow (frames[j + 1] -> frames[j]) and the forward-backward
+        consistency check, in one call (ffb_farneback_sequence_bidir; each frame expanded once): {"flow": f32
+        [n - 1, H, W, 2], "flow_bw": the same, "mask": bool [n - 1, H, W], "n_consistent": int64 [n - 1]}, an output
+        not asked for is None.  "flow" is farneback_sequence's, flow_bw[j] is bit-identical to
+        farneback(frames[j + 1], frames[j]), and mask[j] is True where |f + b|^2 <= alpha (|f|^2 + |b|^2) + beta with b
+        the backward flow sampled bilinearly at the forward target (False for a target outside the frame).  Batches are
+        those of the last configure(), as in farneback_sequence."""
+        frames = np.ascontiguousarray(frames, dtype=np.uint8)
+        if frames.ndim != 3:
+            raise ValueError(f"farneback_sequence_bidir: frames must be uint8 [n, H, W], not {frames.shape}")
+        n, h, w = frames.shape
+        m = max(n - 1, 0)
+        fw = np.empty((m, h, w, 2), np.float32) if forward else None
+        bw = np.empty((m, h, w, 2), np.float32) if backward else None
+        mk = np.empty((m, h, w), np.uint8) if mask else None
+        cnt = self.farneback_sequence_bidir_ptr(frames.ctypes.data, n, w, h, w, w * h, fw, bw, mask=mk, counts=counts,
+                                                alpha=alpha, beta=beta)
+        return {"flow": fw, "flow_bw": bw, "mask": None if mk is None else mk.view(np.bool_), "n_consistent": cnt}
+
+    def farneback_sequence_bidir_ptr(self, frames_ptr: int, n_frames: int, width: int, height: int, pitch: int,
+                                     frame_stride: int, flow=None, flow_bw=None, flow_pitch: int = 0, flow_stride: int = 0,
+                                     mask=None, mask_pitch: int = 0, mask_stride: int = 0, stream: int = 0, *,
+                                     counts: bool = False, alpha: float = 0.01, beta: float = 0.5):
+        """Raw-pointer variant of farneback_sequence_bidir, like farneback_sequence_ptr: `flow` / `flow_bw` pointers
+        (0 = none) sharing flow_pitch / flow_stride, or float32 NumPy arrays [n_frames - 1, H, W, 2]; `mask` a pointer
+        (0 = none) or a uint8 / bool NumPy array [n_frames - 1, H, W]; `stream` a cudaStream_t handle (0 = none).
+        Returns the int64 consistent-pixel counts with counts=True (the call then waits for the device), else None."""
+        n = max(int(n_frames) - 1, 0)
+        ptrs = []
+        for arr in (flow, flow_bw):
+            if isinstance(arr, np.ndarray):
+                assert arr.dtype == np.float32 and arr.flags.c_contiguous and arr.shape == (n, height, width, 2)
+                flow_pitch, flow_stride = width * 8, width * height * 8
+                ptrs.append(arr.ctypes.data)
+            else:
+                ptrs.append(int(arr or 0))
+        if isinstance(mask, np.ndarray):
+            assert mask.dtype in (np.uint8, np.bool_) and mask.flags.c_contiguous and mask.shape == (n, height, width)
+            mask_ptr, mask_pitch, mask_stride = mask.ctypes.data, width, width * height
+        else:
+            mask_ptr = int(mask or 0)
+        cnt = np.empty(max(n, 1), np.int64) if counts else None
+        self._ck(self._lib.ffb_farneback_sequence_bidir(
+            self._h, C.c_void_p(frames_ptr), int(n_frames), int(width), int(height), int(pitch), int(frame_stride),
+            C.c_void_p(ptrs[0] or None), C.c_void_p(ptrs[1] or None), int(flow_pitch), int(flow_stride),
+            C.c_void_p(mask_ptr or None), int(mask_pitch), int(mask_stride), float(alpha), float(beta),
+            None if cnt is None else cnt.ctypes.data_as(C.POINTER(C.c_int64)), C.c_void_p(int(stream) or None)))
+        return None if cnt is None else cnt[:n].copy()
+
     def max_divergence(self, flow: np.ndarray):
         flow = np.ascontiguousarray(flow, dtype=np.float32)
         h, w = flow.shape[:2]
@@ -557,6 +611,18 @@ class FlowContext:
         out = np.empty((h, w, 2), np.float32)
         self._ck(self._lib.ffb_stage_upsample_flow(self._h, _f32(fc), wc, hc, w, h, _f32(out)))
         return out
+
+    def stage_fb_check(self, flow_fw: np.ndarray, flow_bw: np.ndarray, alpha: float = 0.01, beta: float = 0.5):
+        """The forward-backward check of one pair (k_fb_check) on host flows f32 [h, w, 2]: (mask bool [h, w], count)."""
+        fw = np.ascontiguousarray(flow_fw, np.float32)
+        bw = np.ascontiguousarray(flow_bw, np.float32)
+        assert fw.shape == bw.shape and fw.ndim == 3 and fw.shape[2] == 2
+        h, w = fw.shape[:2]
+        mask = np.empty((h, w), np.uint8)
+        n = C.c_int64()
+        self._ck(self._lib.ffb_stage_fb_check(self._h, _f32(fw), _f32(bw), w, h, float(alpha), float(beta), _u8(mask),
+                                              C.byref(n)))
+        return mask.view(np.bool_), int(n.value)
 
     # -- instrumentation
     def profile(self, enable: bool):

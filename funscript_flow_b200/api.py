@@ -14,6 +14,8 @@
     precompute_flow_info_batch(pairs, config)       [precompute_wrapper(p, config) for p in pairs] in one call
     calc_optical_flow_farneback_sequence(frames, None, ...)    the same for every pair of consecutive frames ([n, H, W]
                                                     -> [n - 1, H, W, 2]; each frame expanded once)
+    calc_optical_flow_farneback_sequence_bidirectional(frames, None, ...)   the same plus the backward flows and the
+                                                    forward-backward consistency mask ([n - 1, H, W] bool)
 
 Every entry point that configures a context first sets its Farneback parameters from the settings keys
 flow_pyr_scale, flow_levels, flow_winsize, flow_iterations, flow_poly_n, flow_poly_sigma (farneback_params;
@@ -412,6 +414,58 @@ def calc_optical_flow_farneback_sequence(frames, flow, pyr_scale: float, levels:
     ctx.farneback_sequence_ptr(frames.data_ptr(), n, w, h, w, w * h, out.data_ptr(), w * 8, w * h * 8,
                                torch.cuda.current_stream(frames.device).cuda_stream)
     return out
+
+
+def calc_optical_flow_farneback_sequence_bidirectional(frames, flow, pyr_scale: float, levels: int, winsize: int,
+                                                       iterations: int, poly_n: int, poly_sigma: float, flags: int = 0, *,
+                                                       alpha: float = 0.01, beta: float = 0.5,
+                                                       ctx: Optional[_native.FlowContext] = None):
+    """calc_optical_flow_farneback_sequence plus the backward flow of every pair and the forward-backward consistency
+    mask (Sundaram, Brox & Keutzer, ECCV 2010), in one call with each frame expanded once: returns (forward, backward,
+    mask), float32 [n - 1, H, W, 2] twice and bool [n - 1, H, W].  forward[j] is the flow frames[j] -> frames[j + 1],
+    backward[j] the flow frames[j + 1] -> frames[j] (calc_optical_flow_farneback(frames[j + 1], frames[j], ...) bit for
+    bit), and mask[j] is True where the pixel's forward target lies in the frame and |w + w_b|^2 <= alpha (|w|^2 +
+    |w_b|^2) + beta, w_b the backward flow sampled bilinearly at the target: False marks occlusions, disocclusions and
+    unreliable motion.  Inputs, refusals, the context's configuration and the torch path (tensors on the frames'
+    device, ordered on torch.cuda.current_stream(), no host round trip) are calc_optical_flow_farneback_sequence's."""
+    if flow is not None:
+        raise ValueError("calc_optical_flow_farneback_sequence_bidirectional: flow must be None (an initial flow is not supported)")
+    ctx = ctx or get_context()
+    tensor = _is_torch_tensor(frames)
+    if tensor:
+        import torch
+        if frames.dtype != torch.uint8 or not frames.is_cuda:
+            raise TypeError("calc_optical_flow_farneback_sequence_bidirectional: a tensor must be torch.uint8 on a CUDA device")
+        if frames.device.index != ctx.device:
+            raise ValueError(f"calc_optical_flow_farneback_sequence_bidirectional: frames on {frames.device}, the context on "
+                             f"cuda:{ctx.device}")
+    else:
+        frames = np.asarray(frames)
+        if frames.dtype != np.uint8:
+            raise TypeError("calc_optical_flow_farneback_sequence_bidirectional: frames must be uint8")
+        frames = np.ascontiguousarray(frames)   # the call reads dense frames: a strided view is copied first
+    if frames.ndim != 3:
+        raise ValueError(f"calc_optical_flow_farneback_sequence_bidirectional: frames must be [n, H, W], not {tuple(frames.shape)}")
+    ctx.set_farneback(pyr_scale, levels, winsize, iterations, poly_n, poly_sigma, flags)
+    n, h, w = frames.shape
+    m = max(n - 1, 0)
+    if tensor:
+        frames = frames.contiguous()
+        fw = torch.empty((m, h, w, 2), dtype=torch.float32, device=frames.device)
+        bw = torch.empty_like(fw)
+        mask = torch.empty((m, h, w), dtype=torch.bool, device=frames.device)
+    else:
+        fw, bw, mask = np.empty((m, h, w, 2), np.float32), np.empty((m, h, w, 2), np.float32), np.empty((m, h, w), np.bool_)
+    if n < 2:
+        return fw, bw, mask
+    ctx.configure(w, h, _sequence_batch(w, h, n), 1)
+    if not tensor:
+        ctx.farneback_sequence_bidir_ptr(frames.ctypes.data, n, w, h, w, w * h, fw, bw, mask=mask, alpha=alpha, beta=beta)
+        return fw, bw, mask
+    ctx.farneback_sequence_bidir_ptr(frames.data_ptr(), n, w, h, w, w * h, fw.data_ptr(), bw.data_ptr(), w * 8, w * h * 8,
+                                     mask.data_ptr(), w, w * h, torch.cuda.current_stream(frames.device).cuda_stream,
+                                     alpha=alpha, beta=beta)
+    return fw, bw, mask
 
 
 def process_sequence(frames, params: Optional[Dict] = None, *, ctx: Optional[_native.FlowContext] = None,

@@ -7,7 +7,8 @@
 //     independent pairs as prev_0, next_0, prev_1, ... and reads them with pair stride 2)
 //   --k_flow_iter x iterations per level (flow up-sampling fused, k_upsample_flow otherwise; winsize != 15:
 //     k_flow_matrices + k_box_solve)--> final-flow ring (>= B+8 pairs; ffb_farneback_pairs and ffb_farneback_sequence
-//     copy the flows out of it on s_out, the sequence with a ring of >= 2B+8 pairs)
+//     copy the flows out of it on s_out, the sequence with a ring of >= 2B+8 pairs; ffb_farneback_sequence_bidir also
+//     runs the reversed pairs into a backward final-flow ring and k_fb_check into a mask ring of the same slots)
 //   --k_divmag / k_phase1_finish--> per-pair centre, value, mean magnitude, cut flag (device arrays)
 //   --k_smooth_centers / k_radial / k_radial_finish (lagging 6 pairs)--> per-pair scalar
 // and only the 1-D per-pair results are copied back at ffb_bracket_finish.
@@ -30,7 +31,8 @@ namespace {
 thread_local std::string g_create_error;
 
 const char* const kKernelNames[FFB_K_COUNT] = {"k_pyramid_level", "k_polyexp",  "k_upsample_flow", "k_flow_iter",
-                                               "k_divmag",        "k_radial",   "small",           "k_preprocess"};
+                                               "k_divmag",        "k_radial",   "small",           "k_preprocess",
+                                               "k_fb_check"};
 
 // ------------------------------------------------------------------ host-side constant builders
 int cv_round(double v) { return (int)nearbyint(v); }   // round-half-even in the default FP mode
@@ -249,6 +251,13 @@ struct ffb_ctx {
     size_t r_slot_floats = 0;
     float2* ring = nullptr;
     size_t ring_stride = 0;   // float2 per ring element
+    // ffb_farneback_sequence_bidir, allocated by the first call that needs them: backward final flows and consistency
+    // masks in the slots of the final-flow ring (bw_n / mask_n slots, 0 or ring_n), consistent-pixel counts per pair
+    float2* ring_bw = nullptr;
+    uint8_t* mask_ring = nullptr;
+    int bw_n = 0, mask_n = 0;
+    unsigned* d_ncons = nullptr;
+    int ncons_cap = 0;
     uint8_t* d_u8[2] = {nullptr, nullptr};
     uint8_t* h_pin[2] = {nullptr, nullptr};
     // per-bracket results (device) + partials
@@ -562,9 +571,9 @@ FlowIterPlan flow_iter_plan(int frame_w, int frame_h, int w, int h, const FlowIt
     return p;
 }
 
-template <int NT, int U, int MINB, int HO, int PS>
+template <int NT, int U, int MINB, int HO, int PS, bool REV>
 int launch_flow_iter_t(ffb_ctx* c, const FfbIterArgs& a, int npairs, int level, double bytes, cudaStream_t stream, bool timed) {
-    auto kfn = a.up_src ? k_flow_iter<NT, U, MINB, true, HO, PS> : k_flow_iter<NT, U, MINB, false, HO, PS>;
+    auto kfn = a.up_src ? k_flow_iter<NT, U, MINB, true, HO, PS, REV> : k_flow_iter<NT, U, MINB, false, HO, PS, REV>;
     const size_t smem = ffb_flow_iter_smem<NT, U, HO>();
     if (!c->attr_iter.count((const void*)kfn)) {
         CK(c, cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -584,8 +593,8 @@ struct UpSrc {   // coarser-level flow to be up-sampled inside the iteration ker
     const float2* src = nullptr; size_t stride = 0; int sp = 0, wc = 0, hc = 0;
 };
 
-// the k_flow_iter variant of plan `p` with pair stride PS
-template <int PS>
+// the k_flow_iter variant of plan `p` with pair stride PS and slot order REV
+template <int PS, bool REV>
 int launch_flow_iter_ps(ffb_ctx* c, const FlowIterPlan& p, const FfbIterArgs& a, int npairs, int level, double bytes,
                         cudaStream_t stream, bool timed) {
     // compiled in: 256x4x8, 128x2x4, 160x2x4, 96x2x4, 64x2x4 (the round-2 sweeps measured and dropped 192 / 512-thread
@@ -593,11 +602,11 @@ int launch_flow_iter_ps(ffb_ctx* c, const FlowIterPlan& p, const FfbIterArgs& a,
     // issue of the second row pair, and a barrier-free variant in which neighbouring warps synchronise through
     // shared-memory flags: profiles/r2_sweep_flow_iter.txt)
     switch (p.nt * 100 + p.u * 10 + p.ho) {
-        case 25648: return launch_flow_iter_t<256, 4, 2, 8, PS>(c, a, npairs, level, bytes, stream, timed);
-        case 12824: return launch_flow_iter_t<128, 2, 4, 4, PS>(c, a, npairs, level, bytes, stream, timed);
-        case 16024: return launch_flow_iter_t<160, 2, 3, 4, PS>(c, a, npairs, level, bytes, stream, timed);
-        case 9624:  return launch_flow_iter_t<96, 2, 5, 4, PS>(c, a, npairs, level, bytes, stream, timed);
-        case 6424:  return launch_flow_iter_t<64, 2, 8, 4, PS>(c, a, npairs, level, bytes, stream, timed);
+        case 25648: return launch_flow_iter_t<256, 4, 2, 8, PS, REV>(c, a, npairs, level, bytes, stream, timed);
+        case 12824: return launch_flow_iter_t<128, 2, 4, 4, PS, REV>(c, a, npairs, level, bytes, stream, timed);
+        case 16024: return launch_flow_iter_t<160, 2, 3, 4, PS, REV>(c, a, npairs, level, bytes, stream, timed);
+        case 9624:  return launch_flow_iter_t<96, 2, 5, 4, PS, REV>(c, a, npairs, level, bytes, stream, timed);
+        case 6424:  return launch_flow_iter_t<64, 2, 8, 4, PS, REV>(c, a, npairs, level, bytes, stream, timed);
         default: break;
     }
     return fail(c, FFB_E_INVALID, "FFB_ITER_CFG: no k_flow_iter variant %dx%dx%d (compiled in: 256x4x8, 128x2x4, 160x2x4, 96x2x4, 64x2x4)",
@@ -605,10 +614,11 @@ int launch_flow_iter_ps(ffb_ctx* c, const FlowIterPlan& p, const FfbIterArgs& a,
 }
 
 // One k_flow_iter launch of plan `p` on `stream`, counted under pyramid level `level` (-1: none).  timed = false inside
-// the sliced flow phase, which is timed as a whole.  pair_stride: 1 (bracket) or 2 (independent pairs), see k_flow_iter.
+// the sliced flow phase, which is timed as a whole.  pair_stride: 1 (bracket) or 2 (independent pairs); rev: the backward
+// flows of bracket pairs (pair stride 1), see k_flow_iter.
 int launch_flow_iter(ffb_ctx* c, const FlowIterPlan& p, int level, cudaStream_t stream, bool timed, FfbRing R, size_t plane,
                      int rp, int w, int h, const float2* fin, size_t fin_stride, int fip, FfbRing fout, int fop, int npairs,
-                     const UpSrc* up = nullptr, int pair_stride = 1) {
+                     const UpSrc* up = nullptr, int pair_stride = 1, bool rev = false) {
     FfbIterArgs a;
     a.R = R; a.plane = (int)plane; a.rp = rp; a.w = w; a.h = h;
     a.fin = fin; a.fin_stride = fin_stride; a.fip = fip; a.fout = fout; a.fop = fop;
@@ -624,14 +634,15 @@ int launch_flow_iter(ffb_ctx* c, const FlowIterPlan& p, int level, cudaStream_t 
     // the kernel stores four flow vectors with one 32-byte instruction
     if (fop % 4 != 0 || ((uintptr_t)fout.base | (uintptr_t)fout.stride) % 32 != 0)
         return fail(c, FFB_E_INVALID, "flow output is not 32-byte aligned (pitch %d, stride %zu)", fop, fout.stride);
-    return pair_stride == 2 ? launch_flow_iter_ps<2>(c, p, a, npairs, level, bytes, stream, timed)
-                            : launch_flow_iter_ps<1>(c, p, a, npairs, level, bytes, stream, timed);
+    if (pair_stride == 2) return launch_flow_iter_ps<2, false>(c, p, a, npairs, level, bytes, stream, timed);
+    return rev ? launch_flow_iter_ps<1, true>(c, p, a, npairs, level, bytes, stream, timed)
+               : launch_flow_iter_ps<1, false>(c, p, a, npairs, level, bytes, stream, timed);
 }
 
 // One flow iteration with the context's winsize != 15: k_flow_matrices into the scratch M (npairs x 5 planes), then
 // k_box_solve into fout.  Same arguments, counters and output layout as launch_flow_iter.
 int launch_flow_unfused(ffb_ctx* c, int level, float* M, FfbRing R, size_t plane, int rp, int w, int h, const float2* fin,
-                        size_t fin_stride, int fip, FfbRing fout, int fop, int npairs, int pair_stride = 1) {
+                        size_t fin_stride, int fip, FfbRing fout, int fop, int npairs, int pair_stride = 1, bool rev = false) {
     const int win = c->fb.winsize, r = win / 2;
     if (BOX_NT - 2 * r < 1) return fail(c, FFB_E_INVALID, "winsize %d too large for k_box_solve", win);
     FfbMatrixArgs m;
@@ -642,8 +653,8 @@ int launch_flow_unfused(ffb_ctx* c, int level, float* M, FfbRing R, size_t plane
     const double px = (double)npairs * w * h;
     const ProfMark pm = prof_begin(c, FFB_K_FLOW_ITER, level, px * ((fin ? 48.0 : 40.0) + 20.0), c->s_comp);
     const dim3 mgrid((w + 31) / 32, (h + 7) / 8, npairs);
-    if (pair_stride == 2) FFB_LAUNCH(k_flow_matrices<2>, mgrid, dim3(256), 0, c->s_comp, m);
-    else FFB_LAUNCH(k_flow_matrices<1>, mgrid, dim3(256), 0, c->s_comp, m);
+    auto kfn = pair_stride == 2 ? k_flow_matrices<2, false> : (rev ? k_flow_matrices<1, true> : k_flow_matrices<1, false>);
+    FFB_LAUNCH(kfn, mgrid, dim3(256), 0, c->s_comp, m);
     prof_end(pm);
     CKL(c);
     FfbBoxArgs b;
@@ -685,7 +696,8 @@ void free_batch_group(ffb_ctx* c) {
 }
 void free_ring_group(ffb_ctx* c) {
     dev_free(c->ring); dev_free(c->d_pkey); dev_free(c->d_psum); dev_free(c->d_rpart);
-    c->ring_n = 0;
+    dev_free(c->ring_bw); dev_free(c->mask_ring);
+    c->ring_n = c->bw_n = c->mask_n = 0;
 }
 void free_pairs_group(ffb_ctx* c) {
     dev_free(c->d_cx); dev_free(c->d_cy); dev_free(c->d_val); dev_free(c->d_mm); dev_free(c->d_cut);
@@ -698,6 +710,8 @@ void free_geometry(ffb_ctx* c) {
     free_batch_group(c);
     free_ring_group(c);
     free_pairs_group(c);
+    dev_free(c->d_ncons);
+    c->ncons_cap = 0;
     for (int l = 0; l < FFB_PLAN_LEVELS; ++l) {
         Level& L = c->lev[l];
         dev_free(L.xi); dev_free(L.yi); dev_free(L.uxi); dev_free(L.uyi);
@@ -928,8 +942,9 @@ int launch_divmag(ffb_ctx* c, int p0, int off, int cnt, cudaStream_t stream) {
 // Final flows of np pairs into final-flow ring slots f0 .. (mod ring_n), and their divergence / magnitude partials
 // (divmag = false: flows only).  Pair j reads the expansions in slots r0 + pair_stride * j and the one after it
 // (mod S): bracket pairs [p0, p0 + np) are r0 = f0 = p0 with stride 1, a chunk of independent pairs r0 = 0 with
-// stride 2.
-int flow_pairs(ffb_ctx* c, int r0, int pair_stride, int f0, int np, bool divmag = true) {
+// stride 2.  backward (bracket pairs, divmag = false): the flows of the reversed pairs (R0 = the later frame) into the
+// same slots of the backward final-flow ring.
+int flow_pairs(ffb_ctx* c, int r0, int pair_stride, int f0, int np, bool divmag = true, bool backward = false) {
     // The pairs of a batch are split in two slices whose launch chains run on two streams, so that the short
     // coarse-level launches (and the tail of every launch) of one slice overlap the other slice's work (+4 %; 3-4 slices
     // measured no better).  Every buffer is indexed by pair; the slices share nothing that is written.
@@ -974,7 +989,8 @@ int flow_pairs(ffb_ctx* c, int r0, int pair_stride, int f0, int np, bool divmag 
                 R.mod = c->S;
                 FfbRing toB{(char*)(L.fB + (size_t)off * fstride), fstride * sizeof(float2), 0, 1 << 30};
                 FfbRing toA{(char*)(L.fA + (size_t)off * fstride), fstride * sizeof(float2), 0, 1 << 30};
-                FfbRing toRing{(char*)c->ring, c->ring_stride * sizeof(float2), (f0 + off) % c->ring_n, c->ring_n};
+                FfbRing toRing{(char*)(backward ? c->ring_bw : c->ring), c->ring_stride * sizeof(float2), (f0 + off) % c->ring_n,
+                               c->ring_n};
                 UpSrc up;
                 if (l > 0 && fuse_up) {
                     Level& C = c->lev[l - 1];
@@ -988,10 +1004,10 @@ int flow_pairs(ffb_ctx* c, int r0, int pair_stride, int f0, int np, bool divmag 
                 const FfbRing& fout = it == iters - 1 && last ? toRing : (it % 2 == 0 ? toB : toA);
                 if (fused)
                     TRY(launch_flow_iter(c, L.iter, L.k, streams[sl], !sliced, R, L.plane, L.rp, L.w, L.h, fin, fstride, L.fp,
-                                         fout, L.fp, cnt, it == 0 ? &up : nullptr, pair_stride));
+                                         fout, L.fp, cnt, it == 0 ? &up : nullptr, pair_stride, backward));
                 else
                     TRY(launch_flow_unfused(c, L.k, c->M, R, L.plane, L.rp, L.w, L.h, fin, fstride, L.fp, fout, L.fp, cnt,
-                                            pair_stride));
+                                            pair_stride, backward));
             }
         }
     }
@@ -1020,6 +1036,22 @@ int launch_phase1_finish(ffb_ctx* c, int f0, int out0, int np, int pov, float cu
     f.cx = c->d_cx; f.cy = c->d_cy; f.val = c->d_val; f.mean_mag = c->d_mm; f.cut = c->d_cut;
     const ProfMark pm = prof_begin(c, FFB_K_SMALL, -1, 0, c->s_comp);
     FFB_LAUNCH(k_phase1_finish, dim3(np), dim3(32), 0, c->s_comp, f);
+    prof_end(pm);
+    CKL(c);
+    return FFB_OK;
+}
+
+// k_fb_check of np pairs: forward / backward flows in rings fw / bw (rows fp float2 apart), masks into `mask` (rows mp
+// bytes apart; base NULL: no mask), consistent-pixel counts added to count[0 .. np) (NULL: not counted)
+int launch_fb_check(ffb_ctx* c, FfbRing fw, FfbRing bw, int fp, int w, int h, FfbRing mask, int mp, unsigned* count,
+                    float alpha, float beta, int np) {
+    FfbCheckArgs a;
+    a.fw = fw; a.bw = bw; a.fp = fp; a.w = w; a.h = h;
+    a.mask = mask; a.mp = mp; a.count = count; a.alpha = alpha; a.beta = beta;
+    // algorithmic bytes: the forward flow and, per pixel, one backward vector (the 2x2 footprints of neighbouring
+    // targets overlap), 8 + 8 B/px, plus the mask byte
+    const ProfMark pm = prof_begin(c, FFB_K_FB_CHECK, -1, (double)np * w * h * (mask.base ? 17.0 : 16.0), c->s_comp);
+    FFB_LAUNCH(k_fb_check, dim3((w + 31) / 32, (h + 7) / 8, np), dim3(256), 0, c->s_comp, a);
     prof_end(pm);
     CKL(c);
     return FFB_OK;
@@ -1132,10 +1164,19 @@ int upload_frames(ffb_ctx* c, uint8_t* dst, uint8_t* pin, cudaEvent_t ev_dma, cu
     return FFB_OK;
 }
 
+// Backward pass of a sequence (ffb_farneback_sequence_bidir): after the forward flows of a batch, the backward flows
+// into the backward final-flow ring and, with a mask or counts, k_fb_check into the mask ring / the per-pair counts.
+struct Backward {
+    bool mask = false, count = false;
+    float alpha = 0.f, beta = 0.f;
+};
+
 // One batch of the open bracket (or sequence): upload, expansion, final flows and, with stats, the per-pair results
 // and the radial pass lagging 6 pairs.  stats = false computes the flows only (ffb_farneback_sequence without per-pair
 // outputs): no k_divmag, phase-1 finish, centre smoothing or radial pass, and max_pairs does not bound the pairs.
-int process_batch(ffb_ctx* c, const uint8_t* frames, int nb, size_t pitch, size_t stride, PtrKind kind, bool stats = true) {
+// bw: the backward pass of the batch's pairs (stats = false).
+int process_batch(ffb_ctx* c, const uint8_t* frames, int nb, size_t pitch, size_t stride, PtrKind kind, bool stats = true,
+                  const Backward* bw = nullptr) {
     const int b = c->batch_no & 1;
     const size_t fbytes = (size_t)c->W * c->H;
     const uint8_t* src = frames;
@@ -1160,6 +1201,15 @@ int process_batch(ffb_ctx* c, const uint8_t* frames, int nb, size_t pitch, size_
             return fail(c, FFB_E_INVALID, "shard exceeds the %d pairs announced to ffb_bracket_begin_shard", c->ring_n);
         TRY(flow_pairs(c, p0, 1, p0, np, stats));
         if (stats) TRY(launch_phase1_finish(c, p0, p0, np, c->pov, c->thr));
+        if (bw) {
+            TRY(flow_pairs(c, p0, 1, p0, np, false, true));
+            const size_t fs = c->ring_stride * sizeof(float2), ms = (size_t)c->W * c->H;
+            const int s0 = p0 % c->ring_n;
+            if (bw->mask || bw->count)
+                TRY(launch_fb_check(c, FfbRing{(char*)c->ring, fs, s0, c->ring_n}, FfbRing{(char*)c->ring_bw, fs, s0, c->ring_n},
+                                    c->fp0, c->W, c->H, FfbRing{bw->mask ? (char*)c->mask_ring : nullptr, ms, s0, c->ring_n},
+                                    c->W, bw->count ? c->d_ncons + p0 : nullptr, bw->alpha, bw->beta, np));
+        }
         c->pairs_done += np;
         const int r1 = c->pairs_done - 6;
         if (stats && !c->deferred && r1 > c->radial_done) {
@@ -1693,18 +1743,28 @@ int ffb_farneback(ffb_ctx* c, const uint8_t* prev, const uint8_t* next, int w, i
     return ffb_bracket_get_flow(c, 0, flow);
 }
 
-// Copy on s_out of the final flows in ring slots s0 .. s0 + np - 1 (no wrap) to `dst`: flows flow_stride bytes apart,
-// rows flow_pitch bytes apart, in host memory or on the device (`kind`).
-static int copy_flows_out(ffb_ctx* c, int s0, int np, char* dst, size_t flow_pitch, size_t flow_stride, PtrKind kind) {
+// Per-pair images in the slots of a ring (the final-flow rings, the mask ring): slot s at base + s * slot bytes, H rows
+// of `row` bytes, pitch bytes apart, with slot == H * pitch.
+struct SlotImages { const char* base; size_t slot, pitch, row; };
+static SlotImages flow_slots(const ffb_ctx* c, const float2* ring) {
+    return SlotImages{(const char*)ring, c->ring_stride * sizeof(float2), (size_t)c->fp0 * 8, (size_t)c->W * 8};
+}
+static SlotImages mask_slots(const ffb_ctx* c) {
+    return SlotImages{(const char*)c->mask_ring, (size_t)c->W * c->H, (size_t)c->W, (size_t)c->W};
+}
+
+// Copy on s_out of the images in ring slots s0 .. s0 + np - 1 (no wrap) to `dst`: images `stride` bytes apart, rows
+// `pitch` bytes apart, in host memory or on the device (`kind`).
+static int copy_slots_out(ffb_ctx* c, const SlotImages& r, int s0, int np, char* dst, size_t pitch, size_t stride,
+                          PtrKind kind) {
     const cudaMemcpyKind dir = kind == PTR_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
-    const float2* src = c->ring + (size_t)s0 * c->ring_stride;
-    const size_t row = (size_t)c->W * 8, spitch = (size_t)c->fp0 * 8;
-    if (flow_stride == flow_pitch * c->H)     // the pairs' rows are evenly spaced on both sides
-        CK(c, cudaMemcpy2DAsync(dst, flow_pitch, src, spitch, row, (size_t)np * c->H, dir, c->s_out));
+    const char* src = r.base + (size_t)s0 * r.slot;
+    if (stride == pitch * c->H)     // the pairs' rows are evenly spaced on both sides
+        CK(c, cudaMemcpy2DAsync(dst, pitch, src, r.pitch, r.row, (size_t)np * c->H, dir, c->s_out));
     else
         for (int j = 0; j < np; ++j)
-            CK(c, cudaMemcpy2DAsync(dst + (size_t)j * flow_stride, flow_pitch, src + (size_t)j * c->ring_stride, spitch, row,
-                                    c->H, dir, c->s_out));
+            CK(c, cudaMemcpy2DAsync(dst + (size_t)j * stride, pitch, src + (size_t)j * r.slot, r.pitch, r.row, c->H, dir,
+                                    c->s_out));
     return FFB_OK;
 }
 
@@ -1752,7 +1812,8 @@ int ffb_farneback_pairs(ffb_ctx* c, const uint8_t* prev, const uint8_t* next, in
     // flows of pairs [i0, i0 + np) from ring half `half` to the caller's buffer
     auto copy_out = [&](int i0, int np, int half) -> int {
         CK(c, cudaStreamWaitEvent(c->s_out, c->ev_fin[half], 0));
-        TRY(copy_flows_out(c, half * P, np, (char*)flow + (size_t)i0 * flow_stride, flow_pitch, flow_stride, kf));
+        TRY(copy_slots_out(c, flow_slots(c, c->ring), half * P, np, (char*)flow + (size_t)i0 * flow_stride, flow_pitch,
+                           flow_stride, kf));
         CK(c, cudaEventRecord(c->ev_out[half], c->s_out));
         return FFB_OK;
     };
@@ -1793,60 +1854,75 @@ int ffb_farneback_pairs(ffb_ctx* c, const uint8_t* prev, const uint8_t* next, in
     return FFB_OK;
 }
 
-// Consecutive pairs of a sequence: one bracket over the n_frames frames (the batches of ffb_bracket_push, with the
-// ramp for host input; every frame expanded once; flow_pairs with pair stride 1), whose final flows are also copied
-// out.  Pair p sits in final-flow ring slot p mod ring_n, and the copy-out of batch k on s_out is issued after batch
-// k + 1 has been queued, so it overlaps that batch's kernels.  With ring_n >= 2B + 8, batch k + 1 (at most B pairs)
-// writes no slot of batch k (at most B) nor of the 6 pairs before it that its radial pass still reads; the slots it
-// does overwrite held batch k - 1 or earlier, so it waits for the copy-out of batch k - 1 (ev_out[(k + 1) & 1]).  The
-// radial pass runs on s_comp, in order with every later write.
-int ffb_farneback_sequence(ffb_ctx* c, const uint8_t* frames, int n_frames, int width, int height, size_t pitch,
-                           size_t frame_stride, float* flow, size_t flow_pitch, size_t flow_stride, int pov_mode,
-                           double cut_threshold, double* scalar, uint8_t* cut, int32_t* cx, int32_t* cy, float* val,
-                           float* mean_mag, double* centers, void* stream) {
-    if (!c) return FFB_E_INVALID;
-    if (c->in_bracket) return fail(c, FFB_E_INVALID, "ffb_farneback_sequence inside a bracket");
-    if (n_frames < 0) return fail(c, FFB_E_INVALID, "ffb_farneback_sequence: n_frames %d < 0", n_frames);
-    if (n_frames < 2) return FFB_OK;
-    const int n_pairs = n_frames - 1;
-    if (!frames || width < 1 || height < 1)
-        return fail(c, FFB_E_INVALID, "ffb_farneback_sequence: bad frames (%dx%d)", width, height);
-    if (pitch < (size_t)width) return fail(c, FFB_E_INVALID, "ffb_farneback_sequence: pitch %zu below the width %d", pitch, width);
+// Kind of memory of a caller's buffer (PTR_DEVICE for NULL); device memory must be on the context's device.  `what`
+// names the buffer with its verb ("frames are", "flow is") for the message.
+static int buffer_kind(ffb_ctx* c, const char* fn, const char* what, const void* p, PtrKind* kind) {
+    int dev = c->device;
+    *kind = p ? classify(p, &dev) : PTR_DEVICE;
+    if (*kind == PTR_DEVICE && dev != c->device)
+        return fail(c, FFB_E_INVALID, "%s: %s on device %d, the context on device %d", fn, what, dev, c->device);
+    return FFB_OK;
+}
+
+// The frame and flow arguments of a sequence call (fn: its name in the messages), n_frames >= 2.
+static int check_sequence_args(ffb_ctx* c, const char* fn, const uint8_t* frames, int n_frames, int width, int height,
+                               size_t pitch, size_t frame_stride, bool flow, size_t flow_pitch, size_t flow_stride) {
+    if (!frames || width < 1 || height < 1) return fail(c, FFB_E_INVALID, "%s: bad frames (%dx%d)", fn, width, height);
+    if (pitch < (size_t)width) return fail(c, FFB_E_INVALID, "%s: pitch %zu below the width %d", fn, pitch, width);
     if (frame_stride < pitch * (size_t)(height - 1) + width)
-        return fail(c, FFB_E_INVALID, "ffb_farneback_sequence: frame_stride %zu shorter than a frame", frame_stride);
+        return fail(c, FFB_E_INVALID, "%s: frame_stride %zu shorter than a frame", fn, frame_stride);
     if (flow && flow_pitch < (size_t)width * 8)
-        return fail(c, FFB_E_INVALID, "ffb_farneback_sequence: flow_pitch %zu below 8 * width (%d)", flow_pitch, 8 * width);
-    if (flow && n_pairs > 1 && flow_stride < flow_pitch * (size_t)(height - 1) + (size_t)width * 8)
-        return fail(c, FFB_E_INVALID, "ffb_farneback_sequence: flow_stride %zu shorter than a flow", flow_stride);
-    CK(c, cudaSetDevice(c->device));
-    int dev[2] = {c->device, c->device};
-    const PtrKind kfr = classify(frames, &dev[0]);
-    const PtrKind kf = flow ? classify(flow, &dev[1]) : PTR_DEVICE;
-    if (kfr == PTR_DEVICE && dev[0] != c->device)
-        return fail(c, FFB_E_INVALID, "ffb_farneback_sequence: frames are on device %d, the context on device %d", dev[0], c->device);
-    if (kf == PTR_DEVICE && dev[1] != c->device)
-        return fail(c, FFB_E_INVALID, "ffb_farneback_sequence: flow is on device %d, the context on device %d", dev[1], c->device);
-    const bool stats = scalar || cut || cx || cy || val || mean_mag || centers;
-    // the per-pair results of the whole call stay on the device until the end: max_pairs covers n_pairs
-    const int maxPairs = stats && n_pairs > c->maxPairs ? n_pairs : (c->maxPairs > 0 ? c->maxPairs : 1);
-    const int B = c->B > 0 ? c->B : 2;
-    TRY(configure_checked(c, width, height, B, maxPairs, flow ? 2 * B + 8 : 0));
+        return fail(c, FFB_E_INVALID, "%s: flow_pitch %zu below 8 * width (%d)", fn, flow_pitch, 8 * width);
+    if (flow && n_frames > 2 && flow_stride < flow_pitch * (size_t)(height - 1) + (size_t)width * 8)
+        return fail(c, FFB_E_INVALID, "%s: flow_stride %zu shorter than a flow", fn, flow_stride);
+    return FFB_OK;
+}
+
+// Outputs of a sequence call that leave the final-flow rings (each may be NULL) and the memory each is in.
+struct SequenceOut {
+    float *flow = nullptr, *flow_bw = nullptr;
+    size_t flow_pitch = 0, flow_stride = 0;
+    uint8_t* mask = nullptr;
+    size_t mask_pitch = 0, mask_stride = 0;
+    PtrKind kf = PTR_DEVICE, kb = PTR_DEVICE, km = PTR_DEVICE;
+    bool any() const { return flow || flow_bw || mask; }
+};
+
+// Consecutive pairs of a sequence: one bracket over the n_frames frames (the batches of ffb_bracket_push, with the
+// ramp for host input; every frame expanded once; flow_pairs with pair stride 1), whose final flows -- and with `bw` the
+// backward flows and masks in the same slots of their rings -- are also copied out.  Pair p sits in ring slot
+// p mod ring_n, and the copy-out of batch k on s_out is issued after batch k + 1 has been queued, so it overlaps that
+// batch's kernels.  With ring_n >= 2B + 8, batch k + 1 (at most B pairs) writes no slot of batch k (at most B) nor of
+// the 6 pairs before it that its radial pass still reads; the slots it does overwrite held batch k - 1 or earlier, so
+// it waits for the copy-out of batch k - 1 (ev_out[(k + 1) & 1]).  The radial pass runs on s_comp, in order with every
+// later write.  The geometry is configured by the caller; at the end the caller's stream waits for the call.
+static int sequence_loop(ffb_ctx* c, const uint8_t* frames, int n_frames, size_t pitch, size_t frame_stride, PtrKind kfr,
+                         const SequenceOut& o, bool stats, const Backward* bw, void* stream) {
+    const int n_pairs = n_frames - 1;
+    const bool copy = o.any();
     const cudaStream_t us = (cudaStream_t)stream;
     // ffb_bracket_begin's state; the final-flow ring no longer holds an earlier bracket's flows
     c->deferred = c->phase1_read = false;
     c->pend = 0;
-    c->pov = pov_mode ? 1 : 0;
-    c->thr = (float)cut_threshold;
     c->frames_seen = c->pairs_done = c->radial_done = 0;
     CK(c, cudaEventRecord(c->ev_user, us));
     CK(c, cudaStreamWaitEvent(c->s_copy, c->ev_user, 0));
     CK(c, cudaStreamWaitEvent(c->s_comp, c->ev_user, 0));
-    // flows of pairs [p0, p0 + np) of batch parity `par` to the caller's buffer: one or two runs of ring slots
+    if (bw && bw->count) CK(c, cudaMemsetAsync(c->d_ncons, 0, (size_t)n_pairs * sizeof(unsigned), c->s_comp));
+    // outputs of pairs [p0, p0 + np) of batch parity `par` to the caller's buffers: one or two runs of ring slots each
     auto copy_out = [&](int p0, int np, int par) -> int {
         CK(c, cudaStreamWaitEvent(c->s_out, c->ev_fin[par], 0));
         for (int p = p0; p < p0 + np;) {
             const int s = p % c->ring_n, m = p0 + np - p < c->ring_n - s ? p0 + np - p : c->ring_n - s;
-            TRY(copy_flows_out(c, s, m, (char*)flow + (size_t)p * flow_stride, flow_pitch, flow_stride, kf));
+            if (o.flow)
+                TRY(copy_slots_out(c, flow_slots(c, c->ring), s, m, (char*)o.flow + (size_t)p * o.flow_stride, o.flow_pitch,
+                                   o.flow_stride, o.kf));
+            if (o.flow_bw)
+                TRY(copy_slots_out(c, flow_slots(c, c->ring_bw), s, m, (char*)o.flow_bw + (size_t)p * o.flow_stride,
+                                   o.flow_pitch, o.flow_stride, o.kb));
+            if (o.mask)
+                TRY(copy_slots_out(c, mask_slots(c), s, m, (char*)o.mask + (size_t)p * o.mask_stride, o.mask_pitch,
+                                   o.mask_stride, o.km));
             p += m;
         }
         CK(c, cudaEventRecord(c->ev_out[par], c->s_out));
@@ -1857,10 +1933,10 @@ int ffb_farneback_sequence(ffb_ctx* c, const uint8_t* frames, int n_frames, int 
         const int cap = batch_cap(c, kfr);
         const int nb = n_frames - i < cap ? n_frames - i : cap;
         const int p0 = c->pairs_done;
-        if (flow) CK(c, cudaStreamWaitEvent(c->s_comp, c->ev_out[k & 1], 0));   // copy-out of batch k - 2 done
-        TRY(process_batch(c, frames + (size_t)i * frame_stride, nb, pitch, frame_stride, kfr, stats));
+        if (copy) CK(c, cudaStreamWaitEvent(c->s_comp, c->ev_out[k & 1], 0));   // copy-out of batch k - 2 done
+        TRY(process_batch(c, frames + (size_t)i * frame_stride, nb, pitch, frame_stride, kfr, stats, bw));
         i += nb;
-        if (!flow) continue;
+        if (!copy) continue;
         CK(c, cudaEventRecord(c->ev_fin[k & 1], c->s_comp));
         // issued one batch late: a copy into pageable memory returns only when it is done
         if (pend_np > 0) TRY(copy_out(pend_p0, pend_np, (k - 1) & 1));
@@ -1870,18 +1946,117 @@ int ffb_farneback_sequence(ffb_ctx* c, const uint8_t* frames, int n_frames, int 
     if (stats && n_pairs > c->radial_done) TRY(radial_range(c, c->radial_done, n_pairs, n_pairs));
     if (pend_np > 0) TRY(copy_out(pend_p0, pend_np, (k - 1) & 1));
     c->frames_seen = c->pairs_done = c->radial_done = 0;
-    if (flow) {   // later work of the context (a bracket, the next call) overwrites the ring after the copy-out
+    if (copy) {   // later work of the context (a bracket, the next call) overwrites the rings after the copy-out
         CK(c, cudaEventRecord(c->ev_done, c->s_out));
         CK(c, cudaStreamWaitEvent(c->s_comp, c->ev_done, 0));
     }
     // s_comp has waited for every upload and copy-out: the caller's stream continues when the inputs have been read
-    // and the flows written
+    // and the outputs written
     CK(c, cudaEventRecord(c->ev_done, c->s_comp));
     CK(c, cudaStreamWaitEvent(us, c->ev_done, 0));
-    const bool host_io = kfr != PTR_DEVICE || kf != PTR_DEVICE || stats;
+    return FFB_OK;
+}
+
+int ffb_farneback_sequence(ffb_ctx* c, const uint8_t* frames, int n_frames, int width, int height, size_t pitch,
+                           size_t frame_stride, float* flow, size_t flow_pitch, size_t flow_stride, int pov_mode,
+                           double cut_threshold, double* scalar, uint8_t* cut, int32_t* cx, int32_t* cy, float* val,
+                           float* mean_mag, double* centers, void* stream) {
+    static const char* fn = "ffb_farneback_sequence";
+    if (!c) return FFB_E_INVALID;
+    if (c->in_bracket) return fail(c, FFB_E_INVALID, "ffb_farneback_sequence inside a bracket");
+    if (n_frames < 0) return fail(c, FFB_E_INVALID, "ffb_farneback_sequence: n_frames %d < 0", n_frames);
+    if (n_frames < 2) return FFB_OK;
+    const int n_pairs = n_frames - 1;
+    TRY(check_sequence_args(c, fn, frames, n_frames, width, height, pitch, frame_stride, flow, flow_pitch, flow_stride));
+    CK(c, cudaSetDevice(c->device));
+    PtrKind kfr;
+    SequenceOut o;
+    o.flow = flow; o.flow_pitch = flow_pitch; o.flow_stride = flow_stride;
+    TRY(buffer_kind(c, fn, "frames are", frames, &kfr));
+    TRY(buffer_kind(c, fn, "flow is", flow, &o.kf));
+    const bool stats = scalar || cut || cx || cy || val || mean_mag || centers;
+    // the per-pair results of the whole call stay on the device until the end: max_pairs covers n_pairs
+    const int maxPairs = stats && n_pairs > c->maxPairs ? n_pairs : (c->maxPairs > 0 ? c->maxPairs : 1);
+    const int B = c->B > 0 ? c->B : 2;
+    TRY(configure_checked(c, width, height, B, maxPairs, flow ? 2 * B + 8 : 0));
+    c->pov = pov_mode ? 1 : 0;
+    c->thr = (float)cut_threshold;
+    TRY(sequence_loop(c, frames, n_frames, pitch, frame_stride, kfr, o, stats, nullptr, stream));
+    const bool host_io = kfr != PTR_DEVICE || o.kf != PTR_DEVICE || stats;
     if (stream && !host_io) return FFB_OK;
     if (stats) return fetch_results(c, n_pairs, true, scalar, cut, cx, cy, val, mean_mag, centers);
     CK(c, cudaStreamSynchronize(c->s_comp));
+    return FFB_OK;
+}
+
+// The sequence with the backward flow of every pair as well: a second flow_pairs per batch with the slot order reversed
+// (R0 = frame j + 1, R1 = frame j, the expansions already in the ring) into the backward final-flow ring, then
+// k_fb_check of the batch into the mask ring and the per-pair counts.  The three rings share their slots, and the
+// fences of ffb_farneback_sequence cover the three copy-outs of a batch.
+int ffb_farneback_sequence_bidir(ffb_ctx* c, const uint8_t* frames, int n_frames, int width, int height, size_t pitch,
+                                 size_t frame_stride, float* flow_fw, float* flow_bw, size_t flow_pitch, size_t flow_stride,
+                                 uint8_t* mask, size_t mask_pitch, size_t mask_stride, double alpha, double beta,
+                                 int64_t* n_consistent, void* stream) {
+    static const char* fn = "ffb_farneback_sequence_bidir";
+    if (!c) return FFB_E_INVALID;
+    if (c->in_bracket) return fail(c, FFB_E_INVALID, "ffb_farneback_sequence_bidir inside a bracket");
+    if (n_frames < 0) return fail(c, FFB_E_INVALID, "ffb_farneback_sequence_bidir: n_frames %d < 0", n_frames);
+    if (n_frames < 2) return FFB_OK;
+    const int n_pairs = n_frames - 1;
+    TRY(check_sequence_args(c, fn, frames, n_frames, width, height, pitch, frame_stride, flow_fw || flow_bw, flow_pitch,
+                            flow_stride));
+    if (mask && mask_pitch < (size_t)width)
+        return fail(c, FFB_E_INVALID, "%s: mask_pitch %zu below the width %d", fn, mask_pitch, width);
+    if (mask && n_pairs > 1 && mask_stride < mask_pitch * (size_t)(height - 1) + width)
+        return fail(c, FFB_E_INVALID, "%s: mask_stride %zu shorter than a mask", fn, mask_stride);
+    if (!(alpha >= 0.0 && isfinite(alpha)) || !(beta >= 0.0 && isfinite(beta)))
+        return fail(c, FFB_E_INVALID, "%s: alpha %g and beta %g must be finite and >= 0", fn, alpha, beta);
+    CK(c, cudaSetDevice(c->device));
+    PtrKind kfr;
+    SequenceOut o;
+    o.flow = flow_fw; o.flow_bw = flow_bw; o.flow_pitch = flow_pitch; o.flow_stride = flow_stride;
+    o.mask = mask; o.mask_pitch = mask_pitch; o.mask_stride = mask_stride;
+    TRY(buffer_kind(c, fn, "frames are", frames, &kfr));
+    TRY(buffer_kind(c, fn, "flow_fw is", flow_fw, &o.kf));
+    TRY(buffer_kind(c, fn, "flow_bw is", flow_bw, &o.kb));
+    TRY(buffer_kind(c, fn, "mask is", mask, &o.km));
+    const int B = c->B > 0 ? c->B : 2;
+    TRY(configure_checked(c, width, height, B, c->maxPairs > 0 ? c->maxPairs : 1, o.any() ? 2 * B + 8 : 0));
+    const bool backward = flow_bw || mask || n_consistent;
+    // the backward ring, the mask ring and the counts: grow-only, allocated by the first call that needs them (a new
+    // frame size or a larger final-flow ring frees the rings)
+    if (backward && c->bw_n < c->ring_n) {
+        dev_free(c->ring_bw);
+        c->bw_n = 0;
+        TRY(dev_alloc(c, &c->ring_bw, (size_t)c->ring_n * c->ring_stride));
+        c->bw_n = c->ring_n;
+    }
+    if (mask && c->mask_n < c->ring_n) {
+        dev_free(c->mask_ring);
+        c->mask_n = 0;
+        TRY(dev_alloc(c, &c->mask_ring, (size_t)c->ring_n * width * height));
+        c->mask_n = c->ring_n;
+    }
+    if (n_consistent && c->ncons_cap < n_pairs) {
+        dev_free(c->d_ncons);
+        c->ncons_cap = 0;
+        TRY(dev_alloc(c, &c->d_ncons, (size_t)n_pairs));
+        c->ncons_cap = n_pairs;
+    }
+    Backward bw;
+    bw.mask = mask != nullptr;
+    bw.count = n_consistent != nullptr;
+    bw.alpha = (float)alpha;
+    bw.beta = (float)beta;
+    TRY(sequence_loop(c, frames, n_frames, pitch, frame_stride, kfr, o, false, backward ? &bw : nullptr, stream));
+    const bool host_io = kfr != PTR_DEVICE || o.kf != PTR_DEVICE || o.kb != PTR_DEVICE || o.km != PTR_DEVICE || n_consistent;
+    if (stream && !host_io) return FFB_OK;
+    CK(c, cudaStreamSynchronize(c->s_comp));
+    if (n_consistent) {
+        std::vector<unsigned> h((size_t)n_pairs);
+        CK(c, cudaMemcpy(h.data(), c->d_ncons, (size_t)n_pairs * sizeof(unsigned), cudaMemcpyDeviceToHost));
+        for (int j = 0; j < n_pairs; ++j) n_consistent[j] = h[j];
+    }
     return FFB_OK;
 }
 
@@ -2119,6 +2294,32 @@ int ffb_stage_upsample_flow(ffb_ctx* c, const float* flow_c, int wc, int hc, int
     TRY(launch_upsample(c, dsrc, 0, wc, wc, hc, ddst, 0, w, w, h, dxi, dxa, dyi, dya, 1));
     CK(c, cudaStreamSynchronize(c->s_comp));
     CK(c, cudaMemcpy(out, ddst, (size_t)w * h * 8, cudaMemcpyDeviceToHost));
+    return FFB_OK;
+}
+
+int ffb_stage_fb_check(ffb_ctx* c, const float* flow_fw, const float* flow_bw, int w, int h, double alpha, double beta,
+                       uint8_t* mask, int64_t* n_consistent) {
+    if (!c || !flow_fw || !flow_bw || w < 1 || h < 1 || (double)w * h >= 4294967295.0) return FFB_E_INVALID;
+    if (!(alpha >= 0.0 && isfinite(alpha)) || !(beta >= 0.0 && isfinite(beta)))
+        return fail(c, FFB_E_INVALID, "ffb_stage_fb_check: alpha %g and beta %g must be finite and >= 0", alpha, beta);
+    CK(c, cudaSetDevice(c->device));
+    Scratch s;
+    float2 *dfw = nullptr, *dbw = nullptr;
+    uint8_t* dm = nullptr;
+    unsigned* dn = nullptr;
+    const size_t px = (size_t)w * h;
+    TRY(s.upload(c, &dfw, (const float2*)flow_fw, px));
+    TRY(s.upload(c, &dbw, (const float2*)flow_bw, px));
+    TRY(s.alloc(c, &dm, px));
+    TRY(s.alloc(c, &dn, 1));
+    CK(c, cudaMemsetAsync(dn, 0, sizeof(unsigned), c->s_comp));
+    TRY(launch_fb_check(c, FfbRing{(char*)dfw, 0, 0, 1}, FfbRing{(char*)dbw, 0, 0, 1}, w, w, h, FfbRing{(char*)dm, 0, 0, 1}, w,
+                        dn, (float)alpha, (float)beta, 1));
+    CK(c, cudaStreamSynchronize(c->s_comp));
+    unsigned n = 0;
+    CK(c, cudaMemcpy(&n, dn, sizeof(unsigned), cudaMemcpyDeviceToHost));
+    if (mask) CK(c, cudaMemcpy(mask, dm, px, cudaMemcpyDeviceToHost));
+    if (n_consistent) *n_consistent = n;
     return FFB_OK;
 }
 

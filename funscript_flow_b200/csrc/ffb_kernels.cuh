@@ -739,7 +739,9 @@ __device__ __forceinline__ float2 ffb_solve(float s0, float s1, float s2, float 
 
 // PS (pair stride): pair j reads the expansions in ring elements PS*j and PS*j + 1.  1: consecutive frames of a bracket
 // (frame j+1 is `next` of pair j and `prev` of pair j+1); 2: independent pairs, staged as prev_0, next_0, prev_1, ...
-template <int NT, int U, int MINB, bool UP2X, int HO, int PS>
+// REV (slot order): pair j reads element PS*j + REV as R0 and PS*j + !REV as R1; REV = true is the backward flow of a
+// bracket pair (frame j+1 -> frame j).
+template <int NT, int U, int MINB, bool UP2X, int HO, int PS, bool REV>
 __global__ void __launch_bounds__(NT, MINB) k_flow_iter(FfbIterArgs a) {
     static_assert(HO == 4 || HO == 8, "outputs per horizontal task");
     static_assert(U == 2 || U == 4, "rows per step");
@@ -752,8 +754,8 @@ __global__ void __launch_bounds__(NT, MINB) k_flow_iter(FfbIterArgs a) {
     RingT ring = reinterpret_cast<RingT>(smem_f + NB * U * HL::RSTRIDE);   // [FFB_WIN][5][NT]
     const int tid = threadIdx.x;
     const int pair = blockIdx.x;      // fastest-varying: see the launcher
-    const float4* A0 = reinterpret_cast<const float4*>(ffb_ring_at(a.R, PS * pair));
-    const float4* A1 = reinterpret_cast<const float4*>(ffb_ring_at(a.R, PS * pair + 1));
+    const float4* A0 = reinterpret_cast<const float4*>(ffb_ring_at(a.R, PS * pair + (REV ? 1 : 0)));
+    const float4* A1 = reinterpret_cast<const float4*>(ffb_ring_at(a.R, PS * pair + (REV ? 0 : 1)));
     const float* B0 = reinterpret_cast<const float*>(A0 + a.plane);
     const float* B1 = reinterpret_cast<const float*>(A1 + a.plane);
     const float2* fin = a.fin ? a.fin + (size_t)pair * a.fin_stride : nullptr;
@@ -987,14 +989,14 @@ struct FfbMatrixArgs {
     float* M; size_t m_stride;                       // per pair: 5 planes of `plane` floats
 };
 
-template <int PS>   // pair stride, as k_flow_iter's
+template <int PS, bool REV>   // pair stride and slot order, as k_flow_iter's
 __global__ void __launch_bounds__(256) k_flow_matrices(FfbMatrixArgs a) {
     const int x = blockIdx.x * 32 + (threadIdx.x & 31);
     const int y = blockIdx.y * 8 + (threadIdx.x >> 5);
     if (x >= a.w || y >= a.h) return;
     const int pair = blockIdx.z;
-    const float4* A0 = reinterpret_cast<const float4*>(ffb_ring_at(a.R, PS * pair));
-    const float4* A1 = reinterpret_cast<const float4*>(ffb_ring_at(a.R, PS * pair + 1));
+    const float4* A0 = reinterpret_cast<const float4*>(ffb_ring_at(a.R, PS * pair + (REV ? 1 : 0)));
+    const float4* A1 = reinterpret_cast<const float4*>(ffb_ring_at(a.R, PS * pair + (REV ? 0 : 1)));
     const float* B0 = reinterpret_cast<const float*>(A0 + a.plane);
     const float* B1 = reinterpret_cast<const float*>(A1 + a.plane);
     const float2 d = a.fin ? __ldg(a.fin + (size_t)pair * a.fin_stride + (size_t)y * a.fip + x) : make_float2(0.f, 0.f);
@@ -1062,6 +1064,60 @@ __global__ void __launch_bounds__(BOX_NT) k_box_solve(FfbBoxArgs a) {
             for (int c = 0; c < 5; ++c)
                 vs[c] += (double)__ldg(pin + (size_t)c * a.plane) - (double)__ldg(pout + (size_t)c * a.plane);
         }
+    }
+}
+
+// ======================================================================================
+// K3b forward-backward consistency of pairs whose forward and backward final flows are resident
+// ======================================================================================
+// Sundaram, Brox & Keutzer (ECCV 2010).  One thread per pixel (x, y) of pair j: the forward flow f sends it to
+// t = (x + fx, y + fy).  A target outside [0, w-1] x [0, h-1] (NaN included) is inconsistent; otherwise the backward
+// flow is sampled bilinearly at t (b) and the pixel is consistent when |f + b|^2 <= alpha (|f|^2 + |b|^2) + beta.
+// Every operation is one fp32 rounding in this order, with no contraction, so that a float32 restatement gives the same
+// bits; the consistent pixels of a pair are counted with integer atomics, so the count is deterministic.
+struct FfbCheckArgs {
+    FfbRing fw, bw; int fp;     // forward / backward flows (element = pair), pitch in float2
+    int w, h;
+    FfbRing mask; int mp;       // mask bytes 1 / 0 (element = pair), pitch in bytes; mask.base NULL: no mask
+    unsigned* count;            // consistent pixels of pair j added to count[j] (NULL: not counted)
+    float alpha, beta;
+};
+
+__global__ void __launch_bounds__(256) k_fb_check(FfbCheckArgs a) {
+    const int x = blockIdx.x * 32 + (threadIdx.x & 31);
+    const int y = blockIdx.y * 8 + (threadIdx.x >> 5);
+    const int pair = blockIdx.z;
+    bool ok = false;
+    if (x < a.w && y < a.h) {
+        const float2* F = reinterpret_cast<const float2*>(ffb_ring_at(a.fw, pair));
+        const float2* Bk = reinterpret_cast<const float2*>(ffb_ring_at(a.bw, pair));
+        const float2 f = __ldg(F + (size_t)y * a.fp + x);
+        const float tx = __fadd_rn((float)x, f.x), ty = __fadd_rn((float)y, f.y);
+        if (tx >= 0.f && tx <= (float)(a.w - 1) && ty >= 0.f && ty <= (float)(a.h - 1)) {
+            const float x0f = floorf(tx), y0f = floorf(ty);
+            const int x0 = (int)x0f, y0 = (int)y0f;
+            const int x1 = min(x0 + 1, a.w - 1), y1 = min(y0 + 1, a.h - 1);
+            const float ax = __fsub_rn(tx, x0f), ay = __fsub_rn(ty, y0f);
+            const float rx = __fsub_rn(1.f, ax), ry = __fsub_rn(1.f, ay);
+            const float2 b00 = __ldg(Bk + (size_t)y0 * a.fp + x0), b01 = __ldg(Bk + (size_t)y0 * a.fp + x1);
+            const float2 b10 = __ldg(Bk + (size_t)y1 * a.fp + x0), b11 = __ldg(Bk + (size_t)y1 * a.fp + x1);
+            const float bx = __fadd_rn(__fmul_rn(__fadd_rn(__fmul_rn(b00.x, rx), __fmul_rn(b01.x, ax)), ry),
+                                       __fmul_rn(__fadd_rn(__fmul_rn(b10.x, rx), __fmul_rn(b11.x, ax)), ay));
+            const float by = __fadd_rn(__fmul_rn(__fadd_rn(__fmul_rn(b00.y, rx), __fmul_rn(b01.y, ax)), ry),
+                                       __fmul_rn(__fadd_rn(__fmul_rn(b10.y, rx), __fmul_rn(b11.y, ax)), ay));
+            const float ex = __fadd_rn(f.x, bx), ey = __fadd_rn(f.y, by);
+            const float e = __fadd_rn(__fmul_rn(ex, ex), __fmul_rn(ey, ey));
+            const float nf = __fadd_rn(__fmul_rn(f.x, f.x), __fmul_rn(f.y, f.y));
+            const float nb = __fadd_rn(__fmul_rn(bx, bx), __fmul_rn(by, by));
+            ok = e <= __fadd_rn(__fmul_rn(a.alpha, __fadd_rn(nf, nb)), a.beta);
+        }
+        if (a.mask.base) ffb_ring_at(a.mask, pair)[(size_t)y * a.mp + x] = ok ? 1 : 0;
+    }
+    if (a.count) {      // a warp is one row of 32 pixels: one atomic per warp
+        unsigned n = ok ? 1u : 0u;
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) n += __shfl_xor_sync(0xffffffffu, n, o);
+        if ((threadIdx.x & 31) == 0 && n) atomicAdd(a.count + pair, n);
     }
 }
 

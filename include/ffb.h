@@ -208,6 +208,30 @@ int  ffb_farneback_sequence(ffb_ctx* ctx, const uint8_t* frames, int n_frames, i
                             double cut_threshold, double* scalar, uint8_t* cut, int32_t* cx, int32_t* cy, float* val,
                             float* mean_mag, double* centers, void* stream);
 
+/* ---- sequences with backward flows and a forward-backward consistency mask --------------------------------------
+ * ffb_farneback_sequence for pair j = (frame j, frame j+1), plus its backward flow (frame j+1 -> frame j) and the
+ * forward-backward check (Sundaram, Brox & Keutzer, ECCV 2010).  Outputs may be NULL:
+ *   flow_fw      pair j's flow at flow_fw + j*flow_stride (rows flow_pitch bytes apart): ffb_farneback_sequence's flow
+ *   flow_bw      the backward flow, same layout: bit-identical to ffb_farneback(frame j+1, frame j)
+ *   mask         uint8 [height][width] per pair at mask + j*mask_stride (rows mask_pitch bytes apart): 1 where the
+ *                pixel is consistent, 0 otherwise
+ *   n_consistent int64 per pair (host array): the number of mask bytes that are 1
+ * A pixel (x, y) with forward flow f is consistent when its target t = (x + fx, y + fy) lies in [0, width-1] x
+ * [0, height-1] and the backward flow b sampled there bilinearly satisfies |f + b|^2 <= alpha (|f|^2 + |b|^2) + beta
+ * (alpha and beta rounded to float32; every operation one float32 rounding, no contraction; the reference values are
+ * alpha 0.01, beta 0.5).  Each frame is expanded once: the backward flows re-use the expansions of the forward pass.
+ * frames, the flows and the mask may each be pageable host, pinned host or device memory (of the context's device).
+ * Configuration and the stream contract are ffb_farneback_sequence's (a ring of 2*batch_frames + 8 pairs with a flow or
+ * mask output); the backward ring, the mask ring and the counts are allocated by the first call that needs them and
+ * only grow.  There are no per-pair bracket results.  The flows of an earlier bracket are no longer resident.
+ * FFB_E_INVALID for everything ffb_farneback_sequence refuses, mask_pitch < width, mask_stride shorter than a mask, and
+ * alpha or beta negative or not finite; n_frames of 0 or 1 does nothing. */
+int  ffb_farneback_sequence_bidir(ffb_ctx* ctx, const uint8_t* frames, int n_frames, int width, int height,
+                                  size_t pitch, size_t frame_stride,
+                                  float* flow_fw, float* flow_bw, size_t flow_pitch, size_t flow_stride,
+                                  uint8_t* mask, size_t mask_pitch, size_t mask_stride,
+                                  double alpha, double beta, int64_t* n_consistent, void* stream);
+
 /* ---- per-stage hooks (each runs exactly the production kernel of that stage, for the context's parameters) -----
  * Level geometry of the Farneback pyramid for a frame size with the reference's pyr_scale 0.5, levels 3 (coarsest
  * level first): fills up to 4 entries of w[], h[], ksize[], sigma[]; returns the level count in *n_levels. */
@@ -226,6 +250,10 @@ int  ffb_stage_flow_iter(ffb_ctx* ctx, const float* R0, const float* R1, const f
                          int w, int h, float* flow_out);
 /* A1e: coarse flow [hc][wc][2] -> [h][w][2], bilinear, x (1 / the context's pyr_scale). */
 int  ffb_stage_upsample_flow(ffb_ctx* ctx, const float* flow_c, int wc, int hc, int w, int h, float* out);
+/* Forward-backward check of one pair (ffb_farneback_sequence_bidir's k_fb_check): forward and backward flows
+ * [h][w][2] -> mask [h][w] (1 consistent, 0 not) and its count; mask and n_consistent may be NULL. */
+int  ffb_stage_fb_check(ffb_ctx* ctx, const float* flow_fw, const float* flow_bw, int w, int h, double alpha,
+                        double beta, uint8_t* mask, int64_t* n_consistent);
 
 /* ---- frame pre-processing on the device (SURVEY row N2; replaces F:173-189 + F:1074-1082) ------
  * Decoded BGR frames (3 bytes per pixel, as cv2.VideoCapture returns them) are resized to 256 x 256
@@ -262,7 +290,8 @@ int  ffb_stage_preprocess_window(ffb_ctx* ctx, const uint8_t* bgr, int width, in
 #define FFB_K_RADIAL    5
 #define FFB_K_SMALL     6   /* finish / centre-smoothing kernels */
 #define FFB_K_PREPROC   7
-#define FFB_K_COUNT     8
+#define FFB_K_FB_CHECK  8   /* forward-backward consistency check */
+#define FFB_K_COUNT     9
 /* When enabled, every launch of the kernels above is bracketed by CUDA events on the compute
  * stream; ffb_kernel_stats returns launches, summed device milliseconds and the algorithmic
  * bytes those launches moved (DESIGN.md section "bytes per unit") since the last reset. */

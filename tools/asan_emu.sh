@@ -28,6 +28,18 @@ for (w, h, b) in [(97, 70, 3), (33, 20, 16)]:   # sequences that wrap the final-
     ctx.farneback_sequence_ptr(seq.ctypes.data, 41, w, h, w, w * h, flow.ctypes.data, (w + 3) * 8, (h + 1) * (w + 3) * 8)
     assert np.array_equal(flow[:, :h, :w], r["flow"])
     print(w, h, "sequence ok", float(np.sum(r["scalar"])))
+    # backward flows, masks and counts through the same wrapping rings, into pitched buffers
+    b = ctx.farneback_sequence_bidir(seq)
+    assert np.array_equal(b["flow"], r["flow"])
+    bw = np.zeros((40, h + 1, w + 3, 2), np.float32)
+    mask = np.zeros((40, h + 2, w + 5), np.uint8)
+    cnt = ctx.farneback_sequence_bidir_ptr(seq.ctypes.data, 41, w, h, w, w * h, 0, bw.ctypes.data, (w + 3) * 8,
+                                           (h + 1) * (w + 3) * 8, mask.ctypes.data, w + 5, (h + 2) * (w + 5), counts=True)
+    assert np.array_equal(bw[:, :h, :w], b["flow_bw"]) and np.array_equal(mask[:, :h, :w], b["mask"].view(np.uint8))
+    assert np.array_equal(cnt, b["n_consistent"]) and np.array_equal(cnt, b["mask"].sum(axis=(1, 2)))
+    m, k = ctx.stage_fb_check(b["flow"][3], b["flow_bw"][3])
+    assert np.array_equal(m, b["mask"][3]) and k == cnt[3]
+    print(w, h, "bidirectional ok", int(cnt.sum()))
 pc.check_reductions_random(ctx, n_cases=8, max_side=70)
 pc.check_preprocess(ctx, sizes=((97, 131), (64, 48)))
 pc.check_preprocess_window(ctx)
