@@ -6,7 +6,7 @@ The arithmetic runs only in hand-written CUDA kernels (csrc/) reached through th
 include/ffb.h; importing this package does not need a GPU, calling any processing function does.
 """
 from .api import (BracketPipeline, calc_optical_flow_farneback_batch, calc_optical_flow_farneback_sequence,  # noqa: F401
-                  calc_optical_flow_farneback_sequence_bidirectional,
+                  calc_optical_flow_farneback_batch_bidirectional, calc_optical_flow_farneback_sequence_bidirectional,
                   get_available_backends, get_context, get_gpu_info, max_divergence, precompute_flow_info,
                   precompute_flow_info_batch, precompute_flow_info_gpu, precompute_wrapper, process_bracket,
                   process_bracket_on_contexts, process_sequence, radial_motion_weighted, set_context, smooth_centers)

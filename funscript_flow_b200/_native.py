@@ -70,6 +70,8 @@ def load(path: Optional[str] = None) -> C.CDLL:
                                          f32p, f32p, f64p, vp]),
         "ffb_farneback_sequence_bidir": (i32, [vp, vp, i32, i32, i32, sz, sz, vp, vp, sz, sz, vp, sz, sz, C.c_double,
                                                C.c_double, C.POINTER(C.c_int64), vp]),
+        "ffb_farneback_pairs_bidir": (i32, [vp, vp, vp, i32, i32, i32, sz, sz, vp, vp, sz, sz, vp, sz, sz, C.c_double,
+                                            C.c_double, C.POINTER(C.c_int64), vp]),
         "ffb_max_divergence": (i32, [vp, f32p, i32, i32, i32p, i32p, f32p]),
         "ffb_mean_magnitude": (i32, [vp, f32p, i32, i32, f32p]),
         "ffb_radial_motion": (i32, [vp, f32p, i32, i32, C.c_double, C.c_double, i32, i32, f64p]),
@@ -160,6 +162,26 @@ def _u8(a):
 
 def _f32(a):
     return a.ctypes.data_as(C.POINTER(C.c_float))
+
+
+def _bidir_outputs(n, width, height, flow, flow_bw, flow_pitch, flow_stride, mask, mask_pitch, mask_stride):
+    """The output arguments of a bidirectional call, from pointers (0 = none) with their pitches and strides or from
+    dense NumPy arrays: float32 [n, H, W, 2] flows, a uint8 / bool [n, H, W] mask."""
+    ptrs = []
+    for arr in (flow, flow_bw):
+        if isinstance(arr, np.ndarray):
+            assert arr.dtype == np.float32 and arr.flags.c_contiguous and arr.shape == (n, height, width, 2)
+            flow_pitch, flow_stride = width * 8, width * height * 8
+            ptrs.append(arr.ctypes.data)
+        else:
+            ptrs.append(int(arr or 0))
+    if isinstance(mask, np.ndarray):
+        assert mask.dtype in (np.uint8, np.bool_) and mask.flags.c_contiguous and mask.shape == (n, height, width)
+        mask_ptr, mask_pitch, mask_stride = mask.ctypes.data, width, width * height
+    else:
+        mask_ptr = int(mask or 0)
+    return (C.c_void_p(ptrs[0] or None), C.c_void_p(ptrs[1] or None), int(flow_pitch), int(flow_stride),
+            C.c_void_p(mask_ptr or None), int(mask_pitch), int(mask_stride))
 
 
 class PinnedBuffer:
@@ -521,26 +543,51 @@ class FlowContext:
         (0 = none) or a uint8 / bool NumPy array [n_frames - 1, H, W]; `stream` a cudaStream_t handle (0 = none).
         Returns the int64 consistent-pixel counts with counts=True (the call then waits for the device), else None."""
         n = max(int(n_frames) - 1, 0)
-        ptrs = []
-        for arr in (flow, flow_bw):
-            if isinstance(arr, np.ndarray):
-                assert arr.dtype == np.float32 and arr.flags.c_contiguous and arr.shape == (n, height, width, 2)
-                flow_pitch, flow_stride = width * 8, width * height * 8
-                ptrs.append(arr.ctypes.data)
-            else:
-                ptrs.append(int(arr or 0))
-        if isinstance(mask, np.ndarray):
-            assert mask.dtype in (np.uint8, np.bool_) and mask.flags.c_contiguous and mask.shape == (n, height, width)
-            mask_ptr, mask_pitch, mask_stride = mask.ctypes.data, width, width * height
-        else:
-            mask_ptr = int(mask or 0)
+        out = _bidir_outputs(n, width, height, flow, flow_bw, flow_pitch, flow_stride, mask, mask_pitch, mask_stride)
         cnt = np.empty(max(n, 1), np.int64) if counts else None
         self._ck(self._lib.ffb_farneback_sequence_bidir(
-            self._h, C.c_void_p(frames_ptr), int(n_frames), int(width), int(height), int(pitch), int(frame_stride),
-            C.c_void_p(ptrs[0] or None), C.c_void_p(ptrs[1] or None), int(flow_pitch), int(flow_stride),
-            C.c_void_p(mask_ptr or None), int(mask_pitch), int(mask_stride), float(alpha), float(beta),
-            None if cnt is None else cnt.ctypes.data_as(C.POINTER(C.c_int64)), C.c_void_p(int(stream) or None)))
+            self._h, C.c_void_p(frames_ptr), int(n_frames), int(width), int(height), int(pitch), int(frame_stride), *out,
+            float(alpha), float(beta), None if cnt is None else cnt.ctypes.data_as(C.POINTER(C.c_int64)),
+            C.c_void_p(int(stream) or None)))
         return None if cnt is None else cnt[:n].copy()
+
+    def farneback_pairs_bidir(self, prev: np.ndarray, nxt: np.ndarray, *, forward: bool = True, backward: bool = True,
+                              mask: bool = True, counts: bool = True, alpha: float = 0.01, beta: float = 0.5) -> dict:
+        """farneback_pairs plus, for pair i, the backward flow (nxt[i] -> prev[i]) and the forward-backward consistency
+        check, in one call (ffb_farneback_pairs_bidir; each frame expanded once): {"flow": f32 [n, H, W, 2], "flow_bw":
+        the same, "mask": bool [n, H, W], "n_consistent": int64 [n]}, an output not asked for is None.  "flow" is
+        farneback_pairs', flow_bw[i] is bit-identical to farneback(nxt[i], prev[i]), and the mask and counts are
+        farneback_sequence_bidir's.  Chunks are those of the last configure(), as in farneback_pairs."""
+        prev = np.ascontiguousarray(prev, dtype=np.uint8)
+        nxt = np.ascontiguousarray(nxt, dtype=np.uint8)
+        if prev.shape != nxt.shape or prev.ndim != 3:
+            raise ValueError(f"farneback_pairs_bidir: prev and nxt must be uint8 [n, H, W] of one shape, not {prev.shape} "
+                             f"and {nxt.shape}")
+        n, h, w = prev.shape
+        fw = np.empty((n, h, w, 2), np.float32) if forward else None
+        bw = np.empty((n, h, w, 2), np.float32) if backward else None
+        mk = np.empty((n, h, w), np.uint8) if mask else None
+        cnt = self.farneback_pairs_bidir_ptr(prev.ctypes.data, nxt.ctypes.data, n, w, h, w, w * h, fw, bw, mask=mk,
+                                             counts=counts, alpha=alpha, beta=beta)
+        return {"flow": fw, "flow_bw": bw, "mask": None if mk is None else mk.view(np.bool_), "n_consistent": cnt}
+
+    def farneback_pairs_bidir_ptr(self, prev_ptr: int, next_ptr: int, n: int, width: int, height: int, pitch: int,
+                                  frame_stride: int, flow=None, flow_bw=None, flow_pitch: int = 0, flow_stride: int = 0,
+                                  mask=None, mask_pitch: int = 0, mask_stride: int = 0, stream: int = 0, *,
+                                  counts: bool = False, alpha: float = 0.01, beta: float = 0.5):
+        """Raw-pointer variant of farneback_pairs_bidir, like farneback_pairs_ptr: frames anywhere, `flow` / `flow_bw`
+        pointers (0 = none) sharing flow_pitch / flow_stride, or float32 NumPy arrays [n, H, W, 2]; `mask` a pointer
+        (0 = none) or a uint8 / bool NumPy array [n, H, W]; `stream` a cudaStream_t handle (0 = none).  Returns the int64
+        consistent-pixel counts with counts=True (the call then waits for the device), else None."""
+        n = int(n)
+        out = _bidir_outputs(max(n, 0), width, height, flow, flow_bw, flow_pitch, flow_stride, mask, mask_pitch,
+                             mask_stride)
+        cnt = np.empty(max(n, 1), np.int64) if counts else None
+        self._ck(self._lib.ffb_farneback_pairs_bidir(
+            self._h, C.c_void_p(prev_ptr), C.c_void_p(next_ptr), n, int(width), int(height), int(pitch),
+            int(frame_stride), *out, float(alpha), float(beta),
+            None if cnt is None else cnt.ctypes.data_as(C.POINTER(C.c_int64)), C.c_void_p(int(stream) or None)))
+        return None if cnt is None else cnt[:max(n, 0)].copy()
 
     def max_divergence(self, flow: np.ndarray):
         flow = np.ascontiguousarray(flow, dtype=np.float32)

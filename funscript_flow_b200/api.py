@@ -11,6 +11,8 @@
                                                     cv2's signature (F:878), any parameter set
     calc_optical_flow_farneback_batch(prev, next, None, ...)   the same for n independent pairs ([n, H, W]; NumPy
                                                     arrays or torch CUDA tensors, which stay on the device)
+    calc_optical_flow_farneback_batch_bidirectional(prev, next, None, ...)   the same plus the backward flows and the
+                                                    forward-backward consistency mask ([n, H, W] bool)
     precompute_flow_info_batch(pairs, config)       [precompute_wrapper(p, config) for p in pairs] in one call
     calc_optical_flow_farneback_sequence(frames, None, ...)    the same for every pair of consecutive frames ([n, H, W]
                                                     -> [n - 1, H, W, 2]; each frame expanded once)
@@ -367,6 +369,63 @@ def calc_optical_flow_farneback_batch(prev, next, flow, pyr_scale: float, levels
     ctx.farneback_pairs_ptr(prev.data_ptr(), next.data_ptr(), n, w, h, w, w * h, out.data_ptr(), w * 8, w * h * 8,
                             torch.cuda.current_stream(prev.device).cuda_stream)
     return out
+
+
+def calc_optical_flow_farneback_batch_bidirectional(prev, next, flow, pyr_scale: float, levels: int, winsize: int,
+                                                    iterations: int, poly_n: int, poly_sigma: float, flags: int = 0, *,
+                                                    alpha: float = 0.01, beta: float = 0.5,
+                                                    ctx: Optional[_native.FlowContext] = None):
+    """calc_optical_flow_farneback_batch plus the backward flow of every pair and the forward-backward consistency mask,
+    in one call with each frame expanded once: returns (forward, backward, mask), float32 [n, H, W, 2] twice and bool
+    [n, H, W].  forward[i] is the flow prev[i] -> next[i], backward[i] the flow next[i] -> prev[i]
+    (calc_optical_flow_farneback(next[i], prev[i], ...) bit for bit), and mask[i] is
+    calc_optical_flow_farneback_sequence_bidirectional's: True where the forward target lies in the frame and the
+    backward flow there cancels the forward flow.  For the two eyes of a side-by-side frame it is the left-right check of
+    stereo matching.  Inputs, refusals, the torch path (tensors on the frames' device, ordered on
+    torch.cuda.current_stream(), no host round trip) and the context's batch are calc_optical_flow_farneback_batch's;
+    strided NumPy views are copied to dense frames first.  There are no per-pair results, so max_pairs is not raised."""
+    fn = "calc_optical_flow_farneback_batch_bidirectional"
+    if flow is not None:
+        raise ValueError(f"{fn}: flow must be None (an initial flow is not supported)")
+    ctx = ctx or get_context()
+    tensors = _is_torch_tensor(prev), _is_torch_tensor(next)
+    if tensors[0] != tensors[1]:
+        raise TypeError(f"{fn}: prev and next must both be NumPy arrays or both torch tensors")
+    if tensors[0]:
+        import torch
+        if prev.dtype != torch.uint8 or next.dtype != torch.uint8 or not prev.is_cuda or not next.is_cuda:
+            raise TypeError(f"{fn}: tensors must be torch.uint8 on a CUDA device")
+        if prev.device != next.device or prev.device.index != ctx.device:
+            raise ValueError(f"{fn}: tensors on {prev.device} / {next.device}, the context on cuda:{ctx.device}")
+    else:
+        prev, next = np.asarray(prev), np.asarray(next)
+        if prev.dtype != np.uint8 or next.dtype != np.uint8:
+            raise TypeError(f"{fn}: frames must be uint8")
+        # the call reads dense frames: a strided view (one eye of side-by-side frames, every other frame) is copied first
+        prev, next = np.ascontiguousarray(prev), np.ascontiguousarray(next)
+    if tuple(prev.shape) != tuple(next.shape) or prev.ndim != 3:
+        raise ValueError(f"{fn}: prev and next must be [n, H, W] of one shape, not {tuple(prev.shape)} and "
+                         f"{tuple(next.shape)}")
+    ctx.set_farneback(pyr_scale, levels, winsize, iterations, poly_n, poly_sigma, flags)
+    n, h, w = prev.shape
+    if tensors[0]:
+        prev, next = prev.contiguous(), next.contiguous()
+        fw = torch.empty((n, h, w, 2), dtype=torch.float32, device=prev.device)
+        bw = torch.empty_like(fw)
+        mask = torch.empty((n, h, w), dtype=torch.bool, device=prev.device)
+    else:
+        fw, bw, mask = np.empty((n, h, w, 2), np.float32), np.empty((n, h, w, 2), np.float32), np.empty((n, h, w), np.bool_)
+    if n == 0:
+        return fw, bw, mask
+    ctx.configure(w, h, _pairs_batch(w, h, n), 1)
+    if not tensors[0]:
+        ctx.farneback_pairs_bidir_ptr(prev.ctypes.data, next.ctypes.data, n, w, h, w, w * h, fw, bw, mask=mask, alpha=alpha,
+                                      beta=beta)
+        return fw, bw, mask
+    ctx.farneback_pairs_bidir_ptr(prev.data_ptr(), next.data_ptr(), n, w, h, w, w * h, fw.data_ptr(), bw.data_ptr(), w * 8,
+                                  w * h * 8, mask.data_ptr(), w, w * h, torch.cuda.current_stream(prev.device).cuda_stream,
+                                  alpha=alpha, beta=beta)
+    return fw, bw, mask
 
 
 def _sequence_batch(width: int, height: int, n_frames: int) -> int:

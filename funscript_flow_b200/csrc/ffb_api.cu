@@ -7,8 +7,9 @@
 //     independent pairs as prev_0, next_0, prev_1, ... and reads them with pair stride 2)
 //   --k_flow_iter x iterations per level (flow up-sampling fused, k_upsample_flow otherwise; winsize != 15:
 //     k_flow_matrices + k_box_solve)--> final-flow ring (>= B+8 pairs; ffb_farneback_pairs and ffb_farneback_sequence
-//     copy the flows out of it on s_out, the sequence with a ring of >= 2B+8 pairs; ffb_farneback_sequence_bidir also
-//     runs the reversed pairs into a backward final-flow ring and k_fb_check into a mask ring of the same slots)
+//     copy the flows out of it on s_out, the sequence with a ring of >= 2B+8 pairs; ffb_farneback_sequence_bidir and
+//     ffb_farneback_pairs_bidir also run the reversed pairs into a backward final-flow ring and k_fb_check into a mask
+//     ring of the same slots)
 //   --k_divmag / k_phase1_finish--> per-pair centre, value, mean magnitude, cut flag (device arrays)
 //   --k_smooth_centers / k_radial / k_radial_finish (lagging 6 pairs)--> per-pair scalar
 // and only the 1-D per-pair results are copied back at ffb_bracket_finish.
@@ -251,8 +252,9 @@ struct ffb_ctx {
     size_t r_slot_floats = 0;
     float2* ring = nullptr;
     size_t ring_stride = 0;   // float2 per ring element
-    // ffb_farneback_sequence_bidir, allocated by the first call that needs them: backward final flows and consistency
-    // masks in the slots of the final-flow ring (bw_n / mask_n slots, 0 or ring_n), consistent-pixel counts per pair
+    // ffb_farneback_sequence_bidir / _pairs_bidir, allocated by the first call that needs them (alloc_backward): backward
+    // final flows and consistency masks in the slots of the final-flow ring (bw_n / mask_n slots, 0 or ring_n),
+    // consistent-pixel counts per pair of the call
     float2* ring_bw = nullptr;
     uint8_t* mask_ring = nullptr;
     int bw_n = 0, mask_n = 0;
@@ -615,7 +617,7 @@ int launch_flow_iter_ps(ffb_ctx* c, const FlowIterPlan& p, const FfbIterArgs& a,
 
 // One k_flow_iter launch of plan `p` on `stream`, counted under pyramid level `level` (-1: none).  timed = false inside
 // the sliced flow phase, which is timed as a whole.  pair_stride: 1 (bracket) or 2 (independent pairs); rev: the backward
-// flows of bracket pairs (pair stride 1), see k_flow_iter.
+// flows of the pairs, see k_flow_iter.
 int launch_flow_iter(ffb_ctx* c, const FlowIterPlan& p, int level, cudaStream_t stream, bool timed, FfbRing R, size_t plane,
                      int rp, int w, int h, const float2* fin, size_t fin_stride, int fip, FfbRing fout, int fop, int npairs,
                      const UpSrc* up = nullptr, int pair_stride = 1, bool rev = false) {
@@ -634,7 +636,9 @@ int launch_flow_iter(ffb_ctx* c, const FlowIterPlan& p, int level, cudaStream_t 
     // the kernel stores four flow vectors with one 32-byte instruction
     if (fop % 4 != 0 || ((uintptr_t)fout.base | (uintptr_t)fout.stride) % 32 != 0)
         return fail(c, FFB_E_INVALID, "flow output is not 32-byte aligned (pitch %d, stride %zu)", fop, fout.stride);
-    if (pair_stride == 2) return launch_flow_iter_ps<2, false>(c, p, a, npairs, level, bytes, stream, timed);
+    if (pair_stride == 2)
+        return rev ? launch_flow_iter_ps<2, true>(c, p, a, npairs, level, bytes, stream, timed)
+                   : launch_flow_iter_ps<2, false>(c, p, a, npairs, level, bytes, stream, timed);
     return rev ? launch_flow_iter_ps<1, true>(c, p, a, npairs, level, bytes, stream, timed)
                : launch_flow_iter_ps<1, false>(c, p, a, npairs, level, bytes, stream, timed);
 }
@@ -653,7 +657,8 @@ int launch_flow_unfused(ffb_ctx* c, int level, float* M, FfbRing R, size_t plane
     const double px = (double)npairs * w * h;
     const ProfMark pm = prof_begin(c, FFB_K_FLOW_ITER, level, px * ((fin ? 48.0 : 40.0) + 20.0), c->s_comp);
     const dim3 mgrid((w + 31) / 32, (h + 7) / 8, npairs);
-    auto kfn = pair_stride == 2 ? k_flow_matrices<2, false> : (rev ? k_flow_matrices<1, true> : k_flow_matrices<1, false>);
+    auto kfn = pair_stride == 2 ? (rev ? k_flow_matrices<2, true> : k_flow_matrices<2, false>)
+                                : (rev ? k_flow_matrices<1, true> : k_flow_matrices<1, false>);
     FFB_LAUNCH(kfn, mgrid, dim3(256), 0, c->s_comp, m);
     prof_end(pm);
     CKL(c);
@@ -942,8 +947,8 @@ int launch_divmag(ffb_ctx* c, int p0, int off, int cnt, cudaStream_t stream) {
 // Final flows of np pairs into final-flow ring slots f0 .. (mod ring_n), and their divergence / magnitude partials
 // (divmag = false: flows only).  Pair j reads the expansions in slots r0 + pair_stride * j and the one after it
 // (mod S): bracket pairs [p0, p0 + np) are r0 = f0 = p0 with stride 1, a chunk of independent pairs r0 = 0 with
-// stride 2.  backward (bracket pairs, divmag = false): the flows of the reversed pairs (R0 = the later frame) into the
-// same slots of the backward final-flow ring.
+// stride 2.  backward (divmag = false): the flows of the reversed pairs (R0 = the later frame of a bracket pair, `next`
+// of an independent pair) into the same slots of the backward final-flow ring.
 int flow_pairs(ffb_ctx* c, int r0, int pair_stride, int f0, int np, bool divmag = true, bool backward = false) {
     // The pairs of a batch are split in two slices whose launch chains run on two streams, so that the short
     // coarse-level launches (and the tail of every launch) of one slice overlap the other slice's work (+4 %; 3-4 slices
@@ -1164,12 +1169,25 @@ int upload_frames(ffb_ctx* c, uint8_t* dst, uint8_t* pin, cudaEvent_t ev_dma, cu
     return FFB_OK;
 }
 
-// Backward pass of a sequence (ffb_farneback_sequence_bidir): after the forward flows of a batch, the backward flows
-// into the backward final-flow ring and, with a mask or counts, k_fb_check into the mask ring / the per-pair counts.
+// Backward pass of a bidirectional call (ffb_farneback_sequence_bidir, ffb_farneback_pairs_bidir): after the forward
+// flows of a batch or chunk, the backward flows into the backward final-flow ring and, with a mask or counts,
+// k_fb_check into the mask ring / the per-pair counts.
 struct Backward {
     bool mask = false, count = false;
     float alpha = 0.f, beta = 0.f;
 };
+
+// The backward pass of np pairs whose forward flows are in final-flow ring slots f0 .. (flow_pairs' r0 / pair_stride /
+// f0): their counts go to d_ncons[n0 .. n0 + np).
+int backward_pass(ffb_ctx* c, const Backward& bw, int r0, int pair_stride, int f0, int np, int n0) {
+    TRY(flow_pairs(c, r0, pair_stride, f0, np, false, true));
+    if (!bw.mask && !bw.count) return FFB_OK;
+    const size_t fs = c->ring_stride * sizeof(float2), ms = (size_t)c->W * c->H;
+    const int s0 = f0 % c->ring_n;
+    return launch_fb_check(c, FfbRing{(char*)c->ring, fs, s0, c->ring_n}, FfbRing{(char*)c->ring_bw, fs, s0, c->ring_n},
+                           c->fp0, c->W, c->H, FfbRing{bw.mask ? (char*)c->mask_ring : nullptr, ms, s0, c->ring_n}, c->W,
+                           bw.count ? c->d_ncons + n0 : nullptr, bw.alpha, bw.beta, np);
+}
 
 // One batch of the open bracket (or sequence): upload, expansion, final flows and, with stats, the per-pair results
 // and the radial pass lagging 6 pairs.  stats = false computes the flows only (ffb_farneback_sequence without per-pair
@@ -1201,15 +1219,7 @@ int process_batch(ffb_ctx* c, const uint8_t* frames, int nb, size_t pitch, size_
             return fail(c, FFB_E_INVALID, "shard exceeds the %d pairs announced to ffb_bracket_begin_shard", c->ring_n);
         TRY(flow_pairs(c, p0, 1, p0, np, stats));
         if (stats) TRY(launch_phase1_finish(c, p0, p0, np, c->pov, c->thr));
-        if (bw) {
-            TRY(flow_pairs(c, p0, 1, p0, np, false, true));
-            const size_t fs = c->ring_stride * sizeof(float2), ms = (size_t)c->W * c->H;
-            const int s0 = p0 % c->ring_n;
-            if (bw->mask || bw->count)
-                TRY(launch_fb_check(c, FfbRing{(char*)c->ring, fs, s0, c->ring_n}, FfbRing{(char*)c->ring_bw, fs, s0, c->ring_n},
-                                    c->fp0, c->W, c->H, FfbRing{bw->mask ? (char*)c->mask_ring : nullptr, ms, s0, c->ring_n},
-                                    c->W, bw->count ? c->d_ncons + p0 : nullptr, bw->alpha, bw->beta, np));
-        }
+        if (bw) TRY(backward_pass(c, *bw, p0, 1, p0, np, p0));
         c->pairs_done += np;
         const int r1 = c->pairs_done - 6;
         if (stats && !c->deferred && r1 > c->radial_done) {
@@ -1768,52 +1778,128 @@ static int copy_slots_out(ffb_ctx* c, const SlotImages& r, int s0, int np, char*
     return FFB_OK;
 }
 
+// Kind of memory of a caller's buffer (PTR_DEVICE for NULL); device memory must be on the context's device.  `what`
+// names the buffer with its verb ("frames are", "flow is") for the message.
+static int buffer_kind(ffb_ctx* c, const char* fn, const char* what, const void* p, PtrKind* kind) {
+    int dev = c->device;
+    *kind = p ? classify(p, &dev) : PTR_DEVICE;
+    if (*kind == PTR_DEVICE && dev != c->device)
+        return fail(c, FFB_E_INVALID, "%s: %s on device %d, the context on device %d", fn, what, dev, c->device);
+    return FFB_OK;
+}
+
+// Outputs of a pairs or sequence call that leave the final-flow rings (each may be NULL) and the memory each is in.
+struct RingOut {
+    float *flow = nullptr, *flow_bw = nullptr;
+    size_t flow_pitch = 0, flow_stride = 0;
+    uint8_t* mask = nullptr;
+    size_t mask_pitch = 0, mask_stride = 0;
+    PtrKind kf = PTR_DEVICE, kb = PTR_DEVICE, km = PTR_DEVICE;
+    bool any() const { return flow || flow_bw || mask; }
+};
+
+// Copy on s_out of ring slots s .. s + m - 1 (no wrap) of every output of `o` to pairs i .. i + m - 1 of its buffer.
+static int copy_outputs(ffb_ctx* c, const RingOut& o, int s, int m, int i) {
+    if (o.flow)
+        TRY(copy_slots_out(c, flow_slots(c, c->ring), s, m, (char*)o.flow + (size_t)i * o.flow_stride, o.flow_pitch,
+                           o.flow_stride, o.kf));
+    if (o.flow_bw)
+        TRY(copy_slots_out(c, flow_slots(c, c->ring_bw), s, m, (char*)o.flow_bw + (size_t)i * o.flow_stride, o.flow_pitch,
+                           o.flow_stride, o.kb));
+    if (o.mask)
+        TRY(copy_slots_out(c, mask_slots(c), s, m, (char*)o.mask + (size_t)i * o.mask_stride, o.mask_pitch, o.mask_stride,
+                           o.km));
+    return FFB_OK;
+}
+
+// The mask and check arguments of a bidirectional call (fn: its name in the messages) of n_pairs >= 1 pairs.
+static int check_bidir_args(ffb_ctx* c, const char* fn, int n_pairs, int width, int height, const uint8_t* mask,
+                            size_t mask_pitch, size_t mask_stride, double alpha, double beta) {
+    if (mask && mask_pitch < (size_t)width)
+        return fail(c, FFB_E_INVALID, "%s: mask_pitch %zu below the width %d", fn, mask_pitch, width);
+    if (mask && n_pairs > 1 && mask_stride < mask_pitch * (size_t)(height - 1) + width)
+        return fail(c, FFB_E_INVALID, "%s: mask_stride %zu shorter than a mask", fn, mask_stride);
+    if (!(alpha >= 0.0 && isfinite(alpha)) || !(beta >= 0.0 && isfinite(beta)))
+        return fail(c, FFB_E_INVALID, "%s: alpha %g and beta %g must be finite and >= 0", fn, alpha, beta);
+    return FFB_OK;
+}
+
+// The backward ring (flows), the mask ring (mask) and n_counts per-pair counts of a bidirectional call: grow-only,
+// allocated by the first call that needs them (a new frame size or a larger final-flow ring frees the rings).
+static int alloc_backward(ffb_ctx* c, bool flows, bool mask, int n_counts) {
+    if (flows && c->bw_n < c->ring_n) {
+        dev_free(c->ring_bw);
+        c->bw_n = 0;
+        TRY(dev_alloc(c, &c->ring_bw, (size_t)c->ring_n * c->ring_stride));
+        c->bw_n = c->ring_n;
+    }
+    if (mask && c->mask_n < c->ring_n) {
+        dev_free(c->mask_ring);
+        c->mask_n = 0;
+        TRY(dev_alloc(c, &c->mask_ring, (size_t)c->ring_n * c->W * c->H));
+        c->mask_n = c->ring_n;
+    }
+    if (c->ncons_cap < n_counts) {
+        dev_free(c->d_ncons);
+        c->ncons_cap = 0;
+        TRY(dev_alloc(c, &c->d_ncons, (size_t)n_counts));
+        c->ncons_cap = n_counts;
+    }
+    return FFB_OK;
+}
+
+// End of a bidirectional call of n_pairs pairs (host_in: frames in host memory): with a caller stream and every buffer
+// on the device it returns at once, otherwise when the outputs are complete, with the counts copied out.
+static int finish_bidir(ffb_ctx* c, const RingOut& o, bool host_in, int n_pairs, int64_t* n_consistent, void* stream) {
+    const bool host_io = host_in || o.kf != PTR_DEVICE || o.kb != PTR_DEVICE || o.km != PTR_DEVICE || n_consistent;
+    if (stream && !host_io) return FFB_OK;
+    CK(c, cudaStreamSynchronize(c->s_comp));
+    if (n_consistent) {
+        std::vector<unsigned> h((size_t)n_pairs);
+        CK(c, cudaMemcpy(h.data(), c->d_ncons, (size_t)n_pairs * sizeof(unsigned), cudaMemcpyDeviceToHost));
+        for (int j = 0; j < n_pairs; ++j) n_consistent[j] = h[j];
+    }
+    return FFB_OK;
+}
+
+// The frame and flow arguments of an independent-pairs call (fn: its name in the messages), n_pairs >= 1.
+static int check_pairs_args(ffb_ctx* c, const char* fn, const uint8_t* prev, const uint8_t* next, int n_pairs, int width,
+                            int height, size_t pitch, size_t frame_stride, bool flow, size_t flow_pitch, size_t flow_stride) {
+    if (!prev || !next || width < 1 || height < 1) return fail(c, FFB_E_INVALID, "%s: bad frames (%dx%d)", fn, width, height);
+    if (pitch < (size_t)width) return fail(c, FFB_E_INVALID, "%s: pitch %zu below the width %d", fn, pitch, width);
+    if (n_pairs > 1 && frame_stride < pitch * (size_t)(height - 1) + width)
+        return fail(c, FFB_E_INVALID, "%s: frame_stride %zu shorter than a frame", fn, frame_stride);
+    if (flow && flow_pitch < (size_t)width * 8)
+        return fail(c, FFB_E_INVALID, "%s: flow_pitch %zu below 8 * width (%d)", fn, flow_pitch, 8 * width);
+    if (flow && n_pairs > 1 && flow_stride < flow_pitch * (size_t)(height - 1) + (size_t)width * 8)
+        return fail(c, FFB_E_INVALID, "%s: flow_stride %zu shorter than a flow", fn, flow_stride);
+    return FFB_OK;
+}
+
 // Independent pairs: chunks of P = (B + 1) / 2 pairs.  A chunk stages its 2P frames as prev_0, next_0, prev_1, ... in
 // the frame staging buffer and expands them into expansion slots 0 .. 2P-1; the flow phase reads them with pair stride
-// 2.  Consecutive chunks alternate between the final-flow ring slots [0, P) and [P, 2P) (ring_n >= B + 8 > 2P), so the
-// copy-out of one chunk on s_out overlaps the next chunk's kernels.
-int ffb_farneback_pairs(ffb_ctx* c, const uint8_t* prev, const uint8_t* next, int n_pairs, int width, int height,
-                        size_t pitch, size_t frame_stride, float* flow, size_t flow_pitch, size_t flow_stride,
-                        int pov_mode, double cut_threshold, int32_t* cx, int32_t* cy, float* val, float* mean_mag,
-                        uint8_t* cut, void* stream) {
-    if (!c) return FFB_E_INVALID;
-    if (c->in_bracket) return fail(c, FFB_E_INVALID, "ffb_farneback_pairs inside a bracket");
-    if (n_pairs < 0) return fail(c, FFB_E_INVALID, "ffb_farneback_pairs: n_pairs %d < 0", n_pairs);
-    if (n_pairs == 0) return FFB_OK;
-    if (!prev || !next || width < 1 || height < 1)
-        return fail(c, FFB_E_INVALID, "ffb_farneback_pairs: bad frames (%dx%d)", width, height);
-    if (pitch < (size_t)width) return fail(c, FFB_E_INVALID, "ffb_farneback_pairs: pitch %zu below the width %d", pitch, width);
-    if (n_pairs > 1 && frame_stride < pitch * (size_t)(height - 1) + width)
-        return fail(c, FFB_E_INVALID, "ffb_farneback_pairs: frame_stride %zu shorter than a frame", frame_stride);
-    if (flow && flow_pitch < (size_t)width * 8)
-        return fail(c, FFB_E_INVALID, "ffb_farneback_pairs: flow_pitch %zu below 8 * width (%d)", flow_pitch, 8 * width);
-    if (flow && n_pairs > 1 && flow_stride < flow_pitch * (size_t)(height - 1) + (size_t)width * 8)
-        return fail(c, FFB_E_INVALID, "ffb_farneback_pairs: flow_stride %zu shorter than a flow", flow_stride);
-    CK(c, cudaSetDevice(c->device));
-    int dev[3] = {c->device, c->device, c->device};
-    const PtrKind kp = classify(prev, &dev[0]), kn = classify(next, &dev[1]);
-    const PtrKind kf = flow ? classify(flow, &dev[2]) : PTR_DEVICE;
-    const PtrKind kinds[3] = {kp, kn, kf};
-    for (int i = 0; i < 3; ++i)
-        if (kinds[i] == PTR_DEVICE && dev[i] != c->device)
-            return fail(c, FFB_E_INVALID, "ffb_farneback_pairs: %s is on device %d, the context on device %d",
-                        i == 0 ? "prev" : (i == 1 ? "next" : "flow"), dev[i], c->device);
-    const bool stats = cx || cy || val || mean_mag || cut;
-    // the per-pair results of the whole call stay on the device until the end: max_pairs covers n_pairs
-    const int maxPairs = stats && n_pairs > c->maxPairs ? n_pairs : (c->maxPairs > 0 ? c->maxPairs : 1);
-    TRY(configure_checked(c, width, height, c->B > 0 ? c->B : 2, maxPairs, 0));
+// 2, and with `bw` the backward pass reads them again in reverse slot order.  Consecutive chunks alternate between the
+// slots [0, P) and [P, 2P) of the final-flow ring (ring_n >= B + 8 > 2P) and of the backward and mask rings, so the
+// copy-out of one chunk on s_out overlaps the next chunk's kernels.  divmag: k_divmag after the forward flows; stats:
+// also the per-pair results (pov, thr) into the per-pair arrays.  The geometry is configured by the caller; at the end
+// the caller's stream waits for the call.
+static int pairs_loop(ffb_ctx* c, const uint8_t* prev, const uint8_t* next, int n_pairs, size_t pitch, size_t frame_stride,
+                      PtrKind kp, PtrKind kn, const RingOut& o, bool divmag, bool stats, int pov, float thr,
+                      const Backward* bw, void* stream) {
     const int P = (c->B + 1) / 2;
+    const int width = c->W, height = c->H;
     const size_t fbytes = (size_t)width * height;
+    const bool copy = o.any();
     const cudaStream_t us = (cudaStream_t)stream;
     c->pairs_done = 0;   // the final-flow ring no longer holds a bracket's flows
     CK(c, cudaEventRecord(c->ev_user, us));
     CK(c, cudaStreamWaitEvent(c->s_copy, c->ev_user, 0));
     CK(c, cudaStreamWaitEvent(c->s_comp, c->ev_user, 0));
-    // flows of pairs [i0, i0 + np) from ring half `half` to the caller's buffer
+    if (bw && bw->count) CK(c, cudaMemsetAsync(c->d_ncons, 0, (size_t)n_pairs * sizeof(unsigned), c->s_comp));
+    // outputs of pairs [i0, i0 + np) from ring half `half` to the caller's buffers
     auto copy_out = [&](int i0, int np, int half) -> int {
         CK(c, cudaStreamWaitEvent(c->s_out, c->ev_fin[half], 0));
-        TRY(copy_slots_out(c, flow_slots(c, c->ring), half * P, np, (char*)flow + (size_t)i0 * flow_stride, flow_pitch,
-                           flow_stride, kf));
+        TRY(copy_outputs(c, o, half * P, np, i0));
         CK(c, cudaEventRecord(c->ev_out[half], c->s_out));
         return FFB_OK;
     };
@@ -1830,38 +1916,95 @@ int ffb_farneback_pairs(ffb_ctx* c, const uint8_t* prev, const uint8_t* next, in
         c->batch_no++;
         // ring half `half` is free once the copy-out of chunk k - 2 (or of an earlier call) has read it
         CK(c, cudaStreamWaitEvent(c->s_comp, c->ev_out[half], 0));
-        TRY(flow_pairs(c, 0, 2, half * P, np));
-        if (stats) TRY(launch_phase1_finish(c, half * P, i0, np, pov_mode ? 1 : 0, (float)cut_threshold));
-        if (!flow) continue;
+        TRY(flow_pairs(c, 0, 2, half * P, np, divmag));
+        if (stats) TRY(launch_phase1_finish(c, half * P, i0, np, pov, thr));
+        if (bw) TRY(backward_pass(c, *bw, 0, 2, half * P, np, i0));
+        if (!copy) continue;
         CK(c, cudaEventRecord(c->ev_fin[half], c->s_comp));
         // issued one chunk late: a copy into pageable memory returns only when it is done
         if (pend_i0 >= 0) TRY(copy_out(pend_i0, pend_np, pend_half));
         pend_i0 = i0; pend_np = np; pend_half = half;
     }
     if (pend_i0 >= 0) TRY(copy_out(pend_i0, pend_np, pend_half));
-    if (flow) {   // later work of the context (a bracket, the next call) overwrites the ring after the copy-out
+    if (copy) {   // later work of the context (a bracket, the next call) overwrites the rings after the copy-out
         CK(c, cudaEventRecord(c->ev_done, c->s_out));
         CK(c, cudaStreamWaitEvent(c->s_comp, c->ev_done, 0));
     }
     // s_comp has waited for every upload and copy-out: the caller's stream continues when the inputs have been read
-    // and the flows written
+    // and the outputs written
     CK(c, cudaEventRecord(c->ev_done, c->s_comp));
     CK(c, cudaStreamWaitEvent(us, c->ev_done, 0));
-    const bool host_io = kp != PTR_DEVICE || kn != PTR_DEVICE || kf != PTR_DEVICE || stats;
+    return FFB_OK;
+}
+
+int ffb_farneback_pairs(ffb_ctx* c, const uint8_t* prev, const uint8_t* next, int n_pairs, int width, int height,
+                        size_t pitch, size_t frame_stride, float* flow, size_t flow_pitch, size_t flow_stride,
+                        int pov_mode, double cut_threshold, int32_t* cx, int32_t* cy, float* val, float* mean_mag,
+                        uint8_t* cut, void* stream) {
+    static const char* fn = "ffb_farneback_pairs";
+    if (!c) return FFB_E_INVALID;
+    if (c->in_bracket) return fail(c, FFB_E_INVALID, "ffb_farneback_pairs inside a bracket");
+    if (n_pairs < 0) return fail(c, FFB_E_INVALID, "ffb_farneback_pairs: n_pairs %d < 0", n_pairs);
+    if (n_pairs == 0) return FFB_OK;
+    TRY(check_pairs_args(c, fn, prev, next, n_pairs, width, height, pitch, frame_stride, flow, flow_pitch, flow_stride));
+    CK(c, cudaSetDevice(c->device));
+    PtrKind kp, kn;
+    RingOut o;
+    o.flow = flow; o.flow_pitch = flow_pitch; o.flow_stride = flow_stride;
+    TRY(buffer_kind(c, fn, "prev is", prev, &kp));
+    TRY(buffer_kind(c, fn, "next is", next, &kn));
+    TRY(buffer_kind(c, fn, "flow is", flow, &o.kf));
+    const bool stats = cx || cy || val || mean_mag || cut;
+    // the per-pair results of the whole call stay on the device until the end: max_pairs covers n_pairs
+    const int maxPairs = stats && n_pairs > c->maxPairs ? n_pairs : (c->maxPairs > 0 ? c->maxPairs : 1);
+    TRY(configure_checked(c, width, height, c->B > 0 ? c->B : 2, maxPairs, 0));
+    TRY(pairs_loop(c, prev, next, n_pairs, pitch, frame_stride, kp, kn, o, true, stats, pov_mode ? 1 : 0,
+                   (float)cut_threshold, nullptr, stream));
+    const bool host_io = kp != PTR_DEVICE || kn != PTR_DEVICE || o.kf != PTR_DEVICE || stats;
     if (stream && !host_io) return FFB_OK;
     if (stats) return fetch_results(c, n_pairs, false, nullptr, cut, cx, cy, val, mean_mag, nullptr);
     CK(c, cudaStreamSynchronize(c->s_comp));
     return FFB_OK;
 }
 
-// Kind of memory of a caller's buffer (PTR_DEVICE for NULL); device memory must be on the context's device.  `what`
-// names the buffer with its verb ("frames are", "flow is") for the message.
-static int buffer_kind(ffb_ctx* c, const char* fn, const char* what, const void* p, PtrKind* kind) {
-    int dev = c->device;
-    *kind = p ? classify(p, &dev) : PTR_DEVICE;
-    if (*kind == PTR_DEVICE && dev != c->device)
-        return fail(c, FFB_E_INVALID, "%s: %s on device %d, the context on device %d", fn, what, dev, c->device);
-    return FFB_OK;
+// Independent pairs with the backward flow of every pair as well: after the forward flows of a chunk (no k_divmag: there
+// are no per-pair results), a second flow_pairs with the slot order reversed (R0 = next_i, R1 = prev_i, the chunk's
+// expansions still in their slots) into the backward final-flow ring, then k_fb_check of the chunk into the mask ring
+// and the per-pair counts.  The three rings share their slots, and the fences of ffb_farneback_pairs cover the three
+// copy-outs of a chunk.
+int ffb_farneback_pairs_bidir(ffb_ctx* c, const uint8_t* prev, const uint8_t* next, int n_pairs, int width, int height,
+                              size_t pitch, size_t frame_stride, float* flow_fw, float* flow_bw, size_t flow_pitch,
+                              size_t flow_stride, uint8_t* mask, size_t mask_pitch, size_t mask_stride, double alpha,
+                              double beta, int64_t* n_consistent, void* stream) {
+    static const char* fn = "ffb_farneback_pairs_bidir";
+    if (!c) return FFB_E_INVALID;
+    if (c->in_bracket) return fail(c, FFB_E_INVALID, "ffb_farneback_pairs_bidir inside a bracket");
+    if (n_pairs < 0) return fail(c, FFB_E_INVALID, "ffb_farneback_pairs_bidir: n_pairs %d < 0", n_pairs);
+    if (n_pairs == 0) return FFB_OK;
+    TRY(check_pairs_args(c, fn, prev, next, n_pairs, width, height, pitch, frame_stride, flow_fw || flow_bw, flow_pitch,
+                         flow_stride));
+    TRY(check_bidir_args(c, fn, n_pairs, width, height, mask, mask_pitch, mask_stride, alpha, beta));
+    CK(c, cudaSetDevice(c->device));
+    PtrKind kp, kn;
+    RingOut o;
+    o.flow = flow_fw; o.flow_bw = flow_bw; o.flow_pitch = flow_pitch; o.flow_stride = flow_stride;
+    o.mask = mask; o.mask_pitch = mask_pitch; o.mask_stride = mask_stride;
+    TRY(buffer_kind(c, fn, "prev is", prev, &kp));
+    TRY(buffer_kind(c, fn, "next is", next, &kn));
+    TRY(buffer_kind(c, fn, "flow_fw is", flow_fw, &o.kf));
+    TRY(buffer_kind(c, fn, "flow_bw is", flow_bw, &o.kb));
+    TRY(buffer_kind(c, fn, "mask is", mask, &o.km));
+    TRY(configure_checked(c, width, height, c->B > 0 ? c->B : 2, c->maxPairs > 0 ? c->maxPairs : 1, 0));
+    const bool backward = flow_bw || mask || n_consistent;
+    TRY(alloc_backward(c, backward, mask != nullptr, n_consistent ? n_pairs : 0));
+    Backward bw;
+    bw.mask = mask != nullptr;
+    bw.count = n_consistent != nullptr;
+    bw.alpha = (float)alpha;
+    bw.beta = (float)beta;
+    TRY(pairs_loop(c, prev, next, n_pairs, pitch, frame_stride, kp, kn, o, false, false, 0, 0.f, backward ? &bw : nullptr,
+                   stream));
+    return finish_bidir(c, o, kp != PTR_DEVICE || kn != PTR_DEVICE, n_pairs, n_consistent, stream);
 }
 
 // The frame and flow arguments of a sequence call (fn: its name in the messages), n_frames >= 2.
@@ -1878,16 +2021,6 @@ static int check_sequence_args(ffb_ctx* c, const char* fn, const uint8_t* frames
     return FFB_OK;
 }
 
-// Outputs of a sequence call that leave the final-flow rings (each may be NULL) and the memory each is in.
-struct SequenceOut {
-    float *flow = nullptr, *flow_bw = nullptr;
-    size_t flow_pitch = 0, flow_stride = 0;
-    uint8_t* mask = nullptr;
-    size_t mask_pitch = 0, mask_stride = 0;
-    PtrKind kf = PTR_DEVICE, kb = PTR_DEVICE, km = PTR_DEVICE;
-    bool any() const { return flow || flow_bw || mask; }
-};
-
 // Consecutive pairs of a sequence: one bracket over the n_frames frames (the batches of ffb_bracket_push, with the
 // ramp for host input; every frame expanded once; flow_pairs with pair stride 1), whose final flows -- and with `bw` the
 // backward flows and masks in the same slots of their rings -- are also copied out.  Pair p sits in ring slot
@@ -1897,7 +2030,7 @@ struct SequenceOut {
 // it waits for the copy-out of batch k - 1 (ev_out[(k + 1) & 1]).  The radial pass runs on s_comp, in order with every
 // later write.  The geometry is configured by the caller; at the end the caller's stream waits for the call.
 static int sequence_loop(ffb_ctx* c, const uint8_t* frames, int n_frames, size_t pitch, size_t frame_stride, PtrKind kfr,
-                         const SequenceOut& o, bool stats, const Backward* bw, void* stream) {
+                         const RingOut& o, bool stats, const Backward* bw, void* stream) {
     const int n_pairs = n_frames - 1;
     const bool copy = o.any();
     const cudaStream_t us = (cudaStream_t)stream;
@@ -1914,15 +2047,7 @@ static int sequence_loop(ffb_ctx* c, const uint8_t* frames, int n_frames, size_t
         CK(c, cudaStreamWaitEvent(c->s_out, c->ev_fin[par], 0));
         for (int p = p0; p < p0 + np;) {
             const int s = p % c->ring_n, m = p0 + np - p < c->ring_n - s ? p0 + np - p : c->ring_n - s;
-            if (o.flow)
-                TRY(copy_slots_out(c, flow_slots(c, c->ring), s, m, (char*)o.flow + (size_t)p * o.flow_stride, o.flow_pitch,
-                                   o.flow_stride, o.kf));
-            if (o.flow_bw)
-                TRY(copy_slots_out(c, flow_slots(c, c->ring_bw), s, m, (char*)o.flow_bw + (size_t)p * o.flow_stride,
-                                   o.flow_pitch, o.flow_stride, o.kb));
-            if (o.mask)
-                TRY(copy_slots_out(c, mask_slots(c), s, m, (char*)o.mask + (size_t)p * o.mask_stride, o.mask_pitch,
-                                   o.mask_stride, o.km));
+            TRY(copy_outputs(c, o, s, m, p));
             p += m;
         }
         CK(c, cudaEventRecord(c->ev_out[par], c->s_out));
@@ -1970,7 +2095,7 @@ int ffb_farneback_sequence(ffb_ctx* c, const uint8_t* frames, int n_frames, int 
     TRY(check_sequence_args(c, fn, frames, n_frames, width, height, pitch, frame_stride, flow, flow_pitch, flow_stride));
     CK(c, cudaSetDevice(c->device));
     PtrKind kfr;
-    SequenceOut o;
+    RingOut o;
     o.flow = flow; o.flow_pitch = flow_pitch; o.flow_stride = flow_stride;
     TRY(buffer_kind(c, fn, "frames are", frames, &kfr));
     TRY(buffer_kind(c, fn, "flow is", flow, &o.kf));
@@ -2005,15 +2130,10 @@ int ffb_farneback_sequence_bidir(ffb_ctx* c, const uint8_t* frames, int n_frames
     const int n_pairs = n_frames - 1;
     TRY(check_sequence_args(c, fn, frames, n_frames, width, height, pitch, frame_stride, flow_fw || flow_bw, flow_pitch,
                             flow_stride));
-    if (mask && mask_pitch < (size_t)width)
-        return fail(c, FFB_E_INVALID, "%s: mask_pitch %zu below the width %d", fn, mask_pitch, width);
-    if (mask && n_pairs > 1 && mask_stride < mask_pitch * (size_t)(height - 1) + width)
-        return fail(c, FFB_E_INVALID, "%s: mask_stride %zu shorter than a mask", fn, mask_stride);
-    if (!(alpha >= 0.0 && isfinite(alpha)) || !(beta >= 0.0 && isfinite(beta)))
-        return fail(c, FFB_E_INVALID, "%s: alpha %g and beta %g must be finite and >= 0", fn, alpha, beta);
+    TRY(check_bidir_args(c, fn, n_pairs, width, height, mask, mask_pitch, mask_stride, alpha, beta));
     CK(c, cudaSetDevice(c->device));
     PtrKind kfr;
-    SequenceOut o;
+    RingOut o;
     o.flow = flow_fw; o.flow_bw = flow_bw; o.flow_pitch = flow_pitch; o.flow_stride = flow_stride;
     o.mask = mask; o.mask_pitch = mask_pitch; o.mask_stride = mask_stride;
     TRY(buffer_kind(c, fn, "frames are", frames, &kfr));
@@ -2023,41 +2143,14 @@ int ffb_farneback_sequence_bidir(ffb_ctx* c, const uint8_t* frames, int n_frames
     const int B = c->B > 0 ? c->B : 2;
     TRY(configure_checked(c, width, height, B, c->maxPairs > 0 ? c->maxPairs : 1, o.any() ? 2 * B + 8 : 0));
     const bool backward = flow_bw || mask || n_consistent;
-    // the backward ring, the mask ring and the counts: grow-only, allocated by the first call that needs them (a new
-    // frame size or a larger final-flow ring frees the rings)
-    if (backward && c->bw_n < c->ring_n) {
-        dev_free(c->ring_bw);
-        c->bw_n = 0;
-        TRY(dev_alloc(c, &c->ring_bw, (size_t)c->ring_n * c->ring_stride));
-        c->bw_n = c->ring_n;
-    }
-    if (mask && c->mask_n < c->ring_n) {
-        dev_free(c->mask_ring);
-        c->mask_n = 0;
-        TRY(dev_alloc(c, &c->mask_ring, (size_t)c->ring_n * width * height));
-        c->mask_n = c->ring_n;
-    }
-    if (n_consistent && c->ncons_cap < n_pairs) {
-        dev_free(c->d_ncons);
-        c->ncons_cap = 0;
-        TRY(dev_alloc(c, &c->d_ncons, (size_t)n_pairs));
-        c->ncons_cap = n_pairs;
-    }
+    TRY(alloc_backward(c, backward, mask != nullptr, n_consistent ? n_pairs : 0));
     Backward bw;
     bw.mask = mask != nullptr;
     bw.count = n_consistent != nullptr;
     bw.alpha = (float)alpha;
     bw.beta = (float)beta;
     TRY(sequence_loop(c, frames, n_frames, pitch, frame_stride, kfr, o, false, backward ? &bw : nullptr, stream));
-    const bool host_io = kfr != PTR_DEVICE || o.kf != PTR_DEVICE || o.kb != PTR_DEVICE || o.km != PTR_DEVICE || n_consistent;
-    if (stream && !host_io) return FFB_OK;
-    CK(c, cudaStreamSynchronize(c->s_comp));
-    if (n_consistent) {
-        std::vector<unsigned> h((size_t)n_pairs);
-        CK(c, cudaMemcpy(h.data(), c->d_ncons, (size_t)n_pairs * sizeof(unsigned), cudaMemcpyDeviceToHost));
-        for (int j = 0; j < n_pairs; ++j) n_consistent[j] = h[j];
-    }
-    return FFB_OK;
+    return finish_bidir(c, o, kfr != PTR_DEVICE, n_pairs, n_consistent, stream);
 }
 
 static int upload_flow(ffb_ctx* c, const float* flow, int w, int h) {

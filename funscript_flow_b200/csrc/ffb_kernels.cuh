@@ -740,7 +740,7 @@ __device__ __forceinline__ float2 ffb_solve(float s0, float s1, float s2, float 
 // PS (pair stride): pair j reads the expansions in ring elements PS*j and PS*j + 1.  1: consecutive frames of a bracket
 // (frame j+1 is `next` of pair j and `prev` of pair j+1); 2: independent pairs, staged as prev_0, next_0, prev_1, ...
 // REV (slot order): pair j reads element PS*j + REV as R0 and PS*j + !REV as R1; REV = true is the backward flow of a
-// bracket pair (frame j+1 -> frame j).
+// pair (frame j+1 -> frame j of a bracket, next_j -> prev_j of independent pairs).
 template <int NT, int U, int MINB, bool UP2X, int HO, int PS, bool REV>
 __global__ void __launch_bounds__(NT, MINB) k_flow_iter(FfbIterArgs a) {
     static_assert(HO == 4 || HO == 8, "outputs per horizontal task");

@@ -232,6 +232,28 @@ int  ffb_farneback_sequence_bidir(ffb_ctx* ctx, const uint8_t* frames, int n_fra
                                   uint8_t* mask, size_t mask_pitch, size_t mask_stride,
                                   double alpha, double beta, int64_t* n_consistent, void* stream);
 
+/* ---- independent pairs with backward flows and a forward-backward consistency mask ------------------------------
+ * ffb_farneback_pairs for pair i = (prev + i*frame_stride, next + i*frame_stride), plus its backward flow (next[i] ->
+ * prev[i]) and the forward-backward check; for the two eyes of a side-by-side frame it is the left-right check of
+ * stereo matching.  Outputs may be NULL:
+ *   flow_fw      pair i's flow at flow_fw + i*flow_stride (rows flow_pitch bytes apart): bit-identical to
+ *                ffb_farneback(prev[i], next[i])
+ *   flow_bw      the backward flow, same layout: bit-identical to ffb_farneback(next[i], prev[i])
+ *   mask         uint8 [height][width] per pair at mask + i*mask_stride (rows mask_pitch bytes apart), and
+ *   n_consistent int64 per pair (host array): as in ffb_farneback_sequence_bidir
+ * Each frame is expanded once: the backward flows re-use the expansions of the forward pass.  prev, next, the flows and
+ * the mask may each be pageable host, pinned host or device memory (of the context's device).  Configuration, chunks
+ * and the stream contract are ffb_farneback_pairs'; the backward ring, the mask ring and the counts are allocated by
+ * the first call that needs them and only grow.  There are no per-pair bracket results, and max_pairs does not grow.
+ * The flows of an earlier bracket are no longer resident.  FFB_E_INVALID for everything ffb_farneback_pairs refuses,
+ * mask_pitch < width, mask_stride shorter than a mask, and alpha or beta negative or not finite; n_pairs == 0 does
+ * nothing. */
+int  ffb_farneback_pairs_bidir(ffb_ctx* ctx, const uint8_t* prev, const uint8_t* next, int n_pairs, int width,
+                               int height, size_t pitch, size_t frame_stride,
+                               float* flow_fw, float* flow_bw, size_t flow_pitch, size_t flow_stride,
+                               uint8_t* mask, size_t mask_pitch, size_t mask_stride,
+                               double alpha, double beta, int64_t* n_consistent, void* stream);
+
 /* ---- per-stage hooks (each runs exactly the production kernel of that stage, for the context's parameters) -----
  * Level geometry of the Farneback pyramid for a frame size with the reference's pyr_scale 0.5, levels 3 (coarsest
  * level first): fills up to 4 entries of w[], h[], ksize[], sigma[]; returns the level count in *n_levels. */

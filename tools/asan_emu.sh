@@ -40,6 +40,21 @@ for (w, h, b) in [(97, 70, 3), (33, 20, 16)]:   # sequences that wrap the final-
     m, k = ctx.stage_fb_check(b["flow"][3], b["flow_bw"][3])
     assert np.array_equal(m, b["mask"][3]) and k == cnt[3]
     print(w, h, "bidirectional ok", int(cnt.sum()))
+    # independent pairs with backward flows, masks and counts: chunks alternate ring halves, into pitched buffers
+    prev, nxt = np.ascontiguousarray(seq[0:40:2]), np.ascontiguousarray(seq[40:0:-2])
+    p = ctx.farneback_pairs_bidir(prev, nxt)
+    assert np.array_equal(p["flow"], ctx.farneback_pairs(prev, nxt)["flow"])
+    assert np.array_equal(p["flow_bw"][5], ctx.farneback(nxt[5], prev[5]))
+    fw = np.zeros((20, h + 1, w + 3, 2), np.float32)
+    bw = np.zeros((20, h + 1, w + 3, 2), np.float32)
+    mask = np.zeros((20, h + 2, w + 5), np.uint8)
+    cnt = ctx.farneback_pairs_bidir_ptr(prev.ctypes.data, nxt.ctypes.data, 20, w, h, w, w * h, fw.ctypes.data, bw.ctypes.data,
+                                        (w + 3) * 8, (h + 1) * (w + 3) * 8, mask.ctypes.data, w + 5, (h + 2) * (w + 5),
+                                        counts=True)
+    assert np.array_equal(fw[:, :h, :w], p["flow"]) and np.array_equal(bw[:, :h, :w], p["flow_bw"])
+    assert np.array_equal(mask[:, :h, :w], p["mask"].view(np.uint8)) and np.array_equal(cnt, p["n_consistent"])
+    assert np.array_equal(cnt, p["mask"].sum(axis=(1, 2)))
+    print(w, h, "pairs bidirectional ok", int(cnt.sum()))
 pc.check_reductions_random(ctx, n_cases=8, max_side=70)
 pc.check_preprocess(ctx, sizes=((97, 131), (64, 48)))
 pc.check_preprocess_window(ctx)
