@@ -9,7 +9,8 @@ from .api import (BracketPipeline, calc_optical_flow_farneback_batch, calc_optic
                   calc_optical_flow_farneback_batch_bidirectional, calc_optical_flow_farneback_sequence_bidirectional,
                   get_available_backends, get_context, get_gpu_info, max_divergence, precompute_flow_info,
                   precompute_flow_info_batch, precompute_flow_info_gpu, precompute_wrapper, process_bracket,
-                  process_bracket_on_contexts, process_sequence, radial_motion_weighted, set_context, smooth_centers)
+                  process_bracket_on_contexts, process_sequence, radial_motion_weighted, remap_by_flow, set_context,
+                  smooth_centers)
 from .runner import process_frames, process_many, process_video, run_headless  # noqa: F401
 
 __version__ = "0.2.0"

@@ -15,7 +15,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 DEFAULT_LIB = os.path.join(_HERE, "libffb.so")
 
-K_NAMES = ["pyramid", "polyexp", "upsample", "flow_iter", "divmag", "radial", "small", "preprocess", "fb_check"]
+K_NAMES = ["pyramid", "polyexp", "upsample", "flow_iter", "divmag", "radial", "small", "preprocess", "fb_check", "remap"]
 K_FLOW_ITER = 3
 
 
@@ -72,6 +72,7 @@ def load(path: Optional[str] = None) -> C.CDLL:
                                                C.c_double, C.POINTER(C.c_int64), vp]),
         "ffb_farneback_pairs_bidir": (i32, [vp, vp, vp, i32, i32, i32, sz, sz, vp, vp, sz, sz, vp, sz, sz, C.c_double,
                                             C.c_double, C.POINTER(C.c_int64), vp]),
+        "ffb_remap_flow": (i32, [vp, vp, i32, i32, i32, i32, sz, sz, vp, sz, sz, vp, sz, sz, i32, i32, vp]),
         "ffb_max_divergence": (i32, [vp, f32p, i32, i32, i32p, i32p, f32p]),
         "ffb_mean_magnitude": (i32, [vp, f32p, i32, i32, f32p]),
         "ffb_radial_motion": (i32, [vp, f32p, i32, i32, C.c_double, C.c_double, i32, i32, f64p]),
@@ -588,6 +589,38 @@ class FlowContext:
             int(frame_stride), *out, float(alpha), float(beta),
             None if cnt is None else cnt.ctypes.data_as(C.POINTER(C.c_int64)), C.c_void_p(int(stream) or None)))
         return None if cnt is None else cnt[:max(n, 0)].copy()
+
+    def remap_flow(self, src: np.ndarray, flow: np.ndarray, border_mode: int = 0, border_value: int = 0) -> np.ndarray:
+        """cv2.remap(src, flow, None, cv2.INTER_LINEAR | cv2.WARP_RELATIVE_MAP, border_mode, (v, v, v)) bit for bit
+        (ffb_remap_flow), for one image or a batch: src uint8 [H, W], [H, W, 3], [n, H, W] or [n, H, W, 3], flow float32
+        [H, W, 2] or [n, H, W, 2] (its ndim tells one image from a batch).  border_mode 0 is cv2.BORDER_CONSTANT (value
+        border_value), 1 cv2.BORDER_REPLICATE.  Returns uint8 of src's shape."""
+        src = np.ascontiguousarray(src)
+        flow = np.ascontiguousarray(flow)
+        if src.dtype != np.uint8 or flow.dtype != np.float32:
+            raise TypeError(f"remap_flow: src must be uint8 and flow float32, not {src.dtype} and {flow.dtype}")
+        single = flow.ndim == 3
+        src_b, flow_b = (src[None], flow[None]) if single else (src, flow)
+        if flow_b.ndim != 4 or flow_b.shape[3] != 2 or src_b.shape[:3] != flow_b.shape[:3] or src_b.ndim not in (3, 4) \
+                or (src_b.ndim == 4 and src_b.shape[3] != 3):
+            raise ValueError(f"remap_flow: src {src.shape} and flow {flow.shape} are not [n,] H, W[, 3] and [n,] H, W, 2")
+        n, h, w = flow_b.shape[:3]
+        ch = 3 if src_b.ndim == 4 else 1
+        out = np.empty_like(src_b)
+        self.remap_flow_ptr(src_b.ctypes.data, n, w, h, ch, w * ch, w * h * ch, flow_b.ctypes.data, w * 8, w * h * 8,
+                            out.ctypes.data, w * ch, w * h * ch, border_mode, border_value)
+        return out[0] if single else out
+
+    def remap_flow_ptr(self, src_ptr: int, n: int, width: int, height: int, channels: int, src_pitch: int, src_stride: int,
+                       flow_ptr: int, flow_pitch: int, flow_stride: int, dst_ptr: int, dst_pitch: int, dst_stride: int,
+                       border_mode: int = 0, border_value: int = 0, stream: int = 0):
+        """Raw-pointer variant of remap_flow, like farneback_pairs_ptr: buffers anywhere (e.g. torch_tensor.data_ptr()),
+        pitches and strides in bytes, `stream` a cudaStream_t handle (0 = none)."""
+        self._ck(self._lib.ffb_remap_flow(self._h, C.c_void_p(int(src_ptr) or None), int(n), int(width), int(height),
+                                          int(channels), int(src_pitch), int(src_stride), C.c_void_p(int(flow_ptr) or None),
+                                          int(flow_pitch), int(flow_stride), C.c_void_p(int(dst_ptr) or None),
+                                          int(dst_pitch), int(dst_stride), int(border_mode), int(border_value),
+                                          C.c_void_p(int(stream) or None)))
 
     def max_divergence(self, flow: np.ndarray):
         flow = np.ascontiguousarray(flow, dtype=np.float32)

@@ -18,6 +18,8 @@
                                                     -> [n - 1, H, W, 2]; each frame expanded once)
     calc_optical_flow_farneback_sequence_bidirectional(frames, None, ...)   the same plus the backward flows and the
                                                     forward-backward consistency mask ([n - 1, H, W] bool)
+    remap_by_flow(src, flow, border_mode, border_value)   cv2.remap(src, flow, None, INTER_LINEAR | WARP_RELATIVE_MAP,
+                                                    ...) bit for bit, for one image or a batch (NumPy or torch CUDA)
 
 Every entry point that configures a context first sets its Farneback parameters from the settings keys
 flow_pyr_scale, flow_levels, flow_winsize, flow_iterations, flow_poly_n, flow_poly_sigma (farneback_params;
@@ -525,6 +527,44 @@ def calc_optical_flow_farneback_sequence_bidirectional(frames, flow, pyr_scale: 
                                      mask.data_ptr(), w, w * h, torch.cuda.current_stream(frames.device).cuda_stream,
                                      alpha=alpha, beta=beta)
     return fw, bw, mask
+
+
+def remap_by_flow(src, flow, border_mode: int = 0, border_value: int = 0, *, ctx: Optional[_native.FlowContext] = None):
+    """Warp images by dense flows: cv2.remap(src, flow, None, cv2.INTER_LINEAR | cv2.WARP_RELATIVE_MAP, border_mode,
+    (border_value,) * 3) bit for bit, so dst(x, y) samples src at (x + flow_x, y + flow_y).  src is uint8 [H, W],
+    [H, W, 3], [n, H, W] or [n, H, W, 3], flow float32 [H, W, 2] or [n, H, W, 2]; flow.ndim tells one image from a
+    batch.  border_mode 0 is cv2.BORDER_CONSTANT (value border_value, 0..255), 1 cv2.BORDER_REPLICATE.  The output has
+    src's shape.  NumPy arrays give a NumPy array (strided views are copied to dense arrays first).  torch CUDA tensors
+    (uint8 and float32) on the context's device give a tensor there, ordered on torch.cuda.current_stream(), with no
+    host round trip.  remap_by_flow(frames[1:], calc_optical_flow_farneback_sequence(frames, ...)) warps each next frame
+    onto its previous one.  The context's configuration is left as it is."""
+    fn = "remap_by_flow"
+    ctx = ctx or get_context()
+    tensors = _is_torch_tensor(src), _is_torch_tensor(flow)
+    if tensors[0] != tensors[1]:
+        raise TypeError(f"{fn}: src and flow must both be NumPy arrays or both torch tensors")
+    if not tensors[0]:
+        return ctx.remap_flow(np.asarray(src), np.asarray(flow), border_mode, border_value)
+    import torch
+    if src.dtype != torch.uint8 or flow.dtype != torch.float32 or not src.is_cuda or not flow.is_cuda:
+        raise TypeError(f"{fn}: tensors must be torch.uint8 (src) and torch.float32 (flow) on a CUDA device")
+    if src.device != flow.device or src.device.index != ctx.device:
+        raise ValueError(f"{fn}: tensors on {src.device} / {flow.device}, the context on cuda:{ctx.device}")
+    single = flow.ndim == 3
+    src_b, flow_b = (src[None], flow[None]) if single else (src, flow)
+    if flow_b.ndim != 4 or flow_b.shape[3] != 2 or tuple(src_b.shape[:3]) != tuple(flow_b.shape[:3]) \
+            or src_b.ndim not in (3, 4) or (src_b.ndim == 4 and src_b.shape[3] != 3):
+        raise ValueError(f"{fn}: src {tuple(src.shape)} and flow {tuple(flow.shape)} are not [n,] H, W[, 3] and "
+                         f"[n,] H, W, 2")
+    src_b, flow_b = src_b.contiguous(), flow_b.contiguous()
+    n, h, w = flow_b.shape[:3]
+    ch = 3 if src_b.ndim == 4 else 1
+    out = torch.empty_like(src_b)
+    if n:
+        ctx.remap_flow_ptr(src_b.data_ptr(), n, w, h, ch, w * ch, w * h * ch, flow_b.data_ptr(), w * 8, w * h * 8,
+                           out.data_ptr(), w * ch, w * h * ch, border_mode, border_value,
+                           torch.cuda.current_stream(src.device).cuda_stream)
+    return out[0] if single else out
 
 
 def process_sequence(frames, params: Optional[Dict] = None, *, ctx: Optional[_native.FlowContext] = None,

@@ -33,7 +33,7 @@ thread_local std::string g_create_error;
 
 const char* const kKernelNames[FFB_K_COUNT] = {"k_pyramid_level", "k_polyexp",  "k_upsample_flow", "k_flow_iter",
                                                "k_divmag",        "k_radial",   "small",           "k_preprocess",
-                                               "k_fb_check"};
+                                               "k_fb_check",      "k_remap_flow"};
 
 // ------------------------------------------------------------------ host-side constant builders
 int cv_round(double v) { return (int)nearbyint(v); }   // round-half-even in the default FP mode
@@ -282,6 +282,11 @@ struct ffb_ctx {
     uint8_t* h_color[2] = {nullptr, nullptr};
     cudaEvent_t ev_ch2d[2] = {nullptr, nullptr}, ev_pre[2] = {nullptr, nullptr};
     int color_no = 0;
+    // ffb_remap_flow's staging, grow-only and independent of the geometry: per buffer b of a chunk, the device images
+    // of host (or misaligned) inputs and of a host output, and the pinned copies of pageable inputs
+    uint8_t *rm_src[2] = {nullptr, nullptr}, *rm_flow[2] = {nullptr, nullptr}, *rm_dst[2] = {nullptr, nullptr};
+    uint8_t *rm_hsrc[2] = {nullptr, nullptr}, *rm_hflow[2] = {nullptr, nullptr};
+    size_t rm_src_cap = 0, rm_flow_cap = 0, rm_dst_cap = 0, rm_hsrc_cap = 0, rm_hflow_cap = 0;
     // bracket state
     bool in_bracket = false;
     int pov = 0;
@@ -1062,6 +1067,28 @@ int launch_fb_check(ffb_ctx* c, FfbRing fw, FfbRing bw, int fp, int w, int h, Ff
     return FFB_OK;
 }
 
+// k_remap_flow of n images (n <= 65535) of w x h pixels of ch bytes: sources at src + i * ss (rows sp bytes apart),
+// flows in ring `flow` (rows fp bytes apart), outputs at dst + i * ds (rows dp bytes apart); border 0 constant (value
+// bval), 1 replicate
+int launch_remap(ffb_ctx* c, const uint8_t* src, size_t ss, size_t sp, FfbRing flow, size_t fp, uint8_t* dst, size_t ds,
+                 size_t dp, int w, int h, int ch, int border, int bval, int n) {
+    FfbRemapArgs a;
+    a.src = src; a.src_stride = ss; a.src_pitch = sp;
+    a.flow = flow; a.fp = fp;
+    a.dst = dst; a.dst_stride = ds; a.dst_pitch = dp;
+    a.w = w; a.h = h; a.border_value = bval;
+    a.flow_v8 = ((uintptr_t)flow.base | (n > 1 ? flow.stride : 0) | fp) % 32 == 0;
+    a.dst_v4 = ((uintptr_t)dst | dp | (n > 1 ? ds : 0)) % 4 == 0;
+    // algorithmic bytes: the flow, the taps counted once (neighbouring outputs share their footprints), the output
+    const ProfMark pm = prof_begin(c, FFB_K_REMAP, -1, (double)n * w * h * (8.0 + 2.0 * ch), c->s_comp);
+    auto kfn = ch == 1 ? (border ? k_remap_flow<1, true> : k_remap_flow<1, false>)
+                       : (border ? k_remap_flow<3, true> : k_remap_flow<3, false>);
+    FFB_LAUNCH(kfn, dim3((w + 127) / 128, (h + 7) / 8, n), dim3(256), 0, c->s_comp, a);
+    prof_end(pm);
+    CKL(c);
+    return FFB_OK;
+}
+
 // k_radial + k_radial_finish of ring pairs [j0, j0 + cnt) (cnt <= ring_n): d_scalar[j0 ..] from d_centers and d_cut
 int launch_radial(ffb_ctx* c, int j0, int cnt, int pov) {
     FfbRadArgs r;
@@ -1294,6 +1321,38 @@ void free_preprocess(ffb_ctx* c) {
     c->pre = ffb_ctx::PrePlan();
 }
 
+// Grow-only pair of ffb_remap_flow staging buffers of at least `bytes` each, on the device or pinned on the host.
+static int grow_staging(ffb_ctx* c, uint8_t* (&buf)[2], size_t& cap, size_t bytes, bool pinned) {
+    if (bytes <= cap) return FFB_OK;
+    for (uint8_t*& p : buf) {
+        if (!pinned) dev_free(p);
+        else if (p) cudaFreeHost(p);
+        p = nullptr;
+    }
+    cap = 0;
+    for (uint8_t*& p : buf) {
+        if (pinned) {
+            void* hp = nullptr;
+            TRY(host_alloc(c, &hp, bytes));
+            p = (uint8_t*)hp;
+        } else {
+            TRY(dev_alloc(c, &p, bytes));
+        }
+    }
+    cap = bytes;
+    return FFB_OK;
+}
+
+static void free_remap_staging(ffb_ctx* c) {
+    for (int b = 0; b < 2; ++b) {
+        dev_free(c->rm_src[b]); dev_free(c->rm_flow[b]); dev_free(c->rm_dst[b]);
+        if (c->rm_hsrc[b]) cudaFreeHost(c->rm_hsrc[b]);
+        if (c->rm_hflow[b]) cudaFreeHost(c->rm_hflow[b]);
+        c->rm_hsrc[b] = c->rm_hflow[b] = nullptr;
+    }
+    c->rm_src_cap = c->rm_flow_cap = c->rm_dst_cap = c->rm_hsrc_cap = c->rm_hflow_cap = 0;
+}
+
 int launch_preprocess(ffb_ctx* c, const uint8_t* src, size_t stride, int pitch, uint8_t* dst, const ffb_ctx::PrePlan& p,
                       const int* xt, const int* yt, int n) {
     FfbPreArgs a;
@@ -1415,6 +1474,7 @@ void ffb_destroy(ffb_ctx* c) {
     for (cudaEvent_t e : c->timers) if (e) cudaEventDestroy(e);
     free_geometry(c);
     free_preprocess(c);
+    free_remap_staging(c);
     for (int b = 0; b < 2; ++b) {
         cudaEventDestroy(c->ev_h2d[b]); cudaEventDestroy(c->ev_expand[b]);
         cudaEventDestroy(c->ev_ch2d[b]); cudaEventDestroy(c->ev_pre[b]);
@@ -1753,14 +1813,14 @@ int ffb_farneback(ffb_ctx* c, const uint8_t* prev, const uint8_t* next, int w, i
     return ffb_bracket_get_flow(c, 0, flow);
 }
 
-// Per-pair images in the slots of a ring (the final-flow rings, the mask ring): slot s at base + s * slot bytes, H rows
-// of `row` bytes, pitch bytes apart, with slot == H * pitch.
-struct SlotImages { const char* base; size_t slot, pitch, row; };
+// Per-pair images in the slots of a ring (the final-flow rings, the mask ring, ffb_remap_flow's output staging): slot s
+// at base + s * slot bytes, `rows` rows of `row` bytes, pitch bytes apart, with slot == rows * pitch.
+struct SlotImages { const char* base; size_t slot, pitch, row; int rows; };
 static SlotImages flow_slots(const ffb_ctx* c, const float2* ring) {
-    return SlotImages{(const char*)ring, c->ring_stride * sizeof(float2), (size_t)c->fp0 * 8, (size_t)c->W * 8};
+    return SlotImages{(const char*)ring, c->ring_stride * sizeof(float2), (size_t)c->fp0 * 8, (size_t)c->W * 8, c->H};
 }
 static SlotImages mask_slots(const ffb_ctx* c) {
-    return SlotImages{(const char*)c->mask_ring, (size_t)c->W * c->H, (size_t)c->W, (size_t)c->W};
+    return SlotImages{(const char*)c->mask_ring, (size_t)c->W * c->H, (size_t)c->W, (size_t)c->W, c->H};
 }
 
 // Copy on s_out of the images in ring slots s0 .. s0 + np - 1 (no wrap) to `dst`: images `stride` bytes apart, rows
@@ -1769,11 +1829,11 @@ static int copy_slots_out(ffb_ctx* c, const SlotImages& r, int s0, int np, char*
                           PtrKind kind) {
     const cudaMemcpyKind dir = kind == PTR_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
     const char* src = r.base + (size_t)s0 * r.slot;
-    if (stride == pitch * c->H)     // the pairs' rows are evenly spaced on both sides
-        CK(c, cudaMemcpy2DAsync(dst, pitch, src, r.pitch, r.row, (size_t)np * c->H, dir, c->s_out));
+    if (stride == pitch * r.rows)     // the pairs' rows are evenly spaced on both sides
+        CK(c, cudaMemcpy2DAsync(dst, pitch, src, r.pitch, r.row, (size_t)np * r.rows, dir, c->s_out));
     else
         for (int j = 0; j < np; ++j)
-            CK(c, cudaMemcpy2DAsync(dst + (size_t)j * stride, pitch, src + (size_t)j * r.slot, r.pitch, r.row, c->H, dir,
+            CK(c, cudaMemcpy2DAsync(dst + (size_t)j * stride, pitch, src + (size_t)j * r.slot, r.pitch, r.row, r.rows, dir,
                                     c->s_out));
     return FFB_OK;
 }
@@ -2151,6 +2211,120 @@ int ffb_farneback_sequence_bidir(ffb_ctx* c, const uint8_t* frames, int n_frames
     bw.beta = (float)beta;
     TRY(sequence_loop(c, frames, n_frames, pitch, frame_stride, kfr, o, false, backward ? &bw : nullptr, stream));
     return finish_bidir(c, o, kfr != PTR_DEVICE, n_pairs, n_consistent, stream);
+}
+
+// ---- warping by a flow ---------------------------------------------------------------------------------------------
+// Host buffers move in chunks of images whose source, flow and output take at most kRemapChunkBytes together (at least
+// one image): large enough for full-rate copies, small enough that the copies of one chunk overlap the kernel of the
+// previous one.  All-device calls launch once per 65535 images (the grid's z limit).
+constexpr size_t kRemapChunkBytes = 8u << 20;
+constexpr int kRemapMaxLaunch = 65535;
+
+// cv2.remap(src[i], flow[i], None, INTER_LINEAR | WARP_RELATIVE_MAP, border_mode, (v, v, v)) of n uint8 images
+// (k_remap_flow).  Device buffers are used in place (a device flow whose rows are not 4-byte aligned is copied to the
+// staging first); host inputs are uploaded chunk by chunk on s_copy through staging buffer b = chunk & 1 (pageable ones
+// through its pinned copy), a host output leaves the staging on s_out one chunk late, as in pairs_loop.  The fences are
+// the pairs call's: ev_h2d[b] / ev_h2d_next[b] end the upload of the source / flow into buffer b, ev_expand[b] the
+// kernel that read it, ev_fin[b] / ev_out[b] the kernel that wrote the output staging b and its copy-out.  The call
+// touches neither the geometry, nor the Farneback parameters, nor the final-flow ring.
+int ffb_remap_flow(ffb_ctx* c, const uint8_t* src, int n, int width, int height, int channels, size_t src_pitch,
+                   size_t src_stride, const float* flow, size_t flow_pitch, size_t flow_stride, uint8_t* dst,
+                   size_t dst_pitch, size_t dst_stride, int border_mode, int border_value, void* stream) {
+    static const char* fn = "ffb_remap_flow";
+    if (!c) return FFB_E_INVALID;
+    if (c->in_bracket) return fail(c, FFB_E_INVALID, "ffb_remap_flow inside a bracket");
+    if (n < 0) return fail(c, FFB_E_INVALID, "ffb_remap_flow: n %d < 0", n);
+    if (n == 0) return FFB_OK;
+    if (!src || !flow || !dst || width < 1 || height < 1 || width >= 32767 || height >= 32767)
+        return fail(c, FFB_E_INVALID, "%s: bad images (%dx%d; cv2.remap takes sizes below 32767)", fn, width, height);
+    if (channels != 1 && channels != 3) return fail(c, FFB_E_INVALID, "%s: %d channels (1 or 3)", fn, channels);
+    if (border_mode != 0 && border_mode != 1)
+        return fail(c, FFB_E_INVALID, "%s: border mode %d (0 constant, 1 replicate)", fn, border_mode);
+    if (border_value < 0 || border_value > 255) return fail(c, FFB_E_INVALID, "%s: border value %d outside 0..255", fn, border_value);
+    const size_t row = (size_t)width * channels, frow = (size_t)width * 8;
+    if (src_pitch < row) return fail(c, FFB_E_INVALID, "%s: src_pitch %zu below width * channels (%zu)", fn, src_pitch, row);
+    if (n > 1 && src_stride < src_pitch * (size_t)(height - 1) + row)
+        return fail(c, FFB_E_INVALID, "%s: src_stride %zu shorter than an image", fn, src_stride);
+    if (flow_pitch < frow) return fail(c, FFB_E_INVALID, "%s: flow_pitch %zu below 8 * width (%zu)", fn, flow_pitch, frow);
+    if (n > 1 && flow_stride < flow_pitch * (size_t)(height - 1) + frow)
+        return fail(c, FFB_E_INVALID, "%s: flow_stride %zu shorter than a flow", fn, flow_stride);
+    if (dst_pitch < row) return fail(c, FFB_E_INVALID, "%s: dst_pitch %zu below width * channels (%zu)", fn, dst_pitch, row);
+    if (n > 1 && dst_stride < dst_pitch * (size_t)(height - 1) + row)
+        return fail(c, FFB_E_INVALID, "%s: dst_stride %zu shorter than an image", fn, dst_stride);
+    CK(c, cudaSetDevice(c->device));
+    PtrKind ks, kf, kd;
+    TRY(buffer_kind(c, fn, "src is", src, &ks));
+    TRY(buffer_kind(c, fn, "flow is", flow, &kf));
+    TRY(buffer_kind(c, fn, "dst is", dst, &kd));
+    const size_t img = row * height, fimg = frow * height;
+    const bool flow_aligned = ((uintptr_t)flow | flow_pitch | (n > 1 ? flow_stride : 0)) % 4 == 0;
+    const bool up_src = ks != PTR_DEVICE, up_flow = kf != PTR_DEVICE || !flow_aligned, down = kd != PTR_DEVICE;
+    const bool staged = up_src || up_flow || down;
+    const size_t per = (up_src ? img : 0) + (up_flow ? fimg : 0) + (down ? img : 0);
+    const size_t fit = staged ? kRemapChunkBytes / per : 0;
+    const int K = !staged || fit > (size_t)kRemapMaxLaunch ? kRemapMaxLaunch : (fit < 1 ? 1 : (int)fit);
+    const int k_imgs = K < n ? K : n;
+    if (up_src) TRY(grow_staging(c, c->rm_src, c->rm_src_cap, k_imgs * img, false));
+    if (ks == PTR_PAGEABLE) TRY(grow_staging(c, c->rm_hsrc, c->rm_hsrc_cap, k_imgs * img, true));
+    if (up_flow) TRY(grow_staging(c, c->rm_flow, c->rm_flow_cap, k_imgs * fimg, false));
+    if (up_flow && kf == PTR_PAGEABLE) TRY(grow_staging(c, c->rm_hflow, c->rm_hflow_cap, k_imgs * fimg, true));
+    if (down) TRY(grow_staging(c, c->rm_dst, c->rm_dst_cap, k_imgs * img, false));
+    const cudaStream_t us = (cudaStream_t)stream;
+    CK(c, cudaEventRecord(c->ev_user, us));
+    CK(c, cudaStreamWaitEvent(c->s_copy, c->ev_user, 0));
+    CK(c, cudaStreamWaitEvent(c->s_comp, c->ev_user, 0));
+    // output of images [i0, i0 + m) from output staging b to dst
+    auto copy_out = [&](int i0, int m, int b) -> int {
+        CK(c, cudaStreamWaitEvent(c->s_out, c->ev_fin[b], 0));
+        TRY(copy_slots_out(c, SlotImages{(const char*)c->rm_dst[b], img, row, row, height}, 0, m,
+                           (char*)dst + (size_t)i0 * dst_stride, dst_pitch, dst_stride, kd));
+        CK(c, cudaEventRecord(c->ev_out[b], c->s_out));
+        return FFB_OK;
+    };
+    int pend_i0 = -1, pend_m = 0, pend_b = 0;   // chunk whose copy-out has not been issued yet
+    for (int i0 = 0, k = 0; i0 < n; i0 += K, ++k) {
+        const int m = n - i0 < K ? n - i0 : K, b = k & 1;
+        const uint8_t* s = src + (size_t)i0 * src_stride;
+        size_t ss = src_stride, sp = src_pitch;
+        if (up_src) {
+            TRY(upload_frames(c, c->rm_src[b], c->rm_hsrc[b], c->ev_h2d[b], c->ev_expand[b], s, ks, m, height, row, src_pitch,
+                              src_stride));
+            s = c->rm_src[b]; ss = img; sp = row;
+        }
+        FfbRing fr{(char*)flow + (size_t)i0 * flow_stride, flow_stride, 0, m};
+        size_t fp = flow_pitch;
+        if (up_flow) {
+            TRY(upload_frames(c, c->rm_flow[b], c->rm_hflow[b], c->ev_h2d_next[b], c->ev_expand[b], (const uint8_t*)fr.base,
+                              kf, m, height, frow, flow_pitch, flow_stride));
+            fr = FfbRing{(char*)c->rm_flow[b], fimg, 0, m};
+            fp = frow;
+        }
+        uint8_t* d = dst + (size_t)i0 * dst_stride;
+        size_t ds = dst_stride, dp = dst_pitch;
+        if (down) {
+            CK(c, cudaStreamWaitEvent(c->s_comp, c->ev_out[b], 0));   // the copy-out of chunk k - 2 has read buffer b
+            d = c->rm_dst[b]; ds = img; dp = row;
+        }
+        TRY(launch_remap(c, s, ss, sp, fr, fp, d, ds, dp, width, height, channels, border_mode, border_value, m));
+        if (up_src || up_flow) CK(c, cudaEventRecord(c->ev_expand[b], c->s_comp));
+        if (!down) continue;
+        CK(c, cudaEventRecord(c->ev_fin[b], c->s_comp));
+        // issued one chunk late: a copy into pageable memory returns only when it is done
+        if (pend_i0 >= 0) TRY(copy_out(pend_i0, pend_m, pend_b));
+        pend_i0 = i0; pend_m = m; pend_b = b;
+    }
+    if (pend_i0 >= 0) TRY(copy_out(pend_i0, pend_m, pend_b));
+    if (down) {
+        CK(c, cudaEventRecord(c->ev_done, c->s_out));
+        CK(c, cudaStreamWaitEvent(c->s_comp, c->ev_done, 0));
+    }
+    // s_comp has waited for every upload and copy-out: the caller's stream continues when the inputs have been read
+    // and the outputs written
+    CK(c, cudaEventRecord(c->ev_done, c->s_comp));
+    CK(c, cudaStreamWaitEvent(us, c->ev_done, 0));
+    if (stream && ks == PTR_DEVICE && kf == PTR_DEVICE && kd == PTR_DEVICE) return FFB_OK;
+    CK(c, cudaStreamSynchronize(c->s_comp));
+    return FFB_OK;
 }
 
 static int upload_flow(ffb_ctx* c, const float* flow, int w, int h) {

@@ -13,6 +13,7 @@
 //   k_phase1_finish   A2/A3/A4 finish: centre, value, mean magnitude, cut flag              F:880-894
 //   k_smooth_centers  A5   +-6 centre mean                                                  F:1203-1214
 //   k_radial(+finish) A6   balanced weighted radial projection mean                         F:761-785
+// and, outside the reference's path, k_remap_flow (X9): cv2.remap of uint8 frames by dense flows, bit-exact.
 #pragma once
 #include "ffb_common.h"
 
@@ -1379,4 +1380,100 @@ __global__ void __launch_bounds__(256) k_preprocess(FfbPreArgs a) {
     }
     const int gray = (9798 * rgb[0] + 19235 * rgb[1] + 3735 * rgb[2] + 16384) >> 15;
     a.dst[(size_t)blockIdx.z * a.dst_frame_stride + (size_t)y * a.dst_pitch + x] = (uint8_t)gray;
+}
+
+// ======================================================================================
+// X9  warp by a dense flow: cv2.remap(src, flow, None, INTER_LINEAR | WARP_RELATIVE_MAP) on uint8 frames
+// ======================================================================================
+// cv2's 8-bit arithmetic in integers, bit-exact.  Per axis, with f the flow component at output pixel x:
+//   R  = cvRound(32 f)                    NaN, +-inf and |32 f| >= 2^31 give INT_MIN (cvRound on x86; __float2int_rn
+//                                         would saturate instead, and map NaN to 0)
+//   x0 = saturate_short((R >> 5) + x)     the left tap column (cv2 adds the integer grid after rounding: rounding
+//   ax = R & 31                           x + f in float32 first would differ where that sum rounds)
+// cv2's 15-bit weights are the products (32 - ax | ax) (32 - ay | ay) * 32: exact, summing to 32768 (the entry of
+// ax = ay = 0 holds 32767 and a 1, which still returns the tap itself), so the output
+// (sum w_k v_k + 16384) >> 15 equals (sum W_k v_k + 512) >> 10 with W_k the 10-bit products, per channel.
+// Borders: constant -- a tap outside the frame reads the border value; replicate -- each tap's coordinates are
+// clamped.  Frames are narrower and lower than 32767 px (cv2's limit), so x0 + 1 never overflows a short's range.
+// One thread = 4 consecutive output pixels of a row (a warp = 128 pixels): their flows are one 256-bit load when the
+// flow rows are 32-byte aligned, their outputs one 32-bit store per channel when the output rows are 4-byte aligned.
+struct FfbRemapArgs {
+    const uint8_t* src; size_t src_stride, src_pitch;   // image i at src + i * src_stride, C bytes per pixel
+    FfbRing flow; size_t fp;                           // flow of image i: ring element i, rows fp bytes apart
+    uint8_t* dst; size_t dst_stride, dst_pitch;
+    int w, h;
+    int border_value;
+    bool flow_v8, dst_v4;
+};
+
+__device__ __forceinline__ int ffb_remap_round(float f) {
+    const float s = __fmul_rn(f, 32.f);   // exact: a power of two
+    return s >= -2147483648.f && s < 2147483648.f ? (int)rintf(s) : -2147483647 - 1;
+}
+
+template <int C, bool REPLICATE>
+__device__ __forceinline__ void ffb_remap_px(const FfbRemapArgs& a, const uint8_t* S, int x, int y, float fx, float fy,
+                                             uint8_t* out) {
+    const int rx = ffb_remap_round(fx), ry = ffb_remap_round(fy);
+    const int x0 = ffb_clampi((rx >> 5) + x, -32768, 32767), y0 = ffb_clampi((ry >> 5) + y, -32768, 32767);
+    const int wx[2] = {32 - (rx & 31), rx & 31}, wy[2] = {32 - (ry & 31), ry & 31};
+    int acc[C];
+#pragma unroll
+    for (int c = 0; c < C; ++c) acc[c] = 0;
+#pragma unroll
+    for (int dy = 0; dy < 2; ++dy) {
+#pragma unroll
+        for (int dx = 0; dx < 2; ++dx) {
+            const int w = wx[dx] * wy[dy];
+            int tx = x0 + dx, ty = y0 + dy;
+            if (REPLICATE) {
+                tx = ffb_clampi(tx, 0, a.w - 1);
+                ty = ffb_clampi(ty, 0, a.h - 1);
+            } else if (tx < 0 || tx >= a.w || ty < 0 || ty >= a.h) {
+#pragma unroll
+                for (int c = 0; c < C; ++c) acc[c] += w * a.border_value;
+                continue;
+            }
+            const uint8_t* p = S + (size_t)ty * a.src_pitch + (size_t)tx * C;
+#pragma unroll
+            for (int c = 0; c < C; ++c) acc[c] += w * (int)__ldg(p + c);
+        }
+    }
+#pragma unroll
+    for (int c = 0; c < C; ++c) out[c] = (uint8_t)((acc[c] + 512) >> 10);
+}
+
+template <int C, bool REPLICATE>
+__global__ void __launch_bounds__(256) k_remap_flow(FfbRemapArgs a) {
+    const int x = (blockIdx.x * 32 + (threadIdx.x & 31)) * 4;
+    const int y = blockIdx.y * 8 + (threadIdx.x >> 5);
+    if (x >= a.w || y >= a.h) return;
+    const int img = blockIdx.z;
+    const int n = min(4, a.w - x);
+    const float* F = reinterpret_cast<const float*>(ffb_ring_at(a.flow, img) + (size_t)y * a.fp) + 2 * x;
+    float f[8];
+    if (a.flow_v8 && n == 4) {
+        float4 lo, hi;
+        ffb_load_f8(F, lo, hi);
+        f[0] = lo.x; f[1] = lo.y; f[2] = lo.z; f[3] = lo.w; f[4] = hi.x; f[5] = hi.y; f[6] = hi.z; f[7] = hi.w;
+    } else {
+#pragma unroll
+        for (int i = 0; i < 8; ++i) f[i] = i < 2 * n ? __ldg(F + i) : 0.f;
+    }
+    const uint8_t* S = a.src + (size_t)img * a.src_stride;
+    uint8_t out[4 * C];
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+        if (i < n) ffb_remap_px<C, REPLICATE>(a, S, x + i, y, f[2 * i], f[2 * i + 1], out + i * C);
+    uint8_t* D = a.dst + (size_t)img * a.dst_stride + (size_t)y * a.dst_pitch + (size_t)x * C;
+    if (a.dst_v4 && n == 4) {
+#pragma unroll
+        for (int c = 0; c < C; ++c)
+            reinterpret_cast<unsigned*>(D)[c] = (unsigned)out[4 * c] | (unsigned)out[4 * c + 1] << 8 |
+                                                (unsigned)out[4 * c + 2] << 16 | (unsigned)out[4 * c + 3] << 24;
+    } else {
+#pragma unroll
+        for (int i = 0; i < 4 * C; ++i)
+            if (i < n * C) D[i] = out[i];
+    }
 }

@@ -254,6 +254,29 @@ int  ffb_farneback_pairs_bidir(ffb_ctx* ctx, const uint8_t* prev, const uint8_t*
                                uint8_t* mask, size_t mask_pitch, size_t mask_stride,
                                double alpha, double beta, int64_t* n_consistent, void* stream);
 
+/* ---- warping by a flow: cv2.remap(src, flow, None, INTER_LINEAR | WARP_RELATIVE_MAP, border, (v, v, v)) -------------
+ * For i < n: dst[i] = cv2.remap(src[i], flow[i], None, cv2.INTER_LINEAR | cv2.WARP_RELATIVE_MAP, border_mode,
+ * (border_value,) * 3), bit for bit.  src[i] at src + i*src_stride and dst[i] at dst + i*dst_stride are uint8 width x
+ * height images of `channels` (1 or 3) bytes per pixel, rows src_pitch / dst_pitch bytes apart; flow[i] at
+ * flow + i*flow_stride is float32 [height][width][2] (rows flow_pitch bytes apart), the displacement of each output
+ * pixel: dst(x, y) samples src at (x + fx, y + fy).  The arithmetic is cv2's 8-bit one (DESIGN.md "Warping by flow"):
+ * positions quantised to 1/32 px, 15-bit bilinear weights, non-finite and huge flows as cv2 takes them.  border_mode 0
+ * is cv2.BORDER_CONSTANT (taps outside the image read border_value), 1 cv2.BORDER_REPLICATE.
+ * src, flow and dst may each be pageable host, pinned host or device memory (of the context's device); host buffers
+ * move through the context's own grow-only staging in chunks of images, with uploads and downloads overlapping the
+ * previous chunk's kernel.  The call does not configure the context: its geometry, Farneback parameters and the flows
+ * of the last bracket (ffb_bracket_get_flow) stay as they were.  stream: as in ffb_farneback_pairs -- with a stream
+ * and every buffer on the device the call returns without waiting for the device, otherwise when dst is complete.
+ * FFB_E_INVALID inside a bracket, for n < 0, no buffer, a size of 0 or of 32767 and more (cv2's limit), channels other
+ * than 1 or 3, border_mode other than 0 or 1, border_value outside 0..255, src_pitch or dst_pitch < width*channels,
+ * flow_pitch < 8*width, strides shorter than an image or a flow, and a device pointer on another device; n == 0 does
+ * nothing. */
+int  ffb_remap_flow(ffb_ctx* ctx, const uint8_t* src, int n, int width, int height, int channels,
+                    size_t src_pitch, size_t src_stride,
+                    const float* flow, size_t flow_pitch, size_t flow_stride,
+                    uint8_t* dst, size_t dst_pitch, size_t dst_stride,
+                    int border_mode, int border_value, void* stream);
+
 /* ---- per-stage hooks (each runs exactly the production kernel of that stage, for the context's parameters) -----
  * Level geometry of the Farneback pyramid for a frame size with the reference's pyr_scale 0.5, levels 3 (coarsest
  * level first): fills up to 4 entries of w[], h[], ksize[], sigma[]; returns the level count in *n_levels. */
@@ -313,7 +336,8 @@ int  ffb_stage_preprocess_window(ffb_ctx* ctx, const uint8_t* bgr, int width, in
 #define FFB_K_SMALL     6   /* finish / centre-smoothing kernels */
 #define FFB_K_PREPROC   7
 #define FFB_K_FB_CHECK  8   /* forward-backward consistency check */
-#define FFB_K_COUNT     9
+#define FFB_K_REMAP     9   /* ffb_remap_flow's warp */
+#define FFB_K_COUNT     10
 /* When enabled, every launch of the kernels above is bracketed by CUDA events on the compute
  * stream; ffb_kernel_stats returns launches, summed device milliseconds and the algorithmic
  * bytes those launches moved (DESIGN.md section "bytes per unit") since the last reset. */

@@ -1,7 +1,7 @@
 #!/bin/bash
 # Memory-safety pass over the kernel SOURCES on the CPU: the g++ emulation build (tests/emu) with AddressSanitizer,
 # driven through the C ABI on awkward frame sizes (odd, non-multiple-of-4 widths, frames smaller than a tile), the
-# randomized reductions, the pre-processing windows and the stage hooks.  Run here (no GPU): tools/asan_emu.sh [FFB_ITER_CFG]
+# randomized reductions, the pre-processing windows, the stage hooks and warping by flows.  Run here (no GPU): tools/asan_emu.sh [FFB_ITER_CFG]
 # compute-sanitizer is not available on the GPU pool, so this is the out-of-bounds check of the tiling / halo / padding logic.
 set -e
 ROOT=$(cd "$(dirname "$0")/.." && pwd)
@@ -55,6 +55,23 @@ for (w, h, b) in [(97, 70, 3), (33, 20, 16)]:   # sequences that wrap the final-
     assert np.array_equal(mask[:, :h, :w], p["mask"].view(np.uint8)) and np.array_equal(cnt, p["n_consistent"])
     assert np.array_equal(cnt, p["mask"].sum(axis=(1, 2)))
     print(w, h, "pairs bidirectional ok", int(cnt.sum()))
+# warping by flows at awkward sizes, gray and BGR, both borders, flows far outside the image, pitched buffers; the
+# 300 x 300 gray batch takes two staging chunks
+for (w, h, c, n) in [(1, 1, 1, 3), (37, 1, 3, 3), (1, 29, 1, 3), (97, 70, 3, 3), (131, 5, 1, 4), (300, 300, 1, 12)]:
+    rng = np.random.default_rng(w * h)
+    src = rng.integers(0, 256, (n, h, w) if c == 1 else (n, h, w, 3), dtype=np.uint8)
+    fl = rng.uniform(-2 * max(w, h), 2 * max(w, h), (n, h, w, 2)).astype(np.float32)
+    fl[:, ::3, ::2, 0] = np.nan
+    out = [ctx.remap_flow(src, fl, b, 7) for b in (0, 1)]
+    s_wide = np.zeros((n, h + 1, (w + 3) * c), np.uint8)
+    s_wide[:, :h, :w * c] = src.reshape(n, h, w * c)
+    f_wide = np.zeros((n, h + 1, w + 1, 2), np.float32)
+    f_wide[:, :h, :w] = fl
+    d_wide = np.zeros((n, h + 2, (w + 5) * c), np.uint8)
+    ctx.remap_flow_ptr(s_wide.ctypes.data, n, w, h, c, (w + 3) * c, (h + 1) * (w + 3) * c, f_wide.ctypes.data, (w + 1) * 8,
+                       (h + 1) * (w + 1) * 8, d_wide.ctypes.data, (w + 5) * c, (h + 2) * (w + 5) * c, 1, 7)
+    assert np.array_equal(d_wide[:, :h, :w * c], out[1].reshape(n, h, w * c))
+    print(w, h, c, "remap ok", int(out[0].sum()), int(out[1].sum()))
 pc.check_reductions_random(ctx, n_cases=8, max_side=70)
 pc.check_preprocess(ctx, sizes=((97, 131), (64, 48)))
 pc.check_preprocess_window(ctx)
